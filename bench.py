@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the batched caption-inference hot path (metric of BASELINE.json: captioned images/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|c4] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch per GPU: images -> backbone+FPN+heads -> MT encoder ->
 T KV-cached beam-search steps -> token ids.  Workload (N=1 and per-GPU for N>1, weak scaling) = config C2 of
@@ -21,6 +21,10 @@ random-init weights, V=10000, T=64 decode steps, early stop OFF (fixed work).
   roofline      heaviest kernel of the step (tcgen05 implicit GEMM), algorithmic FLOPs / CUDA-event time, measured
                 live by the engine's per-op profiler right after the timed region.
   cpu_baseline  the oracle's faithful restatement of the reference (per image, uncached decode) on the host cores.
+
+--dump-outputs DIR writes what the timed streaming call returned for its last batch (all ranks' token ids and caption
+lengths after the all-gather) as DIR/ids.npy and DIR/lens.npy in float64, so that two builds can be compared output for
+output: weights and images are seeded, so the same arguments give the same inputs on every run.
 
 --impl reference times that restated reference alone (TensorFlow is not installable here, so the "reference arm"
 is the oracle port; DESIGN.md records this).
@@ -279,6 +283,8 @@ def run_own(args, wl):
     launches = eng.launch_count - l0
     clocks = sampler.stop() if rank == 0 else None
     ids_check = out[0].clone()      # the lanes' output buffers are reused by every later call
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ids=out[0], lens=out[1])
     # ---- one batch at a time (nothing else in flight): the latency of a batch, and the cross-check of the lanes' results
     k1 = max(2, min(args.steps, 6))
     fd.barrier()
@@ -535,6 +541,14 @@ def run_own(args, wl):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(d, **arrays):
+    """DIR/<name>.npy per tensor, as float64 (token ids and lengths are exact in it)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), t.cpu().numpy().astype(np.float64))
+
+
 def quick_workload(key, lanes, dev, opts):
     """Another BASELINE.json config through the same streaming call, device-resident inputs, a short run (driver-visible
     breadth: value, ms per batch and the kernel family with the largest share of the per-op device time)."""
@@ -620,7 +634,13 @@ def main():
     ap.add_argument("--profile-iters", type=int, default=10)
     ap.add_argument("--profile-out", default=None, help="write the engine's per-op profile (JSON) here")
     ap.add_argument("--ncu-step", action="store_true", help="bracket one warm step with cudaProfilerStart/Stop (for ncu launch lists)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the token ids and lengths of the last timed step as DIR/ids.npy and DIR/lens.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl own)")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

@@ -1,6 +1,6 @@
 """Diagnostic: per-op encode profile of the C2 encoder for a few layers (A/B of kernel_opts via DIAG_OPTS)."""
 import os, sys, json
-sys.path.insert(0, "/root/repo/fpn-mt-image-captioning_b200")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "fpn-mt-image-captioning_b200"))
 import torch
 from fpnmt.engine import Engine
 from fpnmt.weights import init_weights
