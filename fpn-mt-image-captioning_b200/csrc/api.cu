@@ -368,3 +368,227 @@ FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, i
 }
 
 }  // extern "C"
+
+// ---- stand-alone encoder bandwidth operators ------------------------------------------------------------
+// Each one uploads fp32 tensors into activations of the requested precision, calls the engine's launcher (which picks the
+// kernel exactly as the engine's program does) and reads the result back.  A tensor of `ld` channels per pixel is one
+// activation of ld channels; the operator sees its first C channels, as through Engine::chan_view.  The output tensor
+// is uploaded too, so columns the kernel must not touch come back unchanged.
+namespace {
+struct OpScratch {
+  cudaStream_t s;
+  bool split;
+  int rc = 0;
+  std::vector<void*> tmp;
+  OpScratch(cudaStream_t st, int precision) : s(st), split(precision == FPNMT_PREC_BF16X3) {}
+  ~OpScratch() {
+    cudaStreamSynchronize(s);
+    for (void* p : tmp) cudaFree(p);
+  }
+  void* alloc(size_t b) {
+    void* p = nullptr;
+    if (cudaMalloc(&p, b ? b : 16) != cudaSuccess) {
+      set_last_error("stand-alone operator: cudaMalloc failed");
+      rc = FPNMT_ERR_CUDA;
+      return nullptr;
+    }
+    tmp.push_back(p);
+    return p;
+  }
+  // host fp32 [n] -> device, zero-padded so that 16-byte vector loads at the end stay inside the allocation
+  const float* upload(const float* h, size_t n) {
+    if (!h) return nullptr;
+    float* d = (float*)alloc((n + 32) * 4);
+    if (!d) return nullptr;
+    cudaMemsetAsync(d, 0, (n + 32) * 4, s);
+    cudaMemcpyAsync(d, h, n * 4, cudaMemcpyHostToDevice, s);
+    return d;
+  }
+  // activation of `ld` channels per row (the engine's layout: hi at [c], lo at [ld + c] in bf16x3), filled from device
+  // fp32 [rows][ld] when src != NULL; the returned view covers the first C channels
+  Act act(size_t rows, int C, int ld, const float* src) {
+    Act a{nullptr, ld, split ? 2 * ld : ld, split ? ld : 0};
+    a.p = (bf16*)alloc(rows * a.ld * 2);
+    if (a.p && src && !rc) rc = launch_f32_to_act(src, rows, ld, a, s);
+    a.C = C;
+    return a;
+  }
+  // device fp32 [rows][ld] <- the whole activation (the columns beyond C included)
+  void read_back(Act a, size_t rows, float* out) {
+    a.C = a.lo ? a.lo : a.ld;
+    if (!rc) rc = launch_act_to_f32(a, rows, out, s);
+  }
+  int finish(const char* name) {
+    const cudaError_t e = cudaStreamSynchronize(s);
+    if (!rc && e != cudaSuccess) {
+      set_last_error(std::string(name) + ": " + cudaGetErrorString(e));
+      return FPNMT_ERR_CUDA;
+    }
+    return rc;
+  }
+};
+
+int op_invalid(const char* msg) {
+  set_last_error(msg);
+  return FPNMT_ERR_INVALID;
+}
+int op_device(int device, const char* name) {
+  FPNMT_CUDA_OK(cudaSetDevice(device));
+  cudaDeviceProp prop;
+  FPNMT_CUDA_OK(cudaGetDeviceProperties(&prop, device));
+  if (prop.major != 10) {
+    set_last_error(std::string(name) + ": device is not sm_100");
+    return FPNMT_ERR_CUDA;
+  }
+  return 0;
+}
+// channels per pixel of a channel-view buffer: 0 means C; must hold C and keep 16-byte rows
+bool view_ld(int C, int* ld) {
+  if (*ld == 0) *ld = C;
+  return C > 0 && C % 8 == 0 && *ld >= C && *ld % 8 == 0;
+}
+bool bad_precision(int precision) { return precision != FPNMT_PREC_BF16 && precision != FPNMT_PREC_BF16X3; }
+}  // namespace
+
+extern "C" {
+
+FPNMT_API int fpnmt_op_depthwise3x3(int device, int precision, const float* x, int N, int H, int W, int C, int in_ld,
+                                    const float* kernel, const float* bias, int stride, int pad_top, int pad_left, int Ho,
+                                    int Wo, int act, float* out, int out_ld, void* stream) {
+  if (!x || !kernel || !out || N < 1 || H < 1 || W < 1 || Ho < 1 || Wo < 1 || (stride != 1 && stride != 2) ||
+      bad_precision(precision) || !view_ld(C, &in_ld) || !view_ld(C, &out_ld))
+    return op_invalid("op_depthwise3x3: bad arguments (C and the lds multiples of 8, stride 1 or 2)");
+  int rc = op_device(device, "op_depthwise3x3");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const float* dw = o.upload(kernel, (size_t)9 * C);
+  const float* db = o.upload(bias, (size_t)C);
+  const size_t ipix = (size_t)N * H * W, opix = (size_t)N * Ho * Wo;
+  Act ax = o.act(ipix, C, in_ld, x), ao = o.act(opix, C, out_ld, out);
+  if (!o.rc) o.rc = launch_depthwise3x3(ax, N, H, W, stride, pad_top, pad_left, Ho, Wo, dw, db, act, ao, o.s);
+  o.read_back(ao, opix, out);
+  return o.finish("op_depthwise3x3");
+}
+
+FPNMT_API int fpnmt_op_pool(int device, int precision, int kind, const float* x, int N, int H, int W, int C, int in_ld, int k,
+                            int stride, int pad_top, int pad_left, int Ho, int Wo, int zero_pad, float* out, int out_ld,
+                            void* stream) {
+  if (!x || !out || N < 1 || H < 1 || W < 1 || Ho < 1 || Wo < 1 || bad_precision(precision) || !view_ld(C, &in_ld) ||
+      !view_ld(C, &out_ld))
+    return op_invalid("op_pool: bad arguments (C and the lds multiples of 8)");
+  if ((kind == 0 && (k < 1 || stride < 1)) || (kind == 1 && (Ho != H / 2 || Wo != W / 2)) ||
+      (kind == 2 && (Ho != (H + 1) / 2 || Wo != (W + 1) / 2)) || kind < 0 || kind > 2)
+    return op_invalid("op_pool: kind 0 (max, k >= 1), 1 (avg 2x2, Ho = H/2) or 2 (subsample, Ho = (H+1)/2)");
+  int rc = op_device(device, "op_pool");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const size_t ipix = (size_t)N * H * W, opix = (size_t)N * Ho * Wo;
+  Act ax = o.act(ipix, C, in_ld, x), ao = o.act(opix, C, out_ld, out);
+  if (!o.rc) {
+    if (kind == 0) o.rc = launch_maxpool(ax, N, H, W, k, stride, pad_top, pad_left, Ho, Wo, zero_pad != 0, ao, o.s);
+    else if (kind == 1) o.rc = launch_avgpool2(ax, N, H, W, ao, o.s);
+    else o.rc = launch_subsample2(ax, N, H, W, ao, o.s);
+  }
+  o.read_back(ao, opix, out);
+  return o.finish("op_pool");
+}
+
+FPNMT_API int fpnmt_op_scale_shift_relu(int device, int precision, const float* x, int64_t pixels, int C, int in_ld,
+                                        const float* scale, const float* shift, float* out, int out_ld, void* stream) {
+  if (!x || !scale || !shift || !out || pixels < 1 || bad_precision(precision) || !view_ld(C, &in_ld) || !view_ld(C, &out_ld))
+    return op_invalid("op_scale_shift_relu: bad arguments (C and the lds multiples of 8)");
+  int rc = op_device(device, "op_scale_shift_relu");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const float *dsc = o.upload(scale, (size_t)C), *dsh = o.upload(shift, (size_t)C);
+  Act ax = o.act((size_t)pixels, C, in_ld, x), ao = o.act((size_t)pixels, C, out_ld, out);
+  if (!o.rc) o.rc = launch_scale_shift_relu(ax, (size_t)pixels, dsc, dsh, ao, o.s);
+  o.read_back(ao, (size_t)pixels, out);
+  return o.finish("op_scale_shift_relu");
+}
+
+FPNMT_API int fpnmt_op_score_conv(int device, int precision, const float* x, int N, int H, int W, const float* kernel,
+                                  const float* bias, float* out, void* stream) {
+  if (precision != FPNMT_PREC_BF16)
+    return op_invalid("op_score_conv: the one-channel score kernel is a bf16-mode kernel (bf16x3 runs op_conv2d with Cout = 1)");
+  if (!x || !kernel || !bias || !out || N < 1 || H < 1 || W < 1 || N > 65535 || (H + 7) / 8 > 65535)
+    return op_invalid("op_score_conv: bad arguments");
+  int rc = op_device(device, "op_score_conv");
+  if (rc) return rc;
+  rc = elementwise_set_attributes();
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const float *dw = o.upload(kernel, (size_t)9 * 256), *db = o.upload(bias, 1);
+  const size_t pix = (size_t)N * H * W;
+  Act ax = o.act(pix, 256, 256, x), ao = o.act(pix, 1, 8, nullptr);
+  if (!o.rc) o.rc = launch_f32_to_act(out, pix, 1, ao, o.s);
+  if (!o.rc) o.rc = launch_conv3x3_c1(ax, dw, db, N, H, W, ao, o.s);
+  if (!o.rc) o.rc = launch_act_to_f32(ao, pix, out, o.s);
+  return o.finish("op_score_conv");
+}
+
+FPNMT_API int fpnmt_op_coattention(int device, int precision, const float* score, const float* cls, int N, int HW, int C,
+                                   float* out, void* stream) {
+  if (!score || !cls || !out || N < 1 || N > 65535 || HW < 1 || bad_precision(precision) || C < 8 || C % 8)
+    return op_invalid("op_coattention: bad arguments (C a multiple of 8)");
+  int rc = op_device(device, "op_coattention");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const size_t pix = (size_t)N * HW;
+  Act as = o.act(pix, 1, 8, nullptr), ac = o.act(pix, C, C, cls), ao = o.act(pix, C, C, out);
+  if (!o.rc) o.rc = launch_f32_to_act(score, pix, 1, as, o.s);
+  if (!o.rc) o.rc = launch_coattention(as, ac, N, HW, ao, o.s);
+  o.read_back(ao, pix, out);
+  return o.finish("op_coattention");
+}
+
+FPNMT_API int fpnmt_op_tokens_ln_pos(int device, int precision, const float* x, int N, int HW, const float* gamma,
+                                     const float* beta, float eps, const float* pos, float* out, void* stream) {
+  if (!x || !gamma || !beta || !pos || !out || N < 1 || HW < 1 || bad_precision(precision))
+    return op_invalid("op_tokens_ln_pos: bad arguments");
+  int rc = op_device(device, "op_tokens_ln_pos");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const float *dg = o.upload(gamma, 512), *db = o.upload(beta, 512), *dp = o.upload(pos, (size_t)HW * 512);
+  const size_t rows = (size_t)N * HW;
+  Act ax = o.act(rows, 512, 512, x), ao = o.act(rows, 512, 512, out);
+  if (!o.rc) o.rc = launch_tokens_ln_pos(ax, N, HW, dg, db, eps, dp, ao, o.s);
+  o.read_back(ao, rows, out);
+  return o.finish("op_tokens_ln_pos");
+}
+
+FPNMT_API int fpnmt_op_enc_attention(int device, int precision, const float* q, const float* const* kv, const int* tk,
+                                     int nviews, int kv_ld, int k_col, int v_col, int B, int Tq, int heads, int force_simt,
+                                     float* out, void* stream) {
+  const int width = heads * 64;
+  if (!q || !kv || !tk || !out || nviews < 1 || nviews > 4 || B < 1 || B > 65535 || Tq < 1 || heads < 1 || heads > 65535 ||
+      bad_precision(precision) || kv_ld % 8 || k_col < 0 || v_col < 0 || k_col % 8 || v_col % 8 || k_col + width > kv_ld ||
+      v_col + width > kv_ld)
+    return op_invalid("op_enc_attention: bad arguments (1..4 views, K/V columns multiples of 8 inside kv_ld)");
+  for (int v = 0; v < nviews; ++v)
+    if (!kv[v] || tk[v] < 1) return op_invalid("op_enc_attention: every view needs K/V and tk >= 1");
+  int rc = op_device(device, "op_enc_attention");
+  if (rc) return rc;
+  rc = attention_set_attributes();
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const size_t qrows = (size_t)B * Tq;
+  const int qw = nviews * width;
+  Act aq = o.act(qrows, qw, qw, q), ao = o.act(qrows, qw, qw, out), akv[4];
+  int cols[4];
+  for (int v = 0; v < nviews; ++v) {
+    akv[v] = o.act((size_t)B * tk[v], kv_ld, kv_ld, kv[v]);
+    cols[v] = v * width;
+  }
+  // kernel choice of Engine::build_mt_encoder: one views launch in bf16 mode, else one launch per view
+  if (!o.rc && !o.split && !force_simt && nviews > 1) {
+    o.rc = launch_enc_attention_views(aq, akv, tk, cols, nviews, k_col, v_col, B, Tq, heads, ao, o.s);
+  } else {
+    for (int v = 0; v < nviews && !o.rc; ++v)
+      o.rc = launch_enc_attention(aq, cols[v], akv[v], k_col, v_col, B, Tq, tk[v], heads, ao, cols[v], force_simt != 0, o.s);
+  }
+  o.read_back(ao, qrows, out);
+  return o.finish("op_enc_attention");
+}
+
+}  // extern "C"

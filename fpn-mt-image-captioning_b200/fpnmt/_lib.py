@@ -63,6 +63,13 @@ SIGNATURES = {
     "fpnmt_op_preprocess": (_i, [_i, _vp, _i, _i, _i, _i, _vp, _vp]),
     "fpnmt_op_decode_jpeg": (_i, [_i, C.POINTER(_vp), C.POINTER(C.c_size_t), _i, _i, _vp, _vp, _vp]),
     "fpnmt_op_dense": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _i, _vp, _vp, _vp, C.c_float, _vp, _i, _vp]),
+    "fpnmt_op_depthwise3x3": (_i, [_i, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
+    "fpnmt_op_pool": (_i, [_i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
+    "fpnmt_op_scale_shift_relu": (_i, [_i, _i, _vp, C.c_int64, _i, _i, _vp, _vp, _vp, _i, _vp]),
+    "fpnmt_op_score_conv": (_i, [_i, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "fpnmt_op_coattention": (_i, [_i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "fpnmt_op_tokens_ln_pos": (_i, [_i, _i, _vp, _i, _i, _vp, _vp, C.c_float, _vp, _vp, _vp]),
+    "fpnmt_op_enc_attention": (_i, [_i, _i, _vp, C.POINTER(_vp), C.POINTER(_i), _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
 }
 
 

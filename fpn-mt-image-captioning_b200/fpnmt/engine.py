@@ -346,6 +346,152 @@ def dense(x: torch.Tensor, kernel: np.ndarray, bias: Optional[np.ndarray] = None
     return out
 
 
+# ---- stand-alone encoder bandwidth operators (kernel parity tests) --------------------------------------------------------
+# Channel views: `x` / `out` may carry more channels per pixel (the last dim, a multiple of 8) than the `channels` the
+# kernel reads and writes, like DenseNet's stage buffers.  `out` is read as well as written (updated in place and
+# returned): what the kernel must not write comes back unchanged.  Without `out` a zero tensor is used.
+def _host32(a):
+    return None if a is None else np.ascontiguousarray(a, dtype=np.float32)
+
+
+def _hptr(a):
+    return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _dev32(t: torch.Tensor) -> torch.Tensor:
+    if t.device.type != "cuda":
+        raise RuntimeError("the stand-alone operators need CUDA tensors; there is no CPU fallback")
+    return t.to(torch.float32).contiguous()
+
+
+def _out32(out: Optional[torch.Tensor], shape, dev) -> torch.Tensor:
+    if out is None:
+        return torch.zeros(shape, dtype=torch.float32, device=dev)
+    if out.dtype != torch.float32 or not out.is_contiguous() or out.device != dev or tuple(out.shape[:-1]) != tuple(shape[:-1]):
+        raise ValueError("out must be a contiguous float32 tensor of shape %s (+ any channel count) on %s" % (tuple(shape[:-1]), dev))
+    return out
+
+
+def depthwise3x3(x: torch.Tensor, kernel: np.ndarray, bias: Optional[np.ndarray] = None, stride: int = 1,
+                 pad: Tuple[int, int] = (1, 1), out_hw: Optional[Tuple[int, int]] = None, act: int = 0,
+                 channels: Optional[int] = None, out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """MobileNetV2 depthwise 3x3 (BN folded): x (N,H,W,ld), kernel (3,3,C,1), bias (C,) -> out (N,Ho,Wo,ld_out)."""
+    x = _dev32(x)
+    n, h, w, ld = x.shape
+    c = channels or ld
+    ho, wo = out_hw or ((h + 2 * pad[0] - 3) // stride + 1, (w + 2 * pad[1] - 3) // stride + 1)
+    out = _out32(out, (n, ho, wo, c), x.device)
+    k, b = _host32(kernel), _host32(bias)
+    _lib.check(_lib.load().fpnmt_op_depthwise3x3(x.device.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), n, h, w, c, ld,
+                                                 _hptr(k), _hptr(b), stride, pad[0], pad[1], ho, wo, act, out.data_ptr(),
+                                                 out.shape[-1], _stream_ptr(x.device)))
+    return out
+
+
+POOL_MAX, POOL_AVG2, POOL_SUBSAMPLE2 = 0, 1, 2
+
+
+def pool(x: torch.Tensor, kind: int, k: int = 2, stride: int = 2, pad: Tuple[int, int] = (0, 0),
+         out_hw: Optional[Tuple[int, int]] = None, zero_pad: bool = False, channels: Optional[int] = None,
+         out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """Max pool k x k / stride (POOL_MAX), 2x2 average pool (POOL_AVG2) or x[:, ::2, ::2] (POOL_SUBSAMPLE2) in NHWC."""
+    x = _dev32(x)
+    n, h, w, ld = x.shape
+    c = channels or ld
+    if out_hw is None:
+        out_hw = {POOL_MAX: ((h + 2 * pad[0] - k) // stride + 1, (w + 2 * pad[1] - k) // stride + 1),
+                  POOL_AVG2: (h // 2, w // 2), POOL_SUBSAMPLE2: ((h + 1) // 2, (w + 1) // 2)}[kind]
+    ho, wo = out_hw
+    out = _out32(out, (n, ho, wo, c), x.device)
+    _lib.check(_lib.load().fpnmt_op_pool(x.device.index or 0, _lib.PREC_IDS[precision], kind, x.data_ptr(), n, h, w, c, ld, k,
+                                         stride, pad[0], pad[1], ho, wo, int(zero_pad), out.data_ptr(), out.shape[-1],
+                                         _stream_ptr(x.device)))
+    return out
+
+
+def scale_shift_relu(x: torch.Tensor, scale: np.ndarray, shift: np.ndarray, channels: Optional[int] = None,
+                     out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """DenseNet pre-activation BN + ReLU over the pixels of x (..., ld): relu(x[..., c] * scale[c] + shift[c])."""
+    x = _dev32(x)
+    ld = x.shape[-1]
+    c = channels or ld
+    pixels = x.numel() // ld
+    out = _out32(out, tuple(x.shape[:-1]) + (c,), x.device)
+    sc, sh = _host32(scale), _host32(shift)
+    _lib.check(_lib.load().fpnmt_op_scale_shift_relu(x.device.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), pixels, c, ld,
+                                                     _hptr(sc), _hptr(sh), out.data_ptr(), out.shape[-1], _stream_ptr(x.device)))
+    return out
+
+
+def score_conv(x: torch.Tensor, kernel: np.ndarray, bias: np.ndarray, out: Optional[torch.Tensor] = None,
+               precision: str = "bf16") -> torch.Tensor:
+    """Co-attention score map: 3x3 'same' convolution of x (N,H,W,256) to one channel -> (N,H,W).  bf16 only."""
+    x = _dev32(x)
+    n, h, w, _ = x.shape
+    if out is None:
+        out = torch.zeros((n, h, w), dtype=torch.float32, device=x.device)
+    elif out.dtype != torch.float32 or not out.is_contiguous() or tuple(out.shape) != (n, h, w):
+        raise ValueError("out must be a contiguous float32 tensor of shape %s" % ((n, h, w),))
+    k, b = _host32(kernel), _host32(np.reshape(bias, (1,)))
+    _lib.check(_lib.load().fpnmt_op_score_conv(x.device.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), n, h, w, _hptr(k),
+                                               _hptr(b), out.data_ptr(), _stream_ptr(x.device)))
+    return out
+
+
+def coattention(score: torch.Tensor, cls: torch.Tensor, out: Optional[torch.Tensor] = None,
+                precision: str = "bf16") -> torch.Tensor:
+    """CoAttention_CNN: softmax over the HW positions of score (N,HW) times cls (N,HW,C) -> (N,HW,C)."""
+    score, cls = _dev32(score), _dev32(cls)
+    n, hw, c = cls.shape
+    if tuple(score.shape) != (n, hw):
+        raise ValueError("score must be (N, HW) to match cls (N, HW, C)")
+    out = _out32(out, (n, hw, c), cls.device)
+    if out.shape[-1] != c:
+        raise ValueError("out must have the C channels of cls")
+    _lib.check(_lib.load().fpnmt_op_coattention(cls.device.index or 0, _lib.PREC_IDS[precision], score.data_ptr(), cls.data_ptr(),
+                                                n, hw, c, out.data_ptr(), _stream_ptr(cls.device)))
+    return out
+
+
+def tokens_ln_pos(x: torch.Tensor, hw: int, gamma: np.ndarray, beta: np.ndarray, pos: np.ndarray, eps: float = 1e-6,
+                  out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """Encoder token pre-amble: LayerNorm(x[n*hw+p]) + pos[p] over rows of x (N*hw, 512)."""
+    x = _dev32(x)
+    rows = x.shape[0]
+    if x.shape[-1] != 512 or rows % hw:
+        raise ValueError("x must be (N*hw, 512)")
+    out = _out32(out, (rows, 512), x.device)
+    if out.shape[-1] != 512:
+        raise ValueError("out must be (N*hw, 512)")
+    g, b, p = _host32(gamma), _host32(beta), _host32(pos)
+    if p.size != hw * 512:
+        raise ValueError("pos must be (hw, 512)")
+    _lib.check(_lib.load().fpnmt_op_tokens_ln_pos(x.device.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), rows // hw, hw,
+                                                  _hptr(g), _hptr(b), eps, _hptr(p), out.data_ptr(), _stream_ptr(x.device)))
+    return out
+
+
+def enc_attention(q: torch.Tensor, kvs: Sequence[torch.Tensor], batch: int, heads: int, k_col: int, v_col: int,
+                  force_simt: bool = False, out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """Cross-level attention of the encoder: q (B*Tq, len(kvs)*heads*64) against the K/V columns [k_col, k_col+heads*64) /
+    [v_col, ...) of each view's kvs[v] (B*Tk_v, kv_ld) -> (B*Tq, len(kvs)*heads*64).  All views share kv_ld."""
+    q = _dev32(q)
+    kvs = [_dev32(t) for t in kvs]
+    nv = len(kvs)
+    if q.shape[0] % batch or any(t.shape[0] % batch or t.shape[1] != kvs[0].shape[1] for t in kvs):
+        raise ValueError("q and every K/V tensor must hold `batch` images, the K/V tensors one width")
+    tq = q.shape[0] // batch
+    out = _out32(out, (q.shape[0], q.shape[1]), q.device)
+    if q.shape[1] != nv * heads * 64 or out.shape[1] != q.shape[1]:
+        raise ValueError("q and out must be (B*Tq, len(kvs)*heads*64)")
+    ptrs = (C.c_void_p * nv)(*[t.data_ptr() for t in kvs])
+    tks = (C.c_int * nv)(*[t.shape[0] // batch for t in kvs])
+    _lib.check(_lib.load().fpnmt_op_enc_attention(q.device.index or 0, _lib.PREC_IDS[precision], q.data_ptr(), ptrs, tks, nv,
+                                                  kvs[0].shape[1], k_col, v_col, batch, tq, heads, int(force_simt),
+                                                  out.data_ptr(), _stream_ptr(q.device)))
+    return out
+
+
 def preprocess(images_u8: torch.Tensor, size: int = cfg.IMAGE_INPUT_SIZE) -> torch.Tensor:
     """GPU `load_image` after the JPEG decode (dataset.py:21-24): uint8 (N,H,W,3) -> float32 (N,size,size,3) in [-1,1]."""
     lib = _lib.load()

@@ -236,6 +236,53 @@ FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, i
                    const float* bias, int act, const float* residual, const float* gamma, const float* beta, float eps,
                    float* out, int force_bn, void* stream);
 
+/* Encoder bandwidth kernels one at a time (the launchers of the engine's program, which choose the kernel by precision
+ * and shape exactly as the engine does).  Activations are DEVICE float32, uploaded into bf16 (or bf16x3 hi + lo)
+ * activations and read back after the kernel.  Channel views: a tensor with ld channels per pixel (in_ld / out_ld,
+ * 0 = C, multiples of 8) of which the kernel reads or writes the first C, as DenseNet's stage buffers are used.  `out`
+ * is read as well as written: its incoming contents are uploaded first, so values the kernel does not write (other
+ * columns, other pixels) come back unchanged.  Host arrays are float32; all calls synchronise `stream`. */
+
+/* MobileNetV2 DepthwiseConv2D 3x3 with BatchNorm folded in (models/retinanet.py backbone): out[n,yo,xo,c] =
+ * act(sum_{ky,kx} x[n, yo*stride+ky-pad_top, xo*stride+kx-pad_left, c] * kernel[ky,kx,c] + bias[c]), taps outside the
+ * image are zero.  x [N,H,W,in_ld]; kernel HOST (3,3,C,1); bias HOST [C] or NULL; out [N,Ho,Wo,out_ld]; stride 1 or 2;
+ * act as fpnmt_op_conv2d.  bf16 stride 1 runs the 4-outputs-per-thread kernel, everything else the generic one. */
+FPNMT_API int fpnmt_op_depthwise3x3(int device, int precision, const float* x, int N, int H, int W, int C, int in_ld,
+                                    const float* kernel, const float* bias, int stride, int pad_top, int pad_left, int Ho,
+                                    int Wo, int act, float* out, int out_ld, void* stream);
+/* kind 0: MaxPooling2D k x k / stride, out-of-image taps ignored (-inf padding) or, with zero_pad, counted as 0
+ * (ZeroPadding2D + valid pool); kind 1: AveragePooling2D 2x2 / 2 (Ho = H/2, Wo = W/2); kind 2: out[n,y,x] = x[n,2y,2x]
+ * (the stride-2 1x1 input of a ResNet stage, Ho = (H+1)/2, Wo = (W+1)/2).  x [N,H,W,in_ld]; out [N,Ho,Wo,out_ld]. */
+FPNMT_API int fpnmt_op_pool(int device, int precision, int kind, const float* x, int N, int H, int W, int C, int in_ld, int k,
+                            int stride, int pad_top, int pad_left, int Ho, int Wo, int zero_pad, float* out, int out_ld,
+                            void* stream);
+/* DenseNet pre-activation BatchNormalization + ReLU: out[p,c] = max(x[p,c] * scale[c] + shift[c], 0).
+ * x [pixels,in_ld]; scale / shift HOST [C]; out [pixels,out_ld]. */
+FPNMT_API int fpnmt_op_scale_shift_relu(int device, int precision, const float* x, int64_t pixels, int C, int in_ld,
+                                        const float* scale, const float* shift, float* out, int out_ld, void* stream);
+/* The co-attention score map, Conv2D(1, 3x3, padding='same') on 256 channels (models/retinanet.py:287): x [N,H,W,256];
+ * kernel HOST (3,3,256,1); bias HOST [1]; out [N,H,W].  bf16 only (the one-channel CUDA-core kernel); bf16x3 runs
+ * fpnmt_op_conv2d with Cout = 1 and is rejected here with FPNMT_ERR_INVALID. */
+FPNMT_API int fpnmt_op_score_conv(int device, int precision, const float* x, int N, int H, int W, const float* kernel,
+                                  const float* bias, float* out, void* stream);
+/* CoAttention_CNN (coattention.py:13-32): out[n,p,c] = softmax_p(score[n,:])[p] * cls[n,p,c].  score [N,HW];
+ * cls and out [N,HW,C]. */
+FPNMT_API int fpnmt_op_coattention(int device, int precision, const float* score, const float* cls, int N, int HW, int C,
+                                   float* out, void* stream);
+/* Encoder token pre-amble (transformer.py:279-296): out[n*HW+p] = LayerNormalization(epsilon=eps)(x[n*HW+p]) + pos[p],
+ * d_model 512.  x and out [N*HW,512]; gamma / beta HOST [512]; pos HOST [HW,512]. */
+FPNMT_API int fpnmt_op_tokens_ln_pos(int device, int precision, const float* x, int N, int HW, const float* gamma,
+                                     const float* beta, float eps, const float* pos, float* out, void* stream);
+/* Cross-level attention of the Multi-Transformer encoder (head dim 64): for view v, head h, image b,
+ * out[b*Tq+i, (v*heads+h)*64 + d] = softmax_j(q_i . k_j / 8) v_j with q_i = q[b*Tq+i, (v*heads+h)*64 ..],
+ * k_j = kv[v][b*tk[v]+j, k_col + h*64 ..], v_j = kv[v][b*tk[v]+j, v_col + h*64 ..].  q and out [B*Tq, nviews*heads*64];
+ * kv HOST array of nviews DEVICE pointers to [B*tk[v], kv_ld]; tk HOST [nviews]; Tq <= 16 (else FPNMT_ERR_INVALID).
+ * Kernel choice as the engine's: bf16 with nviews > 1 one launch of all views, bf16 with one view the tensor-core kernel,
+ * bf16x3 or force_simt the fp32 CUDA-core kernel once per view. */
+FPNMT_API int fpnmt_op_enc_attention(int device, int precision, const float* q, const float* const* kv, const int* tk,
+                                     int nviews, int kv_ld, int k_col, int v_col, int B, int Tq, int heads, int force_simt,
+                                     float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
