@@ -404,6 +404,11 @@ struct OpScratch {
     cudaMemcpyAsync(d, h, n * 4, cudaMemcpyHostToDevice, s);
     return d;
   }
+  const int* upload_i(const int* h, size_t n) {
+    int* d = (int*)alloc(n * 4);
+    if (d) cudaMemcpyAsync(d, h, n * 4, cudaMemcpyHostToDevice, s);
+    return d;
+  }
   // activation of `ld` channels per row (the engine's layout: hi at [c], lo at [ld + c] in bf16x3), filled from device
   // fp32 [rows][ld] when src != NULL; the returned view covers the first C channels
   Act act(size_t rows, int C, int ld, const float* src) {
@@ -448,6 +453,11 @@ bool view_ld(int C, int* ld) {
   return C > 0 && C % 8 == 0 && *ld >= C && *ld % 8 == 0;
 }
 bool bad_precision(int precision) { return precision != FPNMT_PREC_BF16 && precision != FPNMT_PREC_BF16X3; }
+bool all_in(const int* v, size_t n, int lo, int hi) {
+  for (size_t i = 0; i < n; ++i)
+    if (v[i] < lo || v[i] >= hi) return false;
+  return true;
+}
 }  // namespace
 
 extern "C" {
@@ -589,6 +599,169 @@ FPNMT_API int fpnmt_op_enc_attention(int device, int precision, const float* q, 
   }
   o.read_back(ao, qrows, out);
   return o.finish("op_enc_attention");
+}
+
+
+// ---- stand-alone decoder operators ----------------------------------------------------------------------------------
+FPNMT_API int fpnmt_op_dec_self_attention(int device, int precision, const float* qkv, float* kc, float* vc, float* kc2,
+                                          float* vc2, const int* anc, const int* rep, int rows, int T, int t, int heads, int beam,
+                                          int kernel, float* out, void* stream) {
+  if (!qkv || !kc || !vc || !anc || !out || (!kc2) != (!vc2) || rows < 1 || T < 1 || t < 0 || t >= T || heads < 1 ||
+      beam < 1 || beam > 32 || kernel < 0 || kernel > 2 || bad_precision(precision) ||
+      (kernel == DEC_ATT_MMA && precision != FPNMT_PREC_BF16) || (size_t)rows * heads > (1u << 30) || (size_t)rows * T > (1u << 26))
+    return op_invalid("op_dec_self_attention: bad arguments (0 <= t < T, beam 1..32, kernel 0..2, mma only in bf16)");
+  if (!all_in(anc, (size_t)2 * rows * T, 0, rows) || (rep && !all_in(rep, (size_t)2 * rows, 0, rows)))
+    return op_invalid("op_dec_self_attention: anc and rep entries must be rows in [0, rows)");
+  int rc = op_device(device, "op_dec_self_attention");
+  if (rc) return rc;
+  rc = attention_set_attributes();
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const int d = heads * 64;
+  const size_t crows = (size_t)rows * T;
+  const int* danc = o.upload_i(anc, (size_t)2 * rows * T);
+  const int* drep = rep ? o.upload_i(rep, (size_t)2 * rows) : nullptr;
+  const int* dstep = o.upload_i(&t, 1);
+  const Act none{nullptr, 0, 0, 0};
+  Act aq = o.act(rows, 3 * d, 3 * d, qkv), ao = o.act(rows, d, d, out);
+  Act ak = o.act(crows, d, d, kc), av = o.act(crows, d, d, vc);
+  Act ak2 = kc2 ? o.act(crows, d, d, kc2) : none, av2 = vc2 ? o.act(crows, d, d, vc2) : none;
+  if (!o.rc)
+    o.rc = launch_dec_self_attention(aq, ak, av, ak2, av2, danc, crows, dstep, rows, T, heads, ao, o.s, drep,
+                                     drep ? drep + rows : nullptr, beam, (DecAttKernel)kernel);
+  o.read_back(ao, rows, out);
+  o.read_back(ak, crows, kc);
+  o.read_back(av, crows, vc);
+  if (kc2) {
+    o.read_back(ak2, crows, kc2);
+    o.read_back(av2, crows, vc2);
+  }
+  return o.finish("op_dec_self_attention");
+}
+
+FPNMT_API int fpnmt_op_dec_cross_attention(int device, int precision, const float* q, const float* kv, int kv_ld, int k_col,
+                                           int v_col, int rows, int beam, int Tk, int heads, float* out, void* stream) {
+  const int d = heads * 64;
+  if (!q || !kv || !out || rows < 1 || beam < 1 || rows % beam || Tk < 1 || heads < 1 || (size_t)rows * heads > (1u << 30) ||
+      bad_precision(precision) || kv_ld < 8 || kv_ld % 8 || k_col < 0 || v_col < 0 || k_col % 8 || v_col % 8 ||
+      k_col + d > kv_ld || v_col + d > kv_ld)
+    return op_invalid("op_dec_cross_attention: bad arguments (beam divides rows, K/V columns multiples of 8 inside kv_ld)");
+  int rc = op_device(device, "op_dec_cross_attention");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  Act aq = o.act(rows, d, d, q), ao = o.act(rows, d, d, out);
+  Act akv = o.act((size_t)(rows / beam) * Tk, kv_ld, kv_ld, kv);
+  if (!o.rc) o.rc = launch_dec_cross_attention(aq, akv, k_col, v_col, rows, beam, Tk, heads, ao, o.s);
+  o.read_back(ao, rows, out);
+  return o.finish("op_dec_cross_attention");
+}
+
+FPNMT_API int fpnmt_op_xattn(int device, int precision, const float* ckv, const float* wq, const float* bq, const float* wo,
+                             const float* bo, const float* gamma, const float* beta, int Btot, int n_mem, int L, int layer,
+                             int b0, int B, int beam, const float* out1, float* out2, float* Mt, float* Nt, float* sbias,
+                             void* stream) {
+  if (precision != FPNMT_PREC_BF16)
+    return op_invalid("op_xattn: the fused cross-attention block is a bf16-mode kernel (bf16x3 runs the unfused path)");
+  if (!ckv || !wq || !bq || !wo || !bo || !gamma || !beta || !out1 || !out2 || Btot < 1 || Btot > 65535 || n_mem < 1 ||
+      n_mem > 16 || L < 1 || L > 64 || layer < 0 || layer >= L || b0 < 0 || B < 1 || b0 + B > Btot || beam < 1 || beam > 16)
+    return op_invalid("op_xattn: bad arguments (n_mem and beam 1..16, 0 <= layer < L, images [b0, b0 + B) inside Btot)");
+  int rc = op_device(device, "op_xattn");
+  if (rc) return rc;
+  rc = xattn_set_attributes();
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const size_t W = (size_t)512 * 512;
+  std::vector<uint16_t> hwq((size_t)L * W), hwo((size_t)L * W);
+  for (int l = 0; l < L; ++l) xattn_fold_weights(wq + l * W, wo + l * W, &hwq[l * W], &hwo[l * W]);
+  bf16* dq = (bf16*)o.alloc(hwq.size() * 2);
+  bf16* d_o = (bf16*)o.alloc(hwo.size() * 2);
+  const float* dbq = o.upload(bq, (size_t)L * 512);
+  std::vector<const float*> hb(L);
+  for (int l = 0; l < L; ++l) hb[l] = dbq ? dbq + (size_t)l * 512 : nullptr;
+  const float** db = (const float**)o.alloc(L * sizeof(float*));
+  const float *dbo = o.upload(bo, 512), *dg = o.upload(gamma, 512), *dbe = o.upload(beta, 512);
+  bf16* dMt = (bf16*)o.alloc((size_t)L * Btot * 128 * 512 * 2);
+  bf16* dNt = (bf16*)o.alloc((size_t)L * Btot * 512 * 128 * 2);
+  float* dsb = (float*)o.alloc((size_t)L * Btot * 128 * 4);
+  if (o.rc) return o.finish("op_xattn");
+  cudaMemcpyAsync(dq, hwq.data(), hwq.size() * 2, cudaMemcpyHostToDevice, o.s);
+  cudaMemcpyAsync(d_o, hwo.data(), hwo.size() * 2, cudaMemcpyHostToDevice, o.s);
+  cudaMemcpyAsync(db, hb.data(), L * sizeof(float*), cudaMemcpyHostToDevice, o.s);
+  const size_t rows = (size_t)Btot * beam;
+  Act ac = o.act((size_t)Btot * n_mem, L * 1024, L * 1024, ckv);
+  Act ax = o.act(rows, 512, 512, out1), ay = o.act(rows, 512, 512, out2);
+  if (!o.rc) o.rc = launch_xattn_fold(ac, Btot, n_mem, L, dq, db, d_o, dMt, dNt, dsb, o.s);
+  Act xv = ax, yv = ay;                   // row views of the slice, as Engine's build_chain makes them
+  xv.p += (size_t)b0 * beam * ax.ld;
+  yv.p += (size_t)b0 * beam * ay.ld;
+  XattnOp op;
+  if (!o.rc) o.rc = make_xattn_op(&op, dMt, dNt, L, Btot, b0, B, beam, layer, dsb, dbo, dg, dbe, xv, yv);
+  if (!o.rc) o.rc = xattn_launch(op, o.s);
+  o.read_back(ay, rows, out2);
+  if (Mt) o.read_back(Act{dMt, 512, 512, 0}, (size_t)L * Btot * 128, Mt);
+  if (Nt) o.read_back(Act{dNt, 128, 128, 0}, (size_t)L * Btot * 512, Nt);
+  if (sbias && !o.rc) cudaMemcpyAsync(sbias, dsb, (size_t)L * Btot * 128 * 4, cudaMemcpyDeviceToDevice, o.s);
+  return o.finish("op_xattn");
+}
+
+FPNMT_API int fpnmt_op_kv_reorder(int device, int precision, const float* src, float* dst, int ncaches, const int* parent,
+                                  int rows, int beam, int T, int D, int t, void* stream) {
+  if (!src || !dst || !parent || ncaches < 1 || ncaches > 65535 || rows < 1 || beam < 1 || rows % beam || T < 1 || t < 0 ||
+      t > T || D < 8 || D % 8 || bad_precision(precision) || (size_t)rows * T > (1u << 26))
+    return op_invalid("op_kv_reorder: bad arguments (beam divides rows, 0 <= t <= T, D a multiple of 8)");
+  if (!all_in(parent, (size_t)T * rows, 0, beam)) return op_invalid("op_kv_reorder: parent entries must be beams in [0, beam)");
+  int rc = op_device(device, "op_kv_reorder");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const size_t crows = (size_t)rows * T, all = crows * ncaches;
+  const int* dpar = o.upload_i(parent, (size_t)T * rows);
+  const int* dstep = o.upload_i(&t, 1);
+  Act as = o.act(all, D, D, src), ad = o.act(all, D, D, dst);
+  // bufs[parity][cache]: the kernel reads parity (t-1)&1 and writes the other, as after decode step t-1 of the engine
+  const int tt = t - 1;
+  std::vector<const bf16*> hp((size_t)2 * ncaches);
+  for (int c = 0; c < ncaches; ++c) {
+    hp[(size_t)(tt & 1) * ncaches + c] = as.p + c * crows * as.ld;
+    hp[(size_t)((tt + 1) & 1) * ncaches + c] = ad.p + c * crows * ad.ld;
+  }
+  const bf16** dp = (const bf16**)o.alloc(hp.size() * sizeof(bf16*));
+  if (!o.rc) {
+    cudaMemcpyAsync(dp, hp.data(), hp.size() * sizeof(bf16*), cudaMemcpyHostToDevice, o.s);
+    o.rc = launch_kv_reorder(dp, ncaches, dpar, rows, rows, beam, T, as.ld * 2, dstep, o.s);
+  }
+  o.read_back(ad, all, dst);
+  return o.finish("op_kv_reorder");
+}
+
+FPNMT_API int fpnmt_op_embed_pos(int device, int precision, const int* tokens, int rows, const float* emb, int V,
+                                 const float* pos, int T, int C, int t, float* out, void* stream) {
+  if (!tokens || !emb || !pos || !out || rows < 1 || V < 1 || T < 1 || t < 0 || t >= T || C < 8 || C % 8 ||
+      bad_precision(precision) || (size_t)rows * C > (1u << 30))
+    return op_invalid("op_embed_pos: bad arguments (C a multiple of 8, 0 <= t < T)");
+  if (!all_in(tokens, rows, 0, V)) return op_invalid("op_embed_pos: tokens must be in [0, V)");
+  int rc = op_device(device, "op_embed_pos");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const int *dtok = o.upload_i(tokens, rows), *dstep = o.upload_i(&t, 1);
+  const float *demb = o.upload(emb, (size_t)V * C), *dpos = o.upload(pos, (size_t)T * C);
+  Act ao = o.act(rows, C, C, out);
+  if (!o.rc) o.rc = launch_embed_pos(dtok, demb, dpos, dstep, rows, C, ao, o.s);
+  o.read_back(ao, rows, out);
+  return o.finish("op_embed_pos");
+}
+
+FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x, int rows, const float* gamma,
+                                      const float* beta, float eps, float* out, void* stream) {
+  if (!x || !gamma || !beta || !out || rows < 1 || bad_precision(precision))
+    return op_invalid("op_layernorm_rows: bad arguments");
+  int rc = op_device(device, "op_layernorm_rows");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, precision);
+  const float *dg = o.upload(gamma, 512), *db = o.upload(beta, 512);
+  Act ao = o.act(rows, 512, 512, out);
+  if (!o.rc) o.rc = launch_layernorm_rows(x, rows, 512, dg, db, eps, ao, o.s);
+  o.read_back(ao, rows, out);
+  return o.finish("op_layernorm_rows");
 }
 
 }  // extern "C"

@@ -799,19 +799,30 @@ int dec_attention_set_attributes() {
 
 int launch_dec_self_attention(Act qkv, Act kcache, Act vcache, Act kcache2, Act vcache2, const int* anc, size_t anc_stride,
                               const int* step, int rows, int T, int heads, Act out, cudaStream_t s, const int* rep_e,
-                              const int* rep_o, int N) {
+                              const int* rep_o, int N, DecAttKernel kernel) {
   const int warps = rows * heads;
+  const bool plain = !kcache.lo && !qkv.lo && !out.lo;
+  if (kernel == DEC_ATT_MMA && !plain) {
+    set_last_error("dec_self_attention: the mma.sync kernel needs plain bf16 activations");
+    return 1;
+  }
+  const bool simt = kernel == DEC_ATT_SIMT || (kernel == DEC_ATT_AUTO && g_dec_att_simt);
   if (kcache.lo)
     FPNMT_CUDA_OK(launch_k_small(k_dec_self_attention<true>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
                            qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, rows, T, heads, out));
-  else if (qkv.lo || out.lo || g_dec_att_simt)
+  else if (!plain || simt)
     FPNMT_CUDA_OK(launch_k_small(k_dec_self_attention<false>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
                            qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, rows, T, heads, out));
-  else
+  else {
+    // The kernel finds beam n of image b at row b * N + n, so N must divide the rows; otherwise every row is its own image
+    // and its own class (rep_e / rep_o index rows by that layout and would name representatives of other images).
+    const int n = (N >= 1 && rows % N == 0) ? N : 1;
+    const bool classes = n == N && N <= 8;
     FPNMT_CUDA_OK(launch_k_small(k_dec_self_attention_mma, dim3((warps + DEC_MMA_WARPS - 1) / DEC_MMA_WARPS), dim3(DEC_MMA_WARPS * 32),
                                  DEC_MMA_WARPS * sizeof(DecAttTile), s,
-                           qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, (N >= 1 && N <= 8) ? rep_e : nullptr,
-                           (N >= 1 && N <= 8) ? rep_o : nullptr, rows, T, heads, (N >= 1 && rows % N == 0) ? N : 1, out));
+                           qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, classes ? rep_e : nullptr,
+                           classes ? rep_o : nullptr, rows, T, heads, n, out));
+  }
   return 0;
 }
 

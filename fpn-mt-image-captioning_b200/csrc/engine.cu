@@ -188,6 +188,11 @@ static inline uint16_t f2bf(float f) {   // round-to-nearest-even, matches __flo
   u += 0x7fffu + ((u >> 16) & 1u);
   return (uint16_t)(u >> 16);
 }
+void xattn_fold_weights(const float* wq, const float* wo, uint16_t* wq_bf16, uint16_t* woT_bf16) {
+  for (size_t i = 0; i < 512 * 512; ++i) wq_bf16[i] = f2bf(wq[i]);
+  for (int hd = 0; hd < 512; ++hd)
+    for (int f = 0; f < 512; ++f) woT_bf16[(size_t)f * 512 + hd] = f2bf(wo[(size_t)hd * 512 + f]);
+}
 static inline float bf2f(uint16_t h) {
   uint32_t u = (uint32_t)h << 16;
   float f;
@@ -1006,9 +1011,7 @@ int Engine::build_decoder() {
         const HostW *kq = W(m + "/wq/kernel"), *ko = W(m + "/dense/kernel");
         if (!kq || !ko) return FPNMT_ERR_MISSING;
         if (kq->data.size() != 512 * 512 || ko->data.size() != 512 * 512) return fail(FPNMT_ERR_INVALID, m + ": projection kernels must be 512x512");
-        for (size_t i = 0; i < 512 * 512; ++i) hwq[(size_t)l * 512 * 512 + i] = f2bf(kq->data[i]);
-        for (int hd = 0; hd < 512; ++hd)
-          for (int f = 0; f < 512; ++f) hwo[((size_t)l * 512 + f) * 512 + hd] = f2bf(ko->data[(size_t)hd * 512 + f]);
+        xattn_fold_weights(kq->data.data(), ko->data.data(), &hwq[(size_t)l * 512 * 512], &hwo[(size_t)l * 512 * 512]);
         float* b2;
         RC(prep_vec(m + "/wq/bias", &b2));
         hb[l] = b2;

@@ -58,11 +58,15 @@ int launch_enc_attention_views(Act q, const Act* kvs, const int* tks, const int*
 // qkv: [rows][3*d] (q|k|v) of the new position; caches [rows][T][d]; anc [2][..][T] physical row per position, the two
 // step parities `anc_stride` ints apart (rows may be a slice of a larger batch: anc_stride = total rows * T).
 // kcache2 / vcache2 (p != nullptr): physical cache mode - odd steps read and append to the second buffer pair.
+// Kernel choice: DEC_ATT_AUTO is the engine's (bf16x3: the split CUDA-core kernel; bf16: the mma.sync kernel, or the CUDA-core
+// kernel under FPNMT_OPT_DEC_ATT_SIMT); DEC_ATT_SIMT / DEC_ATT_MMA force one of the two bf16 kernels (MMA needs plain bf16).
+enum DecAttKernel { DEC_ATT_AUTO = 0, DEC_ATT_SIMT = 1, DEC_ATT_MMA = 2 };
 int launch_dec_self_attention(Act qkv, Act kcache, Act vcache, Act kcache2, Act vcache2, const int* anc, size_t anc_stride,
                               const int* step, int rows, int T, int heads, Act out, cudaStream_t s, const int* rep_e = nullptr,
-                              const int* rep_o = nullptr, int N = 1);
-// rep_e / rep_o (bf16 tensor-core kernel only, beam N <= 8): BeamState::rep of the two step parities - the warp of a class
-// representative computes every member of its token-history class (members = MMA rows).  nullptr: every row is its own class.
+                              const int* rep_o = nullptr, int N = 1, DecAttKernel kernel = DEC_ATT_AUTO);
+// rep_e / rep_o (bf16 tensor-core kernel only, beam N <= 8 dividing rows): BeamState::rep of the two step parities - the warp
+// of a class representative computes every member of its token-history class (members = MMA rows).  nullptr: every row is
+// its own class.
 // Decoder cross-attention over the 16 memory tokens of the row's image.
 int launch_dec_cross_attention(Act q, Act kv, int k_col, int v_col, int rows, int beam, int Tk, int heads, Act out,
                                cudaStream_t s);

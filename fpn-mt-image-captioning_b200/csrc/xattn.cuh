@@ -49,6 +49,9 @@ int make_xattn_op(XattnOp* op, const bf16* Mt, const bf16* Nt, int L, int Btot, 
 // Folding kernels (once per batch, all layers): ckv = cross K/V activations [B*n_mem][L*2*512] (K at l*1024, V at +512).
 // wq: bf16 [L][512 k][512 (h,d)] (the Dense kernel of mha2/wq as stored, in -> out); woT: bf16 [L][512 f][512 (h,d)] (the
 // mha2 output Dense kernel TRANSPOSED); bq: per-layer fp32 bias pointers.
+// Host side of the fold operands of one layer (512 x 512 each, bf16 bits): wq_bf16 = the mha2/wq Dense kernel as stored,
+// woT_bf16[f][(h,d)] = the mha2 output Dense kernel wo[(h,d)][f] transposed.
+void xattn_fold_weights(const float* wq, const float* wo, uint16_t* wq_bf16, uint16_t* woT_bf16);
 int launch_xattn_fold(const Act& ckv, int B, int n_mem, int L, const bf16* wq, const float* const* bq, const bf16* woT,
                       bf16* Mt, bf16* Nt, float* sbias, cudaStream_t s);
 

@@ -70,6 +70,13 @@ SIGNATURES = {
     "fpnmt_op_coattention": (_i, [_i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "fpnmt_op_tokens_ln_pos": (_i, [_i, _i, _vp, _i, _i, _vp, _vp, C.c_float, _vp, _vp, _vp]),
     "fpnmt_op_enc_attention": (_i, [_i, _i, _vp, C.POINTER(_vp), C.POINTER(_i), _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "fpnmt_op_dec_self_attention": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "fpnmt_op_dec_cross_attention": (_i, [_i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "fpnmt_op_xattn": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp,
+                            _vp]),
+    "fpnmt_op_kv_reorder": (_i, [_i, _i, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp]),
+    "fpnmt_op_embed_pos": (_i, [_i, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _vp, _vp]),
+    "fpnmt_op_layernorm_rows": (_i, [_i, _i, _vp, _i, _vp, _vp, C.c_float, _vp, _vp]),
 }
 
 

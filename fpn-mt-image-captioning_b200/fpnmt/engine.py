@@ -492,6 +492,133 @@ def enc_attention(q: torch.Tensor, kvs: Sequence[torch.Tensor], batch: int, head
     return out
 
 
+# ---- stand-alone decoder operators (kernel parity tests) ------------------------------------------------------------------
+# Tensors the kernel writes (`out`, the caches, `dst`) are updated in place and must already be contiguous float32 CUDA
+# tensors; integer tables are host arrays, checked by the library before upload.
+def _inout32(t: torch.Tensor, shape, name: str) -> torch.Tensor:
+    if t.dtype != torch.float32 or not t.is_contiguous() or t.device.type != "cuda" or tuple(t.shape) != tuple(shape):
+        raise ValueError("%s must be a contiguous float32 CUDA tensor of shape %s" % (name, tuple(shape)))
+    return t
+
+
+def _host_i32(a):
+    return None if a is None else np.ascontiguousarray(a, dtype=np.int32)
+
+
+DEC_ATT_KERNELS = {"auto": 0, "simt": 1, "mma": 2}
+
+
+def dec_self_attention(qkv: torch.Tensor, kc: torch.Tensor, vc: torch.Tensor, anc, t: int, heads: int, beam: int = 1, rep=None,
+                       kc2: Optional[torch.Tensor] = None, vc2: Optional[torch.Tensor] = None, kernel: str = "auto",
+                       out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """Decode self-attention of step t: qkv (rows, 3*heads*64) against the caches kc / vc (rows*T, heads*64) through the
+    ancestry table anc (2, rows, T); appends the new K/V to kc / vc (kc2 / vc2 on odd steps in the physical mode, which
+    passing them selects).  rep (2, rows): token-history class representatives, or None.  Returns out (rows, heads*64)."""
+    qkv = _dev32(qkv)
+    rows, d = qkv.shape[0], heads * 64
+    a = _host_i32(anc)
+    T = a.shape[-1]
+    if a.shape != (2, rows, T) or qkv.shape[1] != 3 * d:
+        raise ValueError("qkv must be (rows, 3*heads*64) and anc (2, rows, T)")
+    r = _host_i32(rep)
+    if r is not None and r.shape != (2, rows):
+        raise ValueError("rep must be (2, rows)")
+    if (kc2 is None) != (vc2 is None):
+        raise ValueError("kc2 and vc2 go together (the physical cache mode)")
+    caches = [_inout32(c, (rows * T, d), n) for c, n in ((kc, "kc"), (vc, "vc"), (kc2, "kc2"), (vc2, "vc2")) if c is not None]
+    out = _out32(out, (rows, d), qkv.device)
+    _lib.check(_lib.load().fpnmt_op_dec_self_attention(
+        qkv.device.index or 0, _lib.PREC_IDS[precision], qkv.data_ptr(), caches[0].data_ptr(), caches[1].data_ptr(),
+        kc2.data_ptr() if kc2 is not None else None, vc2.data_ptr() if vc2 is not None else None, _hptr(a), _hptr(r), rows, T,
+        t, heads, beam, DEC_ATT_KERNELS[kernel], out.data_ptr(), _stream_ptr(qkv.device)))
+    return out
+
+
+def dec_cross_attention(q: torch.Tensor, kv: torch.Tensor, beam: int, heads: int, k_col: int, v_col: int,
+                        out: Optional[torch.Tensor] = None, precision: str = "bf16") -> torch.Tensor:
+    """Decode cross-attention: q (rows, heads*64) against the memory tokens of its image, K/V at columns [k_col, +heads*64)
+    / [v_col, ...) of kv (rows/beam*Tk, kv_ld) -> (rows, heads*64)."""
+    q, kv = _dev32(q), _dev32(kv)
+    rows = q.shape[0]
+    if rows % beam or kv.shape[0] % (rows // beam) or q.shape[1] != heads * 64:
+        raise ValueError("q must be (rows, heads*64), rows a multiple of beam, kv (rows/beam*Tk, kv_ld)")
+    tk = kv.shape[0] // (rows // beam)
+    out = _out32(out, (rows, heads * 64), q.device)
+    _lib.check(_lib.load().fpnmt_op_dec_cross_attention(q.device.index or 0, _lib.PREC_IDS[precision], q.data_ptr(), kv.data_ptr(),
+                                                        kv.shape[1], k_col, v_col, rows, beam, tk, heads, out.data_ptr(),
+                                                        _stream_ptr(q.device)))
+    return out
+
+
+def xattn(ckv: torch.Tensor, wq: np.ndarray, bq: np.ndarray, wo: np.ndarray, bo: np.ndarray, gamma: np.ndarray,
+          beta: np.ndarray, out1: torch.Tensor, beam: int, layer: int, b0: int = 0, images: Optional[int] = None,
+          out2: Optional[torch.Tensor] = None, fold_outputs: bool = False, precision: str = "bf16"):
+    """Fused decoder cross-attention block of `layer` on images [b0, b0 + images) of the batch: ckv (Btot*n_mem, L*1024)
+    memory K/V of all layers; wq / wo (L, 512, 512) Dense kernels as stored; bq (L, 512); bo, gamma, beta (512,) of the
+    layer; out1 (Btot*beam, 512).  Returns out2 (Btot*beam, 512), and with fold_outputs also the fold's (Mt, Nt, sbias)."""
+    ckv, out1 = _dev32(ckv), _dev32(out1)
+    wq, bq, wo = _host32(wq), _host32(bq), _host32(wo)
+    L = wq.shape[0]
+    Btot = out1.shape[0] // beam
+    if out1.shape != (Btot * beam, 512) or ckv.shape[1] != L * 1024 or ckv.shape[0] % Btot or wq.shape != (L, 512, 512) or \
+            wo.shape != (L, 512, 512) or bq.shape != (L, 512):
+        raise ValueError("ckv (Btot*n_mem, L*1024), wq / wo (L, 512, 512), bq (L, 512), out1 (Btot*beam, 512)")
+    n_mem = ckv.shape[0] // Btot
+    images = Btot - b0 if images is None else images
+    out2 = _out32(out2, (Btot * beam, 512), out1.device)
+    dev = out1.device
+    mt = torch.full((L * Btot * 128, 512), float("nan"), device=dev) if fold_outputs else None
+    nt = torch.full((L * Btot * 512, 128), float("nan"), device=dev) if fold_outputs else None
+    sb = torch.full((L * Btot * 128,), float("nan"), device=dev) if fold_outputs else None
+    bo, gamma, beta = _host32(bo), _host32(gamma), _host32(beta)
+    ptr = lambda t: None if t is None else t.data_ptr()
+    _lib.check(_lib.load().fpnmt_op_xattn(dev.index or 0, _lib.PREC_IDS[precision], ckv.data_ptr(), _hptr(wq), _hptr(bq),
+                                          _hptr(wo), _hptr(bo), _hptr(gamma), _hptr(beta), Btot, n_mem, L, layer, b0, images,
+                                          beam, out1.data_ptr(), out2.data_ptr(), ptr(mt), ptr(nt), ptr(sb), _stream_ptr(dev)))
+    return (out2, mt, nt, sb) if fold_outputs else out2
+
+
+def kv_reorder(src: torch.Tensor, dst: torch.Tensor, parent, beam: int, t: int, precision: str = "bf16") -> torch.Tensor:
+    """Physical KV-cache reorder after step t-1: src and dst (ncaches, rows, T, D); dst[c, r, :t] = src[c, (r // beam) * beam
+    + parent[t-1][r], :t] in place; parent (T, rows) beam indices."""
+    src = _dev32(src)
+    nc, rows, T, D = src.shape
+    _inout32(dst, src.shape, "dst")
+    par = _host_i32(parent)
+    if par.shape != (T, rows):
+        raise ValueError("parent must be (T, rows)")
+    _lib.check(_lib.load().fpnmt_op_kv_reorder(src.device.index or 0, _lib.PREC_IDS[precision], src.data_ptr(), dst.data_ptr(), nc,
+                                               _hptr(par), rows, beam, T, D, t, _stream_ptr(src.device)))
+    return dst
+
+
+def embed_pos(tokens, emb: np.ndarray, pos: np.ndarray, t: int, out: Optional[torch.Tensor] = None, precision: str = "bf16",
+              device: int = 0) -> torch.Tensor:
+    """Decoder input of step t: emb[tokens[r]] + pos[t] -> (rows, C); emb (V, C), pos (T, C)."""
+    tok = _host_i32(tokens).reshape(-1)
+    emb, pos = _host32(emb), _host32(pos)
+    (V, Cc), T = emb.shape, pos.shape[0]
+    if pos.shape[1] != Cc:
+        raise ValueError("emb and pos must have the same width")
+    out = _out32(out, (tok.size, Cc), torch.device("cuda", device))
+    _lib.check(_lib.load().fpnmt_op_embed_pos(device, _lib.PREC_IDS[precision], _hptr(tok), tok.size, _hptr(emb), V, _hptr(pos), T,
+                                              Cc, t, out.data_ptr(), _stream_ptr(out.device)))
+    return out
+
+
+def layernorm_rows(x: torch.Tensor, gamma: np.ndarray, beta: np.ndarray, eps: float = 1e-6, out: Optional[torch.Tensor] = None,
+                   precision: str = "bf16") -> torch.Tensor:
+    """LayerNorm of fp32 rows x (rows, 512) into a bf16 / bf16x3 activation, read back as (rows, 512)."""
+    x = _dev32(x)
+    if x.dim() != 2 or x.shape[1] != 512:
+        raise ValueError("x must be (rows, 512)")
+    out = _out32(out, x.shape, x.device)
+    g, b = _host32(gamma), _host32(beta)
+    _lib.check(_lib.load().fpnmt_op_layernorm_rows(x.device.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), x.shape[0],
+                                                   _hptr(g), _hptr(b), eps, out.data_ptr(), _stream_ptr(x.device)))
+    return out
+
+
 def preprocess(images_u8: torch.Tensor, size: int = cfg.IMAGE_INPUT_SIZE) -> torch.Tensor:
     """GPU `load_image` after the JPEG decode (dataset.py:21-24): uint8 (N,H,W,3) -> float32 (N,size,size,3) in [-1,1]."""
     lib = _lib.load()

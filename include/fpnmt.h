@@ -283,6 +283,51 @@ FPNMT_API int fpnmt_op_enc_attention(int device, int precision, const float* q, 
                                      int nviews, int kv_ld, int k_col, int v_col, int B, int Tq, int heads, int force_simt,
                                      float* out, void* stream);
 
+/* Decoder kernels one at a time, with the conventions of the encoder operators above (DEVICE float32 activations uploaded
+ * into bf16 or bf16x3 activations; every tensor the kernel writes is uploaded first and read back whole; integer tables
+ * are HOST int32 and checked on the host, an entry out of range is FPNMT_ERR_INVALID).  Head dim 64, d = heads * 64. */
+
+/* Decode self-attention of step t (transformer.py:131-153 with the KV cache of pipeline.py): for row r and head h,
+ * out[r, h*64 ..] = softmax_j(q . k_j / 8) v_j over the cached positions j < t, K/V read from cache row anc[t&1][r][j] * T + j,
+ * and the new position t with k, v = qkv[r, d + h*64 ..], qkv[r, 2d + h*64 ..]; those are appended to the cache at row
+ * r * T + t.  qkv [rows, 3d]; kc, vc [rows*T, d] (read and written); kc2 / vc2 NULL (ancestry mode) or the second buffer
+ * pair of the physical mode, which odd steps read and append to; anc HOST [2][rows][T] (entries in [0, rows)); rep HOST
+ * [2][rows] (representative row of each row's token-history class per step parity, entries in [0, rows)) or NULL; beam =
+ * rows per image (1..32); out [rows, d].  kernel 0: the engine's choice (bf16x3 the split CUDA-core kernel, bf16 the
+ * mma.sync kernel, which reads rep when beam <= 8 divides rows), 1: the CUDA-core kernel, 2: the mma.sync kernel (bf16 only). */
+FPNMT_API int fpnmt_op_dec_self_attention(int device, int precision, const float* qkv, float* kc, float* vc, float* kc2,
+                                          float* vc2, const int* anc, const int* rep, int rows, int T, int t, int heads, int beam,
+                                          int kernel, float* out, void* stream);
+/* Decode cross-attention over the memory tokens of the row's image (the CUDA-core kernel, split in bf16x3):
+ * out[r, h*64 ..] = softmax_j(q[r, h*64 ..] . k_j / 8) v_j, k_j = kv[(r/beam)*Tk + j, k_col + h*64 ..], v_j likewise at
+ * v_col.  q and out [rows, d]; kv [rows/beam*Tk, kv_ld]. */
+FPNMT_API int fpnmt_op_dec_cross_attention(int device, int precision, const float* q, const float* kv, int kv_ld, int k_col,
+                                           int v_col, int rows, int beam, int Tk, int heads, float* out, void* stream);
+/* The fused decoder cross-attention block (bf16 only, d_model 512, 8 heads) of `layer` on images [b0, b0 + B) of a batch
+ * of Btot: out2 = LayerNorm(softmax_j((out1 . wq + bq)_h K_h^T / 8) V_h . wo + bo + out1) over rows r of those images,
+ * K and V of layer l at columns l*1024 and l*1024 + 512 of ckv [Btot*n_mem, L*1024] (n_mem <= 16, beam <= 16).  First the
+ * fold kernels build the per-image operands of all Btot images and L layers, then one block kernel runs on the slice.
+ * wq, wo HOST [L][512][512] as stored (Dense kernels, in x out); bq HOST [L][512]; bo, gamma, beta HOST [512] of `layer`;
+ * out1 [Btot*beam, 512]; out2 [Btot*beam, 512] (rows outside the slice come back unchanged).  Optional outputs of the
+ * fold: Mt [L*Btot*128, 512], Nt [L*Btot*512, 128], sbias [L*Btot*128] (see csrc/xattn.cuh). */
+FPNMT_API int fpnmt_op_xattn(int device, int precision, const float* ckv, const float* wq, const float* bq, const float* wo,
+                             const float* bo, const float* gamma, const float* beta, int Btot, int n_mem, int L, int layer,
+                             int b0, int B, int beam, const float* out1, float* out2, float* Mt, float* Nt, float* sbias,
+                             void* stream);
+/* Physical KV-cache reorder after decode step tt = t - 1 (pipeline.py:134-137): for each cache c and row r,
+ * dst[c][r*T + j] = src[c][((r/beam)*beam + parent[tt][r])*T + j] for j <= tt; t = 0 copies nothing.  src and dst
+ * [ncaches][rows*T][D] (dst read and written); parent HOST [T][rows], entries in [0, beam). */
+FPNMT_API int fpnmt_op_kv_reorder(int device, int precision, const float* src, float* dst, int ncaches, const int* parent,
+                                  int rows, int beam, int T, int D, int t, void* stream);
+/* Decoder input: out[r] = emb[tokens[r]] + pos[t].  tokens HOST [rows] in [0, V); emb HOST [V][C]; pos HOST [T][C]; t in
+ * [0, T); out [rows, C]. */
+FPNMT_API int fpnmt_op_embed_pos(int device, int precision, const int* tokens, int rows, const float* emb, int V,
+                                 const float* pos, int T, int C, int t, float* out, void* stream);
+/* LayerNormalization(epsilon=eps) of fp32 rows (d_model 512), the unfused decoder's LayerNorm: x [rows, 512] read as
+ * float32; gamma / beta HOST [512]; out [rows, 512]. */
+FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x, int rows, const float* gamma,
+                                      const float* beta, float eps, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

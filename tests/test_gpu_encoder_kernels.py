@@ -16,7 +16,7 @@ of its output, so the bounds are:
   * attention: rel-L2 <= 8e-3 per (view, head) block on the tensor-core path (P is rounded to bf16 before P V), the
     element-wise bound with scale sum_j p_j |v_j| on the fp32 CUDA-core path.
 Outputs must be finite, and every column and pixel the kernel must not write (filled with -3.5 before the call) unchanged.
-FPNMT_KERNEL_ERRORS=<path> writes the worst error of each operator, as a fraction of its bound, to that JSON file.
+FPNMT_KERNEL_ERRORS=<path> merges the worst error of each operator, as a fraction of its bound, into that JSON file.
 
 Measured on one B200 (1000 W power limit), worst error as a fraction of the bound, bf16 / bf16x3:
   max pool, subsample 0 mismatches / 0;  avg pool 0.50 ulp / 0.24;  depthwise 0.99 / 0.23;  scale_shift_relu 1.00 / 0.25;
@@ -25,50 +25,18 @@ Measured on one B200 (1000 W power limit), worst error as a fraction of the boun
 In bf16 the output rounding alone reaches 2^-8 |y| at the bottom of a binade, so ratios near 1 there are that rounding;
 in bf16x3 the hi + lo storage of the output (~2^-17 relative) is a quarter of rtol.  The file runs in about 10 s.
 """
-import json
-import os
-
 import numpy as np
 import pytest
 import torch
 
 import fpnmt_oracle as O
+from kernel_check import RTOL, check_elementwise, error_report, gen, q_act  # noqa: F401 (error_report: autouse fixture)
+from kernel_check import record as _record
 
 pytestmark = pytest.mark.gpu
 
 PRECS = ["bf16", "bf16x3"]
-RTOL = {"bf16": 2.0 ** -8, "bf16x3": 2.0 ** -15}
 SENTINEL = -3.5                  # bf16-exact: any write to a column outside the op's view changes it
-_WORST = {}
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _error_report():
-    yield
-    path = os.environ.get("FPNMT_KERNEL_ERRORS")
-    if path and _WORST:
-        with open(path, "w") as f:
-            json.dump(_WORST, f, indent=1, sort_keys=True)
-
-
-def _record(op, value, bound):
-    cur = _WORST.get(op)
-    if cur is None or value / bound > cur["worst"] / cur["bound"]:
-        _WORST[op] = {"worst": float(value), "bound": float(bound)}
-
-
-def gen(seed):
-    return torch.Generator().manual_seed(seed)
-
-
-def q_act(x, prec):
-    """The values a kernel reads from an activation stored from fp32 x: bf16(x), or hi + lo with hi = bf16(x) and
-    lo = bf16(x - hi) (st_act), summed in fp32 as ld_act does."""
-    x = x.float()
-    hi = x.to(torch.bfloat16).float()
-    if prec == "bf16":
-        return hi
-    return hi + (x - hi).to(torch.bfloat16).float()
 
 
 def view_buffer(shape, C, ld, fill, g):
