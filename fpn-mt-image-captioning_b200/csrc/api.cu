@@ -143,6 +143,15 @@ FPNMT_API int fpnmt_decode_hidden(fpnmt_handle* h, const float* memory, const in
   }
   return h->eng->decode_logits(memory, tokens, t, nullptr, (cudaStream_t)stream, hidden_out);
 }
+FPNMT_API int fpnmt_decode_attention(fpnmt_handle* h, const float* memory, const int32_t* tokens, int t, float* self_out,
+                                     float* cross_out, void* stream) {
+  CHECK_H(h);
+  if (!self_out && !cross_out) {
+    set_last_error("decode_attention: self_out and cross_out are both NULL");
+    return FPNMT_ERR_INVALID;
+  }
+  return h->eng->decode_logits(memory, tokens, t, nullptr, (cudaStream_t)stream, nullptr, self_out, cross_out);
+}
 FPNMT_API int fpnmt_beam_step(fpnmt_handle* h, const float* logits, const float* scores_in, int32_t* parent, int32_t* token,
                     float* scores_out, void* stream) {
   CHECK_H(h);

@@ -3,9 +3,13 @@
 //                         single pass with online softmax; one block per (image, head), 4 queries per warp.
 //   dec_self_attention  : one new query per (row, head) against the KV cache through the beam-ancestry table.
 //   dec_cross_attention : one query per (row, head) against the 16 memory tokens of the row's image.
+//   dec_attention_probs : the normalised probabilities of both for the beam-0 rows (inspection, teacher forcing).
 #include <stdlib.h>
 
+#include <algorithm>
+
 #include "kernels.cuh"
+#include "xattn.cuh"
 
 namespace fpnmt {
 
@@ -863,6 +867,88 @@ int launch_dec_cross_attention(Act q, Act kv, int k_col, int v_col, int rows, in
   else
     FPNMT_CUDA_OK(launch_k(k_dec_cross_attention<false>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
                            q, kv, k_col, v_col, rows, beam, Tk, heads, out));
+  return 0;
+}
+
+// ---- attention probabilities for inspection (Engine::decode_logits with attention outputs) ------------------------------
+// Block (b, h, z): the beam-0 row b * N of image b; z = 0 the self-attention row t = *step of head h, z = 1 the cross-attention
+// row.  Scores are recomputed from the operands the layer's attention kernels read, one warp per key position (lanes split
+// the dot product), then normalised in fp32 over the block.  Runs after the layer's cross-attention block, when the new K of
+// position t is in the cache and q2 / out1 are final.
+__device__ __forceinline__ float dot_row(const float* x, const Act& a, size_t pix, int c0, int K, int lane) {
+  float acc = 0.f;
+  for (int k = lane; k < K; k += 32) acc = fmaf(x[k], ld_act(a, pix, c0 + k), acc);
+  return warp_sum(acc);
+}
+
+constexpr int DP_THREADS = 128;
+
+__global__ void __launch_bounds__(DP_THREADS) k_dec_attention_probs(DecProbArgs a) {
+  extern __shared__ float s_sc[];                     // [max(tlen, n_mem)] scores, then unnormalised probabilities
+  __shared__ float s_x[512];                          // the query (64) or, on the fused path, the out1 row (512)
+  __shared__ float s_red[DP_THREADS / 32];
+  pdl_launch();
+  pdl_wait();
+  const int b = blockIdx.x, h = blockIdx.y, cross = blockIdx.z;
+  float* out = cross ? a.cross_out : a.self_out;
+  if (!out) return;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = DP_THREADS / 32;
+  const int t = *a.step;
+  const size_t row = (size_t)b * a.N;
+  const bool folded = cross && a.Mt;
+  const int kd = folded ? a.q.C : DH;
+  const int n = cross ? a.n_mem : t + 1;
+  if (folded)
+    for (int k = threadIdx.x; k < kd; k += DP_THREADS) s_x[k] = ld_act(a.q, row, k);
+  else
+    for (int k = threadIdx.x; k < DH; k += DP_THREADS) s_x[k] = ld_act(cross ? a.q : a.qkv, row, h * DH + k) * 0.125f;   // 1/sqrt(64)
+  __syncthreads();
+  for (int j = warp; j < n; j += nw) {
+    float s;
+    if (!cross) {
+      const int* anc = a.anc + (size_t)(t & 1) * a.anc_stride + row * a.T;
+      s = dot_row(s_x, a.kc, (size_t)anc[j] * a.T + j, h * DH, DH, lane);
+    } else if (folded) {
+      const Act m{const_cast<bf16*>(a.Mt), kd, kd, 0};
+      const size_t pair = (size_t)b * XA_PAIRS + h * 16 + j;    // (head, token) pairs padded to 16 tokens per head
+      s = dot_row(s_x, m, pair, 0, kd, lane) + a.sbias[pair];
+    } else {
+      s = dot_row(s_x, a.kv, (size_t)b * a.n_mem + j, a.k_col + h * DH, DH, lane);
+    }
+    if (lane == 0) s_sc[j] = s;
+  }
+  __syncthreads();
+  float m = -INFINITY;
+  for (int j = threadIdx.x; j < n; j += DP_THREADS) m = fmaxf(m, s_sc[j]);
+  m = warp_max(m);
+  if (lane == 0) s_red[warp] = m;
+  __syncthreads();
+  m = s_red[0];
+  for (int w = 1; w < nw; ++w) m = fmaxf(m, s_red[w]);
+  __syncthreads();
+  float l = 0.f;
+  for (int j = threadIdx.x; j < n; j += DP_THREADS) {
+    const float e = expf(s_sc[j] - m);
+    s_sc[j] = e;
+    l += e;
+  }
+  l = warp_sum(l);
+  if (lane == 0) s_red[warp] = l;
+  __syncthreads();
+  l = s_red[0];
+  for (int w = 1; w < nw; ++w) l += s_red[w];
+  const int width = cross ? a.n_mem : a.tlen;   // self rows are causal: exact zeros after position t
+  float* dst = out + (((size_t)b * a.heads + h) * a.tlen + t) * width;
+  for (int j = threadIdx.x; j < width; j += DP_THREADS) dst[j] = j < n ? s_sc[j] / l : 0.f;
+}
+
+int launch_dec_attention_probs(const DecProbArgs& a, int B, cudaStream_t s) {
+  if (a.Mt && (a.q.C > 512 || a.n_mem > 16 || a.q.lo)) {
+    set_last_error("dec_attention_probs: unsupported shape");
+    return 1;
+  }
+  const size_t smem = (size_t)std::max(a.tlen, a.n_mem) * sizeof(float);
+  FPNMT_CUDA_OK(launch_k_small(k_dec_attention_probs, dim3(B, a.heads, 2), dim3(DP_THREADS), smem, s, a));
   return 0;
 }
 

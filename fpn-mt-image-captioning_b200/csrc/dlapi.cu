@@ -217,6 +217,29 @@ FPNMT_API int fpnmt_decode_hidden_dl(fpnmt_handle* h, const DLTensor* memory, co
   return fpnmt_decode_hidden(h, (const float*)pm, (const int32_t*)pt, t, (float*)po, stream);
 }
 
+FPNMT_API int fpnmt_decode_attention_dl(fpnmt_handle* h, const DLTensor* memory, const DLTensor* tokens, DLTensor* self_out,
+                                        DLTensor* cross_out, void* stream) {
+  CHECK_HDL(h);
+  void *pm, *pt, *ps = nullptr, *pc = nullptr;
+  int t = 0;
+  int rc = forced_args(h, "decode_attention_dl", memory, tokens, &pm, &pt, &t);
+  if (rc) return rc;
+  const fpnmt_config& c = h->eng->config();
+  const int64_t nm = (int64_t)(c.image_size / 128) * (c.image_size / 128);
+  if (!self_out && !cross_out) return dl_fail("decode_attention_dl: self_out and cross_out are both NULL");
+  if (self_out) {
+    rc = dl_check("decode_attention_dl: self_out", self_out, kDLFloat, h->eng->device(), false, true,
+                  {c.num_layers, c.batch, c.num_heads, t, t}, &ps, nullptr);
+    if (rc) return rc;
+  }
+  if (cross_out) {
+    rc = dl_check("decode_attention_dl: cross_out", cross_out, kDLFloat, h->eng->device(), false, true,
+                  {c.num_layers, c.batch, c.num_heads, t, nm}, &pc, nullptr);
+    if (rc) return rc;
+  }
+  return fpnmt_decode_attention(h, (const float*)pm, (const int32_t*)pt, t, (float*)ps, (float*)pc, stream);
+}
+
 FPNMT_API int fpnmt_generate_dl(fpnmt_handle* h, const DLTensor* images, DLTensor* out_ids, DLTensor* out_len, int early_stop,
                                 DLTensor* step_scores, void* stream) {
   CHECK_HDL(h);

@@ -1093,6 +1093,8 @@ int Engine::build_decoder() {
       }
       const BeamEmbed em{d_emb, d_pos, x.a, D};
       if (em_out) *em_out = em;
+      // attention-probability launches of step_attn_prog_ (whole batch only): position in step_prog they follow, the op
+      std::vector<std::pair<size_t, Op>> prob_ops;
       for (int l = 0; l < L; ++l) {
         LayerW& w = lw[l];
         const std::string ln = "dec" + std::to_string(l);
@@ -1134,6 +1136,7 @@ int Engine::build_decoder() {
           step_prog.push_back(std::move(o));
         }
         RC(dense_res_ln(ln + "_o1+res", ln + "_ln1", att, w.go1, x, w.lnp[0], w.lnp[1], out1));
+        size_t prob_at = 0;   // the probabilities read the new K of position t, q2 / out1: after the cross-attention block
         if (xattn) {
           XattnOp xo;
           RC(make_xattn_op(&xo, xMt, xNt, L, B, b0, Bg, N, l, xSb, w.go2.bias, w.lnp[2], w.lnp[3], out1.a, out2.a));
@@ -1145,6 +1148,7 @@ int Engine::build_decoder() {
           o.bytes = (double)Bg * 2 * 128 * 512 * 2 + (double)Rg * D * 2 * 2;  // folded per-image operands + activations
           o.run = [xo](cudaStream_t s) { return xattn_launch(xo, s); };
           step_prog.push_back(std::move(o));
+          prob_at = step_prog.size();
         } else {
           RC(dense(ln + "_q2", out1, w.gq2, ACT_NONE, q2));
           {
@@ -1154,8 +1158,39 @@ int Engine::build_decoder() {
             const int kcx = l * 2 * D, vcx = l * 2 * D + D, tk = n_base_;
             step_prog.push_back(ew_op(ln + "_cross_attn" + sfx, [=](cudaStream_t s) { return launch_dec_cross_attention(qa, ka, kcx, vcx, Rg, N, tk, H, oa, s); },
                                       (double)Bg * tk * 2 * D * 2, "attention"));
+            prob_at = step_prog.size();
           }
           RC(dense_res_ln(ln + "_o2+res", ln + "_ln2", att2, w.go2, out1, w.lnp[2], w.lnp[3], out2));
+        }
+        if (Bg == B) {
+          DecProbArgs pa{};
+          pa.qkv = qkv.a;
+          pa.kc = kc.a;
+          pa.anc = anc;
+          pa.anc_stride = (size_t)R * T;
+          pa.T = T;
+          pa.q = xattn ? out1.a : q2.a;
+          pa.kv = ckv.a;
+          pa.k_col = l * 2 * D;
+          pa.Mt = xattn ? xMt + (size_t)l * B * 128 * 512 : nullptr;
+          pa.sbias = xattn ? xSb + (size_t)l * B * 128 : nullptr;
+          pa.n_mem = n_base_;
+          pa.step = bs.step;
+          pa.N = N;
+          pa.heads = H;
+          const int nm = n_base_;
+          // output pointers and row count are those of the decode_logits call that runs the program
+          Op o = ew_op(ln + "_attn_probs",
+                       [=](cudaStream_t s) {
+                         DecProbArgs q = pa;
+                         const size_t tl = (size_t)attn_tlen_;
+                         q.tlen = attn_tlen_;
+                         q.self_out = attn_self_ ? attn_self_ + (size_t)l * B * H * tl * tl : nullptr;
+                         q.cross_out = attn_cross_ ? attn_cross_ + (size_t)l * B * H * tl * nm : nullptr;
+                         return launch_dec_attention_probs(q, B, s);
+                       },
+                       (double)B * H * (T / 2 + nm) * D * 2, "attention");
+          prob_ops.emplace_back(prob_at, std::move(o));
         }
         RC(dense(ln + "_ffn1", out2, w.g1, ACT_LEAKY, hdn));
         RC(dense_res_ln(ln + "_ffn2+res", ln + "_ln3", hdn, w.g2, out2, w.lnp[4], w.lnp[5], out3));
@@ -1172,6 +1207,12 @@ int Engine::build_decoder() {
       if (Bg == B) {   // teacher forcing: embed the forced token, then the shared layer stack (whole batch only)
         step_forced_prog_ = embed_prog;
         step_forced_prog_.insert(step_forced_prog_.end(), step_prog.begin(), step_prog.end());
+        step_attn_prog_ = embed_prog;   // the same launches with the probability kernels after the operands they read
+        size_t k = 0;
+        for (size_t i = 0; i < step_prog.size(); ++i) {
+          step_attn_prog_.push_back(step_prog[i]);
+          for (; k < prob_ops.size() && prob_ops[k].first == i + 1; ++k) step_attn_prog_.push_back(prob_ops[k].second);
+        }
       }
       // Logits-free decode tail (bf16 mode, log scores, beam <= 8, wide Dense kernels): the beam-search chain replaces the
       // vocabulary projection's [rows][V] fp32 output (20.5 MB written and read back per step at C2) by per-tile softmax
@@ -1656,10 +1697,14 @@ __global__ void k_anc_identity(int* anc, int rows, int T) {
     anc[j] = (int)((j / T) % rows);
 }
 
-int Engine::decode_logits(const float* memory, const int32_t* tokens, int t, float* logits_out, cudaStream_t s, float* hidden_out) {
+int Engine::decode_logits(const float* memory, const int32_t* tokens, int t, float* logits_out, cudaStream_t s, float* hidden_out,
+                          float* self_out, float* cross_out) {
   if (!finalized_) return fail(FPNMT_ERR_STATE, "decode_logits before finalize_weights");
   if (t < 1 || t > cfg_.max_len) return fail(FPNMT_ERR_INVALID, "decode_logits: t out of range");
-  if (!tokens || (!logits_out && !hidden_out)) return fail(FPNMT_ERR_INVALID, "decode_logits: NULL tokens / output");
+  if (!tokens || (!logits_out && !hidden_out && !self_out && !cross_out)) return fail(FPNMT_ERR_INVALID, "decode_logits: NULL tokens / output");
+  const bool attn = self_out || cross_out;
+  if (attn && use_dstep_)
+    return fail(FPNMT_ERR_STATE, "decode_attention: the fused decoder does not keep attention operands (use decode_path = chain)");
   const Tensor* last = nullptr;
   if (hidden_out) {
     auto it = taps_.find("dec" + std::to_string(cfg_.num_layers - 1) + "_out3");
@@ -1675,6 +1720,9 @@ int Engine::decode_logits(const float* memory, const int32_t* tokens, int t, flo
   FPNMT_CUDA_OK(cudaGetLastError());
   forced_mode_ = true;
   struct Reset { bool& f; ~Reset() { f = false; } } reset{forced_mode_};
+  attn_self_ = self_out;
+  attn_cross_ = cross_out;
+  attn_tlen_ = t;
   for (int i = 0; i < t; ++i) {
     if (use_dstep_) {   // fused decoder, teacher-forcing mode: one step, fp32 logits of every row written out
       DstepParams q = dsp_;
@@ -1684,7 +1732,7 @@ int Engine::decode_logits(const float* memory, const int32_t* tokens, int t, flo
       RC(dstep_launch(q, s));
       launches += 1;
     } else {
-      RC(run_program(step_forced_prog_, s));
+      RC(run_program(attn ? step_attn_prog_ : step_forced_prog_, s));
     }
     if (last) {
       k_forced_hidden<<<cfg_.batch, 128, 0, s>>>(last->a, bs_.step, cfg_.beam, t, hidden_out);

@@ -60,7 +60,10 @@ class Engine {
   int encode(const float* images, int on_host, float* memory_out, cudaStream_t s, bool cnn_only = false);
   int features(const float* images, int on_host, float* const out5[5], cudaStream_t s);
   int get_tap(const char* name, float* out, size_t cap, size_t* count, cudaStream_t s);
-  int decode_logits(const float* memory, const int32_t* tokens, int t, float* logits_out, cudaStream_t s, float* hidden_out = nullptr);
+  // self_out / cross_out (either may be nullptr): attention probabilities of the beam-0 rows, [L][B][heads][t][t] and
+  // [L][B][heads][t][n_mem] (step_attn_prog_; not with the fused decoder)
+  int decode_logits(const float* memory, const int32_t* tokens, int t, float* logits_out, cudaStream_t s, float* hidden_out = nullptr,
+                    float* self_out = nullptr, float* cross_out = nullptr);
   int beam_step(const float* logits, const float* scores_in, int32_t* parent, int32_t* token, float* scores_out,
                 cudaStream_t s);
   int decode(int32_t* out_ids, int32_t* out_len, int on_host, int early_stop, float* step_scores, cudaStream_t s);
@@ -101,6 +104,7 @@ class Engine {
 
   // programs
   Program cnn_prog_, enc_prog_, dec_init_prog_, embed_prog_, step_prog_, step_forced_prog_;
+  Program step_attn_prog_;                // step_forced_prog_ + the attention-probability launches (decode_logits with outputs)
   BeamEmbed beam_embed_{};
   cudaGraphExec_t cnn_graph_ = nullptr, enc_graph_ = nullptr, step_graph_ = nullptr, loop_graph_ = nullptr;
   std::vector<DecGroup> groups_;          // decoder groups (empty: the whole batch is one chain)
@@ -124,6 +128,9 @@ class Engine {
   bool use_dstep_ = false;                // group-stationary fused decoder (dstep.cuh) instead of the per-operator chain
   DstepParams dsp_{};
   bool forced_mode_ = false;              // decode_logits is running (physical cache mode: no buffer alternation)
+  float* attn_self_ = nullptr;            // attention outputs and row count of the running decode_logits (step_attn_prog_)
+  float* attn_cross_ = nullptr;
+  int attn_tlen_ = 0;
   int prof_t_ = 0;                        // step index used by the single-step op of the fused decoder in profile()
   struct F32Tap { const float* p; size_t count; };
   std::map<std::string, F32Tap> taps_f32_;

@@ -70,6 +70,28 @@ int launch_dec_self_attention(Act qkv, Act kcache, Act vcache, Act kcache2, Act 
 // Decoder cross-attention over the 16 memory tokens of the row's image.
 int launch_dec_cross_attention(Act q, Act kv, int k_col, int v_col, int rows, int beam, int Tk, int heads, Act out,
                                cudaStream_t s);
+// Normalised attention probabilities of the beam-0 row b * N of every image at step t = *step, for one decoder layer:
+// self_out[b][h][t][j] = softmax_j(q_h . k_j / 8) for j <= t (K of position j at cache row anc[t & 1][b * N][j] * T + j) and
+// exactly 0 for t < j < tlen; cross_out[b][h][t][j] for the n_mem memory tokens, from q2 against the K columns k_col of kv or,
+// when Mt is set, from the fused cross-attention block's folded operands (scores = Mt . out1 + sbias, padding never read).
+// Either output may be nullptr.  fp32 arithmetic on bf16 / bf16x3 operands.
+struct DecProbArgs {
+  Act qkv, kc;                  // layer's QKV projection [rows][3d] and K cache [rows * T][d]
+  const int* anc;               // ancestry table of the parity 0, the second parity anc_stride ints further
+  size_t anc_stride;
+  int T;
+  Act q;                        // q2 [rows][d] or, with Mt, out1 [rows][512]
+  Act kv;                       // cross K/V of the memory [B * n_mem][..] (unused with Mt)
+  int k_col;
+  const bf16* Mt;               // [B][128 (h,j)][512] folded operand of this layer, or nullptr
+  const float* sbias;           // [B][128] score bias of this layer (with Mt)
+  int n_mem;
+  const int* step;
+  int N, heads, tlen;
+  float* self_out;              // [B][heads][tlen][tlen] of this layer
+  float* cross_out;             // [B][heads][tlen][n_mem] of this layer
+};
+int launch_dec_attention_probs(const DecProbArgs& a, int B, cudaStream_t s);
 
 // ---- beam.cu ------------------------------------------------------------------------------------
 struct BeamState {

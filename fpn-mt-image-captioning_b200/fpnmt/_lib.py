@@ -98,11 +98,13 @@ class DLTensor(C.Structure):
 _dlp = C.POINTER(DLTensor)
 SIGNATURES.update({
     "fpnmt_decode_hidden": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
+    "fpnmt_decode_attention": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "fpnmt_set_weight_dl": (_i, [_vp, C.c_char_p, _dlp]),
     "fpnmt_encode_dl": (_i, [_vp, _dlp, _dlp, _vp]),
     "fpnmt_features_dl": (_i, [_vp, _dlp, C.POINTER(_dlp), _vp]),
     "fpnmt_decode_logits_dl": (_i, [_vp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_decode_hidden_dl": (_i, [_vp, _dlp, _dlp, _dlp, _vp]),
+    "fpnmt_decode_attention_dl": (_i, [_vp, _dlp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_generate_dl": (_i, [_vp, _dlp, _dlp, _dlp, _i, _dlp, _vp]),
     "fpnmt_comm_unique_id": (_i, [_vp]),
     "fpnmt_comm_create": (_i, [_i, _i, _vp, _i, C.POINTER(_vp)]),

@@ -56,7 +56,8 @@ class Engine:
             vocab = int(weights["transformer/final_layer/kernel"].shape[1])
         self.device = torch.device("cuda", device)
         self.backbone, self.batch, self.beam, self.vocab, self.max_len = backbone, batch, beam, vocab, max_len
-        self.image_size, self.d_model, self.num_layers = image_size, d_model, num_layers
+        self.image_size, self.d_model, self.num_layers, self.num_heads = image_size, d_model, num_layers, num_heads
+        self.start_id = start_id
         self.precision = precision
         c = _lib.FpnmtConfig()
         c.backbone = _lib.BACKBONE_IDS[backbone]
@@ -161,6 +162,40 @@ class Engine:
         out = torch.empty((self.batch, t, self.d_model), dtype=torch.float32, device=self.device)
         _lib.check(self.lib.fpnmt_decode_hidden(self._h, mem_ptr, tok.data_ptr(), t, out.data_ptr(), _stream_ptr(self.device)))
         return out
+
+    def decode_attention(self, memory, tokens, self_attention: bool = True, cross_attention: bool = True
+                         ) -> Dict[str, torch.Tensor]:
+        """The attention-weights dict of Decoder.call (transformer.py:337-338) for teacher-forced tokens (B,t):
+        "decoder_layer{i}_block1" (B,heads,t,t) causal self-attention and "decoder_layer{i}_block2" (B,heads,t,n_memory)
+        cross-attention over the memory tokens, i counted from 1; float32 on the device.  memory None = the last encode."""
+        if not (self_attention or cross_attention):
+            raise ValueError("decode_attention: nothing requested")
+        tok = _as_cuda(tokens, torch.int32, self.device)
+        t = int(tok.shape[1])
+        mem_ptr = None
+        if memory is not None:
+            mem = _as_cuda(memory, torch.float32, self.device)
+            mem_ptr = mem.data_ptr()
+        L, H = self.num_layers, self.num_heads
+        so = torch.empty((L, self.batch, H, t, t), dtype=torch.float32, device=self.device) if self_attention else None
+        co = torch.empty((L, self.batch, H, t, self.n_memory), dtype=torch.float32, device=self.device) if cross_attention else None
+        _lib.check(self.lib.fpnmt_decode_attention(self._h, mem_ptr, tok.data_ptr(), t, so.data_ptr() if so is not None else None,
+                                                   co.data_ptr() if co is not None else None, _stream_ptr(self.device)))
+        out = {}
+        for l in range(L):
+            if so is not None:
+                out["decoder_layer%d_block1" % (l + 1)] = so[l]
+            if co is not None:
+                out["decoder_layer%d_block2" % (l + 1)] = co[l]
+        return out
+
+    def caption_attention(self, ids, lens) -> Dict[str, torch.Tensor]:
+        """Attention weights of captions returned by the last `generate` on this engine (ids (B,T), lens (B,)): one
+        teacher-forced pass over [<start>] + caption with the memory that generate left.  Row j of a caption is the attention
+        that predicted its token j (the last row predicted <end> when it fired); rows and columns at or beyond
+        n_b = min(len_b + 1, T) are zero.  What the reference's predict returns for beam row 0 (pipeline.py:82-154)."""
+        tok, n = caption_prefix(_as_cuda(ids, torch.int32, self.device), _as_cuda(lens, torch.int32, self.device), self.start_id)
+        return mask_caption_attention(self.decode_attention(None, tok), n)
 
     def beam_step(self, logits, scores) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """One decode-tail step (pipeline.py:115-141) on caller logits (B*N,V) and scores (B*N,)."""
@@ -302,6 +337,25 @@ class Engine:
     @property
     def launch_count(self) -> int:
         return int(self.lib.fpnmt_launch_count(self._h))
+
+
+def caption_prefix(ids: torch.Tensor, lens: torch.Tensor, start_id: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Decoder input of the pass that gives a caption its attention weights: tokens (B,T) = [<start>] + ids[:, :T-1], and
+    n_b = min(len_b + 1, T) valid positions (the tokens predicted, plus <end> when it fired before the last step)."""
+    T = ids.shape[1]
+    tok = torch.cat([torch.full_like(ids[:, :1], start_id), ids[:, :T - 1]], dim=1)
+    return tok, torch.clamp(lens.to(torch.int64) + 1, max=T)
+
+
+def mask_caption_attention(attn: Dict[str, torch.Tensor], n: torch.Tensor) -> Dict[str, torch.Tensor]:
+    """Zeroes (in place) the rows of every (B,heads,T,.) block at or beyond n_b, and the columns of the self-attention
+    blocks ("_block1") too."""
+    for k, v in attn.items():
+        ok = (torch.arange(v.shape[2], device=v.device)[None, :] < n.to(v.device)[:, None]).to(v.dtype)   # (B,T)
+        v.mul_(ok[:, None, :, None])
+        if k.endswith("_block1"):
+            v.mul_(ok[:, None, None, :])
+    return attn
 
 
 def conv2d(x: torch.Tensor, kernel_hwio: np.ndarray, bias: Optional[np.ndarray] = None, act: int = 0,

@@ -64,18 +64,31 @@ class Pipeline:
 
     # ----------------------------------------------------------------------------------------------
     def predict_batch(self, imgs, max_seq_len: Optional[int] = None, beam: Optional[int] = None,
-                      early_stop: bool = True) -> Tuple[np.ndarray, np.ndarray]:
-        """Batched `predict`: imgs (B,S,S,3) float32 in [-1,1] -> (ids (B,T) int32 zero padded, lengths (B,))."""
+                      early_stop: bool = True, return_attention: bool = False):
+        """Batched `predict`: imgs (B,S,S,3) float32 in [-1,1] -> (ids (B,T) int32 zero padded, lengths (B,)).
+        return_attention: also the captions' attention-weights dict (Engine.caption_attention) as numpy arrays
+        (B,heads,T,T) / (B,heads,T,n_memory), zero at and beyond position min(len + 1, T) -> (ids, lens, attn)."""
         imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
         eng = self.transformer.engine(int(imgs.shape[0]), beam or self.beam, max_seq_len or self.max_seq_len)
         ids, lens = eng.generate(imgs, early_stop=early_stop, to_host=True)
-        return ids.numpy(), lens.numpy()
+        if not return_attention:
+            return ids.numpy(), lens.numpy()
+        attn = {k: v.cpu().numpy() for k, v in eng.caption_attention(ids, lens).items()}
+        return ids.numpy(), lens.numpy(), attn
 
     def predict(self, img, max_seq_len, plot_layer=False):
-        """pipeline.py:82-154: img (H,W,3) -> (1-D int32 ids without <start>/<end>, attention_weights=None)."""
+        """pipeline.py:82-154: img (H,W,3) -> (1-D int32 ids without <start>/<end>, attention_weights).
+        attention_weights is None unless `plot_layer` is truthy; then it is the dict of the reference's last forward pass for
+        the returned caption, n = len + 1 positions when <end> fired and max_seq_len otherwise: "decoder_layer{i}_block1"
+        (1,heads,n,n), "decoder_layer{i}_block2" (1,heads,n,n_memory), numpy float32.  Nothing is plotted."""
         img = torch.as_tensor(img) if not isinstance(img, torch.Tensor) else img
-        ids, lens = self.predict_batch(img[None], max_seq_len)
-        return ids[0, :lens[0]], None
+        if not plot_layer:
+            ids, lens = self.predict_batch(img[None], max_seq_len)
+            return ids[0, :lens[0]], None
+        ids, lens, attn = self.predict_batch(img[None], max_seq_len, return_attention=True)
+        n = min(int(lens[0]) + 1, ids.shape[1])
+        attn = {k: np.ascontiguousarray(v[:, :, :n, :n] if k.endswith("_block1") else v[:, :, :n, :]) for k, v in attn.items()}
+        return ids[0, :lens[0]], attn
 
     def evaluate(self, generator: Iterable, max_seq_len, batch_size: int = 1, lanes: int = 1) -> List[dict]:
         """pipeline.py:156-175: [(img, imgId)] -> [{"image_id", "caption"}] (optionally batched; lanes >= 2 keeps that many

@@ -6,8 +6,8 @@ Same constructor signatures and call conventions as the reference's `Transformer
 
 Deviations from the reference, by design:
 * `training=True` raises (this build is inference-only).
-* attention-weight dicts (transformer.py:337-338) are only consumed by the never-called
-  `plot_attention_weights`; `None` is returned in their place.
+* attention-weight dicts (transformer.py:337-338) are computed on request: `return_attention=True` (keyword-only) runs one
+  more teacher-forced pass that also writes them; by default `None` is returned in their place.
 """
 from __future__ import annotations
 
@@ -89,9 +89,9 @@ class Encoder:
 class Decoder:
     """transformer.py:306-341.  `decoder(x, enc_output, training, look_ahead_mask, padding_mask)`.
 
-    Returns (hidden states (B,t,d_model) of the last decoder layer, None): computed position by position with the KV-cached
-    step program (the causal mask is implicit), read out through fpnmt_decode_hidden.  The attention-weights dict
-    (transformer.py:337-338, only consumed by the never-called plot_attention_weights) is not produced: SURVEY §8b1."""
+    Returns (hidden states (B,t,d_model) of the last decoder layer, attention weights): computed position by position with the
+    KV-cached step program (the causal mask is implicit), read out through fpnmt_decode_hidden.  The attention-weights dict
+    (transformer.py:337-338) is None unless `return_attention=True`, which adds a pass through fpnmt_decode_attention."""
 
     def __init__(self, num_layers, d_model, num_heads, dff, target_vocab_size, rate=0.1, max_position=0, max_seq_len=12,
                  _cache=None):
@@ -99,14 +99,15 @@ class Decoder:
         self.pos_encoding = raw_positional_encoding(max_seq_len + max_position, d_model)
         self._cache = _cache
 
-    def __call__(self, x, enc_output, training=False, look_ahead_mask=None, padding_mask=None):
+    def __call__(self, x, enc_output, training=False, look_ahead_mask=None, padding_mask=None, *, return_attention=False):
         if training:
             raise NotImplementedError("inference-only build: training=True is out of scope")
         if self._cache is None:
             raise RuntimeError("Decoder needs the engine of its Transformer (construct it through Transformer(...))")
         x = torch.as_tensor(x)
         eng = self._cache.get(int(x.shape[0]), 1, max(self.max_seq_len, int(x.shape[1])))
-        return eng.decode_hidden(enc_output, x), None
+        hidden = eng.decode_hidden(enc_output, x)
+        return hidden, (eng.decode_attention(enc_output, x) if return_attention else None)
 
     call = __call__
 
@@ -131,14 +132,15 @@ class Transformer:
                                _cache=self._cache)
         self.final_layer = ("transformer/final_layer/kernel", "transformer/final_layer/bias")
 
-    def __call__(self, inp, tar, training, look_ahead_mask):
+    def __call__(self, inp, tar, training, look_ahead_mask, *, return_attention=False):
         """Inference branch (transformer.py:362-374): `inp` is the pre-computed encoder output (B,16,d);
-        `tar` (B,t) token ids.  Returns (logits (B,t,V), None)."""
+        `tar` (B,t) token ids.  Returns (logits (B,t,V), attention-weights dict or None, see `Decoder`)."""
         if training:
             raise NotImplementedError("inference-only build: training=True is out of scope")
         tar = torch.as_tensor(tar)
         eng = self._cache.get(int(tar.shape[0]), 1, max(self.max_seq_len, int(tar.shape[1])))
-        return eng.decode_logits(inp, tar), None
+        logits = eng.decode_logits(inp, tar)
+        return logits, (eng.decode_attention(inp, tar) if return_attention else None)
 
     call = __call__
 

@@ -153,9 +153,18 @@ FPNMT_API int fpnmt_decode_logits(fpnmt_handle* h, const float* memory, const in
 
 /* Replaces: Decoder.call(x, enc_output, training=False, look_ahead_mask, padding_mask) (models/transformer.py:321-341): the
  * output of the last decoder layer (before final_layer) for teacher-forced tokens; arguments as fpnmt_decode_logits,
- * hidden_out DEVICE float32 [batch, t, d_model].  (The attention-weights dict is not returned: SURVEY §8b1.) */
+ * hidden_out DEVICE float32 [batch, t, d_model].  The attention-weights dict comes from fpnmt_decode_attention. */
 FPNMT_API int fpnmt_decode_hidden(fpnmt_handle* h, const float* memory, const int32_t* tokens, int t, float* hidden_out,
                                   void* stream);
+
+/* The attention-weights dict of Decoder.call (models/transformer.py:337-338) for teacher-forced tokens; memory / tokens /
+ * t as fpnmt_decode_logits (NULL memory = the last encode).  self_out DEVICE float32 [num_layers][batch][heads][t][t]:
+ * "decoder_layer{l+1}_block1", causal softmax(q k^T / 8) with exact zeros above the diagonal; cross_out DEVICE float32
+ * [num_layers][batch][heads][t][n_memory]: "decoder_layer{l+1}_block2", the softmax over the memory tokens (token j = P6
+ * cell (j / w6, j % w6)).  Either output may be NULL, not both.  The probabilities are computed by extra kernels in the
+ * teacher-forced step program; not available with decode_path = FUSED (FPNMT_ERR_STATE). */
+FPNMT_API int fpnmt_decode_attention(fpnmt_handle* h, const float* memory, const int32_t* tokens, int t, float* self_out,
+                                     float* cross_out, void* stream);
 
 /* Replaces: the body of the decode loop, utils/pipeline.py:115-141, on caller-provided logits (the decode-tail
  * kernels alone): logits DEVICE float32 [batch*beam, vocab], scores_in DEVICE float32 [batch*beam];

@@ -53,6 +53,11 @@ FPNMT_API int fpnmt_decode_logits_dl(fpnmt_handle* h, const DLTensor* memory, co
  * hidden_out float32 [batch, t, d_model] on the GPU.  (Raw-pointer twin: fpnmt_decode_hidden in fpnmt.h.) */
 FPNMT_API int fpnmt_decode_hidden_dl(fpnmt_handle* h, const DLTensor* memory, const DLTensor* tokens, DLTensor* hidden_out,
                                      void* stream);
+/* The attention-weights dict of Decoder.call (models/transformer.py:337-338): memory / tokens as above; self_out float32
+ * [num_layers, batch, heads, t, t], cross_out float32 [num_layers, batch, heads, t, n_memory], on the GPU; either may be
+ * NULL, not both.  (Raw-pointer twin: fpnmt_decode_attention in fpnmt.h.) */
+FPNMT_API int fpnmt_decode_attention_dl(fpnmt_handle* h, const DLTensor* memory, const DLTensor* tokens, DLTensor* self_out,
+                                        DLTensor* cross_out, void* stream);
 /* fpnmt_generate (utils/pipeline.py:82-154): images as fpnmt_encode_dl; out_ids int32 [batch, max_len], out_len int32 [batch],
  * both on the GPU or both on the host (host outputs synchronise the stream); step_scores float32 [max_len, batch] on the GPU
  * or NULL. */
