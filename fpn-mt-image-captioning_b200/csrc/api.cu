@@ -163,6 +163,17 @@ FPNMT_API int fpnmt_generate(fpnmt_handle* h, const float* images, int on_host, 
   return h->eng->generate(images, on_host, out_ids, out_len, outputs_on_host, early_stop, step_scores,
                           (cudaStream_t)stream);
 }
+FPNMT_API int fpnmt_sample(fpnmt_handle* h, const float* images, int images_on_host, const fpnmt_sampling* sampling,
+                           int32_t* out_ids, int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
+                           void* stream) {
+  CHECK_H(h);
+  if (!sampling) {
+    set_last_error("sample: NULL sampling parameters");
+    return FPNMT_ERR_INVALID;
+  }
+  return h->eng->sample(images, images_on_host, *sampling, out_ids, out_len, out_logprob, outputs_on_host, early_stop,
+                        (cudaStream_t)stream);
+}
 FPNMT_API int fpnmt_stage_images(fpnmt_handle* h, const float* host_images, int slot) {
   CHECK_H(h);
   return h->eng->stage_images(host_images, slot);
@@ -771,6 +782,34 @@ FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x,
   if (!o.rc) o.rc = launch_layernorm_rows(x, rows, 512, dg, db, eps, ao, o.s);
   o.read_back(ao, rows, out);
   return o.finish("op_layernorm_rows");
+}
+
+FPNMT_API int fpnmt_op_sample_step(int device, const float* logits, int rows, int V, int samples_per_image, int t,
+                                   const fpnmt_sampling* sampling, int32_t* token, float* logprob, float* u_out, void* stream) {
+  if (!logits || !sampling || !token || rows < 1 || V < 1 || V > 51200 || samples_per_image < 1 || t < 0)
+    return op_invalid("op_sample_step: bad arguments (rows >= 1, 1 <= V <= 51200, samples_per_image >= 1, t >= 0)");
+  const fpnmt_sampling& sp = *sampling;
+  if (!(sp.temperature >= 0.f) || !(sp.top_p > 0.f && sp.top_p <= 1.f) || sp.top_k < 0 || sp.top_k > V || sp.reserved[0] ||
+      sp.reserved[1] || sp.reserved[2] || sp.reserved[3])
+    return op_invalid("op_sample_step: temperature >= 0, top_p in (0, 1], 0 <= top_k <= V and reserved words 0");
+  int rc = op_device(device, "op_sample_step");
+  if (rc) return rc;
+  rc = sample_set_attributes();
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, FPNMT_PREC_BF16);
+  const SampleParams prm{sp.temperature, sp.top_k, sp.top_p, 0, (unsigned long long)sp.seed};
+  SampleParams* dp = (SampleParams*)o.alloc(sizeof prm);
+  if (o.rc) return o.finish("op_sample_step");
+  cudaMemcpyAsync(dp, &prm, sizeof prm, cudaMemcpyHostToDevice, o.s);
+  SampleState st{};
+  st.rows = rows; st.V = V; st.N = samples_per_image; st.T = 0;
+  st.params = dp;
+  st.t0 = t;
+  st.tok_out = token;
+  st.lp_out = logprob;
+  st.u_out = u_out;
+  o.rc = launch_sample_step(st, logits, o.s);
+  return o.finish("op_sample_step");
 }
 
 }  // extern "C"

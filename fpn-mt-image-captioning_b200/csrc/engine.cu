@@ -43,6 +43,7 @@ Engine::~Engine() {
   if (enc_graph_) cudaGraphExecDestroy(enc_graph_);
   if (step_graph_) cudaGraphExecDestroy(step_graph_);
   if (loop_graph_) cudaGraphExecDestroy(loop_graph_);
+  if (sample_graph_) cudaGraphExecDestroy(sample_graph_);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
   for (auto st : grp_streams_) cudaStreamDestroy(st);
   for (auto ev : join_ev_) cudaEventDestroy(ev);
@@ -91,6 +92,7 @@ int Engine::init() {
   RC(elementwise_set_attributes());
   RC(attention_set_attributes());
   RC(beam_set_attributes());
+  RC(sample_set_attributes());
   RC(stem_set_attributes());
   use_xattn_ = !(c.kernel_opts & FPNMT_OPT_NO_XATTN);
   use_stem_ = !(c.kernel_opts & FPNMT_OPT_NO_STEM);
@@ -1852,6 +1854,68 @@ int Engine::generate(const float* images, int on_host, int32_t* out_ids, int32_t
                      float* step_scores, cudaStream_t s) {
   RC(encode(images, on_host, nullptr, s, false));
   return decode(out_ids, out_len, out_on_host, early_stop, step_scores, s);
+}
+
+// Sampled decode.  Row r = (image r / N, sample r % N) runs the teacher-forced step program (whole layer stack, fp32 logits
+// of every row, input token = BeamState::last_tok, identity ancestry, no KV-share representatives, first buffer pair) and
+// k_sample_step draws its next token, so the N rows of an image are N independent samples.  The sampling parameters live in a
+// device struct the kernel reads: a captured sample_graph_ serves every parameter set.
+int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len,
+                   float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
+  if (!finalized_) return fail(FPNMT_ERR_STATE, "sample before finalize_weights");
+  if (use_dstep_) return fail(FPNMT_ERR_STATE, "sample: the fused decoder has no sampling tail (use decode_path = chain)");
+  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "sample: this lane still holds a submitted batch (call fpnmt_collect first)");
+  const int B = cfg_.batch, N = cfg_.beam, T = cfg_.max_len, V = cfg_.vocab, R = B * N;
+  if (!(sp.temperature >= 0.f) || !(sp.top_p > 0.f && sp.top_p <= 1.f) || sp.top_k < 0 || sp.top_k > V ||
+      sp.reserved[0] || sp.reserved[1] || sp.reserved[2] || sp.reserved[3])
+    return fail(FPNMT_ERR_INVALID, "sample: temperature >= 0, top_p in (0, 1], 0 <= top_k <= vocab and reserved words 0");
+  if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "sample: NULL out_ids / out_len");
+  FPNMT_CUDA_OK(cudaSetDevice(dev_));
+  if (!ss_.ids) {   // per-row buffers [R][T] + [R] x 3 and the per-image counters, on the first call
+    SampleState st{};
+    st.rows = R; st.V = V; st.N = N; st.T = T;
+    st.start_id = cfg_.start_id; st.end_id = cfg_.end_id;
+    st.params = (const SampleParams*)dalloc(sizeof(SampleParams));
+    st.step = bs_.step;
+    st.last_tok = bs_.last_tok;
+    st.n_done = bs_.n_done;
+    st.ids = (int*)dalloc((size_t)R * T * 4);
+    st.len = (int*)dalloc((size_t)R * 4);
+    st.fin = (int*)dalloc((size_t)R * 4);
+    st.lp = (float*)dalloc((size_t)R * 4);
+    st.img_fin = (int*)dalloc((size_t)B * 4);
+    if (!st.params || !st.ids || !st.len || !st.fin || !st.lp || !st.img_fin) return FPNMT_ERR_CUDA;
+    sample_prog_ = step_forced_prog_;
+    const float* lg = logits_;
+    Op o = ew_op("sample_step", [st, lg](cudaStream_t q) { return launch_sample_step(st, lg, q); },
+                 (double)R * V * 4 + (double)R * 16, "beam");
+    o.idempotent = false;
+    sample_prog_.push_back(std::move(o));
+    ss_ = st;
+  }
+  const SampleParams prm{sp.temperature, sp.top_k, sp.top_p, 0, (unsigned long long)sp.seed};
+  if (images) RC(encode(images, on_host, nullptr, s, false));
+  FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<SampleParams*>(ss_.params), &prm, sizeof prm, cudaMemcpyHostToDevice, s));
+  RC(run_program(dec_init_prog_, s));
+  RC(launch_sample_init(ss_, bs_.anc[0], s));
+  launches += 1;
+  forced_mode_ = true;   // the self-attention launches of the program stay in the first buffer pair, without representatives
+  struct Reset { bool& f; ~Reset() { f = false; } } reset{forced_mode_};
+  if (cfg_.use_graphs && !sample_graph_) RC(capture(sample_prog_, &sample_graph_));
+  for (int t = 0; t < T; ++t) {
+    RC(launch_prog(sample_prog_, sample_graph_, s));
+    if (early_stop && (t % 4 == 3) && t + 1 < T) {
+      FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, bs_.n_done, 4, cudaMemcpyDeviceToHost, s));
+      FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+      if (h_pinned_[0] >= B) break;
+    }
+  }
+  const cudaMemcpyKind kind = out_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, ss_.ids, (size_t)R * T * 4, kind, s));
+  FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, ss_.len, (size_t)R * 4, kind, s));
+  if (out_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, ss_.lp, (size_t)R * 4, kind, s));
+  if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+  return 0;
 }
 
 // Double-buffered input (the role of dataset.py:90-92's map/prefetch in the reference's input pipeline): the copy of the

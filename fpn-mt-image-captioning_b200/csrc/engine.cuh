@@ -69,6 +69,10 @@ class Engine {
   int decode(int32_t* out_ids, int32_t* out_len, int on_host, int early_stop, float* step_scores, cudaStream_t s);
   int generate(const float* images, int on_host, int32_t* out_ids, int32_t* out_len, int out_on_host, int early_stop,
                float* step_scores, cudaStream_t s);
+  // Sampled decode (fpnmt_sample): every row of the batch is one independent sample of its image; the teacher-forced step
+  // program with k_sample_step in place of the teacher-forced tail.  images == nullptr: the memory of the last encode.
+  int sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len, float* out_logprob,
+             int out_on_host, int early_stop, cudaStream_t s);
   int profile(int iters, char* buf, size_t cap);
   int capture_groups(int T);
   int build_dstep(const Tensor& ckv, const float* d_emb, const float* d_pos);
@@ -105,6 +109,9 @@ class Engine {
   // programs
   Program cnn_prog_, enc_prog_, dec_init_prog_, embed_prog_, step_prog_, step_forced_prog_;
   Program step_attn_prog_;                // step_forced_prog_ + the attention-probability launches (decode_logits with outputs)
+  Program sample_prog_;                   // step_forced_prog_ + k_sample_step (sample; built on its first call)
+  SampleState ss_{};                      // sampler state: per-row buffers allocated on the first sample call
+  cudaGraphExec_t sample_graph_ = nullptr;   // sample_prog_ captured with forced_mode_ set (never step_graph_)
   BeamEmbed beam_embed_{};
   cudaGraphExec_t cnn_graph_ = nullptr, enc_graph_ = nullptr, step_graph_ = nullptr, loop_graph_ = nullptr;
   std::vector<DecGroup> groups_;          // decoder groups (empty: the whole batch is one chain)

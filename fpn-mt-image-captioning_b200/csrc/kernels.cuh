@@ -158,4 +158,39 @@ int launch_beam_step(const BeamState& st, const float* logits, int ld, const Bea
 int launch_kv_reorder(const bf16* const* bufs, int ncaches, const int* parent, int rows, int rows_total, int N, int T, int row_bytes,
                       const int* step, cudaStream_t s);
 
+// ---- sample.cu ----------------------------------------------------------------------------------
+// Sampled decoding (fpnmt_sampling, include/fpnmt.h): row r = (image r / N, sample r % N) of fp32 logits [rows][V] draws one
+// token from softmax(z / temperature) restricted to the top-k logits (ties kept) and then to the nucleus of top_p of that
+// mass, with the Philox4x32-10 uniform of counter (t, image, sample, 0) and key (seed lo, seed hi).
+struct SampleParams {       // device copy of fpnmt_sampling read by every step (changing it needs no graph re-capture)
+  float temperature;
+  int top_k;
+  float top_p;
+  int pad;
+  unsigned long long seed;
+};
+struct SampleState {
+  int rows, V, N, T;         // rows = images * N samples, vocab, samples per image, max steps
+  int start_id, end_id;
+  const SampleParams* params;
+  int* step;                 // device step counter (advanced by the kernel), or nullptr: step t0
+  int t0;
+  // engine decode state (ids == nullptr: stand-alone step, nothing below is touched)
+  int* last_tok;             // [rows] token fed to the next step
+  int* ids;                  // [rows][T] caption of each sample, 0 padded (no <start>, no <end>)
+  int* len;                  // [rows]
+  int* fin;                  // [rows] 1 once the sample emitted <end> (or ran T steps)
+  float* lp;                 // [rows] sum of log_softmax(z)[token] (temperature 1) over the emitted steps
+  int* img_fin;              // [images] finished samples of the image
+  int* n_done;               // [2]: finished images, row-completion counter of the step
+  // per-step outputs, each optional
+  int* tok_out;              // [rows]
+  float* lp_out;             // [rows] log_softmax(z)[token] at temperature 1
+  float* u_out;              // [rows] the row's uniform
+};
+int sample_set_attributes();
+// step 0, last_tok = <start>, identity ancestry [2][rows][T] in `anc`, per-row and per-image state cleared
+int launch_sample_init(const SampleState& st, int* anc, cudaStream_t s);
+int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t s);
+
 }  // namespace fpnmt

@@ -30,6 +30,12 @@ class FpnmtConfig(C.Structure):
                            ("lanes", C.c_int32), ("reserved", C.c_int32 * 1)]
 
 
+class FpnmtSampling(C.Structure):
+    """fpnmt_sampling (include/fpnmt.h): temperature, top-k, top-p and seed of a sampled decode."""
+    _fields_ = [("temperature", C.c_float), ("top_k", C.c_int32), ("top_p", C.c_float), ("seed", C.c_uint64),
+                ("reserved", C.c_int32 * 4)]
+
+
 class FpnmtError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__("fpnmt error %d: %s" % (code, msg))
@@ -77,6 +83,8 @@ SIGNATURES = {
     "fpnmt_op_kv_reorder": (_i, [_i, _i, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp]),
     "fpnmt_op_embed_pos": (_i, [_i, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _vp, _vp]),
     "fpnmt_op_layernorm_rows": (_i, [_i, _i, _vp, _i, _vp, _vp, C.c_float, _vp, _vp]),
+    "fpnmt_sample": (_i, [_vp, _vp, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _i, _i, _vp]),
+    "fpnmt_op_sample_step": (_i, [_i, _vp, _i, _i, _i, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _vp]),
 }
 
 
@@ -106,6 +114,7 @@ SIGNATURES.update({
     "fpnmt_decode_hidden_dl": (_i, [_vp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_decode_attention_dl": (_i, [_vp, _dlp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_generate_dl": (_i, [_vp, _dlp, _dlp, _dlp, _i, _dlp, _vp]),
+    "fpnmt_sample_dl": (_i, [_vp, _dlp, C.POINTER(FpnmtSampling), _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_comm_unique_id": (_i, [_vp]),
     "fpnmt_comm_create": (_i, [_i, _i, _vp, _i, C.POINTER(_vp)]),
     "fpnmt_comm_destroy": (_i, [_vp]),
@@ -148,6 +157,13 @@ def load() -> C.CDLL:
         fn.argtypes = args
     _lib = lib
     return lib
+
+
+def sampling(temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0) -> FpnmtSampling:
+    """An fpnmt_sampling with the reserved words zero."""
+    sp = FpnmtSampling()
+    sp.temperature, sp.top_k, sp.top_p, sp.seed = float(temperature), int(top_k), float(top_p), int(seed) & 0xFFFFFFFFFFFFFFFF
+    return sp
 
 
 def check(rc: int) -> None:

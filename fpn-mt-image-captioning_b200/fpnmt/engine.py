@@ -226,6 +226,29 @@ class Engine:
                                            _stream_ptr(self.device)))
         return (ids, lens, scores) if return_scores else (ids, lens)
 
+    def sample(self, images=None, *, temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0,
+               early_stop: bool = True, to_host: bool = True, return_logprobs: bool = False):
+        """`beam` independent sampled captions per image (fpnmt_sample; semantics in include/fpnmt.h): softmax(z / temperature)
+        restricted to the top_k logits (0 = off, ties kept) and then to the nucleus of top_p of that mass (1 = off), drawn with
+        the Philox stream of (seed, step, image, sample).  temperature 0 is greedy.  images None = the memory of the last
+        encode / generate.  Returns ids (B, N, T) int32 zero padded without <start> / <end>, lengths (B, N) and, with
+        return_logprobs, the captions' log-likelihoods (B, N) float32 (log_softmax at temperature 1, <end> included)."""
+        ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
+        B, N, T = self.batch, self.beam, self.max_len
+        if to_host:
+            ids = torch.empty((B, N, T), dtype=torch.int32).pin_memory()
+            lens = torch.empty((B, N), dtype=torch.int32).pin_memory()
+            lp = torch.empty((B, N), dtype=torch.float32).pin_memory() if return_logprobs else None
+        else:
+            ids = torch.empty((B, N, T), dtype=torch.int32, device=self.device)
+            lens = torch.empty((B, N), dtype=torch.int32, device=self.device)
+            lp = torch.empty((B, N), dtype=torch.float32, device=self.device) if return_logprobs else None
+        sp = _lib.sampling(temperature, top_k, top_p, seed)
+        _lib.check(self.lib.fpnmt_sample(self._h, ptr, on_host, C.byref(sp), ids.data_ptr(), lens.data_ptr(),
+                                         lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
+                                         _stream_ptr(self.device)))
+        return (ids, lens, lp) if return_logprobs else (ids, lens)
+
     def stage(self, host_images, slot: int):
         """Enqueue the host->device copy of one batch into staging slot 0/1 on the engine's copy stream (returns at once).
         Returns the host tensor actually handed to the copy; keep it alive until the matching generate_staged is done."""
@@ -671,6 +694,24 @@ def layernorm_rows(x: torch.Tensor, gamma: np.ndarray, beta: np.ndarray, eps: fl
     _lib.check(_lib.load().fpnmt_op_layernorm_rows(x.device.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), x.shape[0],
                                                    _hptr(g), _hptr(b), eps, out.data_ptr(), _stream_ptr(x.device)))
     return out
+
+
+def sample_step(logits: torch.Tensor, samples_per_image: int, t: int, temperature: float = 1.0, top_k: int = 0,
+                top_p: float = 1.0, seed: int = 0) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """One step of the sampling kernel (fpnmt_op_sample_step) on logits (rows, V): row r is sample r % samples_per_image of
+    image r // samples_per_image at step t.  Returns (token (rows,) int32, log_softmax(logits)[token] at temperature 1
+    (rows,) float32, the rows' Philox uniforms (rows,) float32), on the logits' device."""
+    lg = logits if isinstance(logits, torch.Tensor) and logits.is_cuda else _as_cuda(logits, torch.float32, torch.device("cuda", 0))
+    lg = lg.to(torch.float32).contiguous()
+    rows, V = lg.shape
+    device = lg.device.index or 0
+    tok = torch.empty((rows,), dtype=torch.int32, device=lg.device)
+    lp = torch.empty((rows,), dtype=torch.float32, device=lg.device)
+    u = torch.empty((rows,), dtype=torch.float32, device=lg.device)
+    sp = _lib.sampling(temperature, top_k, top_p, seed)
+    _lib.check(_lib.load().fpnmt_op_sample_step(device, lg.data_ptr(), rows, V, int(samples_per_image), int(t), C.byref(sp),
+                                                tok.data_ptr(), lp.data_ptr(), u.data_ptr(), _stream_ptr(lg.device)))
+    return tok, lp, u
 
 
 def preprocess(images_u8: torch.Tensor, size: int = cfg.IMAGE_INPUT_SIZE) -> torch.Tensor:

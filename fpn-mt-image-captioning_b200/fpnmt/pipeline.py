@@ -76,6 +76,17 @@ class Pipeline:
         attn = {k: v.cpu().numpy() for k, v in eng.caption_attention(ids, lens).items()}
         return ids.numpy(), lens.numpy(), attn
 
+    def sample_batch(self, imgs, max_seq_len: Optional[int] = None, num_samples: Optional[int] = None, *,
+                     temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0, return_logprobs: bool = False):
+        """`num_samples` (default: the beam width) independent sampled captions per image (Engine.sample): imgs (B,S,S,3)
+        float32 in [-1,1] -> (ids (B,num_samples,T) int32 zero padded, lengths (B,num_samples)), plus the captions'
+        log-likelihoods (B,num_samples) with return_logprobs.  temperature 0 is greedy."""
+        imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
+        eng = self.transformer.engine(int(imgs.shape[0]), num_samples or self.beam, max_seq_len or self.max_seq_len)
+        out = eng.sample(imgs, temperature=temperature, top_k=top_k, top_p=top_p, seed=seed, early_stop=True, to_host=True,
+                         return_logprobs=return_logprobs)
+        return tuple(o.numpy() for o in out)
+
     def predict(self, img, max_seq_len, plot_layer=False):
         """pipeline.py:82-154: img (H,W,3) -> (1-D int32 ids without <start>/<end>, attention_weights).
         attention_weights is None unless `plot_layer` is truthy; then it is the dict of the reference's last forward pass for

@@ -172,6 +172,41 @@ FPNMT_API int fpnmt_decode_attention(fpnmt_handle* h, const float* memory, const
 FPNMT_API int fpnmt_beam_step(fpnmt_handle* h, const float* logits, const float* scores_in, int32_t* parent, int32_t* token,
                     float* scores_out, void* stream);
 
+/* Sampling parameters of fpnmt_sample / fpnmt_op_sample_step.  Row (image b, sample n) at step t, logits z (fp32, the
+ * vocabulary projection):
+ *   1. p = softmax(z / temperature) over all V tokens.
+ *   2. top-k: K1 = {i : z_i >= z_(k)}, z_(k) the k-th largest logit; every token tied with it is kept (|K1| may exceed k).
+ *   3. top-p: p renormalised over K1; K2 = {i in K1 : p_i >= tau}, tau the largest value for which the tokens of K1 with
+ *      p_j >= tau hold at least top_p of K1's mass.  Ties at tau are kept; K2 always holds the arg-max.
+ *   4. u = (philox4x32_10(counter = (t, b, n, 0), key = (seed & 0xffffffff, seed >> 32))[0] >> 8) * 2^-24.
+ *   5. token = the smallest id i in K2 with sum_{j in K2, j <= i} p_j > u * sum_{K2} p.
+ *   6. log-probability of a sample = sum over its emitted steps, <end> included, of log_softmax(z)[token] at temperature 1
+ *      with no filtering: the caption's log-likelihood under the model.
+ * temperature 0 is greedy: the arg-max, lowest token id on ties (identical for every n; on an engine with the reference beam
+ * initialisation that is the caption fpnmt_generate returns).  Vocabulary entries with logit -1e9 get p = 0 and are never
+ * drawn. */
+typedef struct fpnmt_sampling {
+  float temperature;     /* >= 0; 0 = greedy (arg-max, lowest token id on ties)        */
+  int32_t top_k;         /* 0 = off; else keep tokens whose logit >= the k-th largest  */
+  float top_p;           /* (0, 1]; 1 = off                                            */
+  uint64_t seed;
+  int32_t reserved[4];   /* must be 0 */
+} fpnmt_sampling;
+
+/* N = beam independent sampled captions per image (see fpnmt_sampling): encoder (images != NULL; NULL = the memory of the
+ * last fpnmt_encode / fpnmt_generate) + a decode in which row (b, n) is sample n of image b.  A sample stops at its first
+ * <end>; its row keeps being computed but its tokens are ignored; an image is done when all N of its samples are.
+ * out_ids DEVICE-or-HOST int32 [batch][beam][max_len] (0 padded, no <start>, no <end>), out_len int32 [batch][beam]
+ * (max_len when <end> never fired), out_logprob float32 [batch][beam] or NULL (same side as the others).
+ * outputs_on_host != 0: host outputs, the call synchronises the stream.  early_stop != 0: stop once every sample has
+ * emitted <end> (the result is the same either way).  Errors: FPNMT_ERR_INVALID for temperature < 0, top_p outside (0, 1],
+ * top_k outside [0, vocab] or non-zero reserved words; FPNMT_ERR_STATE with decode_path = FUSED or while lane 0 holds a
+ * submitted batch.  Results are bit-identical run to run, with graphs on or off, early stop on or off and in both cache
+ * modes; the call leaves nothing behind that changes a later fpnmt_generate. */
+FPNMT_API int fpnmt_sample(fpnmt_handle* h, const float* images, int images_on_host, const fpnmt_sampling* sampling,
+                           int32_t* out_ids, int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
+                           void* stream);
+
 /* Replaces: Pipeline.predict (utils/pipeline.py:82-154) for a batch: encoder + beam-search decode.
  * out_ids DEVICE-or-HOST int32 [batch, max_len] (0 padded), out_len int32 [batch]: exactly what predict() returns
  * per image (<start> stripped, trailing <end> stripped).  outputs_on_host != 0: results are copied to host and
@@ -336,6 +371,13 @@ FPNMT_API int fpnmt_op_embed_pos(int device, int precision, const int* tokens, i
  * float32; gamma / beta HOST [512]; out [rows, 512]. */
 FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x, int rows, const float* gamma,
                                       const float* beta, float eps, float* out, void* stream);
+
+/* One sampling step (the kernel of fpnmt_sample) on caller logits: logits DEVICE float32 [rows][V]; row r is sample
+ * r % samples_per_image of image r / samples_per_image at step t; sampling as fpnmt_sample.  Outputs DEVICE: token int32
+ * [rows], logprob float32 [rows] (log_softmax at temperature 1 of the token) or NULL, u_out float32 [rows] (the row's
+ * Philox uniform) or NULL.  V in [1, 51200]. */
+FPNMT_API int fpnmt_op_sample_step(int device, const float* logits, int rows, int V, int samples_per_image, int t,
+                                   const fpnmt_sampling* sampling, int32_t* token, float* logprob, float* u_out, void* stream);
 
 #ifdef __cplusplus
 }

@@ -63,6 +63,11 @@ FPNMT_API int fpnmt_decode_attention_dl(fpnmt_handle* h, const DLTensor* memory,
  * or NULL. */
 FPNMT_API int fpnmt_generate_dl(fpnmt_handle* h, const DLTensor* images, DLTensor* out_ids, DLTensor* out_len, int early_stop,
                                 DLTensor* step_scores, void* stream);
+/* fpnmt_sample: images as fpnmt_encode_dl, or NULL for the memory of the last encode; out_ids int32 [batch, beam, max_len],
+ * out_len int32 [batch, beam], out_logprob float32 [batch, beam] or NULL, all on the GPU or all on the host (host outputs
+ * synchronise the stream). */
+FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpnmt_sampling* sampling, DLTensor* out_ids,
+                              DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream);
 
 /* ---- in-library communicator: the ONE collective of the path (SURVEY §8e) -------------------------------------------
  * Image batches shard across the GPUs of a box; the only exchange is the all-gather of the caption ids.  The library opens
