@@ -16,7 +16,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libfpnmt.so")
-SOURCES = ["api.cu", "engine.cu", "igemm.cu", "tgemm.cu", "tgemmw.cu", "xattn.cu", "dstep.cu", "stem.cu", "tensormap.cu", "elementwise.cu", "attention.cu", "beam.cu", "sample.cu", "jpeg.cu", "dlapi.cu"]
+SOURCES = ["api.cu", "engine.cu", "igemm.cu", "tgemm.cu", "tgemmw.cu", "xattn.cu", "dstep.cu", "stem.cu", "tensormap.cu", "elementwise.cu", "attention.cu", "beam.cu", "sample.cu", "score.cu", "jpeg.cu", "dlapi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
          "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]

@@ -174,6 +174,11 @@ FPNMT_API int fpnmt_sample(fpnmt_handle* h, const float* images, int images_on_h
   return h->eng->sample(images, images_on_host, *sampling, out_ids, out_len, out_logprob, outputs_on_host, early_stop,
                         (cudaStream_t)stream);
 }
+FPNMT_API int fpnmt_score(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* ids, const int32_t* lens, int t,
+                          float* out_logprob, float* out_token_logprob, int outputs_on_host, void* stream) {
+  CHECK_H(h);
+  return h->eng->score(images, images_on_host, ids, lens, t, out_logprob, out_token_logprob, outputs_on_host, (cudaStream_t)stream);
+}
 FPNMT_API int fpnmt_stage_images(fpnmt_handle* h, const float* host_images, int slot) {
   CHECK_H(h);
   return h->eng->stage_images(host_images, slot);

@@ -287,6 +287,36 @@ FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpn
                       stream);
 }
 
+FPNMT_API int fpnmt_score_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* ids, const DLTensor* lens,
+                             DLTensor* out_logprob, DLTensor* out_token_logprob, void* stream) {
+  CHECK_HDL(h);
+  const fpnmt_config& c = h->eng->config();
+  const int64_t S = c.image_size;
+  void *pi = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr, *ptok = nullptr;
+  int img_host = 0, lp_host = 0, tok_host = 0;
+  int rc = 0;
+  if (images) {
+    rc = dl_check("score_dl: images", images, kDLFloat, h->eng->device(), true, true, {c.batch, S, S, 3}, &pi, &img_host);
+    if (rc) return rc;
+  }
+  rc = dl_check("score_dl: ids", ids, kDLInt, h->eng->device(), false, true, {c.batch, c.beam, -1}, &pids, nullptr);
+  if (rc) return rc;
+  const int64_t t = ids->shape[2];
+  if (t < 1 || t > c.max_len) return dl_fail("score_dl: ids must hold 1 .. max_len positions per caption");
+  rc = dl_check("score_dl: lens", lens, kDLInt, h->eng->device(), false, true, {c.batch, c.beam}, &plen, nullptr);
+  if (rc) return rc;
+  rc = dl_check("score_dl: out_logprob", out_logprob, kDLFloat, h->eng->device(), true, true, {c.batch, c.beam}, &plp, &lp_host);
+  if (rc) return rc;
+  if (out_token_logprob) {
+    rc = dl_check("score_dl: out_token_logprob", out_token_logprob, kDLFloat, h->eng->device(), true, true, {c.batch, c.beam, t}, &ptok,
+                  &tok_host);
+    if (rc) return rc;
+    if (tok_host != lp_host) return dl_fail("score_dl: out_token_logprob must live where out_logprob does");
+  }
+  return fpnmt_score(h, (const float*)pi, img_host, (const int32_t*)pids, (const int32_t*)plen, (int)t, (float*)plp, (float*)ptok,
+                     lp_host, stream);
+}
+
 // ---- communicator ---------------------------------------------------------------------------------------------------
 FPNMT_API int fpnmt_comm_unique_id(uint8_t id_out[FPNMT_UNIQUE_ID_BYTES]) {
   if (!id_out) return dl_fail("comm_unique_id: NULL");

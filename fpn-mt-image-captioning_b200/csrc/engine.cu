@@ -44,6 +44,7 @@ Engine::~Engine() {
   if (step_graph_) cudaGraphExecDestroy(step_graph_);
   if (loop_graph_) cudaGraphExecDestroy(loop_graph_);
   if (sample_graph_) cudaGraphExecDestroy(sample_graph_);
+  for (auto& kv : score_graphs_) cudaGraphExecDestroy(kv.second);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
   for (auto st : grp_streams_) cudaStreamDestroy(st);
   for (auto ev : join_ev_) cudaEventDestroy(ev);
@@ -967,6 +968,8 @@ int Engine::build_decoder() {
   float *d_pos, *d_emb;
   RC(upload_f32(pos, &d_pos));
   RC(prep_vec(std::string(TR) + "/decoder/embedding/embeddings", &d_emb));
+  dec_emb_ = d_emb;
+  dec_pos_ = d_pos;
 
   // cross-attention K/V of the memory for all layers: one GEMM [B*16,512] x [512, L*2*512] per batch
   {
@@ -981,6 +984,7 @@ int Engine::build_decoder() {
     Tensor ckv = rows_act(B * n_base_, L * 2 * D);
     RC(add_conv(dec_init_prog_, "dec_cross_kv", enc_out_, g, 1, 1, 0, 0, ACT_NONE, RES_NONE, nullptr, ckv));
     taps_["cross_kv"] = ckv;
+    dec_ckv_ = ckv;
 
     // Group-stationary fused decoder (dstep.cuh): one kernel per decode instead of 38 per step.  Needs the bf16 mode,
     // log-domain scores and the reference beam semantics; everything else takes the per-operator chain below.
@@ -1041,9 +1045,7 @@ int Engine::build_decoder() {
       k_anc_identity<<<148, 256>>>(anc, R, T);
       FPNMT_CUDA_OK(cudaGetLastError());
     }
-    struct LayerW {
-      GemmW gqkv, go1, gq2, go2, g1, g2;
-      float* lnp[6];
+    struct LayerW : DecLayerW {
       Tensor qkv, att, out1, q2, att2, out2, hdn, out3, kc, vc, kc2, vc2;
       float* y;
     };
@@ -1071,6 +1073,8 @@ int Engine::build_decoder() {
     }
     GemmW gf;
     RC(prep_dense_cat({std::string(TR) + "/final_layer"}, &gf));
+    dec_lw_.assign(lw.begin(), lw.end());
+    dec_final_ = gf;
     Tensor x0 = rows_act(R, D);
     auto row_view = [](const Tensor& t, size_t r0, int rows) {
       Tensor v = t;
@@ -1914,6 +1918,132 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
   FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, ss_.ids, (size_t)R * T * 4, kind, s));
   FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, ss_.len, (size_t)R * 4, kind, s));
   if (out_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, ss_.lp, (size_t)R * 4, kind, s));
+  if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// Score program for captions of t positions.  Row r = c * t + j (caption c = b * N + n, position j) of every activation:
+// the Dense layers are igemm in its 1x1 dense geometry at B * N * t rows (LayerNorm layers: fp32 residual output, then
+// layernorm_rows), the self-attention is causal over the caption's own rows, the cross-attention is the step program's kernel
+// with beam := N * t (rows per image).  The vocabulary projection runs in chunks of B * N rows through the [B * N][V] logits
+// buffer of the step programs, each followed by score_rows; score_sum closes the pass.
+int Engine::build_score(int t, Program& p) {
+  const int B = cfg_.batch, N = cfg_.beam, D = cfg_.d_model, H = cfg_.num_heads, V = cfg_.vocab, L = cfg_.num_layers;
+  const int R = B * N, rows = R * t;
+  const double esz = split_ ? 4.0 : 2.0;
+  auto view = [rows](const Tensor& a) {
+    Tensor v = a;
+    v.N = 1; v.H = 1; v.W = rows;
+    return v;
+  };
+  Tensor x = view(sc_.x), qkv = view(sc_.qkv), att = view(sc_.att), out1 = view(sc_.out1), q2 = view(sc_.q2),
+         out2 = view(sc_.out2), hdn = view(sc_.hdn);
+  Tensor none;
+  float* y = sc_.y;
+  const ScoreArgs a{R, t, V, cfg_.start_id, cfg_.end_id, sc_.ids, sc_.lens, sc_.tgt, sc_.bad, sc_.tok_lp, sc_.lp};
+  {
+    const float *emb = dec_emb_, *pos = dec_pos_;
+    const Act xa = x.a;
+    p.push_back(ew_op("score_embed", [=](cudaStream_t s) { return launch_score_embed(a, emb, pos, xa, s); },
+                      (double)rows * D * (8 + esz) + (double)rows * 8));
+  }
+  auto dense_ln = [&](const std::string& nm, const Tensor& in, const GemmW& g, const Tensor& res, const float* gam,
+                      const float* bet, const Tensor& out) -> int {
+    RC(add_conv(p, nm, in, g, 1, 1, 0, 0, ACT_NONE, RES_SAME, &res, none, y, D));
+    const Act oa = out.a;
+    p.push_back(ew_op(nm + "_ln", [=](cudaStream_t s) { return launch_layernorm_rows(y, rows, D, gam, bet, 1e-6f, oa, s); },
+                      (double)rows * D * (4 + esz)));
+    return 0;
+  };
+  for (int l = 0; l < L; ++l) {
+    const DecLayerW& w = dec_lw_[l];
+    const std::string ln = "score_dec" + std::to_string(l);
+    RC(add_conv(p, ln + "_qkv", x, w.gqkv, 1, 1, 0, 0, ACT_NONE, RES_NONE, nullptr, qkv));
+    {
+      const Act qa = qkv.a, oa = att.a;
+      Op o = ew_op(ln + "_self_attn", [=](cudaStream_t s) { return launch_score_self_attention(qa, R, t, H, oa, s); },
+                   (double)rows * D * 4 * esz, "attention");
+      o.flops = 4.0 * R * D * (double)t * (t + 1) / 2;
+      p.push_back(std::move(o));
+    }
+    RC(dense_ln(ln + "_o1+res", att, w.go1, x, w.lnp[0], w.lnp[1], out1));
+    RC(add_conv(p, ln + "_q2", out1, w.gq2, 1, 1, 0, 0, ACT_NONE, RES_NONE, nullptr, q2));
+    {
+      const Act qa = q2.a, oa = att.a, ka = dec_ckv_.a;
+      const int kcx = l * 2 * D, vcx = l * 2 * D + D, tk = n_base_, rows_per_image = N * t;
+      p.push_back(ew_op(ln + "_cross_attn",
+                        [=](cudaStream_t s) { return launch_dec_cross_attention(qa, ka, kcx, vcx, rows, rows_per_image, tk, H, oa, s); },
+                        (double)rows * D * 2 * esz + (double)B * tk * 2 * D * esz, "attention"));
+    }
+    RC(dense_ln(ln + "_o2+res", att, w.go2, out1, w.lnp[2], w.lnp[3], out2));
+    RC(add_conv(p, ln + "_ffn1", out2, w.g1, 1, 1, 0, 0, ACT_LEAKY, RES_NONE, nullptr, hdn));
+    RC(dense_ln(ln + "_ffn2+res", hdn, w.g2, out2, w.lnp[4], w.lnp[5], x));
+  }
+  for (int c = 0; c < t; ++c) {
+    Tensor xc = x;
+    xc.a.p = x.a.p + (size_t)c * R * x.a.ld;
+    xc.W = R;
+    RC(add_conv(p, "score_final_layer", xc, dec_final_, 1, 1, 0, 0, ACT_NONE, RES_NONE, nullptr, none, logits_, V));
+    const int* tg = sc_.tgt + (size_t)c * R;
+    float* tl = sc_.tok_lp + (size_t)c * R;
+    const float* lg = logits_;
+    p.push_back(ew_op("score_rows", [=](cudaStream_t s) { return launch_score_rows(lg, R, V, tg, tl, s); },
+                      (double)R * V * 4 + (double)R * 8));
+  }
+  p.push_back(ew_op("score_sum", [=](cudaStream_t s) { return launch_score_sum(a, s); }, (double)rows * 8 + (double)R * 8));
+  return 0;
+}
+
+int Engine::score(const float* images, int on_host, const int32_t* ids, const int32_t* lens, int t, float* out_logprob,
+                  float* out_token_logprob, int out_on_host, cudaStream_t s) {
+  if (!finalized_) return fail(FPNMT_ERR_STATE, "score before finalize_weights");
+  if (use_dstep_) return fail(FPNMT_ERR_STATE, "score: the fused decoder has no per-layer weights for a parallel pass (use decode_path = chain)");
+  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "score: this lane still holds a submitted batch (call fpnmt_collect first)");
+  if (t < 1 || t > cfg_.max_len) return fail(FPNMT_ERR_INVALID, "score: t must lie in [1, max_len]");
+  if (!ids || !lens || !out_logprob) return fail(FPNMT_ERR_INVALID, "score: NULL ids / lens / out_logprob");
+  FPNMT_CUDA_OK(cudaSetDevice(dev_));
+  const int R = cfg_.batch * cfg_.beam, T = cfg_.max_len, D = cfg_.d_model;
+  if (!sc_.x.a.p) {   // activations of B * N * max_len rows, on the first call
+    const int rows = R * T;
+    sc_.x = rows_act(rows, D); sc_.qkv = rows_act(rows, 3 * D); sc_.att = rows_act(rows, D); sc_.out1 = rows_act(rows, D);
+    sc_.q2 = rows_act(rows, D); sc_.out2 = rows_act(rows, D); sc_.hdn = rows_act(rows, cfg_.dff);
+    sc_.y = (float*)dalloc((size_t)rows * D * 4);
+    sc_.ids = (int*)dalloc((size_t)rows * 4);
+    sc_.lens = (int*)dalloc((size_t)R * 4);
+    sc_.tgt = (int*)dalloc((size_t)rows * 4);
+    sc_.bad = (int*)dalloc((size_t)R * 4);
+    sc_.tok_lp = (float*)dalloc((size_t)rows * 4);
+    sc_.lp = (float*)dalloc((size_t)R * 4);
+    if (!sc_.x.a.p || !sc_.qkv.a.p || !sc_.att.a.p || !sc_.out1.a.p || !sc_.q2.a.p || !sc_.out2.a.p || !sc_.hdn.a.p || !sc_.y ||
+        !sc_.ids || !sc_.lens || !sc_.tgt || !sc_.bad || !sc_.tok_lp || !sc_.lp) {
+      sc_.x.a.p = nullptr;
+      return FPNMT_ERR_CUDA;
+    }
+  }
+  auto it = score_progs_.find(t);
+  if (it == score_progs_.end()) {
+    Program p;
+    RC(build_score(t, p));
+    it = score_progs_.emplace(t, std::move(p)).first;
+  }
+  if (images) RC(encode(images, on_host, nullptr, s, false));
+  FPNMT_CUDA_OK(cudaMemcpyAsync(sc_.ids, ids, (size_t)R * t * 4, cudaMemcpyDeviceToDevice, s));
+  FPNMT_CUDA_OK(cudaMemcpyAsync(sc_.lens, lens, (size_t)R * 4, cudaMemcpyDeviceToDevice, s));
+  RC(run_program(dec_init_prog_, s));
+  cudaGraphExec_t g = nullptr;
+  if (cfg_.use_graphs) {
+    auto gi = score_graphs_.find(t);
+    if (gi == score_graphs_.end()) {
+      RC(capture(it->second, &g));
+      score_graphs_[t] = g;
+    } else {
+      g = gi->second;
+    }
+  }
+  RC(launch_prog(it->second, g, s));
+  const cudaMemcpyKind kind = out_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, sc_.lp, (size_t)R * 4, kind, s));
+  if (out_token_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_token_logprob, sc_.tok_lp, (size_t)R * t * 4, kind, s));
   if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
 }

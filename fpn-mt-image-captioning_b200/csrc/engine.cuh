@@ -28,6 +28,11 @@ struct GemmW {          // device weight matrix [Cout][K] bf16 (split: [Cout][2K
   int Cout = 0, K = 0;
 };
 
+struct DecLayerW {      // device weights of one decoder layer (shared by the step programs and the score pass)
+  GemmW gqkv, go1, gq2, go2, g1, g2;
+  float* lnp[6];        // layernorm{1,2,3} gamma, beta
+};
+
 struct Tensor {         // NHWC activation (dense rows: N=1,H=1,W=rows)
   Act a{nullptr, 0, 0, 0};
   int N = 0, H = 0, W = 0;
@@ -73,6 +78,10 @@ class Engine {
   // program with k_sample_step in place of the teacher-forced tail.  images == nullptr: the memory of the last encode.
   int sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len, float* out_logprob,
              int out_on_host, int early_stop, cudaStream_t s);
+  // Caption scoring (fpnmt_score): the N captions ids [B][N][t] / lens [B][N] (device) of every image through the decoder
+  // as B * N * t rows of one teacher-forced pass.  images == nullptr: the memory of the last encode.
+  int score(const float* images, int on_host, const int32_t* ids, const int32_t* lens, int t, float* out_logprob,
+            float* out_token_logprob, int out_on_host, cudaStream_t s);
   int profile(int iters, char* buf, size_t cap);
   int capture_groups(int T);
   int build_dstep(const Tensor& ckv, const float* d_emb, const float* d_pos);
@@ -112,6 +121,21 @@ class Engine {
   Program sample_prog_;                   // step_forced_prog_ + k_sample_step (sample; built on its first call)
   SampleState ss_{};                      // sampler state: per-row buffers allocated on the first sample call
   cudaGraphExec_t sample_graph_ = nullptr;   // sample_prog_ captured with forced_mode_ set (never step_graph_)
+  // score pass: one program (and graph) per caption length t, built on its first call; activations for B * N * max_len rows
+  // allocated on the first call and shared by all of them (one layer's set is live at a time)
+  struct ScoreBufs {
+    Tensor x, qkv, att, out1, q2, out2, hdn;
+    float* y = nullptr;
+    int *ids = nullptr, *lens = nullptr, *tgt = nullptr, *bad = nullptr;
+    float *tok_lp = nullptr, *lp = nullptr;
+  } sc_;
+  std::map<int, Program> score_progs_;
+  std::map<int, cudaGraphExec_t> score_graphs_;
+  std::vector<DecLayerW> dec_lw_;         // decoder weights prepared by build_decoder (chain decode path)
+  GemmW dec_final_{};
+  const float *dec_emb_ = nullptr, *dec_pos_ = nullptr;   // [V][D] embedding, [max_len][D] positional table
+  Tensor dec_ckv_;                        // cross-attention K/V of the memory, all layers [B * n_mem][L * 2 * D]
+  int build_score(int t, Program& p);
   BeamEmbed beam_embed_{};
   cudaGraphExec_t cnn_graph_ = nullptr, enc_graph_ = nullptr, step_graph_ = nullptr, loop_graph_ = nullptr;
   std::vector<DecGroup> groups_;          // decoder groups (empty: the whole batch is one chain)

@@ -193,4 +193,26 @@ int sample_set_attributes();
 int launch_sample_init(const SampleState& st, int* anc, cudaStream_t s);
 int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t s);
 
+// ---- score.cu -----------------------------------------------------------------------------------
+// Caption scoring (fpnmt_score, include/fpnmt.h): row r = c * t + j is position j of caption c = b * N + n.
+struct ScoreArgs {
+  int caps, t, V;            // captions (B * N), positions per caption, vocab
+  int start_id, end_id;
+  const int* ids;            // [caps][t] caption tokens (no <start>, no <end>)
+  const int* lens;           // [caps]
+  int* tgt;                  // [caps * t] target id of each row (written by score_embed)
+  int* bad;                  // [caps] 1: length outside [0, t] or an id outside [0, V) among the first len
+  float* tok_lp;             // [caps * t] log_softmax(z)[target]
+  float* lp;                 // [caps] sum over the scored positions
+};
+// x[r] = emb[input token] + pos[j] (input: <start> at j = 0, else ids[c][j - 1] clamped to [0, V)), tgt, bad
+int launch_score_embed(const ScoreArgs& a, const float* emb, const float* pos, Act x, cudaStream_t s);
+// causal self-attention of every caption over its own t positions: qkv [caps * t][3d] (q | k | v) -> out [caps * t][d]
+// (fp32 CUDA-core arithmetic on bf16 or split bf16x3 operands)
+int launch_score_self_attention(Act qkv, int caps, int t, int heads, Act out, cudaStream_t s);
+// tok_lp[i] = log_softmax(logits[i])[tgt[i]] for i < rows, fp32 logits [rows][V]
+int launch_score_rows(const float* logits, int rows, int V, const int* tgt, float* tok_lp, cudaStream_t s);
+// lp[c] = sum of tok_lp over the scored positions of caption c; 0 after them; NaN everywhere for a flagged caption
+int launch_score_sum(const ScoreArgs& a, cudaStream_t s);
+
 }  // namespace fpnmt

@@ -85,6 +85,7 @@ SIGNATURES = {
     "fpnmt_op_layernorm_rows": (_i, [_i, _i, _vp, _i, _vp, _vp, C.c_float, _vp, _vp]),
     "fpnmt_sample": (_i, [_vp, _vp, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _i, _i, _vp]),
     "fpnmt_op_sample_step": (_i, [_i, _vp, _i, _i, _i, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _vp]),
+    "fpnmt_score": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp]),
 }
 
 
@@ -115,6 +116,7 @@ SIGNATURES.update({
     "fpnmt_decode_attention_dl": (_i, [_vp, _dlp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_generate_dl": (_i, [_vp, _dlp, _dlp, _dlp, _i, _dlp, _vp]),
     "fpnmt_sample_dl": (_i, [_vp, _dlp, C.POINTER(FpnmtSampling), _dlp, _dlp, _dlp, _i, _vp]),
+    "fpnmt_score_dl": (_i, [_vp, _dlp, _dlp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_comm_unique_id": (_i, [_vp]),
     "fpnmt_comm_create": (_i, [_i, _i, _vp, _i, C.POINTER(_vp)]),
     "fpnmt_comm_destroy": (_i, [_vp]),

@@ -249,6 +249,31 @@ class Engine:
                                          _stream_ptr(self.device)))
         return (ids, lens, lp) if return_logprobs else (ids, lens)
 
+    def score(self, ids, lens, images=None, *, to_host: bool = True, return_token_logprobs: bool = False):
+        """Log-likelihoods of `beam` given captions per image in one teacher-forced pass (fpnmt_score; definition in
+        include/fpnmt.h): ids (B, N, t) int32 in the layout `sample` returns (no <start>, no <end>, 1 <= t <= max_len;
+        `sample`'s ids sliced to t fit), lens (B, N).  Position j predicts ids[..., j] for j < len and <end> at j = len
+        when len < t.  images None = the memory of the last encode / generate / sample.  Returns the captions'
+        log-likelihoods (B, N) float32 and, with return_token_logprobs, the per-position terms (B, N, t), 0 past each
+        caption's scored positions; NaN for a caption with len outside [0, t] or an id outside [0, vocab)."""
+        B, N = self.batch, self.beam
+        tok = _as_cuda(ids, torch.int32, self.device)
+        ln = _as_cuda(lens, torch.int32, self.device)
+        if tok.dim() != 3 or tuple(tok.shape[:2]) != (B, N) or tuple(ln.shape) != (B, N):
+            raise ValueError("score: ids must be (%d, %d, t) and lens (%d, %d), got %s and %s"
+                             % (B, N, B, N, tuple(tok.shape), tuple(ln.shape)))
+        t = int(tok.shape[2])
+        ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
+        if to_host:
+            lp = torch.empty((B, N), dtype=torch.float32).pin_memory()
+            tl = torch.empty((B, N, t), dtype=torch.float32).pin_memory() if return_token_logprobs else None
+        else:
+            lp = torch.empty((B, N), dtype=torch.float32, device=self.device)
+            tl = torch.empty((B, N, t), dtype=torch.float32, device=self.device) if return_token_logprobs else None
+        _lib.check(self.lib.fpnmt_score(self._h, ptr, on_host, tok.data_ptr(), ln.data_ptr(), t, lp.data_ptr(),
+                                        tl.data_ptr() if tl is not None else None, int(to_host), _stream_ptr(self.device)))
+        return (lp, tl) if return_token_logprobs else lp
+
     def stage(self, host_images, slot: int):
         """Enqueue the host->device copy of one batch into staging slot 0/1 on the engine's copy stream (returns at once).
         Returns the host tensor actually handed to the copy; keep it alive until the matching generate_staged is done."""

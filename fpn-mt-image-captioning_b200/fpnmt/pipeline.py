@@ -87,6 +87,37 @@ class Pipeline:
                          return_logprobs=return_logprobs)
         return tuple(o.numpy() for o in out)
 
+    def score_batch(self, imgs, captions, max_seq_len: Optional[int] = None, *, return_token_logprobs: bool = False):
+        """Log-likelihoods of given captions (Engine.score): imgs (B,S,S,3) float32 in [-1,1], captions B lists of N strings
+        (N the same for every image).  Each caption is tokenized with `tokenizer`; a leading <start> and a trailing <end>
+        are dropped.  The pass runs over t = min(longest caption + 1, max_seq_len) positions; a caption longer than
+        max_seq_len tokens raises ValueError.  Returns (B,N) float32 numpy, plus the per-position terms (B,N,t) with
+        return_token_logprobs."""
+        T = max_seq_len or self.max_seq_len
+        if len({len(c) for c in captions}) != 1:
+            raise ValueError("score_batch: every image needs the same number of captions")
+        start, end = self.tokenizer.word_index["<start>"], self.tokenizer.word_index["<end>"]
+        seqs = []
+        for caps in captions:
+            for seq in self.tokenizer.texts_to_sequences(caps):
+                if seq and seq[0] == start:
+                    seq = seq[1:]
+                if seq and seq[-1] == end:
+                    seq = seq[:-1]
+                if len(seq) > T:
+                    raise ValueError("score_batch: a caption of %d tokens exceeds max_seq_len = %d" % (len(seq), T))
+                seqs.append(seq)
+        B, N = len(captions), len(captions[0])
+        t = min(max(len(q) for q in seqs) + 1, T)
+        ids = np.zeros((B * N, t), np.int32)
+        for i, q in enumerate(seqs):
+            ids[i, :len(q)] = q
+        lens = np.array([len(q) for q in seqs], np.int32).reshape(B, N)
+        imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
+        eng = self.transformer.engine(B, N, T)
+        out = eng.score(ids.reshape(B, N, t), lens, imgs, return_token_logprobs=return_token_logprobs)
+        return tuple(o.numpy() for o in out) if return_token_logprobs else out.numpy()
+
     def predict(self, img, max_seq_len, plot_layer=False):
         """pipeline.py:82-154: img (H,W,3) -> (1-D int32 ids without <start>/<end>, attention_weights).
         attention_weights is None unless `plot_layer` is truthy; then it is the dict of the reference's last forward pass for

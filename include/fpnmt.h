@@ -207,6 +207,28 @@ FPNMT_API int fpnmt_sample(fpnmt_handle* h, const float* images, int images_on_h
                            int32_t* out_ids, int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
                            void* stream);
 
+/* Caption scoring: the log-likelihood of N = beam given captions per image, all positions in one teacher-forced decoder pass
+ * (no reference counterpart).  ids DEVICE int32 [batch][beam][t], 1 <= t <= max_len; lens DEVICE int32 [batch][beam].  Row
+ * (b, n) is caption n of image b in the layout fpnmt_sample returns: no <start>, no <end>, entries from position len on
+ * ignored.
+ *   decoder input at position j: <start> for j = 0, else ids[b][n][j-1];
+ *   target at position j: ids[b][n][j] for j < len, and <end> at j = len when len < t;
+ *   scored positions n_bn = len + 1 when len < t; when len == t, t positions and no <end> term (a truncated caption, as a
+ *   sample whose len == max_len).
+ * out_token_logprob[b][n][j] = log_softmax(z_j)[target_j] (temperature 1, no filtering) for j < n_bn, exactly 0 beyond;
+ * out_logprob[b][n] = the sum of those terms in position order.  Scoring a caption fpnmt_sample produced gives that
+ * sample's out_logprob (up to the precision of the two passes).  Position j attends to positions <= j of its caption and to
+ * the memory tokens of its image: the memory of the last fpnmt_encode / fpnmt_generate / fpnmt_sample, or of `images` when
+ * given.  A caption with len outside [0, t], or with an id outside [0, vocab) among its first len entries, gets NaN in both
+ * outputs; ids are clamped before any load and the host never reads ids / lens.  out_logprob float32 [batch][beam],
+ * out_token_logprob float32 [batch][beam][t] or NULL, both on the host (outputs_on_host != 0; the call synchronises the
+ * stream) or both on the device.  Results are bit-identical run to run, with graphs on or off, under any permutation of the
+ * captions among the N slots of an image and for any contents of ids at positions >= len.  The pass leaves nothing behind
+ * that changes a later fpnmt_generate / fpnmt_sample.  Errors: FPNMT_ERR_INVALID for t outside [1, max_len] or NULL ids /
+ * lens / out_logprob; FPNMT_ERR_STATE with decode_path = FUSED or while lane 0 holds a submitted batch. */
+FPNMT_API int fpnmt_score(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* ids, const int32_t* lens, int t,
+                          float* out_logprob, float* out_token_logprob, int outputs_on_host, void* stream);
+
 /* Replaces: Pipeline.predict (utils/pipeline.py:82-154) for a batch: encoder + beam-search decode.
  * out_ids DEVICE-or-HOST int32 [batch, max_len] (0 padded), out_len int32 [batch]: exactly what predict() returns
  * per image (<start> stripped, trailing <end> stripped).  outputs_on_host != 0: results are copied to host and

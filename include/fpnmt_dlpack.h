@@ -68,6 +68,11 @@ FPNMT_API int fpnmt_generate_dl(fpnmt_handle* h, const DLTensor* images, DLTenso
  * synchronise the stream). */
 FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpnmt_sampling* sampling, DLTensor* out_ids,
                               DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream);
+/* fpnmt_score: images as fpnmt_encode_dl, or NULL for the memory of the last encode; ids int32 [batch, beam, t] and lens int32
+ * [batch, beam] on the GPU (t = ids' last dimension); out_logprob float32 [batch, beam] and out_token_logprob float32
+ * [batch, beam, t] or NULL, both on the GPU or both on the host (host outputs synchronise the stream). */
+FPNMT_API int fpnmt_score_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* ids, const DLTensor* lens,
+                             DLTensor* out_logprob, DLTensor* out_token_logprob, void* stream);
 
 /* ---- in-library communicator: the ONE collective of the path (SURVEY §8e) -------------------------------------------
  * Image batches shard across the GPUs of a box; the only exchange is the all-gather of the caption ids.  The library opens
