@@ -157,6 +157,16 @@ FPNMT_API int fpnmt_beam_step(fpnmt_handle* h, const float* logits, const float*
   CHECK_H(h);
   return h->eng->beam_step(logits, scores_in, parent, token, scores_out, (cudaStream_t)stream);
 }
+FPNMT_API int fpnmt_beam_step_vstats(fpnmt_handle* h, const float* stat, const float* val, const int32_t* idx, int tiles,
+                                     const float* scores_in, int32_t* parent, int32_t* token, float* scores_out, void* stream) {
+  CHECK_H(h);
+  if (!stat || !val || !idx || !scores_in || !parent || !token || !scores_out || (((uintptr_t)stat | (uintptr_t)val) & 15)) {
+    set_last_error("beam_step_vstats: NULL argument or stat / val not 16-byte aligned");
+    return FPNMT_ERR_INVALID;
+  }
+  return h->eng->beam_step(nullptr, scores_in, parent, token, scores_out, (cudaStream_t)stream, (const float2*)stat, val, idx,
+                           tiles);
+}
 FPNMT_API int fpnmt_generate(fpnmt_handle* h, const float* images, int on_host, int32_t* out_ids, int32_t* out_len,
                    int outputs_on_host, int early_stop, float* step_scores, void* stream) {
   CHECK_H(h);
@@ -310,6 +320,22 @@ FPNMT_API int fpnmt_op_preprocess(int device, const uint8_t* images_hwc, int N, 
 }
 
 // ---- stand-alone skinny-row Dense operator (tgemm) -----------------------------------------------------
+}  // extern "C"
+// Keras Dense kernel (K, F) -> the engine's [F][K] bf16 weight rows ([F][2K], hi | lo, when split)
+static std::vector<uint16_t> dense_weights(const float* kernel, int K, int F, bool split) {
+  const size_t ldw = split ? 2 * (size_t)K : (size_t)K;
+  std::vector<uint16_t> hw((size_t)F * ldw);
+  for (int k = 0; k < K; ++k)
+    for (int o = 0; o < F; ++o) {
+      const float f = kernel[(size_t)k * F + o];
+      const uint16_t hi = f2bf_host(f);
+      hw[(size_t)o * ldw + k] = hi;
+      if (split) hw[(size_t)o * ldw + K + k] = f2bf_host(f - bf2f_host(hi));
+    }
+  return hw;
+}
+extern "C" {
+
 FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
                    const float* bias, int act, const float* residual, const float* gamma, const float* beta, float eps,
                    float* out, int force_bn, void* stream) {
@@ -334,15 +360,7 @@ FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, i
     set_last_error("op_dense: the wide-row kernel needs bf16 precision and a residual only together with LayerNorm");
     return FPNMT_ERR_INVALID;
   }
-  const size_t ldw = split ? 2 * (size_t)K : (size_t)K;
-  std::vector<uint16_t> hw((size_t)F * ldw);
-  for (int k = 0; k < K; ++k)
-    for (int o = 0; o < F; ++o) {
-      const float f = kernel[(size_t)k * F + o];          // Keras Dense kernel (in, out)
-      const uint16_t hi = f2bf_host(f);
-      hw[(size_t)o * ldw + k] = hi;
-      if (split) hw[(size_t)o * ldw + K + k] = f2bf_host(f - bf2f_host(hi));
-    }
+  const std::vector<uint16_t> hw = dense_weights(kernel, K, F, split);
   std::vector<void*> tmp;
   auto dal = [&](size_t b) {
     void* p = nullptr;
@@ -787,6 +805,35 @@ FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x,
   if (!o.rc) o.rc = launch_layernorm_rows(x, rows, 512, dg, db, eps, ao, o.s);
   o.read_back(ao, rows, out);
   return o.finish("op_layernorm_rows");
+}
+
+FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                   const float* bias, float* stat, float* val, int32_t* idx, void* stream) {
+  if (precision != FPNMT_PREC_BF16)
+    return op_invalid("op_vocab_stats: the logits-free vocabulary projection is a bf16-mode kernel (the wide-row Dense kernel)");
+  if (!x || !kernel || !stat || !val || !idx || R < 1 || K < 8 || K % 8 || F < 8 || F % 8 ||
+      (((uintptr_t)stat | (uintptr_t)val | (uintptr_t)idx) & 15))
+    return op_invalid("op_vocab_stats: bad arguments (K and F multiples of 8, outputs 16-byte aligned)");
+  int rc = op_device(device, "op_vocab_stats");
+  if (rc) return rc;
+  rc = tgemmw_set_attributes();
+  if (rc) return rc;
+  int sms = 0;
+  FPNMT_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+  OpScratch o((cudaStream_t)stream, precision);
+  const std::vector<uint16_t> hw = dense_weights(kernel, K, F, false);
+  bf16* dw = (bf16*)o.alloc(hw.size() * 2);
+  const float* db = o.upload(bias, (size_t)F);
+  Act ax = o.act(R, K, K, x);
+  if (o.rc) return o.finish("op_vocab_stats");
+  cudaMemcpyAsync(dw, hw.data(), hw.size() * 2, cudaMemcpyHostToDevice, o.s);
+  // the op of the engine's beam-search chain (Engine::build_decoder, logits-free tail), writing the caller's buffers
+  const Act none{nullptr, 0, 0, 0};
+  TgemmOp op;
+  o.rc = make_tgemmw_op(&op, R, ax, dw, F, K, db, ACT_NONE, none, nullptr, 0, nullptr, nullptr, nullptr, 1e-6f, sms,
+                        (float2*)stat, val, idx);
+  if (!o.rc) o.rc = tgemm_launch(op, o.s);
+  return o.finish("op_vocab_stats");
 }
 
 FPNMT_API int fpnmt_op_sample_step(int device, const float* logits, int rows, int V, int samples_per_image, int t,

@@ -540,16 +540,29 @@ int beam_set_attributes() {   // per device (Engine::init)
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return 0;
 }
-int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+int check_beam_step(const BeamState& st, int ld) {
   if (st.N > 32 || (ld & 3)) {
     set_last_error("beam_step: beam width must be <= 32 and logits ld a multiple of 4");
     return 1;
   }
-  if (st.vs_stat) {                                         // logits-free tail: merge the vocabulary projection's candidates
+  if (st.vs_stat) {
     if (st.prob_mode || st.N > 8 || st.vs_tiles > 192 || st.vs_tiles < 1) {
       set_last_error("beam_step: the logits-free tail needs log scores, beam <= 8 and <= 192 vocabulary tiles");
       return 1;
     }
+  } else {
+    const int threads = st.V <= 16384 ? 256 : 512;
+    const int nv4 = (st.V + 4 * threads - 1) / (4 * threads);
+    if (nv4 > 32 || (size_t)nv4 * threads * 16 > 200 * 1024) {
+      set_last_error("beam_step: vocabulary too large (max 65536)");
+      return 1;
+    }
+  }
+  return 0;
+}
+int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+  if (check_beam_step(st, ld)) return 1;
+  if (st.vs_stat) {                                         // logits-free tail: merge the vocabulary projection's candidates
     size_t smem = (size_t)st.vs_tiles * 8 * 8;
     if (smem < 12288) smem = 12288;
     FPNMT_CUDA_OK(launch_k_small(k_beam_step<256>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
@@ -559,10 +572,6 @@ int launch_beam_step(const BeamState& st, const float* logits, int ld, const Bea
   const int nv4 = (st.V + 4 * threads - 1) / (4 * threads);
   size_t smem = (size_t)nv4 * threads * 16;
   if (smem < 12288) smem = 12288;                           // phase 2 keeps the N x N merge lists (values, flat ids, keys) there
-  if (nv4 > 32 || smem > 200 * 1024) {
-    set_last_error("beam_step: vocabulary too large (max 65536)");
-    return 1;
-  }
   if (threads == 256)
     FPNMT_CUDA_OK(launch_k_small(k_beam_step<256>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
   else

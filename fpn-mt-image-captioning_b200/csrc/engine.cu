@@ -1753,13 +1753,19 @@ int Engine::decode_logits(const float* memory, const int32_t* tokens, int t, flo
 }
 
 int Engine::beam_step(const float* logits, const float* scores_in, int32_t* parent, int32_t* token, float* scores_out,
-                      cudaStream_t s) {
+                      cudaStream_t s, const float2* vs_stat, const float* vs_val, const int* vs_idx, int vs_tiles) {
   if (!finalized_) return fail(FPNMT_ERR_STATE, "beam_step before finalize_weights");
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   const int R = cfg_.batch * cfg_.beam;
+  BeamState st = bs_;
+  st.vs_stat = vs_stat;
+  st.vs_val = vs_val;
+  st.vs_idx = vs_idx;
+  st.vs_tiles = vs_tiles;
+  RC(check_beam_step(st, cfg_.vocab));                     // a refused step launches nothing
   RC(launch_beam_init(bs_, 0, s));
   FPNMT_CUDA_OK(cudaMemcpyAsync(bs_.score[0], scores_in, (size_t)R * 4, cudaMemcpyDeviceToDevice, s));
-  RC(launch_beam_step(bs_, logits, cfg_.vocab, BeamEmbed{nullptr, nullptr, Act{nullptr, 0, 0, 0}, 0}, s));
+  RC(launch_beam_step(st, logits, cfg_.vocab, BeamEmbed{nullptr, nullptr, Act{nullptr, 0, 0, 0}, 0}, s));
   launches += 2;
   FPNMT_CUDA_OK(cudaMemcpyAsync(parent, bs_.parent_out, (size_t)R * 4, cudaMemcpyDeviceToDevice, s));
   FPNMT_CUDA_OK(cudaMemcpyAsync(token, bs_.token_out, (size_t)R * 4, cudaMemcpyDeviceToDevice, s));

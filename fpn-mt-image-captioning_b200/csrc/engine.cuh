@@ -69,8 +69,10 @@ class Engine {
   // [L][B][heads][t][n_mem] (step_attn_prog_; not with the fused decoder)
   int decode_logits(const float* memory, const int32_t* tokens, int t, float* logits_out, cudaStream_t s, float* hidden_out = nullptr,
                     float* self_out = nullptr, float* cross_out = nullptr);
+  // vs_stat != nullptr: the logits-free tail on the caller's softmax partials and candidates ([B*N][vs_tiles], see BeamState)
   int beam_step(const float* logits, const float* scores_in, int32_t* parent, int32_t* token, float* scores_out,
-                cudaStream_t s);
+                cudaStream_t s, const float2* vs_stat = nullptr, const float* vs_val = nullptr, const int* vs_idx = nullptr,
+                int vs_tiles = 0);
   int decode(int32_t* out_ids, int32_t* out_len, int on_host, int early_stop, float* step_scores, cudaStream_t s);
   int generate(const float* images, int on_host, int32_t* out_ids, int32_t* out_len, int out_on_host, int early_stop,
                float* step_scores, cudaStream_t s);

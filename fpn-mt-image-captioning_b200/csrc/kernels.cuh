@@ -150,6 +150,8 @@ struct BeamEmbed {
 // (last block of each image) merge N x N candidates, emit parents/tokens/scores, reorder sequences + ancestry, handle
 // <end>, write the next decoder input, advance the step counter.  Buffers are double-buffered on (step & 1).
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
+// The refusals of launch_beam_step (set_last_error + 1), for callers that must refuse before launching anything else.
+int check_beam_step(const BeamState& st, int ld);
 // Physical KV-cache reorder by beam parent (pipeline.py:134-137 applied to the cache instead of an indirection table), ALL
 // layers and both of K / V in one launch: after decode step tt = *step - 1, for every row r of the batch
 //   buf[(tt + 1) & 1][c][r][0..tt] = buf[tt & 1][c][(r / N) * N + parent[tt][r]][0..tt]      c = 0 .. ncaches - 1

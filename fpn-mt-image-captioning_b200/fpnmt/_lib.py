@@ -56,6 +56,7 @@ SIGNATURES = {
     "fpnmt_get_tap": (_i, [_vp, C.c_char_p, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "fpnmt_decode_logits": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "fpnmt_beam_step": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "fpnmt_beam_step_vstats": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "fpnmt_generate": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i, _vp, _vp]),
     "fpnmt_stage_images": (_i, [_vp, _vp, _i]),
     "fpnmt_generate_staged": (_i, [_vp, _i, _vp, _vp, _i, _i, _vp, _vp]),
@@ -69,6 +70,7 @@ SIGNATURES = {
     "fpnmt_op_preprocess": (_i, [_i, _vp, _i, _i, _i, _i, _vp, _vp]),
     "fpnmt_op_decode_jpeg": (_i, [_i, C.POINTER(_vp), C.POINTER(C.c_size_t), _i, _i, _vp, _vp, _vp]),
     "fpnmt_op_dense": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _i, _vp, _vp, _vp, C.c_float, _vp, _i, _vp]),
+    "fpnmt_op_vocab_stats": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "fpnmt_op_depthwise3x3": (_i, [_i, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
     "fpnmt_op_pool": (_i, [_i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
     "fpnmt_op_scale_shift_relu": (_i, [_i, _i, _vp, C.c_int64, _i, _i, _vp, _vp, _vp, _i, _vp]),

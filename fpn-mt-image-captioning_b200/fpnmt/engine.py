@@ -209,6 +209,25 @@ class Engine:
                                             out.data_ptr(), _stream_ptr(self.device)))
         return parent, token, out
 
+    def beam_step_vstats(self, stat, val, idx, scores) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """`beam_step` through the logits-free tail: the vocabulary projection's per-tile softmax partials stat (B*N, tiles, 2),
+        candidates val (B*N, tiles, 8) and their token ids idx (B*N, tiles, 8) int32 (what `vocab_stats` returns) instead of
+        the logits."""
+        st = _as_cuda(stat, torch.float32, self.device)
+        vl = _as_cuda(val, torch.float32, self.device)
+        ix = _as_cuda(idx, torch.int32, self.device)
+        sc = _as_cuda(scores, torch.float32, self.device)
+        rows = self.batch * self.beam
+        tiles = int(st.shape[1])
+        if st.shape != (rows, tiles, 2) or vl.shape != (rows, tiles, 8) or ix.shape != (rows, tiles, 8) or sc.shape != (rows,):
+            raise ValueError("beam_step_vstats: stat (%d, tiles, 2), val and idx (%d, tiles, 8), scores (%d,)" % (rows, rows, rows))
+        parent = torch.empty((rows,), dtype=torch.int32, device=self.device)
+        token = torch.empty((rows,), dtype=torch.int32, device=self.device)
+        out = torch.empty((rows,), dtype=torch.float32, device=self.device)
+        _lib.check(self.lib.fpnmt_beam_step_vstats(self._h, st.data_ptr(), vl.data_ptr(), ix.data_ptr(), tiles, sc.data_ptr(),
+                                                   parent.data_ptr(), token.data_ptr(), out.data_ptr(), _stream_ptr(self.device)))
+        return parent, token, out
+
     def generate(self, images, early_stop: bool = True, to_host: bool = True, return_scores: bool = False):
         """Pipeline.predict for a batch (pipeline.py:82-154): ids (B,T) int32 zero-padded, lengths (B,)."""
         ptr, on_host, keep = self._images(images)
@@ -446,6 +465,31 @@ def dense(x: torch.Tensor, kernel: np.ndarray, bias: Optional[np.ndarray] = None
                                   None if res is None else res.data_ptr(), ptr(g), ptr(be), eps, out.data_ptr(), force_bn,
                                   _stream_ptr(dev)))
     return out
+
+
+def vocab_stats(x: torch.Tensor, kernel: np.ndarray, bias: Optional[np.ndarray] = None, stat: Optional[torch.Tensor] = None,
+                val: Optional[torch.Tensor] = None, idx: Optional[torch.Tensor] = None, precision: str = "bf16"
+                ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Vocabulary projection of the logits-free decode tail (fpnmt_op_vocab_stats): x (R, K), kernel (K, F) -> per
+    (row, 128-feature tile) stat (R, ftiles, 2) = (max, sum exp(z - max)), val / idx (R, ftiles, 8) = the tile's 8 largest
+    logits and their feature ids.  stat / val / idx, when given, are updated in place and may have more than R rows: rows
+    from R on are not written."""
+    x = _dev32(x)
+    r, k = x.shape
+    kn = _host32(kernel)
+    f = kn.shape[1]
+    ft = (f + 127) // 128
+    dev = x.device
+    stat = torch.full((r, ft, 2), float("nan"), device=dev) if stat is None else stat
+    val = torch.full((r, ft, 8), float("nan"), device=dev) if val is None else val
+    idx = torch.full((r, ft, 8), -1, dtype=torch.int32, device=dev) if idx is None else idx
+    for t, n, dt, w in ((stat, "stat", torch.float32, 2), (val, "val", torch.float32, 8), (idx, "idx", torch.int32, 8)):
+        if t.dtype != dt or not t.is_contiguous() or t.device != dev or t.dim() != 3 or t.shape[0] < r or tuple(t.shape[1:]) != (ft, w):
+            raise ValueError("%s must be a contiguous %s tensor of shape (>= %d, %d, %d) on %s" % (n, dt, r, ft, w, dev))
+    b = _host32(bias)
+    _lib.check(_lib.load().fpnmt_op_vocab_stats(dev.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), r, k, _hptr(kn), f,
+                                                _hptr(b), stat.data_ptr(), val.data_ptr(), idx.data_ptr(), _stream_ptr(dev)))
+    return stat, val, idx
 
 
 # ---- stand-alone encoder bandwidth operators (kernel parity tests) --------------------------------------------------------

@@ -171,6 +171,15 @@ FPNMT_API int fpnmt_decode_attention(fpnmt_handle* h, const float* memory, const
  * outputs DEVICE int32 parent[batch*beam], token[batch*beam], float32 scores_out[batch*beam]. */
 FPNMT_API int fpnmt_beam_step(fpnmt_handle* h, const float* logits, const float* scores_in, int32_t* parent, int32_t* token,
                     float* scores_out, void* stream);
+/* fpnmt_beam_step through the logits-free decode tail: the same step with the vocabulary projection's per-tile softmax
+ * partials and candidates in place of the logits (what fpnmt_op_vocab_stats writes; the beam-search decode of the bf16 mode
+ * with the wide Dense kernels runs this kernel branch).  stat DEVICE float32 [batch*beam][tiles][2] = (max, sum exp(x - max))
+ * of the tile's valid tokens; val DEVICE float32 [batch*beam][tiles][8] the tile's 8 largest logits, descending, ties lower
+ * id first, -inf padded; idx DEVICE int32 [batch*beam][tiles][8] their token ids in [0, vocab), 0x7fffffff where padded.
+ * stat and val 16-byte aligned.  FPNMT_ERR_INVALID (nothing launched) for score_mode PROB, beam > 8 or tiles outside
+ * 1..192. */
+FPNMT_API int fpnmt_beam_step_vstats(fpnmt_handle* h, const float* stat, const float* val, const int32_t* idx, int tiles,
+                                     const float* scores_in, int32_t* parent, int32_t* token, float* scores_out, void* stream);
 
 /* Sampling parameters of fpnmt_sample / fpnmt_op_sample_step.  Row (image b, sample n) at step t, logits z (fp32, the
  * vocabulary projection):
@@ -301,6 +310,15 @@ FPNMT_API int fpnmt_op_decode_jpeg(int device, const uint8_t* const* jpegs, cons
 FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
                    const float* bias, int act, const float* residual, const float* gamma, const float* beta, float eps,
                    float* out, int force_bn, void* stream);
+/* The vocabulary projection of the logits-free decode tail (bf16 only, the wide-row Dense kernel in its softmax-partials
+ * epilogue): logits z[r, f] = x[r, :] @ kernel[:, f] + bias[f] are never stored; for every row r < R and 128-feature tile t
+ * (ftiles = ceil(F / 128)) the kernel writes stat[r][t] = (max, sum exp(z - max)) over the tile's features f < F,
+ * val[r][t][0..7] the 8 largest z, descending, ties lower f first, -inf padded, and idx[r][t][0..7] their f (0x7fffffff
+ * where padded).  x DEVICE float32 [R, K]; kernel HOST float32 (K, F); bias HOST [F] or NULL; stat / val / idx DEVICE
+ * float32 [.][ftiles][2] / float32 [.][ftiles][8] / int32 [.][ftiles][8], 16-byte aligned, written in place: rows >= R
+ * and anything else the kernel does not write keep their contents.  K and F multiples of 8; bf16x3 is FPNMT_ERR_INVALID. */
+FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                   const float* bias, float* stat, float* val, int32_t* idx, void* stream);
 
 /* Encoder bandwidth kernels one at a time (the launchers of the engine's program, which choose the kernel by precision
  * and shape exactly as the engine does).  Activations are DEVICE float32, uploaded into bf16 (or bf16x3 hi + lo)
