@@ -5,6 +5,8 @@
 //                 phase 2 (last block of each image): merge N x N candidates (ties -> lower flat index n*V+v), emit
 //                 parent/token/score, reorder token sequences and the KV-cache ancestry table by parent, handle <end>
 //                 on the top beam, write the next step's embedding+position rows, advance the device step counter.
+//                 NBEST = true (fpnmt_beam_search) differs only where an image closes: when all N beams are frozen, and
+//                 then with every beam's caption, length and score.
 //   k_kv_reorder            : physical KV-cache reorder by parent, all layers in one launch (the bandwidth-bound
 //                             alternative to the ancestry table; fpnmt_config.cache_mode = FPNMT_CACHE_PHYSICAL).
 #include "kernels.cuh"
@@ -70,7 +72,7 @@ __device__ __forceinline__ void warp_argmax(float& v, int& i) {
 //                          index n*V+v), emit parent/token/score, reorder token sequences and the KV ancestry table,
 //                          handle <end>, write the NEXT step's decoder input rows (embedding + position), and let the
 //                          last image advance the device step counter.
-template <int THREADS>
+template <int THREADS, bool NBEST = false>
 __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(BeamState st, const float* __restrict__ logits, int ld, BeamEmbed em) {
   constexpr int NW = THREADS / 32;
   extern __shared__ float4 s_row4[];                       // the row's logits (later: candidate scores), nv4*THREADS float4
@@ -509,6 +511,30 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
   BDBG(11);
   // top beam is rank 0 (scores are sorted; tf.argmax returns the first maximum) — pipeline.py:143-148
   if (warp == 0) {
+    if constexpr (NBEST) {
+      // N-best: the image is finished once all N beams are frozen (later steps only re-rank the frozen beams in the same
+      // order) or after T steps; every beam is written, in rank order, stripped of <start> and of the <end> it froze on
+      bool all_frozen = true;
+      for (int n = 0; n < N; ++n) all_frozen = all_frozen && st.fin_len[nxt][rows0 + n] > 0;
+      if (!st.done[b] && (all_frozen || t == T - 1)) {
+        for (int n = 0; n < N; ++n) {
+          const int fl = st.fin_len[nxt][rows0 + n];
+          const int len = fl > 0 ? fl - 1 : t + 1;
+          const int* res = st.seq[nxt] + (size_t)(rows0 + n) * (T + 1);
+          int* dst = st.nb.ids + (size_t)(rows0 + n) * T;
+          for (int j = lane; j < T; j += 32) dst[j] = j < len ? res[1 + j] : 0;
+          if (lane == 0) {
+            st.nb.len[rows0 + n] = len;
+            st.nb.score[rows0 + n] = st.score[nxt][rows0 + n];
+          }
+        }
+        __syncwarp();
+        if (lane == 0) {
+          st.done[b] = 1;
+          atomicAdd(st.n_done, 1);
+        }
+      }
+    } else {
     const int top_tok = s_token[0];
     // extension: the image stops when its best beam is a frozen one; its caption ends before the <end> it froze on
     const int top_fin = st.finished_mode ? st.fin_len[nxt][rows0] : 0;
@@ -522,6 +548,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
         st.done[b] = 1;
         atomicAdd(st.n_done, 1);
       }
+    }
     }
     // last image to finish advances the step counter
     if (lane == 0) {
@@ -538,6 +565,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
 int beam_set_attributes() {   // per device (Engine::init)
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return 0;
 }
 int check_beam_step(const BeamState& st, int ld) {
@@ -560,12 +589,13 @@ int check_beam_step(const BeamState& st, int ld) {
   }
   return 0;
 }
-int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+template <bool NBEST>
+static int launch_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
   if (check_beam_step(st, ld)) return 1;
   if (st.vs_stat) {                                         // logits-free tail: merge the vocabulary projection's candidates
     size_t smem = (size_t)st.vs_tiles * 8 * 8;
     if (smem < 12288) smem = 12288;
-    FPNMT_CUDA_OK(launch_k_small(k_beam_step<256>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k_small(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
     return 0;
   }
   const int threads = st.V <= 16384 ? 256 : 512;
@@ -573,10 +603,20 @@ int launch_beam_step(const BeamState& st, const float* logits, int ld, const Bea
   size_t smem = (size_t)nv4 * threads * 16;
   if (smem < 12288) smem = 12288;                           // phase 2 keeps the N x N merge lists (values, flat ids, keys) there
   if (threads == 256)
-    FPNMT_CUDA_OK(launch_k_small(k_beam_step<256>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k_small(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
   else
-    FPNMT_CUDA_OK(launch_k_small(k_beam_step<512>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k_small(k_beam_step<512, NBEST>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
   return 0;
+}
+int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+  return launch_step<false>(st, logits, ld, em, s);
+}
+int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+  if (!st.finished_mode || st.prob_mode || !st.nb.ids || !st.nb.len || !st.nb.score) {
+    set_last_error("beam_step_nbest: needs finished beams, log scores and the N-best outputs");
+    return 1;
+  }
+  return launch_step<true>(st, logits, ld, em, s);
 }
 
 // Physical KV-cache reorder (see kernels.cuh).  grid (rows, ncaches): one block streams the live span of one cache row -

@@ -287,6 +287,34 @@ FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpn
                       stream);
 }
 
+FPNMT_API int fpnmt_beam_search_dl(fpnmt_handle* h, const DLTensor* images, float length_penalty, DLTensor* out_ids,
+                                   DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream) {
+  CHECK_HDL(h);
+  const fpnmt_config& c = h->eng->config();
+  const int64_t S = c.image_size;
+  void *pi = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
+  int img_host = 0, ids_host = 0, len_host = 0, lp_host = 0;
+  int rc = 0;
+  if (images) {
+    rc = dl_check("beam_search_dl: images", images, kDLFloat, h->eng->device(), true, true, {c.batch, S, S, 3}, &pi, &img_host);
+    if (rc) return rc;
+  }
+  rc = dl_check("beam_search_dl: out_ids", out_ids, kDLInt, h->eng->device(), true, true, {c.batch, c.beam, c.max_len}, &pids,
+                &ids_host);
+  if (rc) return rc;
+  rc = dl_check("beam_search_dl: out_len", out_len, kDLInt, h->eng->device(), true, true, {c.batch, c.beam}, &plen, &len_host);
+  if (rc) return rc;
+  if (ids_host != len_host) return dl_fail("beam_search_dl: out_ids and out_len must both be host or both be device tensors");
+  if (out_logprob) {
+    rc = dl_check("beam_search_dl: out_logprob", out_logprob, kDLFloat, h->eng->device(), true, true, {c.batch, c.beam}, &plp,
+                  &lp_host);
+    if (rc) return rc;
+    if (lp_host != ids_host) return dl_fail("beam_search_dl: out_logprob must live where out_ids does");
+  }
+  return fpnmt_beam_search(h, (const float*)pi, img_host, length_penalty, (int32_t*)pids, (int32_t*)plen, (float*)plp, ids_host,
+                           early_stop, stream);
+}
+
 FPNMT_API int fpnmt_score_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* ids, const DLTensor* lens,
                              DLTensor* out_logprob, DLTensor* out_token_logprob, void* stream) {
   CHECK_HDL(h);

@@ -16,6 +16,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 
 namespace fpnmt {
 
@@ -44,6 +45,7 @@ Engine::~Engine() {
   if (step_graph_) cudaGraphExecDestroy(step_graph_);
   if (loop_graph_) cudaGraphExecDestroy(loop_graph_);
   if (sample_graph_) cudaGraphExecDestroy(sample_graph_);
+  if (nbest_graph_) cudaGraphExecDestroy(nbest_graph_);
   for (auto& kv : score_graphs_) cudaGraphExecDestroy(kv.second);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
   for (auto st : grp_streams_) cudaStreamDestroy(st);
@@ -1256,6 +1258,10 @@ int Engine::build_decoder() {
         o.idempotent = false;
         step_prog.push_back(std::move(o));
       }
+      if (Bg == B) {
+        step_beam_at_ = step_prog.size() - 1;
+        step_bsv_ = bsv;
+      }
       if (physical) {
         // KV-cache reorder by beam parent, all layers and K / V in one bandwidth-bound launch (north-star item 3)
         std::vector<const bf16*> hp(2 * 2 * L);
@@ -1924,6 +1930,66 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
   FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, ss_.ids, (size_t)R * T * 4, kind, s));
   FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, ss_.len, (size_t)R * 4, kind, s));
   if (out_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, ss_.lp, (size_t)R * 4, kind, s));
+  if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// N-best beam search.  The whole-batch step program with its beam_step op replaced by the N-best variant (same phases 1 and 2;
+// an image closes when all N beams are frozen, writing all of them).  The variant's state is a copy of the op's own (logits or
+// the logits-free partials, KV ancestry and representatives, physical reorder by parent_out all unchanged) with finished_mode
+// on, its own fin_len and its own length-penalty table, uploaded on every call: one captured graph serves every alpha and
+// bs_.lp, which generate reads, is never touched.
+int Engine::beam_search(const float* images, int on_host, float length_penalty, int32_t* out_ids, int32_t* out_len,
+                        float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
+  if (!finalized_) return fail(FPNMT_ERR_STATE, "beam_search before finalize_weights");
+  if (use_dstep_) return fail(FPNMT_ERR_STATE, "beam_search: the fused decoder has no N-best tail (use decode_path = chain)");
+  if (cfg_.score_mode == FPNMT_SCORE_PROB)
+    return fail(FPNMT_ERR_STATE, "beam_search: the length penalty and the log-likelihoods need score_mode = log");
+  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "beam_search: this lane still holds a submitted batch (call fpnmt_collect first)");
+  if (!std::isfinite(length_penalty)) return fail(FPNMT_ERR_INVALID, "beam_search: length_penalty must be finite");
+  if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "beam_search: NULL out_ids / out_len");
+  FPNMT_CUDA_OK(cudaSetDevice(dev_));
+  const int B = cfg_.batch, T = cfg_.max_len, R = B * cfg_.beam;
+  if (!nbest_bs_.nb.ids) {
+    BeamState st = step_bsv_;
+    st.finished_mode = 1;
+    st.fin_len[0] = (int*)dalloc((size_t)R * 4);
+    st.fin_len[1] = (int*)dalloc((size_t)R * 4);
+    st.lp = (const float*)dalloc((size_t)(T + 2) * 4);
+    st.nb.ids = (int*)dalloc((size_t)R * T * 4);
+    st.nb.len = (int*)dalloc((size_t)R * 4);
+    st.nb.score = (float*)dalloc((size_t)R * 4);
+    if (!st.fin_len[0] || !st.fin_len[1] || !st.lp || !st.nb.ids || !st.nb.len || !st.nb.score) return FPNMT_ERR_CUDA;
+    nbest_prog_ = step_prog_;
+    const float* lg = logits_;
+    const BeamEmbed em = beam_embed_;
+    const int V = cfg_.vocab;
+    Op& o = nbest_prog_[step_beam_at_];
+    o.name = "beam_step(n-best)";
+    o.run = [st, lg, V, em](cudaStream_t q) { return launch_beam_step_nbest(st, lg, V, em, q); };
+    nbest_bs_ = st;
+  }
+  std::vector<float> lp(T + 2);
+  for (int i = 0; i < T + 2; ++i) lp[i] = powf((5.f + (float)i) / 6.f, length_penalty);
+  if (images) RC(encode(images, on_host, nullptr, s, false));
+  FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<float*>(nbest_bs_.lp), lp.data(), lp.size() * 4, cudaMemcpyHostToDevice, s));
+  RC(launch_beam_init(nbest_bs_, 1, s));
+  launches += 1;
+  RC(run_program(dec_init_prog_, s));
+  RC(run_program(embed_prog_, s));
+  if (cfg_.use_graphs && !nbest_graph_) RC(capture(nbest_prog_, &nbest_graph_));
+  for (int t = 0; t < T; ++t) {
+    RC(launch_prog(nbest_prog_, nbest_graph_, s));
+    if (early_stop && (t % 4 == 3) && t + 1 < T) {
+      FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, nbest_bs_.n_done, 4, cudaMemcpyDeviceToHost, s));
+      FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+      if (h_pinned_[0] >= B) break;
+    }
+  }
+  const cudaMemcpyKind kind = out_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, nbest_bs_.nb.ids, (size_t)R * T * 4, kind, s));
+  FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, nbest_bs_.nb.len, (size_t)R * 4, kind, s));
+  if (out_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, nbest_bs_.nb.score, (size_t)R * 4, kind, s));
   if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
 }

@@ -84,6 +84,10 @@ class Engine {
   // as B * N * t rows of one teacher-forced pass.  images == nullptr: the memory of the last encode.
   int score(const float* images, int on_host, const int32_t* ids, const int32_t* lens, int t, float* out_logprob,
             float* out_token_logprob, int out_on_host, cudaStream_t s);
+  // N-best beam search (fpnmt_beam_search): the whole-batch step program with k_beam_step's N-best close, true-beam start,
+  // frozen finished beams and this call's length penalty.  images == nullptr: the memory of the last encode.
+  int beam_search(const float* images, int on_host, float length_penalty, int32_t* out_ids, int32_t* out_len, float* out_logprob,
+                  int out_on_host, int early_stop, cudaStream_t s);
   int profile(int iters, char* buf, size_t cap);
   int capture_groups(int T);
   int build_dstep(const Tensor& ckv, const float* d_emb, const float* d_pos);
@@ -121,6 +125,13 @@ class Engine {
   Program cnn_prog_, enc_prog_, dec_init_prog_, embed_prog_, step_prog_, step_forced_prog_;
   Program step_attn_prog_;                // step_forced_prog_ + the attention-probability launches (decode_logits with outputs)
   Program sample_prog_;                   // step_forced_prog_ + k_sample_step (sample; built on its first call)
+  // beam search: step_prog_ with its beam_step op (index step_beam_at_, state step_bsv_) replaced by the N-best step on
+  // nbest_bs_, a copy of step_bsv_ with its own fin_len, length-penalty table and the N-best outputs (built on its first call)
+  size_t step_beam_at_ = 0;
+  BeamState step_bsv_{};
+  Program nbest_prog_;
+  BeamState nbest_bs_{};
+  cudaGraphExec_t nbest_graph_ = nullptr;
   SampleState ss_{};                      // sampler state: per-row buffers allocated on the first sample call
   cudaGraphExec_t sample_graph_ = nullptr;   // sample_prog_ captured with forced_mode_ set (never step_graph_)
   // score pass: one program (and graph) per caption length t, built on its first call; activations for B * N * max_len rows

@@ -136,7 +136,17 @@ struct BeamState {
   int vs_tiles;
   int physical;              // 1: "physical" KV-cache mode - the ancestry tables stay the identity (never written here) and
                              // launch_kv_reorder moves the cache rows by beam parent after every step
+  // N-best outputs (fpnmt_beam_search; launch_beam_step_nbest, finished_mode = 1): an image closes when all N beams are frozen
+  // or at t = T - 1, and its close writes every beam, in rank order, instead of beam 0 into out_ids / out_len.
+  struct NBest {
+    int* ids;                // [B][N][T] caption of each beam, 0 padded (no <start>, no <end>)
+    int* len;                // [B][N]
+    float* score;            // [B][N] raw beam score (sum of log_softmax terms, <end> included)
+    void* unused;            // 32 bytes in all: the kernel parameters after BeamState keep their 16-byte alignment, so the
+                             // generate instantiations of k_beam_step keep their vector constant loads (same code)
+  } nb;
 };
+static_assert(sizeof(BeamState::NBest) == 32, "see BeamState::NBest::unused");
 // true_beam = 0 reproduces the reference (all beams start identical, pipeline.py:101-102); 1 starts beams 1..N-1 dead
 int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s);
 // Next-step decoder input written by the beam kernel: x[row] = emb[token] + pos[step + 1] (emb == nullptr: skip).
@@ -150,6 +160,8 @@ struct BeamEmbed {
 // (last block of each image) merge N x N candidates, emit parents/tokens/scores, reorder sequences + ancestry, handle
 // <end>, write the next decoder input, advance the step counter.  Buffers are double-buffered on (step & 1).
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
+// The same step with the N-best close (BeamState::nb): needs finished_mode and log scores.
+int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
 // The refusals of launch_beam_step (set_last_error + 1), for callers that must refuse before launching anything else.
 int check_beam_step(const BeamState& st, int ld);
 // Physical KV-cache reorder by beam parent (pipeline.py:134-137 applied to the cache instead of an indirection table), ALL

@@ -268,6 +268,28 @@ class Engine:
                                          _stream_ptr(self.device)))
         return (ids, lens, lp) if return_logprobs else (ids, lens)
 
+    def beam_search(self, images=None, *, length_penalty: float = 0.0, early_stop: bool = True, to_host: bool = True,
+                    return_logprobs: bool = False):
+        """The `beam` most likely captions per image by a true beam search with frozen finished beams (fpnmt_beam_search;
+        definition in include/fpnmt.h), ranked by log-likelihood / ((5 + n) / 6) ** length_penalty, n the scored positions.
+        images None = the memory of the last encode / generate / sample / score.  Returns ids (B, N, T) int32 zero padded
+        without <start> / <end>, in rank order, lengths (B, N) (T: truncated) and, with return_logprobs, the captions'
+        log-likelihoods (B, N) float32 (<end> included): what `score` gives for them with t = T."""
+        ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
+        B, N, T = self.batch, self.beam, self.max_len
+        if to_host:
+            ids = torch.empty((B, N, T), dtype=torch.int32).pin_memory()
+            lens = torch.empty((B, N), dtype=torch.int32).pin_memory()
+            lp = torch.empty((B, N), dtype=torch.float32).pin_memory() if return_logprobs else None
+        else:
+            ids = torch.empty((B, N, T), dtype=torch.int32, device=self.device)
+            lens = torch.empty((B, N), dtype=torch.int32, device=self.device)
+            lp = torch.empty((B, N), dtype=torch.float32, device=self.device) if return_logprobs else None
+        _lib.check(self.lib.fpnmt_beam_search(self._h, ptr, on_host, float(length_penalty), ids.data_ptr(), lens.data_ptr(),
+                                              lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
+                                              _stream_ptr(self.device)))
+        return (ids, lens, lp) if return_logprobs else (ids, lens)
+
     def score(self, ids, lens, images=None, *, to_host: bool = True, return_token_logprobs: bool = False):
         """Log-likelihoods of `beam` given captions per image in one teacher-forced pass (fpnmt_score; definition in
         include/fpnmt.h): ids (B, N, t) int32 in the layout `sample` returns (no <start>, no <end>, 1 <= t <= max_len;

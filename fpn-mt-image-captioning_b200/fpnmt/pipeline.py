@@ -87,6 +87,16 @@ class Pipeline:
                          return_logprobs=return_logprobs)
         return tuple(o.numpy() for o in out)
 
+    def beam_search_batch(self, imgs, max_seq_len: Optional[int] = None, num_beams: Optional[int] = None, *,
+                          length_penalty: float = 0.0, return_logprobs: bool = False):
+        """The `num_beams` (default: the beam width) most likely captions per image (Engine.beam_search): imgs (B,S,S,3)
+        float32 in [-1,1] -> (ids (B,num_beams,T) int32 zero padded, in rank order, lengths (B,num_beams)), plus the captions'
+        log-likelihoods (B,num_beams) with return_logprobs.  Ranking by log-likelihood / ((5 + n) / 6) ** length_penalty."""
+        imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
+        eng = self.transformer.engine(int(imgs.shape[0]), num_beams or self.beam, max_seq_len or self.max_seq_len)
+        out = eng.beam_search(imgs, length_penalty=length_penalty, early_stop=True, to_host=True, return_logprobs=return_logprobs)
+        return tuple(o.numpy() for o in out)
+
     def score_batch(self, imgs, captions, max_seq_len: Optional[int] = None, *, return_token_logprobs: bool = False):
         """Log-likelihoods of given captions (Engine.score): imgs (B,S,S,3) float32 in [-1,1], captions B lists of N strings
         (N the same for every image).  Each caption is tokenized with `tokenizer`; a leading <start> and a trailing <end>

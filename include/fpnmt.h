@@ -238,6 +238,31 @@ FPNMT_API int fpnmt_sample(fpnmt_handle* h, const float* images, int images_on_h
 FPNMT_API int fpnmt_score(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* ids, const int32_t* lens, int t,
                           float* out_logprob, float* out_token_logprob, int outputs_on_host, void* stream);
 
+/* N-best beam search: the N = beam most likely captions of every image with their log-likelihoods (no reference counterpart).
+ * Always a true beam search with frozen finished beams, whatever the handle's true_beam / finished_beams / length_penalty:
+ *   start: at t = 0 only beam 0 is alive (log-score 0, the others -inf);
+ *   a beam that emits <end> is frozen: its only candidate is itself, score unchanged;
+ *   candidates are ranked by raw / lp(n), lp(n) = ((5 + n) / 6)^length_penalty, n = tokens generated including <end> for a
+ *   frozen beam and t + 1 for a live one; ties go to the lower flat index parent * vocab + token.
+ * An image is finished when all N of its beams are frozen (nothing can change after that) or after max_len steps; early_stop
+ * != 0 ends the decode once every image is finished (the host looks every 4 steps), with identical results.
+ * out_ids int32 [batch][beam][max_len]: no <start>, no <end>, 0 from position len on.  out_len int32 [batch][beam]: len <
+ * max_len when the caption ended with <end>, max_len when it was truncated (as fpnmt_sample).  out_logprob float32
+ * [batch][beam] or NULL: the raw beam score, the sum of the log_softmax terms over min(len + 1, max_len) positions, <end>
+ * included; what fpnmt_score returns for that caption with t = max_len.  The N captions of an image come in rank order, by
+ * out_logprob / lp(min(len + 1, max_len)) descending, ties to the lower slot; they are pairwise distinct when vocab >= beam.
+ * With length_penalty = 0, row 0 is what fpnmt_generate returns on a handle created with true_beam = 1, finished_beams = 1
+ * (that decode stops when its top beam freezes, and with alpha = 0 no later beam can overtake it); with length_penalty != 0
+ * row 0 may be a longer caption that fpnmt_generate stopped too early to see.
+ * images as fpnmt_sample (NULL = the memory of the last fpnmt_encode / generate / sample / score; given images are encoded and
+ * become that memory).  Outputs DEVICE, or HOST with outputs_on_host != 0 (the call synchronises the stream).  Results are
+ * bit-identical run to run, with graphs on or off, in both cache modes and with or without FPNMT_OPT_NO_KV_SHARE; the call
+ * leaves nothing behind that changes a later fpnmt_generate / fpnmt_sample / fpnmt_score.  Errors: FPNMT_ERR_INVALID for a
+ * NaN or infinite length_penalty or NULL out_ids / out_len; FPNMT_ERR_STATE with decode_path = FUSED, score_mode = PROB or
+ * while lane 0 holds a submitted batch. */
+FPNMT_API int fpnmt_beam_search(fpnmt_handle* h, const float* images, int images_on_host, float length_penalty, int32_t* out_ids,
+                                int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop, void* stream);
+
 /* Replaces: Pipeline.predict (utils/pipeline.py:82-154) for a batch: encoder + beam-search decode.
  * out_ids DEVICE-or-HOST int32 [batch, max_len] (0 padded), out_len int32 [batch]: exactly what predict() returns
  * per image (<start> stripped, trailing <end> stripped).  outputs_on_host != 0: results are copied to host and

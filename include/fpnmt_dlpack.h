@@ -73,6 +73,11 @@ FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpn
  * [batch, beam, t] or NULL, both on the GPU or both on the host (host outputs synchronise the stream). */
 FPNMT_API int fpnmt_score_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* ids, const DLTensor* lens,
                              DLTensor* out_logprob, DLTensor* out_token_logprob, void* stream);
+/* fpnmt_beam_search: images as fpnmt_encode_dl, or NULL for the memory of the last encode; out_ids int32 [batch, beam,
+ * max_len], out_len int32 [batch, beam], out_logprob float32 [batch, beam] or NULL, all on the GPU or all on the host (host
+ * outputs synchronise the stream). */
+FPNMT_API int fpnmt_beam_search_dl(fpnmt_handle* h, const DLTensor* images, float length_penalty, DLTensor* out_ids,
+                                   DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream);
 
 /* ---- in-library communicator: the ONE collective of the path (SURVEY §8e) -------------------------------------------
  * Image batches shard across the GPUs of a box; the only exchange is the all-gather of the caption ids.  The library opens
