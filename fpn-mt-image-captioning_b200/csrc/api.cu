@@ -192,8 +192,15 @@ FPNMT_API int fpnmt_score(fpnmt_handle* h, const float* images, int images_on_ho
 FPNMT_API int fpnmt_beam_search(fpnmt_handle* h, const float* images, int images_on_host, float length_penalty, int32_t* out_ids,
                                 int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop, void* stream) {
   CHECK_H(h);
-  return h->eng->beam_search(images, images_on_host, length_penalty, out_ids, out_len, out_logprob, outputs_on_host, early_stop,
-                             (cudaStream_t)stream);
+  return h->eng->beam_search(images, images_on_host, 1, 0.f, length_penalty, out_ids, out_len, out_logprob, outputs_on_host,
+                             early_stop, (cudaStream_t)stream);
+}
+FPNMT_API int fpnmt_beam_search_diverse(fpnmt_handle* h, const float* images, int images_on_host, int beam_groups, float diversity,
+                                        float length_penalty, int32_t* out_ids, int32_t* out_len, float* out_logprob,
+                                        int outputs_on_host, int early_stop, void* stream) {
+  CHECK_H(h);
+  return h->eng->beam_search(images, images_on_host, beam_groups, diversity, length_penalty, out_ids, out_len, out_logprob,
+                             outputs_on_host, early_stop, (cudaStream_t)stream);
 }
 FPNMT_API int fpnmt_stage_images(fpnmt_handle* h, const float* host_images, int slot) {
   CHECK_H(h);

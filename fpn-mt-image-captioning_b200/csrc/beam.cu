@@ -5,8 +5,9 @@
 //                 phase 2 (last block of each image): merge N x N candidates (ties -> lower flat index n*V+v), emit
 //                 parent/token/score, reorder token sequences and the KV-cache ancestry table by parent, handle <end>
 //                 on the top beam, write the next step's embedding+position rows, advance the device step counter.
-//                 NBEST = true (fpnmt_beam_search) differs only where an image closes: when all N beams are frozen, and
-//                 then with every beam's caption, length and score.
+//                 NBEST = true (fpnmt_beam_search, fpnmt_beam_search_diverse) ranks the N x N candidates in G groups of
+//                 N / G beams with a diversity penalty (G = 1: one ranking, as above) and differs where an image closes:
+//                 when all N beams are frozen, and then with every beam's caption, length and score.
 //   k_kv_reorder            : physical KV-cache reorder by parent, all layers in one launch (the bandwidth-bound
 //                             alternative to the ancestry table; fpnmt_config.cache_mode = FPNMT_CACHE_PHYSICAL).
 #include "kernels.cuh"
@@ -16,7 +17,7 @@ namespace fpnmt {
 #define LAUNCH_CHECK() FPNMT_CUDA_OK(cudaGetLastError())
 
 
-__global__ void k_beam_init(BeamState st, int true_beam) {
+__global__ void k_beam_init(BeamState st, int true_beam, int beam_groups) {
   pdl_launch();
   pdl_wait();
   const int rows = st.B * st.N;
@@ -34,7 +35,7 @@ __global__ void k_beam_init(BeamState st, int true_beam) {
   if (i < rows) {
     const int n = i % st.N;
     float s0 = st.prob_mode ? 1.f : 0.f;
-    if (true_beam && n > 0) s0 = st.prob_mode ? 0.f : -INFINITY;
+    if (true_beam && n % (st.N / beam_groups) != 0) s0 = st.prob_mode ? 0.f : -INFINITY;   // first beam of each group alive
     st.score[0][i] = s0;
     if (st.finished_mode) st.fin_len[0][i] = 0;
     st.seq[0][(size_t)i * (st.T + 1)] = st.start_id;
@@ -43,9 +44,13 @@ __global__ void k_beam_init(BeamState st, int true_beam) {
   }
   for (size_t j = i; j < (size_t)st.B * st.T; j += (size_t)gridDim.x * blockDim.x) st.out_ids[j] = 0;
 }
-int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s) {
+int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s, int beam_groups) {
+  if (beam_groups < 1 || st.N % beam_groups) {
+    set_last_error("beam_init: beam_groups must divide the beam width");
+    return 1;
+  }
   const int rows = st.B * st.N;
-  FPNMT_CUDA_OK(launch_k(k_beam_init, dim3((rows + 255) / 256), dim3(256), 0, s, st, true_beam));
+  FPNMT_CUDA_OK(launch_k(k_beam_init, dim3((rows + 255) / 256), dim3(256), 0, s, st, true_beam, beam_groups));
   return 0;
 }
 
@@ -439,6 +444,54 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
   }
   __syncthreads();
   BDBG(8);
+  if constexpr (NBEST) {
+    // Beam groups (fpnmt_beam_search_diverse; G = 1 is the single ranking of the branch below): the new beams of group g are
+    // slots [g * M, (g + 1) * M), M = N / G, chosen in group order among the M * N candidates of the group's own rows.  A
+    // live candidate's key loses lambda * h, h = the number of new beams of groups 0 .. g-1 that are live emissions of its
+    // token; a frozen beam is never penalised and never counted.  Phase 1's top-N per row suffices: at most g * M <= N - M
+    // tokens carry a penalty and it only lowers keys, so a row's M best penalised candidates are among its N best raw ones.
+    __shared__ int s_live[32];                              // token of each new beam, -1 for a frozen one
+    const int G = (int)st.nb.groups[0];
+    const float lambda = st.nb.groups[1];
+    const int M = N / G, MN = M * N;
+    for (int g = 0; g < G; ++g) {
+      const int c0 = g * MN;
+      if (g > 0) {
+        __syncthreads();                                    // group g - 1's tokens are in s_live
+        for (int c = c0 + tid; c < c0 + MN; c += THREADS) {
+          const int f = s_ff[c];
+          if (f == 0x7fffffff || st.fin_len[cur][rows0 + c / N] > 0) continue;
+          const int tok = f - (c / N) * V;
+          int h = 0;
+          for (int m = 0; m < g * M; ++m) h += s_live[m] == tok ? 1 : 0;
+          s_key[c] = __fsub_rn(s_key[c], __fmul_rn(lambda, (float)h));
+        }
+        __syncthreads();
+      }
+      for (int c = c0 + tid; c < c0 + MN; c += THREADS) {
+        const int f = s_ff[c];
+        if (f == 0x7fffffff) continue;
+        const float v = s_fv[c], key = s_key[c];
+        int rank = 0;
+        for (int j = c0; j < c0 + MN; ++j) rank += better(s_key[j], s_ff[j], key, f) ? 1 : 0;
+        if (rank < M) {
+          const int n = g * M + rank;                       // new beam n (ties -> lower flat index within the group)
+          const int par = f / V;
+          const int tok = f - par * V;
+          const int fl = st.fin_len[cur][rows0 + par];
+          s_parent[n] = par;
+          s_token[n] = tok;
+          s_live[n] = fl > 0 ? -1 : tok;
+          st.fin_len[nxt][rows0 + n] = fl > 0 ? fl : (tok == st.end_id ? t + 1 : 0);
+          st.score[nxt][rows0 + n] = v;                     // raw: the penalty only ranks, it is never accumulated
+          st.last_tok[rows0 + n] = tok;
+          if (st.parent_out) st.parent_out[(size_t)t * st.Btot * N + rows0 + n] = par;
+          if (st.token_out) st.token_out[(size_t)t * st.Btot * N + rows0 + n] = tok;
+          if (n == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.Btot + b] = v;
+        }
+      }
+    }
+  } else {
   for (int c = tid; c < NN; c += THREADS) {
     const int f = s_ff[c];
     if (f == 0x7fffffff) continue;
@@ -460,6 +513,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       if (st.token_out) st.token_out[(size_t)t * st.Btot * N + rows0 + rank] = tok;
       if (rank == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.Btot + b] = v;
     }
+  }
   }
   __syncthreads();
   BDBG(9);
@@ -513,19 +567,35 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
   if (warp == 0) {
     if constexpr (NBEST) {
       // N-best: the image is finished once all N beams are frozen (later steps only re-rank the frozen beams in the same
-      // order) or after T steps; every beam is written, in rank order, stripped of <start> and of the <end> it froze on
+      // order) or after T steps; every beam is written, in rank order within its group, stripped of <start> and of the
+      // <end> it froze on
       bool all_frozen = true;
       for (int n = 0; n < N; ++n) all_frozen = all_frozen && st.fin_len[nxt][rows0 + n] > 0;
       if (!st.done[b] && (all_frozen || t == T - 1)) {
+        // output slot of lane n's beam: its rank within its group by score / lp(min(len + 1, T)), ties to the lower slot.
+        // This step's keys carried the diversity penalty, so for G > 1 slot order need not be that order; for G = 1 the
+        // keys are exactly the ranking's and this is the identity.
+        const int M = N / (int)st.nb.groups[0];
+        float okey = -INFINITY;
+        if (lane < N) {
+          const int fl = st.fin_len[nxt][rows0 + lane];
+          okey = __fdiv_rn(st.score[nxt][rows0 + lane], st.lp[fl > 0 ? fl : t + 1]);
+        }
+        int oslot = (lane / M) * M;
+        for (int m = 0; m < N; ++m) {
+          const float km = __shfl_sync(0xffffffffu, okey, m);
+          if (m / M == lane / M && (km > okey || (km == okey && m < lane))) ++oslot;
+        }
         for (int n = 0; n < N; ++n) {
+          const int o = rows0 + __shfl_sync(0xffffffffu, oslot, n);
           const int fl = st.fin_len[nxt][rows0 + n];
           const int len = fl > 0 ? fl - 1 : t + 1;
           const int* res = st.seq[nxt] + (size_t)(rows0 + n) * (T + 1);
-          int* dst = st.nb.ids + (size_t)(rows0 + n) * T;
+          int* dst = st.nb.ids + (size_t)o * T;
           for (int j = lane; j < T; j += 32) dst[j] = j < len ? res[1 + j] : 0;
           if (lane == 0) {
-            st.nb.len[rows0 + n] = len;
-            st.nb.score[rows0 + n] = st.score[nxt][rows0 + n];
+            st.nb.len[o] = len;
+            st.nb.score[o] = st.score[nxt][rows0 + n];
           }
         }
         __syncwarp();
@@ -611,9 +681,20 @@ static int launch_step(const BeamState& st, const float* logits, int ld, const B
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
   return launch_step<false>(st, logits, ld, em, s);
 }
+int check_beam_groups(const BeamState& st, int beam_groups, float diversity) {
+  if (beam_groups < 1 || st.N % beam_groups) {
+    set_last_error("beam_search: beam_groups must be >= 1 and divide the beam width");
+    return 1;
+  }
+  if (!(diversity >= 0.f) || diversity == INFINITY) {
+    set_last_error("beam_search: diversity must be finite and >= 0");
+    return 1;
+  }
+  return 0;
+}
 int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
-  if (!st.finished_mode || st.prob_mode || !st.nb.ids || !st.nb.len || !st.nb.score) {
-    set_last_error("beam_step_nbest: needs finished beams, log scores and the N-best outputs");
+  if (!st.finished_mode || st.prob_mode || !st.nb.ids || !st.nb.len || !st.nb.score || !st.nb.groups) {
+    set_last_error("beam_step_nbest: needs finished beams, log scores, the N-best outputs and the beam-group words");
     return 1;
   }
   return launch_step<true>(st, logits, ld, em, s);

@@ -1934,19 +1934,21 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
   return 0;
 }
 
-// N-best beam search.  The whole-batch step program with its beam_step op replaced by the N-best variant (same phases 1 and 2;
-// an image closes when all N beams are frozen, writing all of them).  The variant's state is a copy of the op's own (logits or
-// the logits-free partials, KV ancestry and representatives, physical reorder by parent_out all unchanged) with finished_mode
-// on, its own fin_len and its own length-penalty table, uploaded on every call: one captured graph serves every alpha and
-// bs_.lp, which generate reads, is never touched.
-int Engine::beam_search(const float* images, int on_host, float length_penalty, int32_t* out_ids, int32_t* out_len,
-                        float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
+// N-best and diverse beam search.  The whole-batch step program with its beam_step op replaced by the N-best variant (same
+// phase 1; phase 2 ranks the beams in beam_groups groups with the diversity penalty, and an image closes when all N beams are
+// frozen, writing all of them).  The variant's state is a copy of the op's own (logits or the logits-free partials, KV
+// ancestry and representatives, physical reorder by parent_out all unchanged) with finished_mode on, its own fin_len and its
+// own length-penalty table followed by the (beam_groups, diversity) words, uploaded on every call: one captured graph serves
+// every (G, lambda, alpha) and bs_.lp, which generate reads, is never touched.  fpnmt_beam_search is G = 1.
+int Engine::beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty,
+                        int32_t* out_ids, int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
   if (!finalized_) return fail(FPNMT_ERR_STATE, "beam_search before finalize_weights");
   if (use_dstep_) return fail(FPNMT_ERR_STATE, "beam_search: the fused decoder has no N-best tail (use decode_path = chain)");
   if (cfg_.score_mode == FPNMT_SCORE_PROB)
     return fail(FPNMT_ERR_STATE, "beam_search: the length penalty and the log-likelihoods need score_mode = log");
   if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "beam_search: this lane still holds a submitted batch (call fpnmt_collect first)");
   if (!std::isfinite(length_penalty)) return fail(FPNMT_ERR_INVALID, "beam_search: length_penalty must be finite");
+  if (check_beam_groups(step_bsv_, beam_groups, diversity)) return FPNMT_ERR_INVALID;
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "beam_search: NULL out_ids / out_len");
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   const int B = cfg_.batch, T = cfg_.max_len, R = B * cfg_.beam;
@@ -1955,11 +1957,12 @@ int Engine::beam_search(const float* images, int on_host, float length_penalty, 
     st.finished_mode = 1;
     st.fin_len[0] = (int*)dalloc((size_t)R * 4);
     st.fin_len[1] = (int*)dalloc((size_t)R * 4);
-    st.lp = (const float*)dalloc((size_t)(T + 2) * 4);
+    st.lp = (const float*)dalloc((size_t)(T + 4) * 4);     // lp[0 .. T + 1], then G and lambda (nb.groups)
     st.nb.ids = (int*)dalloc((size_t)R * T * 4);
     st.nb.len = (int*)dalloc((size_t)R * 4);
     st.nb.score = (float*)dalloc((size_t)R * 4);
     if (!st.fin_len[0] || !st.fin_len[1] || !st.lp || !st.nb.ids || !st.nb.len || !st.nb.score) return FPNMT_ERR_CUDA;
+    st.nb.groups = st.lp + T + 2;
     nbest_prog_ = step_prog_;
     const float* lg = logits_;
     const BeamEmbed em = beam_embed_;
@@ -1969,11 +1972,13 @@ int Engine::beam_search(const float* images, int on_host, float length_penalty, 
     o.run = [st, lg, V, em](cudaStream_t q) { return launch_beam_step_nbest(st, lg, V, em, q); };
     nbest_bs_ = st;
   }
-  std::vector<float> lp(T + 2);
+  std::vector<float> lp(T + 4);
   for (int i = 0; i < T + 2; ++i) lp[i] = powf((5.f + (float)i) / 6.f, length_penalty);
+  lp[T + 2] = (float)beam_groups;
+  lp[T + 3] = beam_groups > 1 ? diversity : 0.f;
   if (images) RC(encode(images, on_host, nullptr, s, false));
   FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<float*>(nbest_bs_.lp), lp.data(), lp.size() * 4, cudaMemcpyHostToDevice, s));
-  RC(launch_beam_init(nbest_bs_, 1, s));
+  RC(launch_beam_init(nbest_bs_, 1, s, beam_groups));
   launches += 1;
   RC(run_program(dec_init_prog_, s));
   RC(run_program(embed_prog_, s));

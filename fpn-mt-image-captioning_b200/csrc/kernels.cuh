@@ -142,13 +142,16 @@ struct BeamState {
     int* ids;                // [B][N][T] caption of each beam, 0 padded (no <start>, no <end>)
     int* len;                // [B][N]
     float* score;            // [B][N] raw beam score (sum of log_softmax terms, <end> included)
-    void* unused;            // 32 bytes in all: the kernel parameters after BeamState keep their 16-byte alignment, so the
+    const float* groups;     // [2] beam groups G (an integer, G divides N) and diversity lambda >= 0, uploaded per call:
+                             // the beams form G groups ranked in order with a penalty (see k_beam_step); G = 1: one ranking.
+                             // 32 bytes in all: the kernel parameters after BeamState keep their 16-byte alignment, so the
                              // generate instantiations of k_beam_step keep their vector constant loads (same code)
   } nb;
 };
-static_assert(sizeof(BeamState::NBest) == 32, "see BeamState::NBest::unused");
-// true_beam = 0 reproduces the reference (all beams start identical, pipeline.py:101-102); 1 starts beams 1..N-1 dead
-int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s);
+static_assert(sizeof(BeamState::NBest) == 32, "see BeamState::NBest::groups");
+// true_beam = 0 reproduces the reference (all beams start identical, pipeline.py:101-102); 1 starts only the first beam of
+// each of beam_groups groups of N / beam_groups beams alive (beam_groups = 1: beams 1..N-1 dead)
+int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s, int beam_groups = 1);
 // Next-step decoder input written by the beam kernel: x[row] = emb[token] + pos[step + 1] (emb == nullptr: skip).
 struct BeamEmbed {
   const float* emb;          // [V][D] fp32
@@ -160,8 +163,11 @@ struct BeamEmbed {
 // (last block of each image) merge N x N candidates, emit parents/tokens/scores, reorder sequences + ancestry, handle
 // <end>, write the next decoder input, advance the step counter.  Buffers are double-buffered on (step & 1).
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
-// The same step with the N-best close (BeamState::nb): needs finished_mode and log scores.
+// The same step with beam groups and the N-best close (BeamState::nb): needs finished_mode, log scores and nb.groups.
 int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
+// The refusals of a (beam_groups, diversity) pair for the N-best step (set_last_error + 1): G >= 1 dividing N, lambda finite
+// and >= 0.  The pair lives in device memory (nb.groups), so callers check it here before uploading it.
+int check_beam_groups(const BeamState& st, int beam_groups, float diversity);
 // The refusals of launch_beam_step (set_last_error + 1), for callers that must refuse before launching anything else.
 int check_beam_step(const BeamState& st, int ld);
 // Physical KV-cache reorder by beam parent (pipeline.py:134-137 applied to the cache instead of an indirection table), ALL

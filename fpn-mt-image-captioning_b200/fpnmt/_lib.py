@@ -89,6 +89,7 @@ SIGNATURES = {
     "fpnmt_op_sample_step": (_i, [_i, _vp, _i, _i, _i, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _vp]),
     "fpnmt_score": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp]),
     "fpnmt_beam_search": (_i, [_vp, _vp, _i, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
+    "fpnmt_beam_search_diverse": (_i, [_vp, _vp, _i, _i, C.c_float, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
 }
 
 
@@ -121,6 +122,7 @@ SIGNATURES.update({
     "fpnmt_sample_dl": (_i, [_vp, _dlp, C.POINTER(FpnmtSampling), _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_score_dl": (_i, [_vp, _dlp, _dlp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_beam_search_dl": (_i, [_vp, _dlp, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
+    "fpnmt_beam_search_diverse_dl": (_i, [_vp, _dlp, _i, C.c_float, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_comm_unique_id": (_i, [_vp]),
     "fpnmt_comm_create": (_i, [_i, _i, _vp, _i, C.POINTER(_vp)]),
     "fpnmt_comm_destroy": (_i, [_vp]),

@@ -269,12 +269,15 @@ class Engine:
         return (ids, lens, lp) if return_logprobs else (ids, lens)
 
     def beam_search(self, images=None, *, length_penalty: float = 0.0, early_stop: bool = True, to_host: bool = True,
-                    return_logprobs: bool = False):
+                    return_logprobs: bool = False, beam_groups: int = 1, diversity: float = 0.0):
         """The `beam` most likely captions per image by a true beam search with frozen finished beams (fpnmt_beam_search;
         definition in include/fpnmt.h), ranked by log-likelihood / ((5 + n) / 6) ** length_penalty, n the scored positions.
         images None = the memory of the last encode / generate / sample / score.  Returns ids (B, N, T) int32 zero padded
         without <start> / <end>, in rank order, lengths (B, N) (T: truncated) and, with return_logprobs, the captions'
-        log-likelihoods (B, N) float32 (<end> included): what `score` gives for them with t = T."""
+        log-likelihoods (B, N) float32 (<end> included): what `score` gives for them with t = T.
+        beam_groups G > 1 runs the diverse beam search instead (fpnmt_beam_search_diverse): G groups of N / G beams, each
+        group's candidates lowered by `diversity` per earlier group's beam that chose the same token at the same step.  The
+        output is group-major (beams [g * N / G, (g + 1) * N / G) are group g), rank order within a group."""
         ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
         B, N, T = self.batch, self.beam, self.max_len
         if to_host:
@@ -285,9 +288,15 @@ class Engine:
             ids = torch.empty((B, N, T), dtype=torch.int32, device=self.device)
             lens = torch.empty((B, N), dtype=torch.int32, device=self.device)
             lp = torch.empty((B, N), dtype=torch.float32, device=self.device) if return_logprobs else None
-        _lib.check(self.lib.fpnmt_beam_search(self._h, ptr, on_host, float(length_penalty), ids.data_ptr(), lens.data_ptr(),
-                                              lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
-                                              _stream_ptr(self.device)))
+        if beam_groups == 1:
+            _lib.check(self.lib.fpnmt_beam_search(self._h, ptr, on_host, float(length_penalty), ids.data_ptr(), lens.data_ptr(),
+                                                  lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
+                                                  _stream_ptr(self.device)))
+        else:
+            _lib.check(self.lib.fpnmt_beam_search_diverse(self._h, ptr, on_host, int(beam_groups), float(diversity),
+                                                          float(length_penalty), ids.data_ptr(), lens.data_ptr(),
+                                                          lp.data_ptr() if lp is not None else None, int(to_host),
+                                                          int(early_stop), _stream_ptr(self.device)))
         return (ids, lens, lp) if return_logprobs else (ids, lens)
 
     def score(self, ids, lens, images=None, *, to_host: bool = True, return_token_logprobs: bool = False):

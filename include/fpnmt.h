@@ -263,6 +263,32 @@ FPNMT_API int fpnmt_score(fpnmt_handle* h, const float* images, int images_on_ho
 FPNMT_API int fpnmt_beam_search(fpnmt_handle* h, const float* images, int images_on_host, float length_penalty, int32_t* out_ids,
                                 int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop, void* stream);
 
+/* Diverse beam search (Vijayakumar et al., "Diverse Beam Search"): N = beam captions per image in G = beam_groups groups of
+ * N / G beams, each group a true beam search of width N / G that is pushed away from the tokens the earlier groups chose at
+ * the same step.  It is fpnmt_beam_search with these changes (lambda = diversity):
+ *   groups: G divides N; beam slot n belongs to group n / (N / G).
+ *   start: at t = 0 the first beam of every group is alive (log-score 0), the others are -inf.
+ *   step t: for g = 0 .. G-1 in order, group g's N / G new beams are chosen from the candidates of group g's own rows only.
+ *     A live candidate (parent p, token v) has raw = score[p] + log_softmax(z_p)[v] and ranking key
+ *     raw / lp(t + 1) - lambda * h_g(v), h_g(v) the number of new beams of groups 0 .. g-1 at this step that are live
+ *     emissions of v (<end> counts like any token).  A frozen beam's only candidate is itself, key raw / lp(fin_len), never
+ *     penalised and never counted in h.  Ties go to the lower flat index parent * vocab + token within the group.  The key
+ *     is computed in fp32 as __fsub_rn(__fdiv_rn(raw, lp), __fmul_rn(lambda, (float)h)), without contraction.
+ *   stored score: raw; the penalty is never accumulated, so out_logprob is the caption's log-likelihood and fpnmt_score of a
+ *     returned caption gives it back.
+ *   close: unchanged (all N beams frozen, or max_len steps; early_stop as fpnmt_beam_search).
+ *   output order: group-major, slots [g * N / G, (g + 1) * N / G) hold group g; within a group by
+ *     out_logprob / lp(min(len + 1, max_len)) descending, ties to the lower slot (the last step's keys carried the penalty,
+ *     so the close sorts).
+ * Captions are pairwise distinct within a group (vocab >= beam); across groups they may repeat: with lambda = 0 every group
+ * holds the same list, that of fpnmt_beam_search at width N / G.  G = 1 is fpnmt_beam_search bit for bit (lambda ignored).
+ * Outputs, images, determinism and what the call leaves behind as fpnmt_beam_search.  Errors: FPNMT_ERR_INVALID (nothing
+ * launched) for G < 1, G not dividing beam, a negative, NaN or infinite diversity, a NaN or infinite length_penalty or NULL
+ * out_ids / out_len; FPNMT_ERR_STATE as fpnmt_beam_search (decode_path = FUSED, score_mode = PROB, lane 0 busy). */
+FPNMT_API int fpnmt_beam_search_diverse(fpnmt_handle* h, const float* images, int images_on_host, int beam_groups, float diversity,
+                                        float length_penalty, int32_t* out_ids, int32_t* out_len, float* out_logprob,
+                                        int outputs_on_host, int early_stop, void* stream);
+
 /* Replaces: Pipeline.predict (utils/pipeline.py:82-154) for a batch: encoder + beam-search decode.
  * out_ids DEVICE-or-HOST int32 [batch, max_len] (0 padded), out_len int32 [batch]: exactly what predict() returns
  * per image (<start> stripped, trailing <end> stripped).  outputs_on_host != 0: results are copied to host and

@@ -78,6 +78,10 @@ FPNMT_API int fpnmt_score_dl(fpnmt_handle* h, const DLTensor* images, const DLTe
  * outputs synchronise the stream). */
 FPNMT_API int fpnmt_beam_search_dl(fpnmt_handle* h, const DLTensor* images, float length_penalty, DLTensor* out_ids,
                                    DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream);
+/* fpnmt_beam_search_diverse: tensors and checks as fpnmt_beam_search_dl. */
+FPNMT_API int fpnmt_beam_search_diverse_dl(fpnmt_handle* h, const DLTensor* images, int beam_groups, float diversity,
+                                           float length_penalty, DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob,
+                                           int early_stop, void* stream);
 
 /* ---- in-library communicator: the ONE collective of the path (SURVEY §8e) -------------------------------------------
  * Image batches shard across the GPUs of a box; the only exchange is the all-gather of the caption ids.  The library opens

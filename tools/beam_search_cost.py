@@ -1,15 +1,16 @@
-"""Cost of the N-best beam search at the C2 size (ResNet-50-FPN 512x512, batch 64, beam 8, T = 64, V = 10000, 6 layers,
-bf16, synthetic weights, fixed length).
+"""Cost of the N-best and the diverse beam search at the C2 size (ResNet-50-FPN 512x512, batch 64, beam 8, T = 64, V = 10000,
+6 layers, bf16, synthetic weights, fixed length).
 
     python tools/beam_search_cost.py [--reps 10] [--out result.json]
 
 For the default kernels and for opts=("tgemm_wide",) (the logits-free decode tail), on an engine created with true_beam=1,
 finished_beams=1 (the beam semantics Engine.beam_search always runs):
-1. Engine.beam_search against Engine.generate (both from the images, early_stop=False, device outputs): CUDA events on the
-   launching stream, the two calls alternated, median over --reps.
-2. The beam_step op of both: k_beam_step's kernel time from torch.profiler (CUDA activity, mean over the T launches of one
-   call of each, in a run of its own after the timed one).  generate runs the <.., false> instantiation, beam_search the
-   <.., true> one; they differ only in what the close of an image writes.
+1. Engine.beam_search, Engine.beam_search(beam_groups=G, diversity=0.5) for G = 2, 4, 8 and Engine.generate (all from the
+   images, early_stop=False, device outputs): CUDA events on the launching stream, the calls alternated, median over --reps.
+2. The beam_step op of each: k_beam_step's kernel time from torch.profiler (CUDA activity, mean over the T launches of one
+   call of each, in a run of its own after the timed one).  generate runs the <.., false> instantiation, the searches the
+   <.., true> one; that one ranks the candidates of each image in G sequential group rankings and writes every beam at the
+   close.
 
 The card's name and power limit are read in the same run and printed with the numbers.
 """
@@ -56,6 +57,9 @@ def main():
                      finished_beams=True)
         calls = {"generate": lambda: eng.generate(img, early_stop=False, to_host=False),
                  "beam_search": lambda: eng.beam_search(img, early_stop=False, to_host=False, return_logprobs=True)}
+        for G in (2, 4, 8):
+            calls["diverse_G%d" % G] = (lambda G=G: eng.beam_search(img, early_stop=False, to_host=False, return_logprobs=True,
+                                                                     beam_groups=G, diversity=0.5))
         for f in calls.values():       # warm-up: module loads, graph capture, first-touch of the buffers
             f()
         torch.cuda.synchronize()
