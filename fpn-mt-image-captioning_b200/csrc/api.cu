@@ -1,6 +1,5 @@
 // extern "C" surface of libfpnmt.so (see include/fpnmt.h).
 #include <stdlib.h>
-#include <string.h>
 
 #include <new>
 #include <vector>
@@ -18,12 +17,6 @@ bool pdl_small_enabled() { return g_pdl_mode == 1; }
 }  // namespace fpnmt
 
 using namespace fpnmt;
-
-struct fpnmt_handle {
-  Engine* eng;                   // lane 0: every single-batch entry point runs here
-  std::vector<Engine*> lanes;    // lanes[0] == eng; fpnmt_submit / fpnmt_collect address the others
-  cudaEvent_t last_encode = nullptr;   // encoder-done event of the most recent fpnmt_submit (owned by that lane)
-};
 
 extern "C" {
 
@@ -75,12 +68,6 @@ FPNMT_API int fpnmt_destroy(fpnmt_handle* h) {
   delete h;
   return FPNMT_OK;
 }
-
-#define CHECK_H(h)                                 \
-  if (!(h) || !(h)->eng) {                         \
-    set_last_error("NULL handle");                 \
-    return FPNMT_ERR_INVALID;                      \
-  }
 
 FPNMT_API int fpnmt_set_weight(fpnmt_handle* h, const char* key, const float* data, const int64_t* shape, int ndim) {
   CHECK_H(h);
@@ -227,101 +214,6 @@ FPNMT_API int64_t fpnmt_launch_count(fpnmt_handle* h) {
   return n;
 }
 
-// ---- stand-alone convolution operator -----------------------------------------------------------------
-static inline uint16_t f2bf_host(float f) {
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return 0x7fc0;
-  u += 0x7fffu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
-}
-static inline float bf2f_host(uint16_t h) {
-  uint32_t u = (uint32_t)h << 16;
-  float f;
-  memcpy(&f, &u, 4);
-  return f;
-}
-
-FPNMT_API int fpnmt_op_conv2d(int device, int precision, const float* x, int N, int H, int W, int Cin, const float* kernel, int kh,
-                    int kw, int Cout, int pad_top, int pad_left, const float* bias, int act, const float* residual,
-                    int res_mode, float* out, int force_bn, void* stream) {
-  cudaStream_t s = (cudaStream_t)stream;
-  if (Cin % 8) {
-    set_last_error("op_conv2d: Cin must be a multiple of 8");
-    return FPNMT_ERR_INVALID;
-  }
-  FPNMT_CUDA_OK(cudaSetDevice(device));
-  cudaDeviceProp prop;
-  FPNMT_CUDA_OK(cudaGetDeviceProperties(&prop, device));
-  if (prop.major != 10) {
-    set_last_error("op_conv2d: device is not sm_100");
-    return FPNMT_ERR_CUDA;
-  }
-  int rc = igemm_set_attributes();
-  if (rc) return rc;
-  const bool split = precision == FPNMT_PREC_BF16X3;
-  const int K = kh * kw * Cin;
-  const size_t ldw = split ? 2 * (size_t)K : (size_t)K;
-  std::vector<uint16_t> hw((size_t)Cout * ldw);
-  for (int t = 0; t < kh * kw; ++t)
-    for (int ci = 0; ci < Cin; ++ci)
-      for (int o = 0; o < Cout; ++o) {
-        const float f = kernel[((size_t)t * Cin + ci) * Cout + o];
-        const uint16_t hi = f2bf_host(f);
-        hw[(size_t)o * ldw + (size_t)t * Cin + ci] = hi;
-        if (split) hw[(size_t)o * ldw + K + (size_t)t * Cin + ci] = f2bf_host(f - bf2f_host(hi));
-      }
-  std::vector<void*> tmp;
-  auto dal = [&](size_t b) {
-    void* p = nullptr;
-    cudaMalloc(&p, b ? b : 16);
-    tmp.push_back(p);
-    return p;
-  };
-  auto cleanup = [&]() {
-    for (void* p : tmp) cudaFree(p);
-  };
-  bf16* dw = (bf16*)dal(hw.size() * 2);
-  float* dbias = nullptr;
-  if (bias) {
-    dbias = (float*)dal((size_t)(Cout + 32) * 4);
-    cudaMemsetAsync(dbias, 0, (size_t)(Cout + 32) * 4, s);
-    cudaMemcpyAsync(dbias, bias, (size_t)Cout * 4, cudaMemcpyHostToDevice, s);
-  }
-  cudaMemcpyAsync(dw, hw.data(), hw.size() * 2, cudaMemcpyHostToDevice, s);
-  auto mk = [&](size_t pix, int C) {
-    Act a;
-    const int cs = C < 8 ? 8 : (C + 7) / 8 * 8;
-    a.C = C;
-    a.ld = split ? 2 * cs : cs;
-    a.lo = split ? cs : 0;
-    a.p = (bf16*)dal(pix * a.ld * 2);
-    return a;
-  };
-  const size_t pix = (size_t)N * H * W;
-  Act ax = mk(pix, Cin), ao = mk(pix, Cout), ar{nullptr, 0, 0, 0};
-  rc = launch_f32_to_act(x, pix, Cin, ax, s);
-  if (!rc && residual) {
-    const size_t rpix = res_mode == RES_UP2 ? (size_t)N * (H / 2) * (W / 2) : pix;
-    ar = mk(rpix, Cout);
-    rc = launch_f32_to_act(residual, rpix, Cout, ar, s);
-  }
-  IgemmOp op;
-  ConvGeom g{N, H, W, Cin, Cout, kh, kw, pad_top, pad_left};
-  if (!rc)
-    rc = make_igemm_op(&op, g, ax, dw, split, dbias, act, ao, nullptr, 0, residual ? res_mode : RES_NONE, ar,
-                       prop.multiProcessorCount, force_bn);
-  if (!rc) rc = igemm_launch(op, s);
-  if (!rc) rc = launch_act_to_f32(ao, pix, out, s);
-  cudaError_t e = cudaStreamSynchronize(s);
-  cleanup();
-  if (!rc && e != cudaSuccess) {
-    set_last_error(std::string("op_conv2d: ") + cudaGetErrorString(e));
-    return FPNMT_ERR_CUDA;
-  }
-  return rc;
-}
-
 // ---- input preprocessing operator ------------------------------------------------------------------------
 FPNMT_API int fpnmt_op_preprocess(int device, const uint8_t* images_hwc, int N, int H, int W, int S, float* out, void* stream) {
   if (!images_hwc || !out || N < 1 || H < 1 || W < 1 || S < 1) {
@@ -332,104 +224,11 @@ FPNMT_API int fpnmt_op_preprocess(int device, const uint8_t* images_hwc, int N, 
   return launch_preprocess(images_hwc, N, H, W, S, out, (cudaStream_t)stream);
 }
 
-// ---- stand-alone skinny-row Dense operator (tgemm) -----------------------------------------------------
-}  // extern "C"
-// Keras Dense kernel (K, F) -> the engine's [F][K] bf16 weight rows ([F][2K], hi | lo, when split)
-static std::vector<uint16_t> dense_weights(const float* kernel, int K, int F, bool split) {
-  const size_t ldw = split ? 2 * (size_t)K : (size_t)K;
-  std::vector<uint16_t> hw((size_t)F * ldw);
-  for (int k = 0; k < K; ++k)
-    for (int o = 0; o < F; ++o) {
-      const float f = kernel[(size_t)k * F + o];
-      const uint16_t hi = f2bf_host(f);
-      hw[(size_t)o * ldw + k] = hi;
-      if (split) hw[(size_t)o * ldw + K + k] = f2bf_host(f - bf2f_host(hi));
-    }
-  return hw;
-}
-extern "C" {
-
-FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
-                   const float* bias, int act, const float* residual, const float* gamma, const float* beta, float eps,
-                   float* out, int force_bn, void* stream) {
-  cudaStream_t s = (cudaStream_t)stream;
-  if (K % 8 || F % 8) {
-    set_last_error("op_dense: K and F must be multiples of 8");
-    return FPNMT_ERR_INVALID;
-  }
-  FPNMT_CUDA_OK(cudaSetDevice(device));
-  cudaDeviceProp prop;
-  FPNMT_CUDA_OK(cudaGetDeviceProperties(&prop, device));
-  if (prop.major != 10) {
-    set_last_error("op_dense: device is not sm_100");
-    return FPNMT_ERR_CUDA;
-  }
-  int rc = tgemm_set_attributes();
-  if (!rc) rc = tgemmw_set_attributes();
-  if (rc) return rc;
-  const bool split = precision == FPNMT_PREC_BF16X3;
-  const bool wide = force_bn >= 128;          // the wide-row two-CTAs-per-SM kernel (tgemmw.cu)
-  if (wide && !tgemmw_supports(split, residual != nullptr, gamma != nullptr, F, K)) {
-    set_last_error("op_dense: the wide-row kernel needs bf16 precision and a residual only together with LayerNorm");
-    return FPNMT_ERR_INVALID;
-  }
-  const std::vector<uint16_t> hw = dense_weights(kernel, K, F, split);
-  std::vector<void*> tmp;
-  auto dal = [&](size_t b) {
-    void* p = nullptr;
-    cudaMalloc(&p, b ? b : 16);
-    tmp.push_back(p);
-    return p;
-  };
-  bf16* dw = (bf16*)dal(hw.size() * 2);
-  cudaMemcpyAsync(dw, hw.data(), hw.size() * 2, cudaMemcpyHostToDevice, s);
-  auto upl = [&](const float* h, int n) {
-    float* d = (float*)dal((size_t)(n + 128) * 4);
-    cudaMemsetAsync(d, 0, (size_t)(n + 128) * 4, s);
-    cudaMemcpyAsync(d, h, (size_t)n * 4, cudaMemcpyHostToDevice, s);
-    return d;
-  };
-  float* dbias = bias ? upl(bias, F) : nullptr;
-  float* dg = gamma ? upl(gamma, F) : nullptr;
-  float* db = beta ? upl(beta, F) : nullptr;
-  auto mk = [&](size_t rows, int C) {
-    Act a;
-    a.C = C;
-    a.ld = split ? 2 * C : C;
-    a.lo = split ? C : 0;
-    a.p = (bf16*)dal(rows * a.ld * 2);
-    return a;
-  };
-  Act ax = mk(R, K), ao = mk(R, F), ar{nullptr, 0, 0, 0};
-  rc = launch_f32_to_act(x, R, K, ax, s);
-  if (!rc && residual) {
-    ar = mk(R, F);
-    rc = launch_f32_to_act(residual, R, F, ar, s);
-  }
-  TgemmOp op;
-  if (!rc && wide)
-    rc = make_tgemmw_op(&op, R, ax, dw, F, K, dbias, act, ao, nullptr, 0, residual ? &ar : nullptr, dg, db, eps, prop.multiProcessorCount);
-  else if (!rc)
-    rc = make_tgemm_op(&op, R, ax, dw, F, K, split, dbias, act, ao, nullptr, 0, residual ? &ar : nullptr, dg, db, eps,
-                       prop.multiProcessorCount, force_bn);
-  if (!rc) rc = tgemm_launch(op, s);
-  if (!rc) rc = launch_act_to_f32(ao, R, out, s);
-  cudaError_t e = cudaStreamSynchronize(s);
-  for (void* p : tmp) cudaFree(p);
-  if (!rc && e != cudaSuccess) {
-    set_last_error(std::string("op_dense: ") + cudaGetErrorString(e));
-    return FPNMT_ERR_CUDA;
-  }
-  return rc;
-}
-
 }  // extern "C"
 
-// ---- stand-alone encoder bandwidth operators ------------------------------------------------------------
+// ---- stand-alone operators ------------------------------------------------------------------------------
 // Each one uploads fp32 tensors into activations of the requested precision, calls the engine's launcher (which picks the
-// kernel exactly as the engine's program does) and reads the result back.  A tensor of `ld` channels per pixel is one
-// activation of ld channels; the operator sees its first C channels, as through Engine::chan_view.  The output tensor
-// is uploaded too, so columns the kernel must not touch come back unchanged.
+// kernel exactly as the engine's program does) and reads the result back.
 namespace {
 struct OpScratch {
   cudaStream_t s;
@@ -451,12 +250,12 @@ struct OpScratch {
     tmp.push_back(p);
     return p;
   }
-  // host fp32 [n] -> device, zero-padded so that 16-byte vector loads at the end stay inside the allocation
-  const float* upload(const float* h, size_t n) {
+  // host fp32 [n] -> device, zero-padded by `pad` floats so that 16-byte vector loads at the end stay inside the allocation
+  const float* upload(const float* h, size_t n, size_t pad = 32) {
     if (!h) return nullptr;
-    float* d = (float*)alloc((n + 32) * 4);
+    float* d = (float*)alloc((n + pad) * 4);
     if (!d) return nullptr;
-    cudaMemsetAsync(d, 0, (n + 32) * 4, s);
+    cudaMemsetAsync(d, 0, (n + pad) * 4, s);
     cudaMemcpyAsync(d, h, n * 4, cudaMemcpyHostToDevice, s);
     return d;
   }
@@ -514,9 +313,95 @@ bool all_in(const int* v, size_t n, int lo, int hi) {
     if (v[i] < lo || v[i] >= hi) return false;
   return true;
 }
+// Keras Dense kernel (K, F) -> the engine's [F][K] bf16 weight rows ([F][2K], hi | lo, when split)
+std::vector<uint16_t> dense_weights(const float* kernel, int K, int F, bool split) {
+  const size_t ldw = split ? 2 * (size_t)K : (size_t)K;
+  std::vector<uint16_t> hw((size_t)F * ldw);
+  for (int k = 0; k < K; ++k)
+    for (int o = 0; o < F; ++o) {
+      const float f = kernel[(size_t)k * F + o];
+      const uint16_t hi = f2bf(f);
+      hw[(size_t)o * ldw + k] = hi;
+      if (split) hw[(size_t)o * ldw + K + k] = f2bf(f - bf2f(hi));
+    }
+  return hw;
+}
 }  // namespace
 
 extern "C" {
+
+// ---- convolution (igemm) and skinny-row Dense (tgemm) --------------------------------------------------------------
+FPNMT_API int fpnmt_op_conv2d(int device, int precision, const float* x, int N, int H, int W, int Cin, const float* kernel, int kh,
+                    int kw, int Cout, int pad_top, int pad_left, const float* bias, int act, const float* residual,
+                    int res_mode, float* out, int force_bn, void* stream) {
+  if (Cin % 8) return op_invalid("op_conv2d: Cin must be a multiple of 8");
+  int rc = op_device(device, "op_conv2d");
+  if (rc) return rc;
+  rc = igemm_set_attributes();
+  if (rc) return rc;
+  int sms = 0;
+  FPNMT_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+  OpScratch o((cudaStream_t)stream, precision);
+  const std::vector<uint16_t> hw = dense_weights(kernel, kh * kw * Cin, Cout, o.split);
+  bf16* dw = (bf16*)o.alloc(hw.size() * 2);
+  const float* dbias = o.upload(bias, (size_t)Cout);
+  // activations of C logical channels (channel stride rounded up to 8), filled at width C: Cout need not be a multiple of 8
+  auto act_c = [&o](size_t pix, int C, const float* src) {
+    Act a = o.act(pix, C, C < 8 ? 8 : (C + 7) / 8 * 8, nullptr);
+    if (src && !o.rc) o.rc = launch_f32_to_act(src, pix, C, a, o.s);
+    return a;
+  };
+  const size_t pix = (size_t)N * H * W;
+  const size_t rpix = res_mode == RES_UP2 ? (size_t)N * (H / 2) * (W / 2) : pix;
+  Act ax = act_c(pix, Cin, x), ao = act_c(pix, Cout, nullptr);
+  Act ar = residual ? act_c(rpix, Cout, residual) : Act{nullptr, 0, 0, 0};
+  if (o.rc) return o.finish("op_conv2d");
+  cudaMemcpyAsync(dw, hw.data(), hw.size() * 2, cudaMemcpyHostToDevice, o.s);
+  IgemmOp op;
+  ConvGeom g{N, H, W, Cin, Cout, kh, kw, pad_top, pad_left};
+  o.rc = make_igemm_op(&op, g, ax, dw, o.split, dbias, act, ao, nullptr, 0, residual ? res_mode : RES_NONE, ar, sms, force_bn);
+  if (!o.rc) o.rc = igemm_launch(op, o.s);
+  if (!o.rc) o.rc = launch_act_to_f32(ao, pix, out, o.s);
+  return o.finish("op_conv2d");
+}
+
+FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                   const float* bias, int act, const float* residual, const float* gamma, const float* beta, float eps,
+                   float* out, int force_bn, void* stream) {
+  if (K % 8 || F % 8) return op_invalid("op_dense: K and F must be multiples of 8");
+  int rc = op_device(device, "op_dense");
+  if (rc) return rc;
+  rc = tgemm_set_attributes();
+  if (!rc) rc = tgemmw_set_attributes();
+  if (rc) return rc;
+  const bool wide = force_bn >= 128;          // the wide-row two-CTAs-per-SM kernel (tgemmw.cu)
+  if (wide && !tgemmw_supports(precision == FPNMT_PREC_BF16X3, residual != nullptr, gamma != nullptr, F, K))
+    return op_invalid("op_dense: the wide-row kernel needs bf16 precision and a residual only together with LayerNorm");
+  int sms = 0;
+  FPNMT_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+  OpScratch o((cudaStream_t)stream, precision);
+  const std::vector<uint16_t> hw = dense_weights(kernel, K, F, o.split);
+  bf16* dw = (bf16*)o.alloc(hw.size() * 2);
+  // the tgemm epilogues read bias, gamma and beta in whole 128-feature tiles
+  const float *dbias = o.upload(bias, (size_t)F, 128), *dg = o.upload(gamma, (size_t)F, 128), *db = o.upload(beta, (size_t)F, 128);
+  Act ax = o.act(R, K, K, x), ao = o.act(R, F, F, nullptr);
+  Act ar = residual ? o.act(R, F, F, residual) : Act{nullptr, 0, 0, 0};
+  if (o.rc) return o.finish("op_dense");
+  cudaMemcpyAsync(dw, hw.data(), hw.size() * 2, cudaMemcpyHostToDevice, o.s);
+  TgemmOp op;
+  if (wide)
+    o.rc = make_tgemmw_op(&op, R, ax, dw, F, K, dbias, act, ao, nullptr, 0, residual ? &ar : nullptr, dg, db, eps, sms);
+  else
+    o.rc = make_tgemm_op(&op, R, ax, dw, F, K, o.split, dbias, act, ao, nullptr, 0, residual ? &ar : nullptr, dg, db, eps, sms,
+                         force_bn);
+  if (!o.rc) o.rc = tgemm_launch(op, o.s);
+  o.read_back(ao, R, out);
+  return o.finish("op_dense");
+}
+
+// ---- encoder bandwidth operators -----------------------------------------------------------------------------------
+// A tensor of `ld` channels per pixel is one activation of ld channels; the operator sees its first C channels, as through
+// Engine::chan_view.  The output tensor is uploaded too, so columns the kernel must not touch come back unchanged.
 
 FPNMT_API int fpnmt_op_depthwise3x3(int device, int precision, const float* x, int N, int H, int W, int C, int in_ld,
                                     const float* kernel, const float* bias, int stride, int pad_top, int pad_left, int Ho,
@@ -854,8 +739,7 @@ FPNMT_API int fpnmt_op_sample_step(int device, const float* logits, int rows, in
   if (!logits || !sampling || !token || rows < 1 || V < 1 || V > 51200 || samples_per_image < 1 || t < 0)
     return op_invalid("op_sample_step: bad arguments (rows >= 1, 1 <= V <= 51200, samples_per_image >= 1, t >= 0)");
   const fpnmt_sampling& sp = *sampling;
-  if (!(sp.temperature >= 0.f) || !(sp.top_p > 0.f && sp.top_p <= 1.f) || sp.top_k < 0 || sp.top_k > V || sp.reserved[0] ||
-      sp.reserved[1] || sp.reserved[2] || sp.reserved[3])
+  if (check_sampling(sp, V))
     return op_invalid("op_sample_step: temperature >= 0, top_p in (0, 1], 0 <= top_k <= V and reserved words 0");
   int rc = op_device(device, "op_sample_step");
   if (rc) return rc;

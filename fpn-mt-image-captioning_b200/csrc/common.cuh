@@ -6,12 +6,28 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <string.h>
 
 #include <string>
 
 namespace fpnmt {
 
 typedef __nv_bfloat16 bf16;
+
+// host bf16 conversion of weights: round-to-nearest-even, matches __float2bfloat16_rn for finite values
+inline uint16_t f2bf(float f) {
+  uint32_t u;
+  memcpy(&u, &f, 4);
+  if ((u & 0x7fffffffu) > 0x7f800000u) return 0x7fc0;
+  u += 0x7fffu + ((u >> 16) & 1u);
+  return (uint16_t)(u >> 16);
+}
+inline float bf2f(uint16_t h) {
+  uint32_t u = (uint32_t)h << 16;
+  float f;
+  memcpy(&f, &u, 4);
+  return f;
+}
 
 // ------------------------------------------------------------------------------------------------
 // error plumbing (host)

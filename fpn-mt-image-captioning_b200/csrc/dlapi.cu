@@ -10,12 +10,6 @@
 #include "../../include/fpnmt_dlpack.h"
 #include "engine.cuh"
 
-struct fpnmt_handle {          // same layout as in api.cu
-  fpnmt::Engine* eng;
-  std::vector<fpnmt::Engine*> lanes;
-  cudaEvent_t last_encode = nullptr;
-};
-
 namespace fpnmt {
 
 static int dl_fail(const std::string& m) {
@@ -120,16 +114,10 @@ struct fpnmt_comm {
 
 static_assert(sizeof(ncclUniqueId) == FPNMT_UNIQUE_ID_BYTES, "ncclUniqueId is 128 bytes");
 
-#define CHECK_HDL(h)                               \
-  if (!(h) || !(h)->eng) {                         \
-    set_last_error("NULL handle");                 \
-    return FPNMT_ERR_INVALID;                      \
-  }
-
 extern "C" {
 
 FPNMT_API int fpnmt_set_weight_dl(fpnmt_handle* h, const char* key, const DLTensor* w) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   if (!key || !w || !w->data) return dl_fail("set_weight_dl: NULL key / tensor");
   if (w->ndim < 1 || w->ndim > 4) return dl_fail(std::string("set_weight_dl(") + key + "): rank must be 1..4");
   void* p = nullptr;
@@ -141,7 +129,7 @@ FPNMT_API int fpnmt_set_weight_dl(fpnmt_handle* h, const char* key, const DLTens
 }
 
 FPNMT_API int fpnmt_encode_dl(fpnmt_handle* h, const DLTensor* images, DLTensor* memory_out, void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   const fpnmt_config& c = h->eng->config();
   const int64_t S = c.image_size, nm = (int64_t)(S / 128) * (S / 128);
   void *pi = nullptr, *pm = nullptr;
@@ -156,7 +144,7 @@ FPNMT_API int fpnmt_encode_dl(fpnmt_handle* h, const DLTensor* images, DLTensor*
 }
 
 FPNMT_API int fpnmt_features_dl(fpnmt_handle* h, const DLTensor* images, DLTensor* const out5[5], void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   const fpnmt_config& c = h->eng->config();
   const int64_t S = c.image_size;
   void* pi = nullptr;
@@ -191,9 +179,37 @@ static int forced_args(fpnmt_handle* h, const char* fn, const DLTensor* memory, 
   return 0;
 }
 
+// images of an entry point that takes NULL for the memory of the last encode: [batch][S][S][3], host or device
+static int dl_images_opt(fpnmt_handle* h, const std::string& fn, const DLTensor* images, void** ptr, int* on_host) {
+  if (!images) return 0;
+  const fpnmt_config& c = h->eng->config();
+  return dl_check((fn + ": images").c_str(), images, kDLFloat, h->eng->device(), true, true,
+                  {c.batch, c.image_size, c.image_size, 3}, ptr, on_host);
+}
+
+// N captions per image: out_ids int32 [batch][beam][max_len], out_len int32 [batch][beam] and out_logprob float32
+// [batch][beam] or NULL, all host or all device (*on_host)
+static int dl_captions(fpnmt_handle* h, const std::string& fn, DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob,
+                       void** pids, void** plen, void** plp, int* on_host) {
+  const fpnmt_config& c = h->eng->config();
+  int len_host = 0, lp_host = 0;
+  int rc = dl_check((fn + ": out_ids").c_str(), out_ids, kDLInt, h->eng->device(), true, true, {c.batch, c.beam, c.max_len}, pids,
+                    on_host);
+  if (rc) return rc;
+  rc = dl_check((fn + ": out_len").c_str(), out_len, kDLInt, h->eng->device(), true, true, {c.batch, c.beam}, plen, &len_host);
+  if (rc) return rc;
+  if (*on_host != len_host) return dl_fail(fn + ": out_ids and out_len must both be host or both be device tensors");
+  if (!out_logprob) return 0;
+  rc = dl_check((fn + ": out_logprob").c_str(), out_logprob, kDLFloat, h->eng->device(), true, true, {c.batch, c.beam}, plp,
+                &lp_host);
+  if (rc) return rc;
+  if (lp_host != *on_host) return dl_fail(fn + ": out_logprob must live where out_ids does");
+  return 0;
+}
+
 FPNMT_API int fpnmt_decode_logits_dl(fpnmt_handle* h, const DLTensor* memory, const DLTensor* tokens, DLTensor* logits_out,
                                      void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   void *pm, *pt, *po = nullptr;
   int t = 0;
   int rc = forced_args(h, "decode_logits_dl", memory, tokens, &pm, &pt, &t);
@@ -206,7 +222,7 @@ FPNMT_API int fpnmt_decode_logits_dl(fpnmt_handle* h, const DLTensor* memory, co
 
 FPNMT_API int fpnmt_decode_hidden_dl(fpnmt_handle* h, const DLTensor* memory, const DLTensor* tokens, DLTensor* hidden_out,
                                      void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   void *pm, *pt, *po = nullptr;
   int t = 0;
   int rc = forced_args(h, "decode_hidden_dl", memory, tokens, &pm, &pt, &t);
@@ -219,7 +235,7 @@ FPNMT_API int fpnmt_decode_hidden_dl(fpnmt_handle* h, const DLTensor* memory, co
 
 FPNMT_API int fpnmt_decode_attention_dl(fpnmt_handle* h, const DLTensor* memory, const DLTensor* tokens, DLTensor* self_out,
                                         DLTensor* cross_out, void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   void *pm, *pt, *ps = nullptr, *pc = nullptr;
   int t = 0;
   int rc = forced_args(h, "decode_attention_dl", memory, tokens, &pm, &pt, &t);
@@ -242,7 +258,7 @@ FPNMT_API int fpnmt_decode_attention_dl(fpnmt_handle* h, const DLTensor* memory,
 
 FPNMT_API int fpnmt_generate_dl(fpnmt_handle* h, const DLTensor* images, DLTensor* out_ids, DLTensor* out_len, int early_stop,
                                 DLTensor* step_scores, void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   const fpnmt_config& c = h->eng->config();
   const int64_t S = c.image_size;
   void *pi = nullptr, *pids = nullptr, *plen = nullptr, *psc = nullptr;
@@ -263,26 +279,12 @@ FPNMT_API int fpnmt_generate_dl(fpnmt_handle* h, const DLTensor* images, DLTenso
 
 FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpnmt_sampling* sampling, DLTensor* out_ids,
                               DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream) {
-  CHECK_HDL(h);
-  const fpnmt_config& c = h->eng->config();
-  const int64_t S = c.image_size;
+  CHECK_H(h);
   void *pi = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
-  int img_host = 0, ids_host = 0, len_host = 0, lp_host = 0;
-  int rc = 0;
-  if (images) {
-    rc = dl_check("sample_dl: images", images, kDLFloat, h->eng->device(), true, true, {c.batch, S, S, 3}, &pi, &img_host);
-    if (rc) return rc;
-  }
-  rc = dl_check("sample_dl: out_ids", out_ids, kDLInt, h->eng->device(), true, true, {c.batch, c.beam, c.max_len}, &pids, &ids_host);
+  int img_host = 0, ids_host = 0;
+  int rc = dl_images_opt(h, "sample_dl", images, &pi, &img_host);
+  if (!rc) rc = dl_captions(h, "sample_dl", out_ids, out_len, out_logprob, &pids, &plen, &plp, &ids_host);
   if (rc) return rc;
-  rc = dl_check("sample_dl: out_len", out_len, kDLInt, h->eng->device(), true, true, {c.batch, c.beam}, &plen, &len_host);
-  if (rc) return rc;
-  if (ids_host != len_host) return dl_fail("sample_dl: out_ids and out_len must both be host or both be device tensors");
-  if (out_logprob) {
-    rc = dl_check("sample_dl: out_logprob", out_logprob, kDLFloat, h->eng->device(), true, true, {c.batch, c.beam}, &plp, &lp_host);
-    if (rc) return rc;
-    if (lp_host != ids_host) return dl_fail("sample_dl: out_logprob must live where out_ids does");
-  }
   return fpnmt_sample(h, (const float*)pi, img_host, sampling, (int32_t*)pids, (int32_t*)plen, (float*)plp, ids_host, early_stop,
                       stream);
 }
@@ -292,29 +294,12 @@ FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpn
 static int beam_search_dl(const char* name, fpnmt_handle* h, const DLTensor* images, int beam_groups, float diversity,
                           float length_penalty, DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob, int early_stop,
                           void* stream) {
-  CHECK_HDL(h);
-  const fpnmt_config& c = h->eng->config();
-  const int64_t S = c.image_size;
-  const std::string n = name;
+  CHECK_H(h);
   void *pi = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
-  int img_host = 0, ids_host = 0, len_host = 0, lp_host = 0;
-  int rc = 0;
-  if (images) {
-    rc = dl_check((n + ": images").c_str(), images, kDLFloat, h->eng->device(), true, true, {c.batch, S, S, 3}, &pi, &img_host);
-    if (rc) return rc;
-  }
-  rc = dl_check((n + ": out_ids").c_str(), out_ids, kDLInt, h->eng->device(), true, true, {c.batch, c.beam, c.max_len}, &pids,
-                &ids_host);
+  int img_host = 0, ids_host = 0;
+  int rc = dl_images_opt(h, name, images, &pi, &img_host);
+  if (!rc) rc = dl_captions(h, name, out_ids, out_len, out_logprob, &pids, &plen, &plp, &ids_host);
   if (rc) return rc;
-  rc = dl_check((n + ": out_len").c_str(), out_len, kDLInt, h->eng->device(), true, true, {c.batch, c.beam}, &plen, &len_host);
-  if (rc) return rc;
-  if (ids_host != len_host) return dl_fail(n + ": out_ids and out_len must both be host or both be device tensors");
-  if (out_logprob) {
-    rc = dl_check((n + ": out_logprob").c_str(), out_logprob, kDLFloat, h->eng->device(), true, true, {c.batch, c.beam}, &plp,
-                  &lp_host);
-    if (rc) return rc;
-    if (lp_host != ids_host) return dl_fail(n + ": out_logprob must live where out_ids does");
-  }
   return fpnmt_beam_search_diverse(h, (const float*)pi, img_host, beam_groups, diversity, length_penalty, (int32_t*)pids,
                                    (int32_t*)plen, (float*)plp, ids_host, early_stop, stream);
 }
@@ -333,16 +318,12 @@ FPNMT_API int fpnmt_beam_search_diverse_dl(fpnmt_handle* h, const DLTensor* imag
 
 FPNMT_API int fpnmt_score_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* ids, const DLTensor* lens,
                              DLTensor* out_logprob, DLTensor* out_token_logprob, void* stream) {
-  CHECK_HDL(h);
+  CHECK_H(h);
   const fpnmt_config& c = h->eng->config();
-  const int64_t S = c.image_size;
   void *pi = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr, *ptok = nullptr;
   int img_host = 0, lp_host = 0, tok_host = 0;
-  int rc = 0;
-  if (images) {
-    rc = dl_check("score_dl: images", images, kDLFloat, h->eng->device(), true, true, {c.batch, S, S, 3}, &pi, &img_host);
-    if (rc) return rc;
-  }
+  int rc = dl_images_opt(h, "score_dl", images, &pi, &img_host);
+  if (rc) return rc;
   rc = dl_check("score_dl: ids", ids, kDLInt, h->eng->device(), false, true, {c.batch, c.beam, -1}, &pids, nullptr);
   if (rc) return rc;
   const int64_t t = ids->shape[2];

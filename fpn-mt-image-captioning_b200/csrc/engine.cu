@@ -46,7 +46,8 @@ Engine::~Engine() {
   if (loop_graph_) cudaGraphExecDestroy(loop_graph_);
   if (sample_graph_) cudaGraphExecDestroy(sample_graph_);
   if (nbest_graph_) cudaGraphExecDestroy(nbest_graph_);
-  for (auto& kv : score_graphs_) cudaGraphExecDestroy(kv.second);
+  for (auto& kv : score_graphs_)
+    if (kv.second) cudaGraphExecDestroy(kv.second);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
   for (auto st : grp_streams_) cudaStreamDestroy(st);
   for (auto ev : join_ev_) cudaEventDestroy(ev);
@@ -186,23 +187,10 @@ int Engine::prep_vec(const std::string& key, float** out) {
   return upload_f32(w->data, out);
 }
 
-static inline uint16_t f2bf(float f) {   // round-to-nearest-even, matches __float2bfloat16_rn for finite values
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return 0x7fc0;
-  u += 0x7fffu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
-}
 void xattn_fold_weights(const float* wq, const float* wo, uint16_t* wq_bf16, uint16_t* woT_bf16) {
   for (size_t i = 0; i < 512 * 512; ++i) wq_bf16[i] = f2bf(wq[i]);
   for (int hd = 0; hd < 512; ++hd)
     for (int f = 0; f < 512; ++f) woT_bf16[(size_t)f * 512 + hd] = f2bf(wo[(size_t)hd * 512 + f]);
-}
-static inline float bf2f(uint16_t h) {
-  uint32_t u = (uint32_t)h << 16;
-  float f;
-  memcpy(&f, &u, 4);
-  return f;
 }
 
 int Engine::upload_gemm(const std::vector<float>& wt, const std::vector<float>& bias, int Cout, int K, GemmW* out) {
@@ -1596,6 +1584,55 @@ int Engine::launch_prog(Program& p, cudaGraphExec_t g, cudaStream_t s) {
   return run_program(p, s);
 }
 
+int Engine::launch_graph(Program& p, cudaGraphExec_t& g, cudaStream_t s) {
+  if (cfg_.use_graphs && !g) RC(capture(p, &g));
+  return launch_prog(p, g, s);
+}
+
+int Engine::poll_done(const int* n_done, cudaStream_t s, bool* done) {
+  FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, n_done, 4, cudaMemcpyDeviceToHost, s));
+  FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+  *done = h_pinned_[0] >= cfg_.batch;
+  return 0;
+}
+
+// max_len replays of a step program; with early stop the host reads the finished-image counter every 4 steps and stops
+// once every image has finished
+int Engine::run_steps(Program& p, cudaGraphExec_t& g, const int* n_done, int early_stop, cudaStream_t s) {
+  const int T = cfg_.max_len;
+  for (int t = 0; t < T; ++t) {
+    RC(launch_graph(p, g, s));
+    if (early_stop && (t % 4 == 3) && t + 1 < T) {
+      bool done = false;
+      RC(poll_done(n_done, s, &done));
+      if (done) break;
+    }
+  }
+  return 0;
+}
+
+// the refusals shared by the decode modes that need the per-operator chain and the lane's own buffers
+int Engine::check_decode_entry(const char* entry, const char* fused_reason) {
+  const std::string e = entry;
+  if (!finalized_) return fail(FPNMT_ERR_STATE, e + " before finalize_weights");
+  if (use_dstep_) return fail(FPNMT_ERR_STATE, e + ": the fused decoder " + fused_reason + " (use decode_path = chain)");
+  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, e + ": this lane still holds a submitted batch (call fpnmt_collect first)");
+  return 0;
+}
+
+// result handoff: device src -> dst on the host (on_host) or the device; nothing for a NULL dst
+static int copy_out(void* dst, const void* src, size_t bytes, int on_host, cudaStream_t s) {
+  if (dst) FPNMT_CUDA_OK(cudaMemcpyAsync(dst, src, bytes, on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, s));
+  return 0;
+}
+
+// sets a flag for the guard's lifetime (forced_mode_ while a teacher-forced step program is enqueued or captured)
+struct FlagGuard {
+  bool& f;
+  explicit FlagGuard(bool& flag) : f(flag) { f = true; }
+  ~FlagGuard() { f = false; }
+};
+
 int Engine::set_images(const float* images, int on_host, cudaStream_t s) {
   const size_t n = (size_t)cfg_.batch * cfg_.image_size * cfg_.image_size * 3;
   const float* dptr = images;
@@ -1618,12 +1655,8 @@ int Engine::encode(const float* images, int on_host, float* memory_out, cudaStre
   if (!images) return fail(FPNMT_ERR_INVALID, "images is NULL");
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   RC(set_images(images, on_host, s));
-  if (cfg_.use_graphs) {
-    if (cnn_only && !cnn_graph_) RC(capture(cnn_prog_, &cnn_graph_));
-    if (!cnn_only && !enc_graph_) RC(capture(enc_prog_, &enc_graph_));
-  }
-  if (cnn_only) RC(launch_prog(cnn_prog_, cnn_graph_, s));
-  else RC(launch_prog(enc_prog_, enc_graph_, s));
+  if (cnn_only) RC(launch_graph(cnn_prog_, cnn_graph_, s));
+  else RC(launch_graph(enc_prog_, enc_graph_, s));
   if (memory_out && !cnn_only) RC(launch_act_to_f32(enc_out_.a, enc_out_.pixels(), memory_out, s));
   return 0;
 }
@@ -1730,8 +1763,7 @@ int Engine::decode_logits(const float* memory, const int32_t* tokens, int t, flo
   RC(run_program(dec_init_prog_, s));
   k_forced_init<<<(R + 255) / 256, 256, 0, s>>>(bs_, tokens, t);
   FPNMT_CUDA_OK(cudaGetLastError());
-  forced_mode_ = true;
-  struct Reset { bool& f; ~Reset() { f = false; } } reset{forced_mode_};
+  FlagGuard forced(forced_mode_);
   attn_self_ = self_out;
   attn_cross_ = cross_out;
   attn_tlen_ = t;
@@ -1797,9 +1829,9 @@ int Engine::decode(int32_t* out_ids, int32_t* out_len, int on_host, int early_st
       RC(dstep_launch(q, s));
       launches += 1;
       if (early_stop && t0 + chunk < T) {
-        FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, bs_.n_done, 4, cudaMemcpyDeviceToHost, s));
-        FPNMT_CUDA_OK(cudaStreamSynchronize(s));
-        if (h_pinned_[0] >= B) break;
+        bool done = false;
+        RC(poll_done(bs_.n_done, s, &done));
+        if (done) break;
       }
     }
   } else if (cfg_.use_graphs && !early_stop && groups_.size() > 1) {
@@ -1847,21 +1879,12 @@ int Engine::decode(int32_t* out_ids, int32_t* out_len, int on_host, int early_st
     FPNMT_CUDA_OK(cudaGraphLaunch(loop_graph_, s));
     launches += (int64_t)T * (int64_t)step_prog_.size();
   } else {
-  if (cfg_.use_graphs && !step_graph_) RC(capture(step_prog_, &step_graph_));
-  for (int t = 0; t < T; ++t) {
-    RC(launch_prog(step_prog_, step_graph_, s));
-    if (early_stop && (t % 4 == 3) && t + 1 < T) {
-      FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, bs_.n_done, 4, cudaMemcpyDeviceToHost, s));
-      FPNMT_CUDA_OK(cudaStreamSynchronize(s));
-      if (h_pinned_[0] >= B) break;
-    }
+    RC(run_steps(step_prog_, step_graph_, bs_.n_done, early_stop, s));
   }
   }
-  }
-  const cudaMemcpyKind kind = on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  if (out_ids) FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, bs_.out_ids, (size_t)B * T * 4, kind, s));
-  if (out_len) FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, bs_.out_len, (size_t)B * 4, kind, s));
-  if (step_scores) FPNMT_CUDA_OK(cudaMemcpyAsync(step_scores, step_scores_, (size_t)T * B * 4, cudaMemcpyDeviceToDevice, s));
+  RC(copy_out(out_ids, bs_.out_ids, (size_t)B * T * 4, on_host, s));
+  RC(copy_out(out_len, bs_.out_len, (size_t)B * 4, on_host, s));
+  RC(copy_out(step_scores, step_scores_, (size_t)T * B * 4, 0, s));
   if (on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
 }
@@ -1878,12 +1901,9 @@ int Engine::generate(const float* images, int on_host, int32_t* out_ids, int32_t
 // device struct the kernel reads: a captured sample_graph_ serves every parameter set.
 int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len,
                    float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
-  if (!finalized_) return fail(FPNMT_ERR_STATE, "sample before finalize_weights");
-  if (use_dstep_) return fail(FPNMT_ERR_STATE, "sample: the fused decoder has no sampling tail (use decode_path = chain)");
-  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "sample: this lane still holds a submitted batch (call fpnmt_collect first)");
+  RC(check_decode_entry("sample", "has no sampling tail"));
   const int B = cfg_.batch, N = cfg_.beam, T = cfg_.max_len, V = cfg_.vocab, R = B * N;
-  if (!(sp.temperature >= 0.f) || !(sp.top_p > 0.f && sp.top_p <= 1.f) || sp.top_k < 0 || sp.top_k > V ||
-      sp.reserved[0] || sp.reserved[1] || sp.reserved[2] || sp.reserved[3])
+  if (check_sampling(sp, V))
     return fail(FPNMT_ERR_INVALID, "sample: temperature >= 0, top_p in (0, 1], 0 <= top_k <= vocab and reserved words 0");
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "sample: NULL out_ids / out_len");
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
@@ -1915,21 +1935,11 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
   RC(run_program(dec_init_prog_, s));
   RC(launch_sample_init(ss_, bs_.anc[0], s));
   launches += 1;
-  forced_mode_ = true;   // the self-attention launches of the program stay in the first buffer pair, without representatives
-  struct Reset { bool& f; ~Reset() { f = false; } } reset{forced_mode_};
-  if (cfg_.use_graphs && !sample_graph_) RC(capture(sample_prog_, &sample_graph_));
-  for (int t = 0; t < T; ++t) {
-    RC(launch_prog(sample_prog_, sample_graph_, s));
-    if (early_stop && (t % 4 == 3) && t + 1 < T) {
-      FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, bs_.n_done, 4, cudaMemcpyDeviceToHost, s));
-      FPNMT_CUDA_OK(cudaStreamSynchronize(s));
-      if (h_pinned_[0] >= B) break;
-    }
-  }
-  const cudaMemcpyKind kind = out_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, ss_.ids, (size_t)R * T * 4, kind, s));
-  FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, ss_.len, (size_t)R * 4, kind, s));
-  if (out_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, ss_.lp, (size_t)R * 4, kind, s));
+  FlagGuard forced(forced_mode_);   // the self-attention launches of the program stay in the first buffer pair, without representatives
+  RC(run_steps(sample_prog_, sample_graph_, bs_.n_done, early_stop, s));
+  RC(copy_out(out_ids, ss_.ids, (size_t)R * T * 4, out_on_host, s));
+  RC(copy_out(out_len, ss_.len, (size_t)R * 4, out_on_host, s));
+  RC(copy_out(out_logprob, ss_.lp, (size_t)R * 4, out_on_host, s));
   if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
 }
@@ -1942,11 +1952,9 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
 // every (G, lambda, alpha) and bs_.lp, which generate reads, is never touched.  fpnmt_beam_search is G = 1.
 int Engine::beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty,
                         int32_t* out_ids, int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
-  if (!finalized_) return fail(FPNMT_ERR_STATE, "beam_search before finalize_weights");
-  if (use_dstep_) return fail(FPNMT_ERR_STATE, "beam_search: the fused decoder has no N-best tail (use decode_path = chain)");
+  RC(check_decode_entry("beam_search", "has no N-best tail"));
   if (cfg_.score_mode == FPNMT_SCORE_PROB)
     return fail(FPNMT_ERR_STATE, "beam_search: the length penalty and the log-likelihoods need score_mode = log");
-  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "beam_search: this lane still holds a submitted batch (call fpnmt_collect first)");
   if (!std::isfinite(length_penalty)) return fail(FPNMT_ERR_INVALID, "beam_search: length_penalty must be finite");
   if (check_beam_groups(step_bsv_, beam_groups, diversity)) return FPNMT_ERR_INVALID;
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "beam_search: NULL out_ids / out_len");
@@ -1982,19 +1990,10 @@ int Engine::beam_search(const float* images, int on_host, int beam_groups, float
   launches += 1;
   RC(run_program(dec_init_prog_, s));
   RC(run_program(embed_prog_, s));
-  if (cfg_.use_graphs && !nbest_graph_) RC(capture(nbest_prog_, &nbest_graph_));
-  for (int t = 0; t < T; ++t) {
-    RC(launch_prog(nbest_prog_, nbest_graph_, s));
-    if (early_stop && (t % 4 == 3) && t + 1 < T) {
-      FPNMT_CUDA_OK(cudaMemcpyAsync(h_pinned_, nbest_bs_.n_done, 4, cudaMemcpyDeviceToHost, s));
-      FPNMT_CUDA_OK(cudaStreamSynchronize(s));
-      if (h_pinned_[0] >= B) break;
-    }
-  }
-  const cudaMemcpyKind kind = out_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, nbest_bs_.nb.ids, (size_t)R * T * 4, kind, s));
-  FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, nbest_bs_.nb.len, (size_t)R * 4, kind, s));
-  if (out_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, nbest_bs_.nb.score, (size_t)R * 4, kind, s));
+  RC(run_steps(nbest_prog_, nbest_graph_, nbest_bs_.n_done, early_stop, s));
+  RC(copy_out(out_ids, nbest_bs_.nb.ids, (size_t)R * T * 4, out_on_host, s));
+  RC(copy_out(out_len, nbest_bs_.nb.len, (size_t)R * 4, out_on_host, s));
+  RC(copy_out(out_logprob, nbest_bs_.nb.score, (size_t)R * 4, out_on_host, s));
   if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
 }
@@ -2073,9 +2072,7 @@ int Engine::build_score(int t, Program& p) {
 
 int Engine::score(const float* images, int on_host, const int32_t* ids, const int32_t* lens, int t, float* out_logprob,
                   float* out_token_logprob, int out_on_host, cudaStream_t s) {
-  if (!finalized_) return fail(FPNMT_ERR_STATE, "score before finalize_weights");
-  if (use_dstep_) return fail(FPNMT_ERR_STATE, "score: the fused decoder has no per-layer weights for a parallel pass (use decode_path = chain)");
-  if (lane_state_ != 0) return fail(FPNMT_ERR_STATE, "score: this lane still holds a submitted batch (call fpnmt_collect first)");
+  RC(check_decode_entry("score", "has no per-layer weights for a parallel pass"));
   if (t < 1 || t > cfg_.max_len) return fail(FPNMT_ERR_INVALID, "score: t must lie in [1, max_len]");
   if (!ids || !lens || !out_logprob) return fail(FPNMT_ERR_INVALID, "score: NULL ids / lens / out_logprob");
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
@@ -2107,20 +2104,9 @@ int Engine::score(const float* images, int on_host, const int32_t* ids, const in
   FPNMT_CUDA_OK(cudaMemcpyAsync(sc_.ids, ids, (size_t)R * t * 4, cudaMemcpyDeviceToDevice, s));
   FPNMT_CUDA_OK(cudaMemcpyAsync(sc_.lens, lens, (size_t)R * 4, cudaMemcpyDeviceToDevice, s));
   RC(run_program(dec_init_prog_, s));
-  cudaGraphExec_t g = nullptr;
-  if (cfg_.use_graphs) {
-    auto gi = score_graphs_.find(t);
-    if (gi == score_graphs_.end()) {
-      RC(capture(it->second, &g));
-      score_graphs_[t] = g;
-    } else {
-      g = gi->second;
-    }
-  }
-  RC(launch_prog(it->second, g, s));
-  const cudaMemcpyKind kind = out_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  FPNMT_CUDA_OK(cudaMemcpyAsync(out_logprob, sc_.lp, (size_t)R * 4, kind, s));
-  if (out_token_logprob) FPNMT_CUDA_OK(cudaMemcpyAsync(out_token_logprob, sc_.tok_lp, (size_t)R * t * 4, kind, s));
+  RC(launch_graph(it->second, score_graphs_[t], s));
+  RC(copy_out(out_logprob, sc_.lp, (size_t)R * 4, out_on_host, s));
+  RC(copy_out(out_token_logprob, sc_.tok_lp, (size_t)R * t * 4, out_on_host, s));
   if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
 }
@@ -2190,8 +2176,7 @@ int Engine::submit(const float* images, int on_host, int early_stop, cudaStream_
   // for.  Without the chain the overlap depends on when the host happens to submit (measured: 2 920 -> 2 960 images/s, and
   // the run-to-run spread of the device-resident figure shrinks).
   if (prev_encode_done) FPNMT_CUDA_OK(cudaStreamWaitEvent(lane_stream_, prev_encode_done, 0));
-  if (cfg_.use_graphs && !enc_graph_) RC(capture(enc_prog_, &enc_graph_));
-  RC(launch_prog(enc_prog_, enc_graph_, lane_stream_));
+  RC(launch_graph(enc_prog_, enc_graph_, lane_stream_));
   FPNMT_CUDA_OK(cudaEventRecord(lane_enc_ev_, lane_stream_));
   FPNMT_CUDA_OK(cudaStreamWaitEvent(lane_dec_stream_, lane_enc_ev_, 0));
   if (early_stop) {
@@ -2213,9 +2198,8 @@ int Engine::collect(int32_t* out_ids, int32_t* out_len, int on_host, cudaStream_
   if (st == 2) {
     RC(decode(out_ids, out_len, on_host, 1, nullptr, lane_dec_stream_));
   } else {
-    const cudaMemcpyKind kind = on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-    if (out_ids) FPNMT_CUDA_OK(cudaMemcpyAsync(out_ids, bs_.out_ids, (size_t)B * T * 4, kind, lane_dec_stream_));
-    if (out_len) FPNMT_CUDA_OK(cudaMemcpyAsync(out_len, bs_.out_len, (size_t)B * 4, kind, lane_dec_stream_));
+    RC(copy_out(out_ids, bs_.out_ids, (size_t)B * T * 4, on_host, lane_dec_stream_));
+    RC(copy_out(out_len, bs_.out_len, (size_t)B * 4, on_host, lane_dec_stream_));
   }
   FPNMT_CUDA_OK(cudaEventRecord(lane_out_ev_, lane_dec_stream_));
   if (on_host) {

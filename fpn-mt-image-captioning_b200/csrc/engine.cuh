@@ -232,8 +232,25 @@ class Engine {
   int run_program(Program& p, cudaStream_t s);
   int capture(Program& p, cudaGraphExec_t* out);
   int launch_prog(Program& p, cudaGraphExec_t g, cudaStream_t s);
+  int launch_graph(Program& p, cudaGraphExec_t& g, cudaStream_t s);     // capture g on first use (use_graphs), then launch
+  int poll_done(const int* n_done, cudaStream_t s, bool* done);         // synchronises s; done: every image has finished
+  int run_steps(Program& p, cudaGraphExec_t& g, const int* n_done, int early_stop, cudaStream_t s);
+  int check_decode_entry(const char* entry, const char* fused_reason);
   int set_images(const float* images, int on_host, cudaStream_t s);
   int profile_program(Program& p, int iters, std::string& json, const char* label);
 };
 
 }  // namespace fpnmt
+
+// The object behind the C ABI's opaque handle (api.cu, dlapi.cu).
+struct fpnmt_handle {
+  fpnmt::Engine* eng;                   // lane 0: every single-batch entry point runs here
+  std::vector<fpnmt::Engine*> lanes;    // lanes[0] == eng; fpnmt_submit / fpnmt_collect address the others
+  cudaEvent_t last_encode = nullptr;    // encoder-done event of the most recent fpnmt_submit (owned by that lane)
+};
+
+#define CHECK_H(h)                                 \
+  if (!(h) || !(h)->eng) {                         \
+    ::fpnmt::set_last_error("NULL handle");        \
+    return FPNMT_ERR_INVALID;                      \
+  }

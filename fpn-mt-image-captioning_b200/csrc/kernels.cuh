@@ -2,6 +2,8 @@
 #pragma once
 #include "common.cuh"
 
+struct fpnmt_sampling;   // include/fpnmt.h
+
 namespace fpnmt {
 
 // Opt-in shared-memory sizes are a per-DEVICE function attribute: Engine::init calls these for its device (a static
@@ -189,8 +191,11 @@ struct SampleParams {       // device copy of fpnmt_sampling read by every step 
   int pad;
   unsigned long long seed;
 };
+// 1 when sampling parameters are out of range for a vocabulary of V (callers set their own message): temperature >= 0,
+// top_p in (0, 1], 0 <= top_k <= V and the reserved words 0
+int check_sampling(const fpnmt_sampling& sp, int V);
 struct SampleState {
-  int rows, V, N, T;         // rows = images * N samples, vocab, samples per image, max steps
+  int rows, V, N, T;       // rows = images * N samples, vocab, samples per image, max steps
   int start_id, end_id;
   const SampleParams* params;
   int* step;                 // device step counter (advanced by the kernel), or nullptr: step t0

@@ -8,6 +8,7 @@
 //                   fed to the next step, frozen flag / length / log-probability / caption of the sample, the image's
 //                   finished-sample counter, and the device step counter (last CTA).
 //   k_sample_init   step 0, <start> fed to every row, identity ancestry in both step parities, per-row state cleared.
+#include "../../include/fpnmt.h"
 #include "kernels.cuh"
 
 namespace fpnmt {
@@ -340,6 +341,11 @@ __global__ void k_sample_init(SampleState st, int* anc) {
 int sample_set_attributes() {   // per device
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_sample_step, cudaFuncAttributeMaxDynamicSharedMemorySize, SAMPLE_MAX_SMEM));
   return 0;
+}
+
+int check_sampling(const fpnmt_sampling& sp, int V) {
+  return !(sp.temperature >= 0.f) || !(sp.top_p > 0.f && sp.top_p <= 1.f) || sp.top_k < 0 || sp.top_k > V || sp.reserved[0] ||
+         sp.reserved[1] || sp.reserved[2] || sp.reserved[3];
 }
 
 int launch_sample_init(const SampleState& st, int* anc, cudaStream_t s) {

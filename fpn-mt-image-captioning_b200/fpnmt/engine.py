@@ -115,6 +115,23 @@ class Engine:
             raise ValueError("images must be NHWC (%d,%d,%d,3), got %s" % (self.batch, s, s, tuple(t.shape)))
         return t.data_ptr(), 0, t
 
+    def _images_opt(self, images) -> Tuple[Optional[int], int, object]:
+        """`_images`, or (None, 0, None) for images None: the memory of the last encode."""
+        return (None, 0, None) if images is None else self._images(images)
+
+    def _memory(self, memory) -> Tuple[Optional[int], object]:
+        """(pointer, keepalive) of a memory argument (B, n_memory, d_model); (None, None) for None: the last encode's."""
+        if memory is None:
+            return None, None
+        mem = _as_cuda(memory, torch.float32, self.device)
+        return mem.data_ptr(), mem
+
+    def _result(self, shape, dtype, to_host: bool) -> torch.Tensor:
+        """Output buffer of a call: pinned host memory for to_host (the call synchronises), else device memory."""
+        if to_host:
+            return torch.empty(shape, dtype=dtype).pin_memory()
+        return torch.empty(shape, dtype=dtype, device=self.device)
+
     def encode(self, images) -> torch.Tensor:
         """Encoder.call (transformer.py:266-303): (B,S,S,3) -> (B, n_memory, d_model) float32 on device."""
         ptr, on_host, keep = self._images(images)
@@ -142,10 +159,7 @@ class Engine:
         """Transformer.call(enc_output, tar, False, mask) (transformer.py:359-374) -> logits (B,t,V)."""
         tok = _as_cuda(tokens, torch.int32, self.device)
         t = int(tok.shape[1])
-        mem_ptr = None
-        if memory is not None:
-            mem = _as_cuda(memory, torch.float32, self.device)
-            mem_ptr = mem.data_ptr()
+        mem_ptr, keep = self._memory(memory)
         out = torch.empty((self.batch, t, self.vocab), dtype=torch.float32, device=self.device)
         _lib.check(self.lib.fpnmt_decode_logits(self._h, mem_ptr, tok.data_ptr(), t, out.data_ptr(),
                                                 _stream_ptr(self.device)))
@@ -155,10 +169,7 @@ class Engine:
         """Decoder.call(x, enc_output, False, mask, None) (transformer.py:321-341) -> last decoder layer's output (B,t,d)."""
         tok = _as_cuda(tokens, torch.int32, self.device)
         t = int(tok.shape[1])
-        mem_ptr = None
-        if memory is not None:
-            mem = _as_cuda(memory, torch.float32, self.device)
-            mem_ptr = mem.data_ptr()
+        mem_ptr, keep = self._memory(memory)
         out = torch.empty((self.batch, t, self.d_model), dtype=torch.float32, device=self.device)
         _lib.check(self.lib.fpnmt_decode_hidden(self._h, mem_ptr, tok.data_ptr(), t, out.data_ptr(), _stream_ptr(self.device)))
         return out
@@ -172,10 +183,7 @@ class Engine:
             raise ValueError("decode_attention: nothing requested")
         tok = _as_cuda(tokens, torch.int32, self.device)
         t = int(tok.shape[1])
-        mem_ptr = None
-        if memory is not None:
-            mem = _as_cuda(memory, torch.float32, self.device)
-            mem_ptr = mem.data_ptr()
+        mem_ptr, keep = self._memory(memory)
         L, H = self.num_layers, self.num_heads
         so = torch.empty((L, self.batch, H, t, t), dtype=torch.float32, device=self.device) if self_attention else None
         co = torch.empty((L, self.batch, H, t, self.n_memory), dtype=torch.float32, device=self.device) if cross_attention else None
@@ -231,12 +239,8 @@ class Engine:
     def generate(self, images, early_stop: bool = True, to_host: bool = True, return_scores: bool = False):
         """Pipeline.predict for a batch (pipeline.py:82-154): ids (B,T) int32 zero-padded, lengths (B,)."""
         ptr, on_host, keep = self._images(images)
-        if to_host:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32).pin_memory()
-            lens = torch.empty((self.batch,), dtype=torch.int32).pin_memory()
-        else:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32, device=self.device)
-            lens = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
+        ids = self._result((self.batch, self.max_len), torch.int32, to_host)
+        lens = self._result((self.batch,), torch.int32, to_host)
         scores = None
         if return_scores:
             scores = torch.zeros((self.max_len, self.batch), dtype=torch.float32, device=self.device)
@@ -252,16 +256,11 @@ class Engine:
         the Philox stream of (seed, step, image, sample).  temperature 0 is greedy.  images None = the memory of the last
         encode / generate.  Returns ids (B, N, T) int32 zero padded without <start> / <end>, lengths (B, N) and, with
         return_logprobs, the captions' log-likelihoods (B, N) float32 (log_softmax at temperature 1, <end> included)."""
-        ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
+        ptr, on_host, keep = self._images_opt(images)
         B, N, T = self.batch, self.beam, self.max_len
-        if to_host:
-            ids = torch.empty((B, N, T), dtype=torch.int32).pin_memory()
-            lens = torch.empty((B, N), dtype=torch.int32).pin_memory()
-            lp = torch.empty((B, N), dtype=torch.float32).pin_memory() if return_logprobs else None
-        else:
-            ids = torch.empty((B, N, T), dtype=torch.int32, device=self.device)
-            lens = torch.empty((B, N), dtype=torch.int32, device=self.device)
-            lp = torch.empty((B, N), dtype=torch.float32, device=self.device) if return_logprobs else None
+        ids = self._result((B, N, T), torch.int32, to_host)
+        lens = self._result((B, N), torch.int32, to_host)
+        lp = self._result((B, N), torch.float32, to_host) if return_logprobs else None
         sp = _lib.sampling(temperature, top_k, top_p, seed)
         _lib.check(self.lib.fpnmt_sample(self._h, ptr, on_host, C.byref(sp), ids.data_ptr(), lens.data_ptr(),
                                          lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
@@ -278,16 +277,11 @@ class Engine:
         beam_groups G > 1 runs the diverse beam search instead (fpnmt_beam_search_diverse): G groups of N / G beams, each
         group's candidates lowered by `diversity` per earlier group's beam that chose the same token at the same step.  The
         output is group-major (beams [g * N / G, (g + 1) * N / G) are group g), rank order within a group."""
-        ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
+        ptr, on_host, keep = self._images_opt(images)
         B, N, T = self.batch, self.beam, self.max_len
-        if to_host:
-            ids = torch.empty((B, N, T), dtype=torch.int32).pin_memory()
-            lens = torch.empty((B, N), dtype=torch.int32).pin_memory()
-            lp = torch.empty((B, N), dtype=torch.float32).pin_memory() if return_logprobs else None
-        else:
-            ids = torch.empty((B, N, T), dtype=torch.int32, device=self.device)
-            lens = torch.empty((B, N), dtype=torch.int32, device=self.device)
-            lp = torch.empty((B, N), dtype=torch.float32, device=self.device) if return_logprobs else None
+        ids = self._result((B, N, T), torch.int32, to_host)
+        lens = self._result((B, N), torch.int32, to_host)
+        lp = self._result((B, N), torch.float32, to_host) if return_logprobs else None
         if beam_groups == 1:
             _lib.check(self.lib.fpnmt_beam_search(self._h, ptr, on_host, float(length_penalty), ids.data_ptr(), lens.data_ptr(),
                                                   lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
@@ -313,13 +307,9 @@ class Engine:
             raise ValueError("score: ids must be (%d, %d, t) and lens (%d, %d), got %s and %s"
                              % (B, N, B, N, tuple(tok.shape), tuple(ln.shape)))
         t = int(tok.shape[2])
-        ptr, on_host, keep = (None, 0, None) if images is None else self._images(images)
-        if to_host:
-            lp = torch.empty((B, N), dtype=torch.float32).pin_memory()
-            tl = torch.empty((B, N, t), dtype=torch.float32).pin_memory() if return_token_logprobs else None
-        else:
-            lp = torch.empty((B, N), dtype=torch.float32, device=self.device)
-            tl = torch.empty((B, N, t), dtype=torch.float32, device=self.device) if return_token_logprobs else None
+        ptr, on_host, keep = self._images_opt(images)
+        lp = self._result((B, N), torch.float32, to_host)
+        tl = self._result((B, N, t), torch.float32, to_host) if return_token_logprobs else None
         _lib.check(self.lib.fpnmt_score(self._h, ptr, on_host, tok.data_ptr(), ln.data_ptr(), t, lp.data_ptr(),
                                         tl.data_ptr() if tl is not None else None, int(to_host), _stream_ptr(self.device)))
         return (lp, tl) if return_token_logprobs else lp
@@ -340,12 +330,8 @@ class Engine:
 
     def generate_staged(self, slot: int, early_stop: bool = True, to_host: bool = True):
         """`generate` on a batch previously handed to `stage(…, slot)`."""
-        if to_host:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32).pin_memory()
-            lens = torch.empty((self.batch,), dtype=torch.int32).pin_memory()
-        else:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32, device=self.device)
-            lens = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
+        ids = self._result((self.batch, self.max_len), torch.int32, to_host)
+        lens = self._result((self.batch,), torch.int32, to_host)
         _lib.check(self.lib.fpnmt_generate_staged(self._h, int(slot), ids.data_ptr(), lens.data_ptr(), int(to_host),
                                                   int(early_stop), None, _stream_ptr(self.device)))
         return ids, lens
@@ -353,26 +339,17 @@ class Engine:
     def submit(self, lane: int, images, early_stop: bool = False):
         """Enqueue one whole batch on lane `lane` (fpnmt_submit) and return at once.  Returns a keep-alive object: the images
         must stay valid until `collect(lane)`."""
-        ptr, on_host, keep = self._images_nocopy(images)
+        ptr, on_host, keep = self._images(images)
         _lib.check(self.lib.fpnmt_submit(self._h, int(lane), ptr, on_host, int(early_stop), _stream_ptr(self.device)))
         return keep
 
     def collect(self, lane: int, to_host: bool = True):
         """Result of the batch submitted on `lane` (fpnmt_collect): ids (B,T) int32 zero-padded, lengths (B,)."""
-        if to_host:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32).pin_memory()
-            lens = torch.empty((self.batch,), dtype=torch.int32).pin_memory()
-        else:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32, device=self.device)
-            lens = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
+        ids = self._result((self.batch, self.max_len), torch.int32, to_host)
+        lens = self._result((self.batch,), torch.int32, to_host)
         _lib.check(self.lib.fpnmt_collect(self._h, int(lane), ids.data_ptr(), lens.data_ptr(), int(to_host),
                                           _stream_ptr(self.device)))
         return ids, lens
-
-    def _images_nocopy(self, images):
-        """(pointer, on_host, keepalive) for submit: host batches go as they are (the lane copies them on its own stream),
-        device batches are used in place."""
-        return self._images(images)
 
     def generate_stream(self, batches, early_stop: bool = True, to_host: bool = True):
         """Captions for an iterable of batches (HOST tensors: pinned memory makes the copies asynchronous; or device tensors),
@@ -417,12 +394,8 @@ class Engine:
 
     def decode(self, early_stop: bool = True, to_host: bool = True):
         """Decode half only, from the memory left by the last `encode`."""
-        if to_host:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32).pin_memory()
-            lens = torch.empty((self.batch,), dtype=torch.int32).pin_memory()
-        else:
-            ids = torch.empty((self.batch, self.max_len), dtype=torch.int32, device=self.device)
-            lens = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
+        ids = self._result((self.batch, self.max_len), torch.int32, to_host)
+        lens = self._result((self.batch,), torch.int32, to_host)
         _lib.check(self.lib.fpnmt_decode(self._h, ids.data_ptr(), lens.data_ptr(), int(to_host), int(early_stop), None,
                                          _stream_ptr(self.device)))
         return ids, lens
