@@ -10,10 +10,9 @@
 namespace fpnmt {
 static thread_local std::string g_last_error;
 void set_last_error(const std::string& s) { g_last_error = s; }
-static int g_pdl_mode = 1;   // 0 = off, 1 = every kernel, 2 = tcgen05 GEMM kernels only (fpnmt_config.kernel_opts)
-void set_pdl_mode(int mode) { g_pdl_mode = mode; }
-bool pdl_enabled() { return g_pdl_mode != 0; }
-bool pdl_small_enabled() { return g_pdl_mode == 1; }
+static bool g_pdl = true;   // fpnmt_config.kernel_opts FPNMT_OPT_NO_PDL clears it
+void set_pdl_enabled(bool on) { g_pdl = on; }
+bool pdl_enabled() { return g_pdl; }
 }  // namespace fpnmt
 
 using namespace fpnmt;

@@ -644,18 +644,18 @@ int launch_dec_self_attention(Act qkv, Act kcache, Act vcache, Act kcache2, Act 
   }
   const bool simt = kernel == DEC_ATT_SIMT || (kernel == DEC_ATT_AUTO && g_dec_att_simt);
   if (kcache.lo)
-    FPNMT_CUDA_OK(launch_k_small(k_dec_self_attention<true>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
+    FPNMT_CUDA_OK(launch_k(k_dec_self_attention<true>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
                            qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, rows, T, heads, out));
   else if (!plain || simt)
-    FPNMT_CUDA_OK(launch_k_small(k_dec_self_attention<false>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
+    FPNMT_CUDA_OK(launch_k(k_dec_self_attention<false>, dim3((warps + DEC_WARPS - 1) / DEC_WARPS), dim3(DEC_WARPS * 32), 0, s,
                            qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, rows, T, heads, out));
   else {
     // The kernel finds beam n of image b at row b * N + n, so N must divide the rows; otherwise every row is its own image
     // and its own class (rep_e / rep_o index rows by that layout and would name representatives of other images).
     const int n = (N >= 1 && rows % N == 0) ? N : 1;
     const bool classes = n == N && N <= 8;
-    FPNMT_CUDA_OK(launch_k_small(k_dec_self_attention_mma, dim3((warps + DEC_MMA_WARPS - 1) / DEC_MMA_WARPS), dim3(DEC_MMA_WARPS * 32),
-                                 DEC_MMA_WARPS * sizeof(DecAttTile), s,
+    FPNMT_CUDA_OK(launch_k(k_dec_self_attention_mma, dim3((warps + DEC_MMA_WARPS - 1) / DEC_MMA_WARPS), dim3(DEC_MMA_WARPS * 32),
+                           DEC_MMA_WARPS * sizeof(DecAttTile), s,
                            qkv, kcache, vcache, kcache2, vcache2, anc, anc_stride, step, classes ? rep_e : nullptr,
                            classes ? rep_o : nullptr, rows, T, heads, n, out));
   }
@@ -780,7 +780,7 @@ int launch_dec_attention_probs(const DecProbArgs& a, int B, cudaStream_t s) {
     return 1;
   }
   const size_t smem = (size_t)std::max(a.tlen, a.n_mem) * sizeof(float);
-  FPNMT_CUDA_OK(launch_k_small(k_dec_attention_probs, dim3(B, a.heads, 2), dim3(DP_THREADS), smem, s, a));
+  FPNMT_CUDA_OK(launch_k(k_dec_attention_probs, dim3(B, a.heads, 2), dim3(DP_THREADS), smem, s, a));
   return 0;
 }
 

@@ -485,9 +485,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
           st.fin_len[nxt][rows0 + n] = fl > 0 ? fl : (tok == st.end_id ? t + 1 : 0);
           st.score[nxt][rows0 + n] = v;                     // raw: the penalty only ranks, it is never accumulated
           st.last_tok[rows0 + n] = tok;
-          if (st.parent_out) st.parent_out[(size_t)t * st.Btot * N + rows0 + n] = par;
-          if (st.token_out) st.token_out[(size_t)t * st.Btot * N + rows0 + n] = tok;
-          if (n == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.Btot + b] = v;
+          if (st.parent_out) st.parent_out[(size_t)t * st.B * N + rows0 + n] = par;
+          if (st.token_out) st.token_out[(size_t)t * st.B * N + rows0 + n] = tok;
+          if (n == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.B + b] = v;
         }
       }
     }
@@ -509,9 +509,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       }
       st.score[nxt][rows0 + rank] = v;
       st.last_tok[rows0 + rank] = tok;
-      if (st.parent_out) st.parent_out[(size_t)t * st.Btot * N + rows0 + rank] = par;
-      if (st.token_out) st.token_out[(size_t)t * st.Btot * N + rows0 + rank] = tok;
-      if (rank == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.Btot + b] = v;
+      if (st.parent_out) st.parent_out[(size_t)t * st.B * N + rows0 + rank] = par;
+      if (st.token_out) st.token_out[(size_t)t * st.B * N + rows0 + rank] = tok;
+      if (rank == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.B + b] = v;
     }
   }
   }
@@ -665,7 +665,7 @@ static int launch_step(const BeamState& st, const float* logits, int ld, const B
   if (st.vs_stat) {                                         // logits-free tail: merge the vocabulary projection's candidates
     size_t smem = (size_t)st.vs_tiles * 8 * 8;
     if (smem < 12288) smem = 12288;
-    FPNMT_CUDA_OK(launch_k_small(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
     return 0;
   }
   const int threads = st.V <= 16384 ? 256 : 512;
@@ -673,9 +673,9 @@ static int launch_step(const BeamState& st, const float* logits, int ld, const B
   size_t smem = (size_t)nv4 * threads * 16;
   if (smem < 12288) smem = 12288;                           // phase 2 keeps the N x N merge lists (values, flat ids, keys) there
   if (threads == 256)
-    FPNMT_CUDA_OK(launch_k_small(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
   else
-    FPNMT_CUDA_OK(launch_k_small(k_beam_step<512, NBEST>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<512, NBEST>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
   return 0;
 }
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {

@@ -124,10 +124,8 @@ __device__ __forceinline__ void st_act8(const Act& a, size_t pix, int c, const f
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-bool pdl_enabled();         // FPNMT_OPT_NO_PDL disables the launch attribute (api.cu)
-bool pdl_small_enabled();   // FPNMT_OPT_PDL_GEMM_ONLY: only the tcgen05 GEMM kernels launch early; the small-footprint kernels
-                            // of the decode step (attention, beam) start after their predecessor has finished
-void set_pdl_mode(int mode);   // process-wide; Engine::init sets it from fpnmt_config.kernel_opts
+bool pdl_enabled();            // FPNMT_OPT_NO_PDL disables the launch attribute (api.cu)
+void set_pdl_enabled(bool on);   // process-wide; Engine::init sets it from fpnmt_config.kernel_opts
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_k_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
@@ -148,11 +146,6 @@ template <typename... KArgs, typename... Args>
 inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                             Args... args) {
   return launch_k_pdl(pdl_enabled(), kernel, grid, block, smem, stream, args...);
-}
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_k_small(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                                  Args... args) {
-  return launch_k_pdl(pdl_small_enabled(), kernel, grid, block, smem, stream, args...);
 }
 
 // ------------------------------------------------------------------------------------------------

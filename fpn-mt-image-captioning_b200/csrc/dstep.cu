@@ -127,7 +127,7 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dstep_kernel(const __grid_const
     const int total = p.nsteps * per_step;
     constexpr int DS_AHEAD = 12;
     auto l2_prefetch = [&](int n) {
-      if (n < total && leader && !(p.exp & 2))
+      if (n < total && leader)
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p.wstream + (size_t)group_row(n % per_step) * 128), "n"(DS_GROUP) : "memory");
     };
     for (int n = 0; n < DS_AHEAD; ++n) l2_prefetch(n);
@@ -671,25 +671,6 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dstep_kernel(const __grid_const
             }
             if (lane < 8) *reinterpret_cast<uint4*>(p.x_att + (xrow0 + lr) * 512 + cta * 64 + lane * 8) = pack8(o);
           }
-          // (A/B switch, off: L2 prefetch of the K/V lines of the NEXT attention phase.  Measured on C2: the burst of ~4000
-          // 128-byte prefetches per CTA queues in front of the weight TMA loads - GEMM phases 2-3x slower - and the attention
-          // phase itself does not get faster, the K/V of a layer at t ~ 64 being half of the L2.)
-          if (p.exp & 1) {
-            const int ln = (l + 1 < p.L) ? l + 1 : 0;
-            const bf16* kn = p.kcache + (size_t)ln * p.R * p.T * 512 + cta * 64;
-            const bf16* vn = p.vcache + (size_t)ln * p.R * p.T * 512 + cta * 64;
-            for (int rr = 0; rr < 2; ++rr) {
-              const int lr = ww * 2 + rr;
-              if (lr >= nrows) break;
-              const int* anc = p.st.anc[cur] + (size_t)(row_base + lr) * p.T;
-              for (int pos = lane; pos < t; pos += 32) {
-                const int arow = anc_smem ? row_base + (int)ANC8[lr * DS_ANC_T + pos] : __ldcg(anc + pos);
-                const size_t off = ((size_t)arow * p.T + pos) * 512;
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(kn + off));
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(vn + off));
-              }
-            }
-          }
         }
         DSTAMPL();   // self-attention done
         xsync();                                                    // A: attention heads of all CTAs
@@ -1131,9 +1112,9 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dstep_kernel(const __grid_const
             s_token[rank] = tok;
             p.st.score[nxt][rows0 + rank] = c;
             p.st.last_tok[rows0 + rank] = tok;
-            if (p.st.parent_out) p.st.parent_out[(size_t)t * p.st.Btot * N + rows0 + rank] = par;
-            if (p.st.token_out) p.st.token_out[(size_t)t * p.st.Btot * N + rows0 + rank] = tok;
-            if (rank == 0 && p.st.step_logprob) p.st.step_logprob[(size_t)t * p.st.Btot + rows0 / N] = c;
+            if (p.st.parent_out) p.st.parent_out[(size_t)t * p.st.B * N + rows0 + rank] = par;
+            if (p.st.token_out) p.st.token_out[(size_t)t * p.st.B * N + rows0 + rank] = tok;
+            if (rank == 0 && p.st.step_logprob) p.st.step_logprob[(size_t)t * p.st.B + rows0 / N] = c;
           }
         }
         ds_worker_sync();

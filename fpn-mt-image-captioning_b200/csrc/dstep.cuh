@@ -71,8 +71,6 @@ struct DstepParams {
                              // the reference's beam initialisation (all beams identical, pipeline.py:101-102) one set of K/V
                              // lines per image instead of one per beam.  Every row still computes everything else itself.
   int mode;                  // 0 = beam search; 1 = teacher forcing: write the fp32 logits of every row, no beam tail
-  int exp;                   // developer A/B switches (fpnmt_config.reserved[0]): 1 = L2-prefetch next layer's K/V lines,
-                             // 2 = no L2 prefetch of the weight stream
   const uint8_t* wstream;    // [L][8] layer streams, then [8] final-layer streams of ntv * 8 * 16 KB: plain [rows][64] bf16 tiles
   size_t final_off;          // byte offset of the final-layer streams
   size_t stream_bytes;       // total bytes

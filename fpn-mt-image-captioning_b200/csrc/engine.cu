@@ -49,9 +49,6 @@ Engine::~Engine() {
   for (auto& kv : score_graphs_)
     if (kv.second) cudaGraphExecDestroy(kv.second);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
-  for (auto st : grp_streams_) cudaStreamDestroy(st);
-  for (auto ev : join_ev_) cudaEventDestroy(ev);
-  if (fork_ev_) cudaEventDestroy(fork_ev_);
   if (copy_stream_) {
     cudaStreamSynchronize(copy_stream_);
     cudaStreamDestroy(copy_stream_);
@@ -84,6 +81,14 @@ int Engine::init() {
   if (c.image_size < 256 || c.image_size % 256) return fail(FPNMT_ERR_INVALID, "image_size must be a multiple of 256");
   if (c.dff % 8) return fail(FPNMT_ERR_INVALID, "dff must be a multiple of 8");
   if (c.backbone < 0 || c.backbone > 2) return fail(FPNMT_ERR_INVALID, "unknown backbone");
+  // a word or bit that selects nothing is refused rather than silently running the defaults
+  const int32_t known_opts = FPNMT_OPT_NO_XATTN | FPNMT_OPT_NO_STEM | FPNMT_OPT_NO_TGEMM | FPNMT_OPT_ENC_ATT_SIMT | FPNMT_OPT_NO_PDL |
+                             FPNMT_OPT_DEC_ATT_SIMT | FPNMT_OPT_TGEMM_WIDE | FPNMT_OPT_NO_TGEMM_WIDE | FPNMT_OPT_NO_DENSE_1X1 |
+                             FPNMT_OPT_NO_B_STATIONARY | FPNMT_OPT_NO_TMA_STORE | FPNMT_OPT_NO_VSTATS | FPNMT_OPT_NO_KV_SHARE |
+                             FPNMT_OPT_DSTEP_TAPS;
+  if (c.kernel_opts & ~known_opts) return fail(FPNMT_ERR_INVALID, "kernel_opts sets a bit that no FPNMT_OPT_* defines");
+  if (c.dec_groups < 0 || c.dec_groups > 1) return fail(FPNMT_ERR_INVALID, "dec_groups must be 0 or 1 (the batch decodes as one chain)");
+  if (c.reserved[0]) return fail(FPNMT_ERR_INVALID, "fpnmt_config.reserved must be 0");
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   cudaDeviceProp prop;
   FPNMT_CUDA_OK(cudaGetDeviceProperties(&prop, dev_));
@@ -102,9 +107,9 @@ int Engine::init() {
   use_stem_ = !(c.kernel_opts & FPNMT_OPT_NO_STEM);
   use_tgemm_ = !(c.kernel_opts & FPNMT_OPT_NO_TGEMM);
   set_dec_att_simt((c.kernel_opts & FPNMT_OPT_DEC_ATT_SIMT) != 0);   // process-wide, like the PDL mode
-  set_pdl_mode((c.kernel_opts & FPNMT_OPT_NO_PDL) ? 0 : (c.kernel_opts & FPNMT_OPT_PDL_GEMM_ONLY) ? 2 : 1);
-  if (c.cache_mode < 0 || c.cache_mode > 1 || c.decode_path < 0 || c.decode_path > 2 || c.dec_groups < 0 || c.length_penalty < 0.f)
-    return fail(FPNMT_ERR_INVALID, "bad cache_mode / decode_path / dec_groups / length_penalty");
+  set_pdl_enabled(!(c.kernel_opts & FPNMT_OPT_NO_PDL));
+  if (c.cache_mode < 0 || c.cache_mode > 1 || c.decode_path < 0 || c.decode_path > 2 || c.length_penalty < 0.f)
+    return fail(FPNMT_ERR_INVALID, "bad cache_mode / decode_path / length_penalty");
   FPNMT_CUDA_OK(cudaStreamCreateWithFlags(&cap_stream_, cudaStreamNonBlocking));
   FPNMT_CUDA_OK(cudaMallocHost(&h_pinned_, 64));
   return 0;
@@ -392,7 +397,7 @@ int Engine::add_dense(Program& prog, const std::string& name, const Tensor& in, 
                       1e-6f, num_sms_));
   else
     RC(make_tgemm_op(&op, R, in.a, gw.w, gw.Cout, gw.K, split_, gw.bias, act, out.a, out_f32, ld_f32, res ? &res->a : nullptr,
-                     gamma, beta, 1e-6f, num_sms_, 0, (cfg_.kernel_opts & FPNMT_OPT_KSPLIT2) != 0));
+                     gamma, beta, 1e-6f, num_sms_));
   op.p.dbg = dbg_timeline(name);
   Op o;
   o.name = name;
@@ -897,7 +902,7 @@ int Engine::build_decoder() {
   const int V = cfg_.vocab, T = cfg_.max_len;
   const int R = B * N;
   // beam state
-  bs_.B = B; bs_.N = N; bs_.V = V; bs_.T = T; bs_.Btot = B;
+  bs_.B = B; bs_.N = N; bs_.V = V; bs_.T = T;
   bs_.start_id = cfg_.start_id; bs_.end_id = cfg_.end_id;
   bs_.prob_mode = cfg_.score_mode == FPNMT_SCORE_PROB;
   for (int i = 0; i < 2; ++i) {
@@ -1027,9 +1032,8 @@ int Engine::build_decoder() {
       dec_init_prog_.push_back(std::move(o));
     }
 
-    // ---- per-layer weights and full-batch buffers (allocated once; chains below work on row slices of them)
+    // ---- per-layer weights and buffers
     const bool physical = cfg_.cache_mode == FPNMT_CACHE_PHYSICAL;
-    if (physical && cfg_.dec_groups > 1) return fail(FPNMT_ERR_INVALID, "cache_mode PHYSICAL does not combine with dec_groups");
     bs_.physical = physical ? 1 : 0;
     if (physical) {   // the ancestry tables stay the identity in this mode
       k_anc_identity<<<148, 256>>>(anc, R, T);
@@ -1065,254 +1069,187 @@ int Engine::build_decoder() {
     RC(prep_dense_cat({std::string(TR) + "/final_layer"}, &gf));
     dec_lw_.assign(lw.begin(), lw.end());
     dec_final_ = gf;
-    Tensor x0 = rows_act(R, D);
-    auto row_view = [](const Tensor& t, size_t r0, int rows) {
-      Tensor v = t;
-      v.a.p = t.a.p + r0 * (size_t)t.a.ld;
-      v.N = 1; v.H = 1; v.W = rows;
-      return v;
-    };
+    Tensor x = rows_act(R, D);
     Tensor none;
+    bs_.dbg = dbg_timeline("beam_step");
 
-    // One decode chain over the images [b0, b0 + Bg): step-0 embedding program + the program of one step.  The whole
-    // batch is chain (0, B); with decoder groups the batch is cut into independent chains that run concurrently
-    // (every kernel of the step is latency-bound at these row counts and fills less than half of the SMs).
-    auto build_chain = [&](int b0, int Bg, const BeamState& bs, Program& embed_prog, Program& step_prog, BeamEmbed* em_out) -> int {
-      const int r0 = b0 * N, Rg = Bg * N;
-      const std::string sfx = (Bg == B) ? std::string() : "@" + std::to_string(b0);
-      Tensor x = row_view(x0, r0, Rg);
-      {   // step 0 input (embedding of <start> + pos[0]); later steps' inputs are written by the beam kernel
-        Act xa = x.a;
-        const int* tok = bs.last_tok;
-        const int* step = bs.step;
-        embed_prog.push_back(ew_op("embed_pos" + sfx, [=](cudaStream_t s) { return launch_embed_pos(tok, d_emb, d_pos, step, Rg, D, xa, s); }, (double)Rg * D * 6));
+    // ---- the step-0 embedding program and the program of one step
+    {   // step 0 input (embedding of <start> + pos[0]); later steps' inputs are written by the beam kernel
+      Act xa = x.a;
+      const int* tok = bs_.last_tok;
+      const int* step = bs_.step;
+      embed_prog_.push_back(ew_op("embed_pos", [=](cudaStream_t s) { return launch_embed_pos(tok, d_emb, d_pos, step, R, D, xa, s); }, (double)R * D * 6));
+    }
+    const BeamEmbed em{d_emb, d_pos, x.a, D};
+    beam_embed_ = em;
+    // attention-probability launches of step_attn_prog_: position in step_prog_ they follow, the op
+    std::vector<std::pair<size_t, Op>> prob_ops;
+    for (int l = 0; l < L; ++l) {
+      LayerW& w = lw[l];
+      const std::string ln = "dec" + std::to_string(l);
+      // Dense layers of the step: skinny-row tgemm (weights prefetched before the grid dependency, LayerNorm fused
+      // into the epilogue by a 4-CTA cluster) or, with FPNMT_TGEMM=0, the generic igemm + separate LayerNorm kernels.
+      auto dense = [&](const std::string& nm, const Tensor& in, const GemmW& g, int act, const Tensor& out) -> int {
+        if (use_tgemm_) return add_dense(step_prog_, nm, in, g, act, nullptr, out);
+        return add_conv(step_prog_, nm, in, g, 1, 1, 0, 0, act, RES_NONE, nullptr, out);
+      };
+      auto dense_res_ln = [&](const std::string& nm, const std::string& lnn2, const Tensor& in, const GemmW& g, const Tensor& res,
+                              float* gam, float* bet, const Tensor& out) -> int {
+        if (use_tgemm_) return add_dense(step_prog_, nm + "+ln", in, g, ACT_NONE, &res, out, nullptr, 0, gam, bet);
+        float* y = w.y;
+        RC(add_conv(step_prog_, nm, in, g, 1, 1, 0, 0, ACT_NONE, RES_SAME, &res, none, y, D));
+        Act oa = out.a;
+        step_prog_.push_back(ew_op(lnn2, [=](cudaStream_t s) { return launch_layernorm_rows(y, R, D, gam, bet, 1e-6f, oa, s); }, (double)R * D * 6));
+        return 0;
+      };
+      RC(dense(ln + "_qkv", x, w.gqkv, ACT_NONE, w.qkv));
+      {
+        Act qa = w.qkv.a, ka = w.kc.a, va = w.vc.a, oa = w.att.a, ka2 = w.kc2.a, va2 = w.vc2.a;
+        const size_t anc_stride = (size_t)R * T;
+        const int* step = bs_.step;
+        const int *rep_e = bs_.rep[0], *rep_o = bs_.rep[1];
+        Op o = ew_op(ln + "_self_attn",
+                     [=](cudaStream_t s) {
+                       // teacher forcing (decode_logits) has no beam step and therefore no reorder: it stays in the first buffer pair
+                       const Act none{nullptr, 0, 0, 0};
+                       return launch_dec_self_attention(qa, ka, va, forced_mode_ ? none : ka2, forced_mode_ ? none : va2, anc, anc_stride, step, R, T, H, oa, s,
+                                                        forced_mode_ ? nullptr : rep_e, forced_mode_ ? nullptr : rep_o, N);
+                     },
+                     (double)R * (T / 2) * 2 * D * 2, "attention");
+        step_prog_.push_back(std::move(o));
       }
-      const BeamEmbed em{d_emb, d_pos, x.a, D};
-      if (em_out) *em_out = em;
-      // attention-probability launches of step_attn_prog_ (whole batch only): position in step_prog they follow, the op
-      std::vector<std::pair<size_t, Op>> prob_ops;
-      for (int l = 0; l < L; ++l) {
-        LayerW& w = lw[l];
-        const std::string ln = "dec" + std::to_string(l);
-        Tensor qkv = row_view(w.qkv, r0, Rg), att = row_view(w.att, r0, Rg), out1 = row_view(w.out1, r0, Rg),
-               q2 = row_view(w.q2, r0, Rg), att2 = row_view(w.att2, r0, Rg), out2 = row_view(w.out2, r0, Rg),
-               hdn = row_view(w.hdn, r0, Rg), out3 = row_view(w.out3, r0, Rg);
-        Tensor kc = row_view(w.kc, (size_t)r0 * T, Rg * T), vc = row_view(w.vc, (size_t)r0 * T, Rg * T);
-        Tensor kc2 = physical ? row_view(w.kc2, (size_t)r0 * T, Rg * T) : Tensor(), vc2 = physical ? row_view(w.vc2, (size_t)r0 * T, Rg * T) : Tensor();
-        float* y = w.y + (size_t)r0 * D;
-        // Dense layers of the step: skinny-row tgemm (weights prefetched before the grid dependency, LayerNorm fused
-        // into the epilogue by a 4-CTA cluster) or, with FPNMT_TGEMM=0, the generic igemm + separate LayerNorm kernels.
-        auto dense = [&](const std::string& nm, const Tensor& in, const GemmW& g, int act, const Tensor& out) -> int {
-          if (use_tgemm_) return add_dense(step_prog, nm + sfx, in, g, act, nullptr, out);
-          return add_conv(step_prog, nm + sfx, in, g, 1, 1, 0, 0, act, RES_NONE, nullptr, out);
-        };
-        auto dense_res_ln = [&](const std::string& nm, const std::string& lnn2, const Tensor& in, const GemmW& g, const Tensor& res,
-                                float* gam, float* bet, const Tensor& out) -> int {
-          if (use_tgemm_) return add_dense(step_prog, nm + "+ln" + sfx, in, g, ACT_NONE, &res, out, nullptr, 0, gam, bet);
-          RC(add_conv(step_prog, nm + sfx, in, g, 1, 1, 0, 0, ACT_NONE, RES_SAME, &res, none, y, D));
-          Act oa = out.a;
-          step_prog.push_back(ew_op(lnn2 + sfx, [=](cudaStream_t s) { return launch_layernorm_rows(y, Rg, D, gam, bet, 1e-6f, oa, s); }, (double)Rg * D * 6));
-          return 0;
-        };
-        RC(dense(ln + "_qkv", x, w.gqkv, ACT_NONE, qkv));
-        {
-          Act qa = qkv.a, ka = kc.a, va = vc.a, oa = att.a, ka2 = kc2.a, va2 = vc2.a;
-          const int* ancp = anc + (size_t)r0 * T;
-          const size_t anc_stride = (size_t)R * T;
-          const int* step = bs.step;
-          const int *rep_e = bs.rep[0], *rep_o = bs.rep[1];
-          Op o = ew_op(ln + "_self_attn" + sfx,
-                       [=](cudaStream_t s) {
-                         // teacher forcing (decode_logits) has no beam step and therefore no reorder: it stays in the first buffer pair
-                         const Act none{nullptr, 0, 0, 0};
-                         return launch_dec_self_attention(qa, ka, va, forced_mode_ ? none : ka2, forced_mode_ ? none : va2, ancp, anc_stride, step, Rg, T, H, oa, s,
-                                                          forced_mode_ ? nullptr : rep_e, forced_mode_ ? nullptr : rep_o, N);
-                       },
-                       (double)Rg * (T / 2) * 2 * D * 2, "attention");
-          step_prog.push_back(std::move(o));
-        }
-        RC(dense_res_ln(ln + "_o1+res", ln + "_ln1", att, w.go1, x, w.lnp[0], w.lnp[1], out1));
-        size_t prob_at = 0;   // the probabilities read the new K of position t, q2 / out1: after the cross-attention block
-        if (xattn) {
-          XattnOp xo;
-          RC(make_xattn_op(&xo, xMt, xNt, L, B, b0, Bg, N, l, xSb, w.go2.bias, w.lnp[2], w.lnp[3], out1.a, out2.a));
-          xo.p.dbg = dbg_timeline(ln + "_xattn");
-          Op o;
-          o.name = ln + "_xattn(q2+cross_attn+o2+res+ln)" + sfx;
-          o.kind = "xattn";
-          o.flops = 2.0 * Rg * D * D * 2.0 + 4.0 * Rg * n_base_ * D;          // the two projections + the attention proper
-          o.bytes = (double)Bg * 2 * 128 * 512 * 2 + (double)Rg * D * 2 * 2;  // folded per-image operands + activations
-          o.run = [xo](cudaStream_t s) { return xattn_launch(xo, s); };
-          step_prog.push_back(std::move(o));
-          prob_at = step_prog.size();
-        } else {
-          RC(dense(ln + "_q2", out1, w.gq2, ACT_NONE, q2));
-          {
-            Act qa = q2.a, oa = att2.a;
-            Act ka = ckv.a;
-            ka.p = ckv.a.p + (size_t)b0 * n_base_ * ckv.a.ld;
-            const int kcx = l * 2 * D, vcx = l * 2 * D + D, tk = n_base_;
-            step_prog.push_back(ew_op(ln + "_cross_attn" + sfx, [=](cudaStream_t s) { return launch_dec_cross_attention(qa, ka, kcx, vcx, Rg, N, tk, H, oa, s); },
-                                      (double)Bg * tk * 2 * D * 2, "attention"));
-            prob_at = step_prog.size();
-          }
-          RC(dense_res_ln(ln + "_o2+res", ln + "_ln2", att2, w.go2, out1, w.lnp[2], w.lnp[3], out2));
-        }
-        if (Bg == B) {
-          DecProbArgs pa{};
-          pa.qkv = qkv.a;
-          pa.kc = kc.a;
-          pa.anc = anc;
-          pa.anc_stride = (size_t)R * T;
-          pa.T = T;
-          pa.q = xattn ? out1.a : q2.a;
-          pa.kv = ckv.a;
-          pa.k_col = l * 2 * D;
-          pa.Mt = xattn ? xMt + (size_t)l * B * 128 * 512 : nullptr;
-          pa.sbias = xattn ? xSb + (size_t)l * B * 128 : nullptr;
-          pa.n_mem = n_base_;
-          pa.step = bs.step;
-          pa.N = N;
-          pa.heads = H;
-          const int nm = n_base_;
-          // output pointers and row count are those of the decode_logits call that runs the program
-          Op o = ew_op(ln + "_attn_probs",
-                       [=](cudaStream_t s) {
-                         DecProbArgs q = pa;
-                         const size_t tl = (size_t)attn_tlen_;
-                         q.tlen = attn_tlen_;
-                         q.self_out = attn_self_ ? attn_self_ + (size_t)l * B * H * tl * tl : nullptr;
-                         q.cross_out = attn_cross_ ? attn_cross_ + (size_t)l * B * H * tl * nm : nullptr;
-                         return launch_dec_attention_probs(q, B, s);
-                       },
-                       (double)B * H * (T / 2 + nm) * D * 2, "attention");
-          prob_ops.emplace_back(prob_at, std::move(o));
-        }
-        RC(dense(ln + "_ffn1", out2, w.g1, ACT_LEAKY, hdn));
-        RC(dense_res_ln(ln + "_ffn2+res", ln + "_ln3", hdn, w.g2, out2, w.lnp[4], w.lnp[5], out3));
-        if (Bg == B) {   // per-layer decoder states of the last executed step (parity taps, same names in the fused decoder)
-          taps_[ln + "_out1"] = out1;
-          taps_[ln + "_out2"] = out2;
-          taps_[ln + "_out3"] = out3;
-        }
-        x = out3;
-      }
-      float* lg = logits_ + (size_t)r0 * V;
-      if (use_tgemm_) RC(add_dense(step_prog, "final_layer" + sfx, x, gf, ACT_NONE, nullptr, none, lg, V));
-      else RC(add_conv(step_prog, "final_layer" + sfx, x, gf, 1, 1, 0, 0, ACT_NONE, RES_NONE, nullptr, none, lg, V));
-      if (Bg == B) {   // teacher forcing: embed the forced token, then the shared layer stack (whole batch only)
-        step_forced_prog_ = embed_prog;
-        step_forced_prog_.insert(step_forced_prog_.end(), step_prog.begin(), step_prog.end());
-        step_attn_prog_ = embed_prog;   // the same launches with the probability kernels after the operands they read
-        size_t k = 0;
-        for (size_t i = 0; i < step_prog.size(); ++i) {
-          step_attn_prog_.push_back(step_prog[i]);
-          for (; k < prob_ops.size() && prob_ops[k].first == i + 1; ++k) step_attn_prog_.push_back(prob_ops[k].second);
-        }
-      }
-      // Logits-free decode tail (bf16 mode, log scores, beam <= 8, wide Dense kernels): the beam-search chain replaces the
-      // vocabulary projection's [rows][V] fp32 output (20.5 MB written and read back per step at C2) by per-tile softmax
-      // partials + 8 candidates (2.9 MB); teacher forcing (decode_logits) keeps the logits version built above.
-      const int vtiles = (V + TG_BM - 1) / TG_BM;
-      const bool want_wide = (cfg_.kernel_opts & FPNMT_OPT_TGEMM_WIDE) || (cfg_.lanes >= 2 && !(cfg_.kernel_opts & FPNMT_OPT_NO_TGEMM_WIDE));
-      const bool vstats = use_tgemm_ && want_wide && !split_ && !bs.prob_mode && N <= TG_VS_N && vtiles <= 192 && Bg == B &&
-                          !(cfg_.kernel_opts & FPNMT_OPT_NO_VSTATS);
-      BeamState bsv = bs;
-      if (vstats) {
-        float2* vst = (float2*)dalloc((size_t)Rg * vtiles * sizeof(float2));
-        float* vval = (float*)dalloc((size_t)Rg * vtiles * TG_VS_N * sizeof(float));
-        int* vidx = (int*)dalloc((size_t)Rg * vtiles * TG_VS_N * sizeof(int));
-        if (!vst || !vval || !vidx) return FPNMT_ERR_CUDA;
-        TgemmOp op;
-        RC(make_tgemmw_op(&op, Rg, x.a, gf.w, gf.Cout, gf.K, gf.bias, ACT_NONE, none.a, nullptr, 0, nullptr, nullptr, nullptr, 1e-6f,
-                          num_sms_, vst, vval, vidx));
-        op.p.dbg = dbg_timeline("final_layer");
+      RC(dense_res_ln(ln + "_o1+res", ln + "_ln1", w.att, w.go1, x, w.lnp[0], w.lnp[1], w.out1));
+      size_t prob_at = 0;   // the probabilities read the new K of position t, q2 / out1: after the cross-attention block
+      if (xattn) {
+        XattnOp xo;
+        RC(make_xattn_op(&xo, xMt, xNt, L, B, 0, B, N, l, xSb, w.go2.bias, w.lnp[2], w.lnp[3], w.out1.a, w.out2.a));
+        xo.p.dbg = dbg_timeline(ln + "_xattn");
         Op o;
-        o.name = "final_layer(softmax partials + candidates)" + sfx;
-        o.kind = "tgemm";
-        o.flops = op.flops;
-        o.bytes = (double)Rg * gf.K * 2 + (double)gf.Cout * gf.K * 2 + (double)Rg * vtiles * (8 + 8 * TG_VS_N);
-        o.run = [op](cudaStream_t s) { return tgemm_launch(op, s); };
-        step_prog.back() = std::move(o);                      // replaces the logits version in the beam-search chain
-        bsv.vs_stat = vst;
-        bsv.vs_val = vval;
-        bsv.vs_idx = vidx;
-        bsv.vs_tiles = vtiles;
+        o.name = ln + "_xattn(q2+cross_attn+o2+res+ln)";
+        o.kind = "xattn";
+        o.flops = 2.0 * R * D * D * 2.0 + 4.0 * R * n_base_ * D;          // the two projections + the attention proper
+        o.bytes = (double)B * 2 * 128 * 512 * 2 + (double)R * D * 2 * 2;  // folded per-image operands + activations
+        o.run = [xo](cudaStream_t s) { return xattn_launch(xo, s); };
+        step_prog_.push_back(std::move(o));
+        prob_at = step_prog_.size();
+      } else {
+        RC(dense(ln + "_q2", w.out1, w.gq2, ACT_NONE, w.q2));
+        {
+          Act qa = w.q2.a, oa = w.att2.a, ka = ckv.a;
+          const int kcx = l * 2 * D, vcx = l * 2 * D + D, tk = n_base_;
+          step_prog_.push_back(ew_op(ln + "_cross_attn", [=](cudaStream_t s) { return launch_dec_cross_attention(qa, ka, kcx, vcx, R, N, tk, H, oa, s); },
+                                     (double)B * tk * 2 * D * 2, "attention"));
+          prob_at = step_prog_.size();
+        }
+        RC(dense_res_ln(ln + "_o2+res", ln + "_ln2", w.att2, w.go2, w.out1, w.lnp[2], w.lnp[3], w.out2));
       }
       {
-        Op o = ew_op("beam_step" + sfx, [=](cudaStream_t s) { return launch_beam_step(bsv, lg, V, em, s); },
-                     vstats ? (double)Rg * vtiles * (8 + 8 * TG_VS_N) + (double)Rg * (T + 1) * 8
-                            : (double)Rg * V * 4 + (double)Rg * (T + 1) * 8, "beam");
-        o.idempotent = false;
-        step_prog.push_back(std::move(o));
+        DecProbArgs pa{};
+        pa.qkv = w.qkv.a;
+        pa.kc = w.kc.a;
+        pa.anc = anc;
+        pa.anc_stride = (size_t)R * T;
+        pa.T = T;
+        pa.q = xattn ? w.out1.a : w.q2.a;
+        pa.kv = ckv.a;
+        pa.k_col = l * 2 * D;
+        pa.Mt = xattn ? xMt + (size_t)l * B * 128 * 512 : nullptr;
+        pa.sbias = xattn ? xSb + (size_t)l * B * 128 : nullptr;
+        pa.n_mem = n_base_;
+        pa.step = bs_.step;
+        pa.N = N;
+        pa.heads = H;
+        const int nm = n_base_;
+        // output pointers and row count are those of the decode_logits call that runs the program
+        Op o = ew_op(ln + "_attn_probs",
+                     [=](cudaStream_t s) {
+                       DecProbArgs q = pa;
+                       const size_t tl = (size_t)attn_tlen_;
+                       q.tlen = attn_tlen_;
+                       q.self_out = attn_self_ ? attn_self_ + (size_t)l * B * H * tl * tl : nullptr;
+                       q.cross_out = attn_cross_ ? attn_cross_ + (size_t)l * B * H * tl * nm : nullptr;
+                       return launch_dec_attention_probs(q, B, s);
+                     },
+                     (double)B * H * (T / 2 + nm) * D * 2, "attention");
+        prob_ops.emplace_back(prob_at, std::move(o));
       }
-      if (Bg == B) {
-        step_beam_at_ = step_prog.size() - 1;
-        step_bsv_ = bsv;
+      RC(dense(ln + "_ffn1", w.out2, w.g1, ACT_LEAKY, w.hdn));
+      RC(dense_res_ln(ln + "_ffn2+res", ln + "_ln3", w.hdn, w.g2, w.out2, w.lnp[4], w.lnp[5], w.out3));
+      // per-layer decoder states of the last executed step (parity taps, same names in the fused decoder)
+      taps_[ln + "_out1"] = w.out1;
+      taps_[ln + "_out2"] = w.out2;
+      taps_[ln + "_out3"] = w.out3;
+      x = w.out3;
+    }
+    float* lg = logits_;
+    if (use_tgemm_) RC(add_dense(step_prog_, "final_layer", x, gf, ACT_NONE, nullptr, none, lg, V));
+    else RC(add_conv(step_prog_, "final_layer", x, gf, 1, 1, 0, 0, ACT_NONE, RES_NONE, nullptr, none, lg, V));
+    // teacher forcing: embed the forced token, then the shared layer stack
+    step_forced_prog_ = embed_prog_;
+    step_forced_prog_.insert(step_forced_prog_.end(), step_prog_.begin(), step_prog_.end());
+    step_attn_prog_ = embed_prog_;   // the same launches with the probability kernels after the operands they read
+    size_t k = 0;
+    for (size_t i = 0; i < step_prog_.size(); ++i) {
+      step_attn_prog_.push_back(step_prog_[i]);
+      for (; k < prob_ops.size() && prob_ops[k].first == i + 1; ++k) step_attn_prog_.push_back(prob_ops[k].second);
+    }
+    // Logits-free decode tail (bf16 mode, log scores, beam <= 8, wide Dense kernels): the beam-search chain replaces the
+    // vocabulary projection's [rows][V] fp32 output (20.5 MB written and read back per step at C2) by per-tile softmax
+    // partials + 8 candidates (2.9 MB); teacher forcing (decode_logits) keeps the logits version built above.
+    const int vtiles = (V + TG_BM - 1) / TG_BM;
+    const bool want_wide = (cfg_.kernel_opts & FPNMT_OPT_TGEMM_WIDE) || (cfg_.lanes >= 2 && !(cfg_.kernel_opts & FPNMT_OPT_NO_TGEMM_WIDE));
+    const bool vstats = use_tgemm_ && want_wide && !split_ && !bs_.prob_mode && N <= TG_VS_N && vtiles <= 192 &&
+                        !(cfg_.kernel_opts & FPNMT_OPT_NO_VSTATS);
+    BeamState bsv = bs_;
+    if (vstats) {
+      float2* vst = (float2*)dalloc((size_t)R * vtiles * sizeof(float2));
+      float* vval = (float*)dalloc((size_t)R * vtiles * TG_VS_N * sizeof(float));
+      int* vidx = (int*)dalloc((size_t)R * vtiles * TG_VS_N * sizeof(int));
+      if (!vst || !vval || !vidx) return FPNMT_ERR_CUDA;
+      TgemmOp op;
+      RC(make_tgemmw_op(&op, R, x.a, gf.w, gf.Cout, gf.K, gf.bias, ACT_NONE, none.a, nullptr, 0, nullptr, nullptr, nullptr, 1e-6f,
+                        num_sms_, vst, vval, vidx));
+      op.p.dbg = dbg_timeline("final_layer");
+      Op o;
+      o.name = "final_layer(softmax partials + candidates)";
+      o.kind = "tgemm";
+      o.flops = op.flops;
+      o.bytes = (double)R * gf.K * 2 + (double)gf.Cout * gf.K * 2 + (double)R * vtiles * (8 + 8 * TG_VS_N);
+      o.run = [op](cudaStream_t s) { return tgemm_launch(op, s); };
+      step_prog_.back() = std::move(o);                      // replaces the logits version in the beam-search chain
+      bsv.vs_stat = vst;
+      bsv.vs_val = vval;
+      bsv.vs_idx = vidx;
+      bsv.vs_tiles = vtiles;
+    }
+    {
+      Op o = ew_op("beam_step", [=](cudaStream_t s) { return launch_beam_step(bsv, lg, V, em, s); },
+                   vstats ? (double)R * vtiles * (8 + 8 * TG_VS_N) + (double)R * (T + 1) * 8
+                          : (double)R * V * 4 + (double)R * (T + 1) * 8, "beam");
+      o.idempotent = false;
+      step_prog_.push_back(std::move(o));
+    }
+    step_beam_at_ = step_prog_.size() - 1;
+    step_bsv_ = bsv;
+    if (physical) {
+      // KV-cache reorder by beam parent, all layers and K / V in one bandwidth-bound launch (north-star item 3)
+      std::vector<const bf16*> hp(2 * 2 * L);
+      for (int l = 0; l < L; ++l) {
+        hp[2 * l] = lw[l].kc.a.p;
+        hp[2 * l + 1] = lw[l].vc.a.p;
+        hp[2 * L + 2 * l] = lw[l].kc2.a.p;
+        hp[2 * L + 2 * l + 1] = lw[l].vc2.a.p;
       }
-      if (physical) {
-        // KV-cache reorder by beam parent, all layers and K / V in one bandwidth-bound launch (north-star item 3)
-        std::vector<const bf16*> hp(2 * 2 * L);
-        for (int l = 0; l < L; ++l) {
-          hp[2 * l] = lw[l].kc.a.p;
-          hp[2 * l + 1] = lw[l].vc.a.p;
-          hp[2 * L + 2 * l] = lw[l].kc2.a.p;
-          hp[2 * L + 2 * l + 1] = lw[l].vc2.a.p;
-        }
-        const bf16** dp = (const bf16**)dalloc(hp.size() * sizeof(bf16*));
-        if (!dp) return FPNMT_ERR_CUDA;
-        FPNMT_CUDA_OK(cudaMemcpy(dp, hp.data(), hp.size() * sizeof(bf16*), cudaMemcpyHostToDevice));
-        const int row_bytes = lw[0].kc.a.ld * 2;
-        const int* par = bs.parent_out;
-        const int* step = bs.step;
-        Op o = ew_op("kv_reorder_physical", [=](cudaStream_t s) { return launch_kv_reorder(dp, 2 * L, par, R, R, N, T, row_bytes, step, s); },
-                     2.0 * 2 * L * (double)R * (T / 2 + 1) * row_bytes, "kvreorder");
-        o.idempotent = false;
-        step_prog.push_back(std::move(o));
-      }
-      return 0;
-    };
-    bs_.dbg = dbg_timeline("beam_step");
-    RC(build_chain(0, B, bs_, embed_prog_, step_prog_, &beam_embed_));
-
-    // ---- decoder groups (opt-in, FPNMT_DEC_GROUPS=G): G independent chains over image slices, run as parallel branches
-    // of the decode graph.  Measured on C2 (B200): a half-batch chain alone takes 331 us per step against 385 us for the
-    // whole batch, but two of them co-running take 374 us (four quarter chains: 373 us) - about 1 % faster than one
-    // chain, so the default stays one chain.
-    int G = cfg_.dec_groups;
-    G = std::max(1, std::min(std::min(G, 8), B));
-    if (G > 1) {
-      groups_.resize(G);
-      for (int g = 0; g < G; ++g) {
-        DecGroup& dg = groups_[g];
-        dg.b0 = (int)((long long)g * B / G);
-        dg.Bg = (int)((long long)(g + 1) * B / G) - dg.b0;
-        const int b0 = dg.b0, r0 = b0 * N;
-        BeamState st = bs_;
-        st.B = dg.Bg;
-        st.Btot = B;
-        for (int i = 0; i < 2; ++i) {
-          st.score[i] = bs_.score[i] + r0;
-          st.seq[i] = bs_.seq[i] + (size_t)r0 * (T + 1);
-          st.anc[i] = bs_.anc[i] + (size_t)r0 * T;
-          st.rep[i] = bs_.rep[i] ? bs_.rep[i] + r0 : nullptr;
-        }
-        st.last_tok = bs_.last_tok + r0;
-        st.step = (int*)dalloc(16);
-        st.n_done = (int*)dalloc(16);
-        if (!st.step || !st.n_done) return FPNMT_ERR_CUDA;
-        st.done = bs_.done + b0;
-        st.img_count = bs_.img_count + b0;
-        st.out_ids = bs_.out_ids + (size_t)b0 * T;
-        st.out_len = bs_.out_len + b0;
-        st.cand_val = bs_.cand_val + (size_t)r0 * N;
-        st.cand_idx = bs_.cand_idx + (size_t)r0 * N;
-        st.step_logprob = bs_.step_logprob + b0;
-        st.parent_out = bs_.parent_out + r0;
-        st.token_out = bs_.token_out + r0;
-        dg.bs = st;
-        RC(build_chain(dg.b0, dg.Bg, dg.bs, dg.embed, dg.step, nullptr));
-      }
+      const bf16** dp = (const bf16**)dalloc(hp.size() * sizeof(bf16*));
+      if (!dp) return FPNMT_ERR_CUDA;
+      FPNMT_CUDA_OK(cudaMemcpy(dp, hp.data(), hp.size() * sizeof(bf16*), cudaMemcpyHostToDevice));
+      const int row_bytes = lw[0].kc.a.ld * 2;
+      const int* par = bs_.parent_out;
+      const int* step = bs_.step;
+      Op o = ew_op("kv_reorder_physical", [=](cudaStream_t s) { return launch_kv_reorder(dp, 2 * L, par, R, R, N, T, row_bytes, step, s); },
+                   2.0 * 2 * L * (double)R * (T / 2 + 1) * row_bytes, "kvreorder");
+      o.idempotent = false;
+      step_prog_.push_back(std::move(o));
     }
   }
   return 0;
@@ -1465,7 +1402,6 @@ int Engine::build_dstep(const Tensor& ckv, const float* d_emb, const float* d_po
   }
   p.st = bs_;
   p.mode = 0;
-  p.exp = cfg_.reserved[0];
   p.timeline = dbg_timeline("dstep");
   RC(dstep_set_attributes());
   // one-step op for the per-op profiler (the product decode is ONE launch of all steps)
@@ -1532,45 +1468,6 @@ int Engine::capture(Program& p, cudaGraphExec_t* out) {
   if (rc) return rc;
   FPNMT_CUDA_OK(e);
   FPNMT_CUDA_OK(cudaGraphInstantiate(out, g, 0));
-  FPNMT_CUDA_OK(cudaGraphDestroy(g));
-  return 0;
-}
-
-// Decode graph with decoder groups: the chains of the groups are captured on separate streams between a fork and a
-// join event, so the graph holds G independent branches (each a programmatic-launch chain of embed + T steps).
-int Engine::capture_groups(int T) {
-  const size_t G = groups_.size();
-  if (!fork_ev_) FPNMT_CUDA_OK(cudaEventCreateWithFlags(&fork_ev_, cudaEventDisableTiming));
-  while (grp_streams_.size() + 1 < G) {
-    cudaStream_t st;
-    cudaEvent_t ev;
-    FPNMT_CUDA_OK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    FPNMT_CUDA_OK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    grp_streams_.push_back(st);
-    join_ev_.push_back(ev);
-  }
-  cudaGraph_t g;
-  FPNMT_CUDA_OK(cudaStreamBeginCapture(cap_stream_, cudaStreamCaptureModeThreadLocal));
-  int rc = 0;
-  cudaError_t ce = cudaEventRecord(fork_ev_, cap_stream_);
-  for (size_t i = 0; i < G && !rc && ce == cudaSuccess; ++i) {
-    cudaStream_t st = i == 0 ? cap_stream_ : grp_streams_[i - 1];
-    if (i > 0) ce = cudaStreamWaitEvent(st, fork_ev_, 0);
-    for (auto& op : groups_[i].embed)
-      if (!rc) rc = op.run(st);
-    for (int t = 0; t < T && !rc; ++t)
-      for (auto& op : groups_[i].step) {
-        rc = op.run(st);
-        if (rc) break;
-      }
-    if (i > 0 && ce == cudaSuccess) ce = cudaEventRecord(join_ev_[i - 1], st);
-  }
-  for (size_t i = 1; i < G && ce == cudaSuccess; ++i) ce = cudaStreamWaitEvent(cap_stream_, join_ev_[i - 1], 0);
-  cudaError_t e = cudaStreamEndCapture(cap_stream_, &g);
-  if (rc) return rc;
-  FPNMT_CUDA_OK(ce);
-  FPNMT_CUDA_OK(e);
-  FPNMT_CUDA_OK(cudaGraphInstantiate(&loop_graph_, g, 0));
   FPNMT_CUDA_OK(cudaGraphDestroy(g));
   return 0;
 }
@@ -1834,15 +1731,6 @@ int Engine::decode(int32_t* out_ids, int32_t* out_len, int on_host, int early_st
         if (done) break;
       }
     }
-  } else if (cfg_.use_graphs && !early_stop && groups_.size() > 1) {
-    // fixed-length decode with decoder groups: ONE graph = fork -> per group (step-0 embedding, T steps) -> join
-    RC(launch_beam_init(bs_, cfg_.true_beam, s));            // whole-batch state (outputs, flags) ...
-    for (auto& g : groups_) RC(launch_beam_init(g.bs, cfg_.true_beam, s));   // ... and every group's own step counters
-    launches += 1 + (int64_t)groups_.size();
-    RC(run_program(dec_init_prog_, s));
-    if (!loop_graph_) RC(capture_groups(T));
-    FPNMT_CUDA_OK(cudaGraphLaunch(loop_graph_, s));
-    for (auto& g : groups_) launches += (int64_t)g.embed.size() + (int64_t)T * (int64_t)g.step.size();
   } else {
   RC(launch_beam_init(bs_, cfg_.true_beam, s));
   launches += 1;
@@ -2271,17 +2159,9 @@ int Engine::profile(int iters, char* buf, size_t cap) {
   RC(profile_program(dec_init_prog_, iters, json, "decode_init"));
   json += ", ";
   RC(profile_program(step_prog_, iters, json, "decode_step"));
-  if (groups_.size() > 1) {   // the chain of ONE decoder group (the fixed-length decode runs groups_.size() of them concurrently)
-    DecGroup& g0 = groups_[0];
-    RC(launch_beam_init(g0.bs, cfg_.true_beam, s));
-    RC(run_program(g0.embed, s));
-    for (int t = 0; t < warm; ++t) RC(run_program(g0.step, s));
-    json += ", ";
-    RC(profile_program(g0.step, iters, json, "decode_group_step"));
-  }
   char tail[240];
-  snprintf(tail, sizeof tail, ", \"decode_step_t\": %d, \"decode_groups\": %d, \"device_bytes\": %zu, \"dstep_groups_per_launch\": %d}", warm,
-           (int)std::max<size_t>(1, groups_.size()), alloc_bytes_, use_dstep_ ? dstep_max_groups(num_sms_) : 0);
+  snprintf(tail, sizeof tail, ", \"decode_step_t\": %d, \"device_bytes\": %zu, \"dstep_groups_per_launch\": %d}", warm,
+           alloc_bytes_, use_dstep_ ? dstep_max_groups(num_sms_) : 0);
   json += tail;
   FPNMT_CUDA_OK(cudaStreamSynchronize(s));
   if (dbg_buf_ && use_dstep_ && dsp_.timeline) {   // FPNMT_DBG_OP=dstep: phase stamps of the last profiled step (cluster 0, CTA 0)

@@ -49,12 +49,6 @@ struct Op {
 };
 typedef std::vector<Op> Program;
 
-struct DecGroup {        // one independent decode chain over the images [b0, b0 + Bg) of the batch
-  int b0 = 0, Bg = 0;
-  BeamState bs{};
-  Program embed, step;
-};
-
 class Engine {
  public:
   Engine(const fpnmt_config& cfg, int device);
@@ -90,7 +84,6 @@ class Engine {
   int beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty, int32_t* out_ids,
                   int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s);
   int profile(int iters, char* buf, size_t cap);
-  int capture_groups(int T);
   int build_dstep(const Tensor& ckv, const float* d_emb, const float* d_pos);
   int get_tap_f32(const std::string& name, float* out, size_t cap, size_t* count, cudaStream_t s);
   int add_stem(Program& p, const std::string& name, int kh, int pad, int cout, const GemmW& gw, int Kp, int act, const Tensor& out);
@@ -153,10 +146,6 @@ class Engine {
   int build_score(int t, Program& p);
   BeamEmbed beam_embed_{};
   cudaGraphExec_t cnn_graph_ = nullptr, enc_graph_ = nullptr, step_graph_ = nullptr, loop_graph_ = nullptr;
-  std::vector<DecGroup> groups_;          // decoder groups (empty: the whole batch is one chain)
-  std::vector<cudaStream_t> grp_streams_; // capture streams of groups 1..G-1
-  cudaEvent_t fork_ev_ = nullptr;
-  std::vector<cudaEvent_t> join_ev_;
   cudaStream_t cap_stream_ = nullptr;
 
   // buffers referenced at run time

@@ -98,7 +98,6 @@ int launch_dec_attention_probs(const DecProbArgs& a, int B, cudaStream_t s);
 // ---- beam.cu ------------------------------------------------------------------------------------
 struct BeamState {
   int B, N, V, T;            // images, beam width, vocab, max steps
-  int Btot;                  // images of the whole batch when this state is a slice of it (stride of the [T][..] logs)
   int start_id, end_id;
   int prob_mode;             // 1: product of probabilities (reference), 0: sum of log-probs
   float* score[2];           // [B*N] double-buffered beam scores

@@ -349,7 +349,7 @@ int check_sampling(const fpnmt_sampling& sp, int V) {
 }
 
 int launch_sample_init(const SampleState& st, int* anc, cudaStream_t s) {
-  FPNMT_CUDA_OK(launch_k_small(k_sample_init, dim3(148), dim3(256), 0, s, st, anc));
+  FPNMT_CUDA_OK(launch_k(k_sample_init, dim3(148), dim3(256), 0, s, st, anc));
   return 0;
 }
 
@@ -359,7 +359,7 @@ int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t 
     set_last_error("sample_step: vocabulary must be 1 .. 51200 and rows >= 1");
     return 1;
   }
-  FPNMT_CUDA_OK(launch_k_small(k_sample_step, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits));
+  FPNMT_CUDA_OK(launch_k(k_sample_step, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits));
   return 0;
 }
 

@@ -69,10 +69,8 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
   const bool is_ln = p.gamma != nullptr;
 
   const int item = blockIdx.x;
-  const int per_rt = p.ftiles * p.ksplit;            // CTAs per row group (== cluster size in the LayerNorm variants)
-  const int ftile = (item % per_rt) % p.ftiles;
-  const int ks = (item % per_rt) / p.ftiles;         // which half of the K range (split-K)
-  const int rgroup = item / per_rt;
+  const int ftile = item % p.ftiles;                 // the ftiles CTAs of a row group form the LayerNorm cluster
+  const int rgroup = item / p.ftiles;
   const int rt0 = rgroup * p.rt_per_item;
   const int rt1 = min(p.rtiles, rt0 + p.rt_per_item);
   const int kiters = p.nterms * p.kchunks;
@@ -122,20 +120,14 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
   // critical path of a latency-bound kernel, so one wait / one commit per 16 tcgen05.mma instead of per 4.
   constexpr int G = 4;                             // k-chunks per group
   constexpr int NG = TG_A_SLOTS / G;               // groups resident per operand (2)
-  const int ngroups_all = (kiters + G - 1) / G;
-  const int g_begin = ks * (ngroups_all / p.ksplit);           // this CTA's groups: [g_begin, g_begin + ngroups)
-  const int ngroups = p.ksplit == 1 ? ngroups_all : ngroups_all / p.ksplit;
-  // Single-tile K = 512 kernels (every decoder projection): the two activation groups are issued by two different
-  // threads (TMA warp: group 0, first epilogue warp: group 1) so that the second group's four TMA instructions do not
-  // queue behind the first group's in one thread's instruction stream (~80 ns per TMA issue on the critical path).
-  const bool helper_b = false;   // measured slower on B200 (qkv 6.7 -> 7.6 us): a second issuing thread does not help
+  const int ngroups = (kiters + G - 1) / G;
   if (warp == 0) {
     // ---------------------------------------------------------------------------------- TMA producer
     // convergent warp, one elected lane issues (see umma_bf16_pred in common.cuh)
     const uint32_t leader = elect_one() ? 1u : 0u;
     {
-      auto load_a_group = [&](int g, int slot) {   // chunks (g_begin+g)*G .. of the weight panel -> A slots slot*G ..
-        const int c0 = (g_begin + g) * G, n = min(G, kiters - c0);
+      auto load_a_group = [&](int g, int slot) {   // chunks g*G .. of the weight panel -> A slots slot*G ..
+        const int c0 = g * G, n = min(G, kiters - c0);
         mbar_expect_tx_pred(&fullA[slot], n * TG_A_BYTES, leader);
         int term = c0 / p.kchunks, kc = c0 % p.kchunks;
         for (int i = 0; i < n; ++i) {
@@ -159,12 +151,8 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
             ++gA;
           }
           const int sb = gB % NG;
-          if (helper_b && g == 1) {                // group 1 of the activation panel is issued by an epilogue warp
-            ++gB;
-            continue;
-          }
           if (gB >= NG) mbar_wait(&emptyB[sb], ((gB / NG) & 1) ^ 1);
-          const int c0 = (g_begin + g) * G, n = min(G, kiters - c0);
+          const int c0 = g * G, n = min(G, kiters - c0);
           mbar_expect_tx_pred(&fullB[sb], n * B_BYTES, leader);
           int term = c0 / p.kchunks, kc = c0 % p.kchunks;
           for (int i = 0; i < n; ++i) {
@@ -202,7 +190,7 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
           tc_fence_after();
           if (g == 0 && rt == rt0 && leader) DBG(3);
           if (g == 0 && rt > rt0 && rt - rt0 <= 4 && leader) DBG(8 + (rt - rt0));
-          const int n = min(G, kiters - (g_begin + g) * G);
+          const int n = min(G, kiters - g * G);
           const uint64_t adesc0 = umma_desc_sw128(smem_u32(sA + sa * G * TG_A_BYTES));
           const uint64_t bdesc0 = umma_desc_sw128(smem_u32(sB + sb * G * B_BYTES));
           if (n == G) {                            // full group: 16 back-to-back MMAs, descriptors advance by constants
@@ -240,7 +228,7 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
     const int quarter = warp & 3;           // TMEM lane window of this warp
     const int fl = quarter * 32 + lane;     // phase A: feature within the tile == TMEM lane
     const int f = ftile * TG_BM + fl;
-    const float bias = (p.bias && f < p.F && ks == 0) ? __ldg(p.bias + f) : 0.f;   // split-K: added once (ks == 0)
+    const float bias = (p.bias && f < p.F) ? __ldg(p.bias + f) : 0.f;
     const int fo = ftile * TG_BM + e * 32;  // phase B: first of this thread's 32 features
     int acc = 0;
     uint32_t acc_phase = 0;
@@ -251,15 +239,6 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
       asm volatile("cp.async.commit_group;" ::: "memory");
     }
     pdl_wait();
-    if (helper_b && e == 0 && lane == 0) {
-      const int n = kiters - G;
-      mbar_expect_tx(&fullB[1], n * B_BYTES);
-      int term = G / p.kchunks, kc = G % p.kchunks;
-      for (int i = 0; i < n; ++i) {
-        tma_load_2d(sB + (G + i) * B_BYTES, term == 2 ? &tmX_lo : &tmX_hi, &fullB[1], kc * TG_BK, rt0 * BN);
-        if (++kc == p.kchunks) { kc = 0; ++term; }
-      }
-    }
     __syncwarp();
     for (int rt = rt0; rt < rt1; ++rt) {
 #pragma unroll 1
@@ -269,7 +248,7 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
         uint4 rh[4], rl[4];
 #pragma unroll
         for (int g = 0; g < 4; ++g) rh[g] = rl[g] = make_uint4(0u, 0u, 0u, 0u);
-        if (p.has_res && row_ok && ks == 0) {   // in flight while the MMAs of the tile are still running
+        if (p.has_res && row_ok) {   // in flight while the MMAs of the tile are still running
           const bf16* q = p.res.p + (size_t)row * p.res.ld + fo;
 #pragma unroll
           for (int g = 0; g < 4; ++g)
@@ -331,24 +310,6 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
         for (int i = 0; i < 8; ++i) {
           const float4 q4 = *reinterpret_cast<const float4*>(sLN + lane * TG_LN_STRIDE + e * 32 + i * 4);
           x[4 * i] = q4.x; x[4 * i + 1] = q4.y; x[4 * i + 2] = q4.z; x[4 * i + 3] = q4.w;
-        }
-        if (p.ksplit == 2) {                 // split-K: add the partial sums of the CTA that owns the other K half
-          cluster_sync_all();                // #0: both halves' partial tiles are in their shared-memory scratch
-          if (ks == 0) {
-            uint32_t peer;
-            asm volatile("mapa.shared::cluster.u32 %0, %1, %2;"
-                         : "=r"(peer) : "r"(smem_u32(sLN + lane * TG_LN_STRIDE + e * 32)), "r"((uint32_t)(ftile + p.ftiles)));
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-              float y;
-              asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(y) : "r"(peer + 4 * i) : "memory");
-              x[i] += y;
-            }
-          } else {                           // ks == 1: its work is done; keep its shared memory alive until #2
-            cluster_sync_all();
-            cluster_sync_all();
-            continue;
-          }
         }
         if (p.has_res) {
 #pragma unroll
@@ -449,7 +410,6 @@ tgemm_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CU
     }
   }
   if (is_ln && warp < 2) {   // the TMA / MMA warps take part in the cluster barriers of the LN epilogue
-    if (p.ksplit == 2) cluster_sync_all();
     cluster_sync_all();
     cluster_sync_all();
   }
@@ -507,7 +467,7 @@ int tgemm_set_attributes() {
 
 int make_tgemm_op(TgemmOp* op, int R, const Act& x, const bf16* wt, int F, int K, bool split, const float* bias, int act,
                   const Act& out, float* out_f32, int ld_f32, const Act* res, const float* gamma, const float* beta,
-                  float eps, int num_sms, int force_bn, bool ksplit2) {
+                  float eps, int num_sms, int force_bn) {
   TgemmParams& p = op->p;
   p = TgemmParams{};
   if (x.C != K) {
@@ -539,13 +499,6 @@ int make_tgemm_op(TgemmOp* op, int R, const Act& x, const bf16* wt, int F, int K
   p.rt_per_item = (p.rtiles + rgroups - 1) / rgroups;
   rgroups = (p.rtiles + p.rt_per_item - 1) / p.rt_per_item;
   p.stationary = (p.nterms * p.kchunks <= TG_A_SLOTS) ? 1 : 0;
-  p.ksplit = 1;
-  {
-    const int groups_all = (p.nterms * p.kchunks + 3) / 4;
-    // Split-K over an 8-CTA cluster is implemented and parity-tested (FPNMT_OPT_KSPLIT2) but OFF by default: on B200 the
-    // 8-CTA clusters of 211 KB CTAs schedule so much later that FFN2 went from 12 us to 25 us.
-    if (ksplit2 && ln && !p.stationary && groups_all >= 4 && groups_all % 2 == 0) p.ksplit = 2;
-  }
   p.bias = bias;
   p.act = act;
   p.out = out;
@@ -558,8 +511,8 @@ int make_tgemm_op(TgemmOp* op, int R, const Act& x, const bf16* wt, int F, int K
   p.eps = eps;
   op->BN = BN;
   op->wide = 0;
-  op->grid = p.ftiles * p.ksplit * rgroups;
-  op->cluster = ln ? 4 * p.ksplit : 1;
+  op->grid = p.ftiles * rgroups;
+  op->cluster = ln ? 4 : 1;
   op->flops = 2.0 * (double)R * (double)F * (double)K;
   const uint64_t kw_total = split ? 2 * (uint64_t)K : (uint64_t)K;
   int rc = encode_tmap_2d(&op->tmW, wt, kw_total, (uint64_t)F, kw_total, TG_BM);

@@ -29,8 +29,6 @@ struct TgemmParams {
   int ftiles, rtiles;    // ceil(F / 128), ceil(R / BN)
   int rt_per_item;       // row tiles handled by one CTA (consecutive)
   int stationary;        // 1: the weight panel (<= 8 chunks) stays in shared memory for all row tiles of the CTA
-  int ksplit;            // 1, or 2: the K range is split over two CTAs of the (8-CTA) LayerNorm cluster, partial sums
-                         // are added through distributed shared memory (long-K layers: FFN2, K = 2048)
   const float* bias;     // [F] (padded to a multiple of 128) or nullptr
   int act;
   Act out;               // bf16 output view [R][ld] (p may be nullptr)
@@ -56,7 +54,7 @@ struct TgemmOp {
   int BN;        // 32 or 64 (tgemm_kernel); 64 or 128 (tgemmw_kernel)
   int wide;      // 1: tgemmw_kernel (tgemmw.cu)
   int grid;
-  int cluster;   // 1, 4 (LayerNorm) or 8 (LayerNorm + split-K)
+  int cluster;   // 1, or 4 (LayerNorm)
   double flops;
 };
 
@@ -67,7 +65,7 @@ int tgemm_set_attributes();
 // x: activation view [R][ld] (C == K); wt: [F][K] bf16 (split: [F][2K]).  BN = 0 selects automatically.
 int make_tgemm_op(TgemmOp* op, int R, const Act& x, const bf16* wt, int F, int K, bool split, const float* bias, int act,
                   const Act& out, float* out_f32, int ld_f32, const Act* res, const float* gamma, const float* beta,
-                  float eps, int num_sms, int force_bn = 0, bool ksplit2 = false);
+                  float eps, int num_sms, int force_bn = 0);
 
 // Wide-row, two-CTAs-per-SM variant (tgemmw.cu): BN = 128 rows per CTA, K streamed through a 96 KB ring, bf16 mode only.
 size_t tgemmw_smem_bytes(int BN);

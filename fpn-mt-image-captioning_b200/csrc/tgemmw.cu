@@ -559,7 +559,6 @@ int make_tgemmw_op(TgemmOp* op, int R, const Act& x, const bf16* wt, int F, int 
   p.rt_per_item = (p.rtiles + rgroups - 1) / rgroups;
   rgroups = (p.rtiles + p.rt_per_item - 1) / p.rt_per_item;
   p.stationary = 0;
-  p.ksplit = 1;
   p.bias = bias;
   p.act = act;
   p.out = out;

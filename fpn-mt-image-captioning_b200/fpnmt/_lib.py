@@ -18,8 +18,7 @@ SCORE_IDS = {"log": 0, "prob": 1}
 CACHE_IDS = {"ancestry": 0, "physical": 1}
 DECODE_IDS = {"auto": 0, "chain": 1, "fused": 2}
 # fpnmt_config.kernel_opts bits (include/fpnmt.h FPNMT_OPT_*): each switches one fused kernel back to its unfused equivalent
-OPT_BITS = {"no_xattn": 1, "no_stem": 2, "no_tgemm": 4, "enc_att_simt": 8, "ksplit2": 16, "no_pdl": 32, "pdl_gemm_only": 64,
-            "dstep_taps": 128, "dec_att_simt": 256, "tgemm_wide": 512, "no_tgemm_wide": 1024, "no_kv_share": 2048, "no_vstats": 4096, "no_dense_1x1": 8192, "no_tma_store": 16384, "no_b_stationary": 32768}
+OPT_BITS = {"no_xattn": 1, "no_stem": 2, "no_tgemm": 4, "enc_att_simt": 8, "no_pdl": 32, "dstep_taps": 128, "dec_att_simt": 256, "tgemm_wide": 512, "no_tgemm_wide": 1024, "no_kv_share": 2048, "no_vstats": 4096, "no_dense_1x1": 8192, "no_tma_store": 16384, "no_b_stationary": 32768}
 
 
 class FpnmtConfig(C.Structure):

@@ -43,7 +43,7 @@ class Engine:
                  score_mode: str = "log", start_id: int = cfg.START_ID, end_id: int = cfg.END_ID,
                  true_beam: bool = False, use_graphs: bool = True, device: int = 0, opts: Sequence[str] = (),
                  cache_mode: str = "ancestry", decode_path: str = "auto", length_penalty: float = 0.0,
-                 finished_beams: bool = False, dec_groups: int = 0, lanes: int = 1, _exp: int = 0):
+                 finished_beams: bool = False, lanes: int = 1):
         """opts: names from _lib.OPT_BITS (e.g. "no_xattn") - each turns one fused kernel back into its unfused equivalent;
         cache_mode "ancestry" | "physical"; decode_path "auto" (today: the per-operator chain) | "chain" | "fused" (one
         dstep_kernel launch runs every layer, the vocabulary projection and the beam tail of all steps); length_penalty / finished_beams: flagged extensions, 0 = reference;
@@ -71,10 +71,9 @@ class Engine:
         for o in opts:
             c.kernel_opts |= _lib.OPT_BITS[o]
         c.cache_mode, c.decode_path = _lib.CACHE_IDS[cache_mode], _lib.DECODE_IDS[decode_path]
-        c.length_penalty, c.finished_beams, c.dec_groups = float(length_penalty), int(finished_beams), int(dec_groups)
+        c.length_penalty, c.finished_beams = float(length_penalty), int(finished_beams)
         c.lanes = int(lanes)
         self.lanes = max(1, int(lanes))
-        c.reserved[0] = int(_exp)          # developer A/B switches of the fused decoder (dstep.cuh), 0 in product use
         self._h = C.c_void_p()
         torch.cuda.init()
         with torch.cuda.device(self.device):

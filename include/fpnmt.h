@@ -48,9 +48,7 @@ enum { FPNMT_OPT_NO_XATTN = 1,       /* separate q2 / cross-attention / o2+LN ke
        FPNMT_OPT_NO_STEM = 2,        /* explicit im2col + GEMM stem instead of stem_kernel                              */
        FPNMT_OPT_NO_TGEMM = 4,       /* decoder Dense layers through igemm + separate LayerNorm                         */
        FPNMT_OPT_ENC_ATT_SIMT = 8,   /* CUDA-core encoder attention instead of the tensor-core flash kernel             */
-       FPNMT_OPT_KSPLIT2 = 16,       /* split-K over an 8-CTA cluster for the K = 2048 LayerNorm Dense (slower on B200)  */
        FPNMT_OPT_NO_PDL = 32,        /* no programmatic dependent launch (process-wide: the last created engine wins)    */
-       FPNMT_OPT_PDL_GEMM_ONLY = 64, /* only the tcgen05 GEMM kernels launch early                                      */
        FPNMT_OPT_DEC_ATT_SIMT = 256, /* CUDA-core decode self-attention in bf16 mode (instead of the mma.sync kernel)          */
        FPNMT_OPT_TGEMM_WIDE = 512,   /* bf16 Dense layers on tgemmw_kernel (128 rows per CTA, two CTAs per SM, TMA-store
                                         epilogue: least SM time, best when several lanes share the GPU) even with lanes < 2.
@@ -93,7 +91,7 @@ typedef struct fpnmt_config {
   int32_t true_beam;     /* 0 = reference init (all beams identical, pipeline.py:101-102); 1 = only beam 0 alive  */
   int32_t use_graphs;    /* 1 = replay the encode / decode-step programs as CUDA graphs                          */
   /* ---- the eight words below were `reserved[8]` in ABI 0.1; all-zero selects the defaults ---- */
-  int32_t kernel_opts;   /* FPNMT_OPT_* bit mask                                                                  */
+  int32_t kernel_opts;   /* FPNMT_OPT_* bit mask; a bit not defined above is refused (FPNMT_ERR_INVALID)          */
   int32_t cache_mode;    /* FPNMT_CACHE_*                                                                         */
   int32_t decode_path;   /* FPNMT_DECODE_*                                                                        */
   float length_penalty;  /* EXTENSION (not in the reference): alpha of the length normalisation applied when a beam
@@ -101,12 +99,12 @@ typedef struct fpnmt_config {
   int32_t finished_beams;/* EXTENSION: 1 = a beam that emitted <end> is frozen and competes with its final score;
                             the image stops when its best beam is a finished one.  0 = reference (pipeline.py:143-148:
                             stop the moment the top beam emits <end>, finished lower beams keep decoding)          */
-  int32_t dec_groups;    /* DECODE_CHAIN only: cut the batch into this many concurrently decoded chains (0/1 = one) */
+  int32_t dec_groups;    /* unused, must be 0 or 1 (the batch is decoded as one chain); kept so the layout does not change */
   int32_t lanes;         /* batches in flight (fpnmt_submit / fpnmt_collect): the handle holds this many complete engines
                             (own activations, KV cache, beam state, streams; ONE shared copy of the GEMM weights) on the one GPU, 0/1 = one,
                             at most 16.  Two lanes overlap
                             the throughput-bound encoder of batch i+1 with the latency-bound decode of batch i.            */
-  int32_t reserved[1];
+  int32_t reserved[1];   /* must be 0                                                                               */
 } fpnmt_config;
 
 typedef struct fpnmt_handle fpnmt_handle;

@@ -13,7 +13,7 @@ from fpnmt.weights import init_weights
 def main():
     bb, B, N, V, T = "mobilenet224_1.0", int(os.environ.get("DIAG_B", "64")), 8, 10000, 64
     w = init_weights(bb, vocab=V, seed=0)
-    eng = Engine(w, backbone=bb, batch=B, beam=N, vocab=V, max_len=T, decode_path="fused", _exp=int(os.environ.get("DIAG_EXP", "0")))
+    eng = Engine(w, backbone=bb, batch=B, beam=N, vocab=V, max_len=T, decode_path="fused")
     img = (torch.rand(B, 512, 512, 3) * 2 - 1).cuda()
     eng.generate(img, early_stop=False)
     torch.cuda.synchronize()

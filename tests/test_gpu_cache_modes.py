@@ -48,8 +48,6 @@ def test_physical_mode_is_rejected_where_it_cannot_run():
     w = O.caption_weights(BB, vocab=512, layers=L, seed=1)
     with pytest.raises(FpnmtError):
         Engine(w, backbone=BB, batch=2, beam=4, vocab=512, max_len=8, num_layers=L, image_size=S, cache_mode="physical", decode_path="fused")
-    with pytest.raises(FpnmtError):
-        Engine(w, backbone=BB, batch=4, beam=4, vocab=512, max_len=8, num_layers=L, image_size=S, cache_mode="physical", dec_groups=2)
 
 
 @pytest.mark.parametrize("true_beam,finished", [(False, False), (True, False), (True, True)])

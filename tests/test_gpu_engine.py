@@ -387,24 +387,34 @@ def test_double_buffered_host_input_matches_one_shot_generate():
     eng.close()
 
 
-@pytest.mark.parametrize("groups", [2, 3])
-def test_decoder_groups_match_single_chain(groups):
-    """fpnmt_config.dec_groups (per-operator decode chain) cuts the batch into independent decode chains (parallel branches of the decode graph over row
-    slices of the same buffers): identical ids, lengths and per-step scores as the single chain."""
-    from fpnmt.engine import Engine
-    bb = "mobilenet224_1.0"
-    w = small_weights(bb, V, L, seed=8)
-    img = O.test_images(5, S, seed=12).cuda()
-    res = {}
-    for g in (1, groups):
-        eng = Engine(w, backbone=bb, batch=5, beam=N, vocab=V, max_len=T, num_layers=L, image_size=S, precision="bf16",
-                     use_graphs=True, decode_path="chain", dec_groups=g)
-        res[g] = eng.generate(img, early_stop=False, return_scores=True)
-        again = eng.generate(img, early_stop=False)
-        assert torch.equal(again[0], res[g][0])
-        eng.close()
-    assert torch.equal(res[1][0], res[groups][0]) and torch.equal(res[1][1], res[groups][1])
-    assert torch.allclose(res[1][2].cpu(), res[groups][2].cpu(), rtol=0, atol=0)
+def test_config_words_that_select_nothing_are_refused():
+    """fpnmt_create refuses a dec_groups above 1, a kernel_opts bit that no FPNMT_OPT_* defines (16 and 64 included) and a
+    non-zero reserved word with FPNMT_ERR_INVALID and a message, instead of silently building the default engine."""
+    import ctypes as C
+    from fpnmt import _lib
+    lib = _lib.load()
+
+    def create(**words):
+        c = _lib.FpnmtConfig()
+        c.backbone, c.image_size, c.batch, c.beam, c.vocab, c.max_len = 0, S, B, N, V, T
+        c.num_layers, c.d_model, c.num_heads, c.dff, c.start_id, c.end_id = L, 512, 8, 2048, 2, 3
+        for k, v in words.items():
+            if k == "reserved0":
+                c.reserved[0] = v
+            else:
+                setattr(c, k, v)
+        h = C.c_void_p()
+        rc = lib.fpnmt_create(C.byref(c), 0, C.byref(h))
+        msg = lib.fpnmt_last_error().decode()
+        if rc == _lib.OK:
+            lib.fpnmt_destroy(h)
+        return rc, msg
+
+    assert create(dec_groups=1)[0] == _lib.OK
+    for words, word in (({"dec_groups": 2}, "dec_groups"), ({"kernel_opts": 16}, "kernel_opts"), ({"kernel_opts": 64}, "kernel_opts"),
+                        ({"reserved0": 1}, "reserved")):
+        rc, msg = create(**words)
+        assert rc == _lib.ERR_INVALID and word in msg, (words, rc, msg)
 
 
 @pytest.mark.parametrize("bb", BACKBONES)
