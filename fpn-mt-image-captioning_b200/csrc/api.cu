@@ -170,6 +170,18 @@ FPNMT_API int fpnmt_sample(fpnmt_handle* h, const float* images, int images_on_h
   return h->eng->sample(images, images_on_host, *sampling, out_ids, out_len, out_logprob, outputs_on_host, early_stop,
                         (cudaStream_t)stream);
 }
+FPNMT_API int fpnmt_sample_prefix(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                  const int32_t* prefix_len, int p, const fpnmt_sampling* sampling, int32_t* out_ids,
+                                  int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop, void* stream) {
+  CHECK_H(h);
+  if (!sampling) {
+    set_last_error("sample_prefix: NULL sampling parameters");
+    return FPNMT_ERR_INVALID;
+  }
+  const PrefixArg pa{prefix_ids, prefix_len, p};
+  return h->eng->sample(images, images_on_host, *sampling, out_ids, out_len, out_logprob, outputs_on_host, early_stop,
+                        (cudaStream_t)stream, &pa);
+}
 FPNMT_API int fpnmt_score(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* ids, const int32_t* lens, int t,
                           float* out_logprob, float* out_token_logprob, int outputs_on_host, void* stream) {
   CHECK_H(h);
@@ -187,6 +199,15 @@ FPNMT_API int fpnmt_beam_search_diverse(fpnmt_handle* h, const float* images, in
   CHECK_H(h);
   return h->eng->beam_search(images, images_on_host, beam_groups, diversity, length_penalty, out_ids, out_len, out_logprob,
                              outputs_on_host, early_stop, (cudaStream_t)stream);
+}
+FPNMT_API int fpnmt_beam_search_prefix(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                       const int32_t* prefix_len, int p, int beam_groups, float diversity, float length_penalty,
+                                       int32_t* out_ids, int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
+                                       void* stream) {
+  CHECK_H(h);
+  const PrefixArg pa{prefix_ids, prefix_len, p};
+  return h->eng->beam_search(images, images_on_host, beam_groups, diversity, length_penalty, out_ids, out_len, out_logprob,
+                             outputs_on_host, early_stop, (cudaStream_t)stream, &pa);
 }
 FPNMT_API int fpnmt_stage_images(fpnmt_handle* h, const float* host_images, int slot) {
   CHECK_H(h);
@@ -704,13 +725,17 @@ FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x,
   return o.finish("op_layernorm_rows");
 }
 
-FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
-                                   const float* bias, float* stat, float* val, int32_t* idx, void* stream) {
+}  // extern "C"
+
+// fpnmt_op_vocab_stats and, with target != nullptr, fpnmt_op_vocab_stats_target (tgemmw_target_kernel)
+static int op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F, const float* bias,
+                          const int32_t* target, float* target_logit, float* stat, float* val, int32_t* idx, void* stream) {
   if (precision != FPNMT_PREC_BF16)
     return op_invalid("op_vocab_stats: the logits-free vocabulary projection is a bf16-mode kernel (the wide-row Dense kernel)");
   if (!x || !kernel || !stat || !val || !idx || R < 1 || K < 8 || K % 8 || F < 8 || F % 8 ||
       (((uintptr_t)stat | (uintptr_t)val | (uintptr_t)idx) & 15))
     return op_invalid("op_vocab_stats: bad arguments (K and F multiples of 8, outputs 16-byte aligned)");
+  if ((!target) != (!target_logit)) return op_invalid("op_vocab_stats_target: NULL target / target_logit");
   int rc = op_device(device, "op_vocab_stats");
   if (rc) return rc;
   rc = tgemmw_set_attributes();
@@ -729,8 +754,24 @@ FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, in
   TgemmOp op;
   o.rc = make_tgemmw_op(&op, R, ax, dw, F, K, db, ACT_NONE, none, nullptr, 0, nullptr, nullptr, nullptr, 1e-6f, sms,
                         (float2*)stat, val, idx);
+  op.tgt = target;
+  op.tgt_logit = target_logit;
   if (!o.rc) o.rc = tgemm_launch(op, o.s);
   return o.finish("op_vocab_stats");
+}
+
+extern "C" {
+
+FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                   const float* bias, float* stat, float* val, int32_t* idx, void* stream) {
+  return op_vocab_stats(device, precision, x, R, K, kernel, F, bias, nullptr, nullptr, stat, val, idx, stream);
+}
+
+FPNMT_API int fpnmt_op_vocab_stats_target(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                          const float* bias, const int32_t* target, float* stat, float* val, int32_t* idx,
+                                          float* target_logit, void* stream) {
+  if (!target || !target_logit) return op_invalid("op_vocab_stats_target: NULL target / target_logit");
+  return op_vocab_stats(device, precision, x, R, K, kernel, F, bias, target, target_logit, stat, val, idx, stream);
 }
 
 FPNMT_API int fpnmt_op_sample_step(int device, const float* logits, int rows, int V, int samples_per_image, int t,

@@ -41,6 +41,7 @@ __global__ void k_beam_init(BeamState st, int true_beam, int beam_groups) {
     st.seq[0][(size_t)i * (st.T + 1)] = st.start_id;
     st.last_tok[i] = st.start_id;
     if (st.rep[0]) st.rep[0][i] = i - n;                   // every beam starts from <start>: one history per image
+    if (st.pf.tgt) st.pf.tgt[i] = st.pf.len[i / st.N] > 0 ? st.pf.ids[(size_t)(i / st.N) * st.T] : -1;   // step 0's targets
   }
   for (size_t j = i; j < (size_t)st.B * st.T; j += (size_t)gridDim.x * blockDim.x) st.out_ids[j] = 0;
 }
@@ -77,7 +78,9 @@ __device__ __forceinline__ void warp_argmax(float& v, int& i) {
 //                          index n*V+v), emit parent/token/score, reorder token sequences and the KV ancestry table,
 //                          handle <end>, write the NEXT step's decoder input rows (embedding + position), and let the
 //                          last image advance the device step counter.
-template <int THREADS, bool NBEST = false>
+//   PREFIX (prompted N-best decode, BeamState::pf): at a step inside the image's prefix every row's one candidate is the prefix
+//                          token, scored with the expression of the free branch, and phase 2 keeps every beam on its own row.
+template <int THREADS, bool NBEST = false, bool PREFIX = false>
 __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(BeamState st, const float* __restrict__ logits, int ld, BeamEmbed em) {
   constexpr int NW = THREADS / 32;
   extern __shared__ float4 s_row4[];                       // the row's logits (later: candidate scores), nv4*THREADS float4
@@ -104,6 +107,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
   const float* x = logits + (size_t)row * ld;
   // finished-beam extension: a frozen beam's only candidate is itself (token <end>, score unchanged)
   const bool row_frozen = st.finished_mode && st.fin_len[t & 1][row] > 0;
+  int ftok = -1;                                           // forced token of the image at this step (prompted decode), or -1
+  if constexpr (PREFIX) {
+    if (t < st.pf.len[row / N]) ftok = st.pf.ids[(size_t)(row / N) * T + t];
+  }
   if (row_frozen) {
     if (tid < N) {
       st.cand_val[(size_t)row * N + tid] = tid == 0 ? score : -INFINITY;
@@ -150,6 +157,12 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
 #pragma unroll
     for (int w = 0; w < NW; ++w) sum += s_m[w] > -INFINITY ? s_s[w] * __expf(s_m[w] - m) : 0.f;
     const float lse = m + logf(sum);
+    if (PREFIX && ftok >= 0) {                               // forced step: the prefix token is the row's one candidate
+      if (tid < N) {
+        st.cand_val[(size_t)row * N + tid] = tid == 0 ? score + (__ldcg(st.pf.tgt_logit + row) - lse) : -INFINITY;
+        st.cand_idx[(size_t)row * N + tid] = tid == 0 ? ftok : 0x7fffffff;
+      }
+    } else {
     for (int i = tid; i < nt; i += THREADS) {
       const float g = s_cv[i];
       int rank = 0;
@@ -186,6 +199,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       st.cand_val[(size_t)row * N + tid] = -INFINITY;
       st.cand_idx[(size_t)row * N + tid] = 0x7fffffff;
     }
+    }   // !forced
   } else {
   const int nv4 = (V + 4 * THREADS - 1) / (4 * THREADS);  // float4 slots per thread; slot i of thread tid = elements
   float* s_row = reinterpret_cast<float*>(s_row4);        //   (i*THREADS + tid)*4 .. +3 (conflict-free, coalesced)
@@ -258,6 +272,12 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
   const float lse = m + logf(sum);
   const bool prob = st.prob_mode != 0;
   auto cand = [&](float vv) -> float { return prob ? (expf(vv - m) / sum) * score : score + (vv - lse); };
+  if (PREFIX && ftok >= 0) {                                 // forced step: the prefix token is the row's one candidate
+    if (tid < N) {
+      st.cand_val[(size_t)row * N + tid] = tid == 0 ? cand(s_row[ftok]) : -INFINITY;
+      st.cand_idx[(size_t)row * N + tid] = tid == 0 ? ftok : 0x7fffffff;
+    }
+  } else {
 
   // ---- row-local top-N (tf.math.top_k order: value descending, lower index first).
   // Fast path: the 32 "lane groups" (threads with the same lane id, one per warp) hold 32 disjoint parts of the row; the
@@ -402,6 +422,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       }
     }
   }
+  }   // !forced
   }   // !row_frozen
   __syncthreads();
   if (row == 0) BDBG(5);
@@ -454,6 +475,22 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
     const int G = (int)st.nb.groups[0];
     const float lambda = st.nb.groups[1];
     const int M = N / G, MN = M * N;
+    if (PREFIX && ftok >= 0) {
+      // forced step: new beam n is row n's one candidate (parent = n, the prefix token); no ranking, no penalty
+      if (tid < N) {
+        const int n = tid;
+        const float v = s_fv[n * N];
+        const int fl = st.fin_len[cur][rows0 + n];
+        s_parent[n] = n;
+        s_token[n] = ftok;
+        st.fin_len[nxt][rows0 + n] = fl > 0 ? fl : (ftok == st.end_id ? t + 1 : 0);
+        st.score[nxt][rows0 + n] = v;
+        st.last_tok[rows0 + n] = ftok;
+        if (st.parent_out) st.parent_out[(size_t)t * st.B * N + rows0 + n] = n;
+        if (st.token_out) st.token_out[(size_t)t * st.B * N + rows0 + n] = ftok;
+        if (n == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.B + b] = v;
+      }
+    } else
     for (int g = 0; g < G; ++g) {
       const int c0 = g * MN;
       if (g > 0) {
@@ -514,6 +551,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       if (rank == 0 && st.step_logprob) st.step_logprob[(size_t)t * st.B + b] = v;
     }
   }
+  }
+  if constexpr (PREFIX) {                                    // the token whose logit step t + 1's vocabulary projection reports
+    if (st.pf.tgt && tid < N)
+      st.pf.tgt[rows0 + tid] = t + 1 < st.pf.len[b] ? st.pf.ids[(size_t)b * T + t + 1] : -1;
   }
   __syncthreads();
   BDBG(9);
@@ -637,6 +678,8 @@ int beam_set_attributes() {   // per device (Engine::init)
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<256, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return 0;
 }
 int check_beam_step(const BeamState& st, int ld) {
@@ -659,13 +702,13 @@ int check_beam_step(const BeamState& st, int ld) {
   }
   return 0;
 }
-template <bool NBEST>
+template <bool NBEST, bool PREFIX = false>
 static int launch_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
   if (check_beam_step(st, ld)) return 1;
   if (st.vs_stat) {                                         // logits-free tail: merge the vocabulary projection's candidates
     size_t smem = (size_t)st.vs_tiles * 8 * 8;
     if (smem < 12288) smem = 12288;
-    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST, PREFIX>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
     return 0;
   }
   const int threads = st.V <= 16384 ? 256 : 512;
@@ -673,9 +716,9 @@ static int launch_step(const BeamState& st, const float* logits, int ld, const B
   size_t smem = (size_t)nv4 * threads * 16;
   if (smem < 12288) smem = 12288;                           // phase 2 keeps the N x N merge lists (values, flat ids, keys) there
   if (threads == 256)
-    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST, PREFIX>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
   else
-    FPNMT_CUDA_OK(launch_k(k_beam_step<512, NBEST>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<512, NBEST, PREFIX>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
   return 0;
 }
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
@@ -698,6 +741,67 @@ int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, con
     return 1;
   }
   return launch_step<true>(st, logits, ld, em, s);
+}
+int launch_beam_step_prefix(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+  if (!st.pf.ids || !st.pf.len || (st.vs_stat && (!st.pf.tgt || !st.pf.tgt_logit))) {
+    set_last_error("beam_step_prefix: needs the prefix buffers (and on the logits-free tail the target ids and logits)");
+    return 1;
+  }
+  if (!st.finished_mode || st.prob_mode || !st.nb.ids || !st.nb.len || !st.nb.score || !st.nb.groups) {
+    set_last_error("beam_step_prefix: needs finished beams, log scores, the N-best outputs and the beam-group words");
+    return 1;
+  }
+  return launch_step<true, true>(st, logits, ld, em, s);
+}
+
+// Prompted decode: one block per image copies and checks its prefix (see kernels.cuh)
+__global__ void k_prefix_load(const int* __restrict__ prefix_ids, const int* __restrict__ prefix_len, int p, int T, int V,
+                              int end_id, int* __restrict__ dst_ids, int* __restrict__ dst_len, int* __restrict__ bad) {
+  const int b = blockIdx.x;
+  const int len = prefix_len[b];
+  const bool len_bad = len < 0 || len > p;
+  const int n = len_bad ? 0 : len;
+  int bad_id = 0;
+  for (int j = threadIdx.x; j < T; j += blockDim.x) {
+    int v = 0;
+    if (j < n) {
+      const int id = prefix_ids[(size_t)b * p + j];
+      bad_id |= (id < 0 || id >= V || id == end_id) ? 1 : 0;
+      v = min(max(id, 0), V - 1);
+    }
+    dst_ids[(size_t)b * T + j] = v;
+  }
+  const int any_bad = __syncthreads_or(bad_id) || len_bad;
+  if (threadIdx.x == 0) {
+    bad[b] = any_bad ? 1 : 0;
+    dst_len[b] = any_bad ? 0 : n;
+  }
+}
+int launch_prefix_load(const int* prefix_ids, const int* prefix_len, int p, int B, int T, int V, int end_id, int* dst_ids,
+                       int* dst_len, int* bad, cudaStream_t s) {
+  if (p < 1 || p > T) {
+    set_last_error("prefix_load: prefix width must be 1 .. max_len");
+    return 1;
+  }
+  k_prefix_load<<<B, 128, 0, s>>>(prefix_ids, prefix_len, p, T, V, end_id, dst_ids, dst_len, bad);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+__global__ void k_prefix_flag(const int* __restrict__ bad, int N, int T, int* __restrict__ ids, int* __restrict__ len,
+                              float* __restrict__ logprob) {
+  const int b = blockIdx.x;
+  if (!bad[b]) return;
+  for (int j = threadIdx.x; j < N * T; j += blockDim.x) ids[(size_t)b * N * T + j] = 0;
+  if (threadIdx.x < N) {
+    len[b * N + threadIdx.x] = 0;
+    logprob[b * N + threadIdx.x] = __int_as_float(0x7fc00000);
+  }
+}
+int launch_prefix_flag(const int* bad, int B, int N, int T, int* ids, int* len, float* logprob, cudaStream_t s) {
+  k_prefix_flag<<<B, 128, 0, s>>>(bad, N, T, ids, len, logprob);
+  LAUNCH_CHECK();
+  return 0;
 }
 
 // Physical KV-cache reorder (see kernels.cuh).  grid (rows, ncaches): one block streams the live span of one cache row -

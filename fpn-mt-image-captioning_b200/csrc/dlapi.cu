@@ -289,6 +289,45 @@ FPNMT_API int fpnmt_sample_dl(fpnmt_handle* h, const DLTensor* images, const fpn
                       stream);
 }
 
+// prefix_ids int32 [batch][p] and prefix_len int32 [batch] on the engine's GPU (p = prefix_ids' last dimension; the entry point
+// refuses p outside 1 .. max_len - 1)
+static int dl_prefix(fpnmt_handle* h, const std::string& fn, const DLTensor* prefix_ids, const DLTensor* prefix_len, void** pids,
+                     void** plen, int* p) {
+  const fpnmt_config& c = h->eng->config();
+  int rc = dl_check((fn + ": prefix_ids").c_str(), prefix_ids, kDLInt, h->eng->device(), false, true, {c.batch, -1}, pids, nullptr);
+  if (rc) return rc;
+  *p = (int)prefix_ids->shape[1];
+  return dl_check((fn + ": prefix_len").c_str(), prefix_len, kDLInt, h->eng->device(), false, true, {c.batch}, plen, nullptr);
+}
+
+FPNMT_API int fpnmt_sample_prefix_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids, const DLTensor* prefix_len,
+                                     const fpnmt_sampling* sampling, DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob,
+                                     int early_stop, void* stream) {
+  CHECK_H(h);
+  void *pi = nullptr, *pp = nullptr, *pl = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
+  int img_host = 0, ids_host = 0, p = 0;
+  int rc = dl_images_opt(h, "sample_prefix_dl", images, &pi, &img_host);
+  if (!rc) rc = dl_prefix(h, "sample_prefix_dl", prefix_ids, prefix_len, &pp, &pl, &p);
+  if (!rc) rc = dl_captions(h, "sample_prefix_dl", out_ids, out_len, out_logprob, &pids, &plen, &plp, &ids_host);
+  if (rc) return rc;
+  return fpnmt_sample_prefix(h, (const float*)pi, img_host, (const int32_t*)pp, (const int32_t*)pl, p, sampling, (int32_t*)pids,
+                             (int32_t*)plen, (float*)plp, ids_host, early_stop, stream);
+}
+
+FPNMT_API int fpnmt_beam_search_prefix_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
+                                          const DLTensor* prefix_len, int beam_groups, float diversity, float length_penalty,
+                                          DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream) {
+  CHECK_H(h);
+  void *pi = nullptr, *pp = nullptr, *pl = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
+  int img_host = 0, ids_host = 0, p = 0;
+  int rc = dl_images_opt(h, "beam_search_prefix_dl", images, &pi, &img_host);
+  if (!rc) rc = dl_prefix(h, "beam_search_prefix_dl", prefix_ids, prefix_len, &pp, &pl, &p);
+  if (!rc) rc = dl_captions(h, "beam_search_prefix_dl", out_ids, out_len, out_logprob, &pids, &plen, &plp, &ids_host);
+  if (rc) return rc;
+  return fpnmt_beam_search_prefix(h, (const float*)pi, img_host, (const int32_t*)pp, (const int32_t*)pl, p, beam_groups, diversity,
+                                  length_penalty, (int32_t*)pids, (int32_t*)plen, (float*)plp, ids_host, early_stop, stream);
+}
+
 // fpnmt_beam_search_dl and fpnmt_beam_search_diverse_dl: the same shape checks, then the diverse entry (G = 1 is
 // fpnmt_beam_search)
 static int beam_search_dl(const char* name, fpnmt_handle* h, const DLTensor* images, int beam_groups, float diversity,

@@ -46,6 +46,8 @@ Engine::~Engine() {
   if (loop_graph_) cudaGraphExecDestroy(loop_graph_);
   if (sample_graph_) cudaGraphExecDestroy(sample_graph_);
   if (nbest_graph_) cudaGraphExecDestroy(nbest_graph_);
+  if (nbest_pfx_graph_) cudaGraphExecDestroy(nbest_pfx_graph_);
+  if (sample_pfx_graph_) cudaGraphExecDestroy(sample_pfx_graph_);
   for (auto& kv : score_graphs_)
     if (kv.second) cudaGraphExecDestroy(kv.second);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
@@ -1217,6 +1219,8 @@ int Engine::build_decoder() {
       o.bytes = (double)R * gf.K * 2 + (double)gf.Cout * gf.K * 2 + (double)R * vtiles * (8 + 8 * TG_VS_N);
       o.run = [op](cudaStream_t s) { return tgemm_launch(op, s); };
       step_prog_.back() = std::move(o);                      // replaces the logits version in the beam-search chain
+      step_final_at_ = step_prog_.size() - 1;
+      vs_final_op_ = op;
       bsv.vs_stat = vst;
       bsv.vs_val = vval;
       bsv.vs_idx = vidx;
@@ -1788,12 +1792,13 @@ int Engine::generate(const float* images, int on_host, int32_t* out_ids, int32_t
 // k_sample_step draws its next token, so the N rows of an image are N independent samples.  The sampling parameters live in a
 // device struct the kernel reads: a captured sample_graph_ serves every parameter set.
 int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len,
-                   float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
+                   float* out_logprob, int out_on_host, int early_stop, cudaStream_t s, const PrefixArg* prefix) {
   RC(check_decode_entry("sample", "has no sampling tail"));
   const int B = cfg_.batch, N = cfg_.beam, T = cfg_.max_len, V = cfg_.vocab, R = B * N;
   if (check_sampling(sp, V))
     return fail(FPNMT_ERR_INVALID, "sample: temperature >= 0, top_p in (0, 1], 0 <= top_k <= vocab and reserved words 0");
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "sample: NULL out_ids / out_len");
+  RC(check_prefix("sample_prefix", prefix));
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   if (!ss_.ids) {   // per-row buffers [R][T] + [R] x 3 and the per-image counters, on the first call
     SampleState st{};
@@ -1817,14 +1822,30 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
     sample_prog_.push_back(std::move(o));
     ss_ = st;
   }
+  if (prefix && sample_pfx_prog_.empty()) {   // prompted: the same program with the forced-capable sample op
+    const SampleState st = ss_;
+    const float* lg = logits_;
+    const int *pid = pfx_ids_, *pln = pfx_len_;
+    sample_pfx_prog_ = sample_prog_;
+    Op& o = sample_pfx_prog_.back();
+    o.name = "sample_step(prefix)";
+    o.run = [st, lg, pid, pln](cudaStream_t q) { return launch_sample_step_prefix(st, pid, pln, lg, q); };
+  }
   const SampleParams prm{sp.temperature, sp.top_k, sp.top_p, 0, (unsigned long long)sp.seed};
   if (images) RC(encode(images, on_host, nullptr, s, false));
   FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<SampleParams*>(ss_.params), &prm, sizeof prm, cudaMemcpyHostToDevice, s));
   RC(run_program(dec_init_prog_, s));
+  if (prefix) RC(load_prefix(*prefix, s));
   RC(launch_sample_init(ss_, bs_.anc[0], s));
   launches += 1;
   FlagGuard forced(forced_mode_);   // the self-attention launches of the program stay in the first buffer pair, without representatives
-  RC(run_steps(sample_prog_, sample_graph_, bs_.n_done, early_stop, s));
+  if (prefix) {
+    RC(run_steps(sample_pfx_prog_, sample_pfx_graph_, bs_.n_done, early_stop, s));
+    RC(launch_prefix_flag(pfx_bad_, B, N, T, ss_.ids, ss_.len, ss_.lp, s));
+    launches += 1;
+  } else {
+    RC(run_steps(sample_prog_, sample_graph_, bs_.n_done, early_stop, s));
+  }
   RC(copy_out(out_ids, ss_.ids, (size_t)R * T * 4, out_on_host, s));
   RC(copy_out(out_len, ss_.len, (size_t)R * 4, out_on_host, s));
   RC(copy_out(out_logprob, ss_.lp, (size_t)R * 4, out_on_host, s));
@@ -1839,13 +1860,15 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
 // own length-penalty table followed by the (beam_groups, diversity) words, uploaded on every call: one captured graph serves
 // every (G, lambda, alpha) and bs_.lp, which generate reads, is never touched.  fpnmt_beam_search is G = 1.
 int Engine::beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty,
-                        int32_t* out_ids, int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s) {
+                        int32_t* out_ids, int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s,
+                        const PrefixArg* prefix) {
   RC(check_decode_entry("beam_search", "has no N-best tail"));
   if (cfg_.score_mode == FPNMT_SCORE_PROB)
     return fail(FPNMT_ERR_STATE, "beam_search: the length penalty and the log-likelihoods need score_mode = log");
   if (!std::isfinite(length_penalty)) return fail(FPNMT_ERR_INVALID, "beam_search: length_penalty must be finite");
   if (check_beam_groups(step_bsv_, beam_groups, diversity)) return FPNMT_ERR_INVALID;
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "beam_search: NULL out_ids / out_len");
+  RC(check_prefix("beam_search_prefix", prefix));
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   const int B = cfg_.batch, T = cfg_.max_len, R = B * cfg_.beam;
   if (!nbest_bs_.nb.ids) {
@@ -1868,21 +1891,80 @@ int Engine::beam_search(const float* images, int on_host, int beam_groups, float
     o.run = [st, lg, V, em](cudaStream_t q) { return launch_beam_step_nbest(st, lg, V, em, q); };
     nbest_bs_ = st;
   }
+  if (prefix && nbest_pfx_prog_.empty()) {
+    // prompted: the forced-capable beam op on nbest_bs_ + the prefix buffers; on the logits-free tail the vocabulary
+    // projection also reports the logit of each row's forced token
+    BeamState st = nbest_bs_;
+    st.pf.ids = pfx_ids_;
+    st.pf.len = pfx_len_;
+    nbest_pfx_prog_ = nbest_prog_;
+    if (st.vs_stat) {
+      st.pf.tgt = pfx_tgt_;
+      st.pf.tgt_logit = pfx_tgt_logit_;
+      TgemmOp op = vs_final_op_;
+      op.tgt = pfx_tgt_;
+      op.tgt_logit = pfx_tgt_logit_;
+      Op& f = nbest_pfx_prog_[step_final_at_];
+      f.name = "final_layer(softmax partials + candidates + target logit)";
+      f.run = [op](cudaStream_t q) { return tgemm_launch(op, q); };
+    }
+    const float* lg = logits_;
+    const BeamEmbed em = beam_embed_;
+    const int V = cfg_.vocab;
+    Op& o = nbest_pfx_prog_[step_beam_at_];
+    o.name = "beam_step(n-best, prefix)";
+    o.run = [st, lg, V, em](cudaStream_t q) { return launch_beam_step_prefix(st, lg, V, em, q); };
+    nbest_pfx_bs_ = st;
+  }
   std::vector<float> lp(T + 4);
   for (int i = 0; i < T + 2; ++i) lp[i] = powf((5.f + (float)i) / 6.f, length_penalty);
   lp[T + 2] = (float)beam_groups;
   lp[T + 3] = beam_groups > 1 ? diversity : 0.f;
   if (images) RC(encode(images, on_host, nullptr, s, false));
   FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<float*>(nbest_bs_.lp), lp.data(), lp.size() * 4, cudaMemcpyHostToDevice, s));
-  RC(launch_beam_init(nbest_bs_, 1, s, beam_groups));
+  if (prefix) RC(load_prefix(*prefix, s));                  // before the init kernel, which writes step 0's targets
+  RC(launch_beam_init(prefix ? nbest_pfx_bs_ : nbest_bs_, 1, s, beam_groups));
   launches += 1;
   RC(run_program(dec_init_prog_, s));
   RC(run_program(embed_prog_, s));
-  RC(run_steps(nbest_prog_, nbest_graph_, nbest_bs_.n_done, early_stop, s));
+  if (prefix) {
+    RC(run_steps(nbest_pfx_prog_, nbest_pfx_graph_, nbest_bs_.n_done, early_stop, s));
+    RC(launch_prefix_flag(pfx_bad_, B, cfg_.beam, T, nbest_bs_.nb.ids, nbest_bs_.nb.len, nbest_bs_.nb.score, s));
+    launches += 1;
+  } else {
+    RC(run_steps(nbest_prog_, nbest_graph_, nbest_bs_.n_done, early_stop, s));
+  }
   RC(copy_out(out_ids, nbest_bs_.nb.ids, (size_t)R * T * 4, out_on_host, s));
   RC(copy_out(out_len, nbest_bs_.nb.len, (size_t)R * 4, out_on_host, s));
   RC(copy_out(out_logprob, nbest_bs_.nb.score, (size_t)R * 4, out_on_host, s));
   if (out_on_host) FPNMT_CUDA_OK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// The refusals of a prefix argument (nothing launched) and, on the first prompted call, the engine's prefix buffers.
+int Engine::check_prefix(const char* entry, const PrefixArg* prefix) {
+  if (!prefix) return 0;
+  const std::string e = entry;
+  if (!prefix->ids || !prefix->len) return fail(FPNMT_ERR_INVALID, e + ": NULL prefix_ids / prefix_len");
+  if (prefix->p < 1 || prefix->p > cfg_.max_len - 1) return fail(FPNMT_ERR_INVALID, e + ": p must be 1 .. max_len - 1");
+  if (!pfx_ids_) {
+    FPNMT_CUDA_OK(cudaSetDevice(dev_));
+    const int B = cfg_.batch, R = B * cfg_.beam;
+    pfx_ids_ = (int*)dalloc((size_t)B * cfg_.max_len * 4);
+    pfx_len_ = (int*)dalloc((size_t)B * 4);
+    pfx_bad_ = (int*)dalloc((size_t)B * 4);
+    pfx_tgt_ = (int*)dalloc((size_t)R * 4);
+    pfx_tgt_logit_ = (float*)dalloc((size_t)R * 4);
+    if (!pfx_ids_ || !pfx_len_ || !pfx_bad_ || !pfx_tgt_ || !pfx_tgt_logit_) return FPNMT_ERR_CUDA;
+  }
+  return 0;
+}
+
+// the caller's prefixes -> pfx_ids_ / pfx_len_ / pfx_bad_ (checked and clamped on the device)
+int Engine::load_prefix(const PrefixArg& prefix, cudaStream_t s) {
+  RC(launch_prefix_load(prefix.ids, prefix.len, prefix.p, cfg_.batch, cfg_.max_len, cfg_.vocab, cfg_.end_id, pfx_ids_, pfx_len_,
+                        pfx_bad_, s));
+  launches += 1;
   return 0;
 }
 

@@ -49,6 +49,14 @@ struct Op {
 };
 typedef std::vector<Op> Program;
 
+// The caption prefixes of a prompted decode (fpnmt_sample_prefix / fpnmt_beam_search_prefix): DEVICE ids [batch][p] and
+// len [batch], never read by the host.
+struct PrefixArg {
+  const int32_t* ids;
+  const int32_t* len;
+  int p;
+};
+
 class Engine {
  public:
   Engine(const fpnmt_config& cfg, int device);
@@ -72,8 +80,9 @@ class Engine {
                float* step_scores, cudaStream_t s);
   // Sampled decode (fpnmt_sample): every row of the batch is one independent sample of its image; the teacher-forced step
   // program with k_sample_step in place of the teacher-forced tail.  images == nullptr: the memory of the last encode.
+  // prefix != nullptr: the prompted decode (fpnmt_sample_prefix) on sample_pfx_prog_.
   int sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len, float* out_logprob,
-             int out_on_host, int early_stop, cudaStream_t s);
+             int out_on_host, int early_stop, cudaStream_t s, const PrefixArg* prefix = nullptr);
   // Caption scoring (fpnmt_score): the N captions ids [B][N][t] / lens [B][N] (device) of every image through the decoder
   // as B * N * t rows of one teacher-forced pass.  images == nullptr: the memory of the last encode.
   int score(const float* images, int on_host, const int32_t* ids, const int32_t* lens, int t, float* out_logprob,
@@ -81,8 +90,10 @@ class Engine {
   // N-best beam search (fpnmt_beam_search: beam_groups = 1) and diverse beam search (fpnmt_beam_search_diverse): the
   // whole-batch step program with k_beam_step's group ranking and N-best close, true-beam start (first beam of every group),
   // frozen finished beams and this call's length penalty.  images == nullptr: the memory of the last encode.
+  // prefix != nullptr: the prompted search (fpnmt_beam_search_prefix) on nbest_pfx_prog_.
   int beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty, int32_t* out_ids,
-                  int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s);
+                  int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s,
+                  const PrefixArg* prefix = nullptr);
   int profile(int iters, char* buf, size_t cap);
   int build_dstep(const Tensor& ckv, const float* d_emb, const float* d_pos);
   int get_tap_f32(const std::string& name, float* out, size_t cap, size_t* count, cudaStream_t s);
@@ -127,6 +138,19 @@ class Engine {
   Program nbest_prog_;
   BeamState nbest_bs_{};
   cudaGraphExec_t nbest_graph_ = nullptr;
+  // prompted decode (built on its first call): nbest_prog_ with the beam op replaced by the forced-capable one on nbest_pfx_bs_
+  // (nbest_bs_ + the prefix buffers) and, on the logits-free tail, the vocabulary projection (index step_final_at_, op
+  // vs_final_op_) by its target variant; sample_pfx_prog_ is sample_prog_ with the forced-capable sample op.  The prefixes
+  // are copied into pfx_ids_ / pfx_len_ on every call, so one captured graph serves every prefix.
+  size_t step_final_at_ = 0;
+  TgemmOp vs_final_op_{};
+  Program nbest_pfx_prog_, sample_pfx_prog_;
+  BeamState nbest_pfx_bs_{};
+  cudaGraphExec_t nbest_pfx_graph_ = nullptr, sample_pfx_graph_ = nullptr;
+  int *pfx_ids_ = nullptr, *pfx_len_ = nullptr, *pfx_bad_ = nullptr, *pfx_tgt_ = nullptr;   // [B][T], [B], [B], [B*N]
+  float* pfx_tgt_logit_ = nullptr;                                                          // [B*N]
+  int check_prefix(const char* entry, const PrefixArg* prefix);
+  int load_prefix(const PrefixArg& prefix, cudaStream_t s);
   SampleState ss_{};                      // sampler state: per-row buffers allocated on the first sample call
   cudaGraphExec_t sample_graph_ = nullptr;   // sample_prog_ captured with forced_mode_ set (never step_graph_)
   // score pass: one program (and graph) per caption length t, built on its first call; activations for B * N * max_len rows

@@ -148,8 +148,18 @@ struct BeamState {
                              // 32 bytes in all: the kernel parameters after BeamState keep their 16-byte alignment, so the
                              // generate instantiations of k_beam_step keep their vector constant loads (same code)
   } nb;
+  // Prompted decode (fpnmt_beam_search_prefix; launch_beam_step_prefix): at a step t < len[b] every row of image b takes the
+  // token ids[b][t] with parent = itself, nothing ranked.  32 bytes, for the alignment reason of NBest.
+  struct Prefix {
+    const int* ids;          // [B][T] the engine's copy of the prefixes (launch_prefix_load), 0 padded
+    const int* len;          // [B] prefix length, 0 for an image whose prefix was refused
+    int* tgt;                // [B*N] logits-free tail: the token whose logit the next step's vocabulary projection reports
+                             // (-1: none), written by k_beam_init for step 0 and by the beam kernel of step t for t + 1
+    const float* tgt_logit;  // [B*N] that logit (tgemmw_kernel's target epilogue), read by the forced rows of the vstats path
+  } pf;
 };
 static_assert(sizeof(BeamState::NBest) == 32, "see BeamState::NBest::groups");
+static_assert(sizeof(BeamState::Prefix) == 32, "see BeamState::NBest::groups");
 // true_beam = 0 reproduces the reference (all beams start identical, pipeline.py:101-102); 1 starts only the first beam of
 // each of beam_groups groups of N / beam_groups beams alive (beam_groups = 1: beams 1..N-1 dead)
 int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s, int beam_groups = 1);
@@ -166,6 +176,15 @@ struct BeamEmbed {
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
 // The same step with beam groups and the N-best close (BeamState::nb): needs finished_mode, log scores and nb.groups.
 int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
+// The N-best step of a prompted decode: forced steps inside each image's prefix (BeamState::pf), the N-best step after it.
+int launch_beam_step_prefix(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
+// Prompted decode, before the first step: dst_ids[b][j] = prefix_ids[b][j] for j < prefix_len[b] (ids clamped to [0, V)
+// before they are stored), 0 elsewhere ([B][T]); bad[b] = 1 when prefix_len[b] is outside [0, p] or one of its first
+// prefix_len[b] ids is outside [0, V) or equals end_id; dst_len[b] = bad[b] ? 0 : prefix_len[b].  prefix_ids DEVICE [B][p].
+int launch_prefix_load(const int* prefix_ids, const int* prefix_len, int p, int B, int T, int V, int end_id, int* dst_ids,
+                       int* dst_len, int* bad, cudaStream_t s);
+// After a prompted decode: every row of an image with bad[b] set gets ids 0, len 0 and logprob NaN (rows = B * N, ids [rows][T]).
+int launch_prefix_flag(const int* bad, int B, int N, int T, int* ids, int* len, float* logprob, cudaStream_t s);
 // The refusals of a (beam_groups, diversity) pair for the N-best step (set_last_error + 1): G >= 1 dividing N, lambda finite
 // and >= 0.  The pair lives in device memory (nb.groups), so callers check it here before uploading it.
 int check_beam_groups(const BeamState& st, int beam_groups, float diversity);
@@ -216,6 +235,9 @@ int sample_set_attributes();
 // step 0, last_tok = <start>, identity ancestry [2][rows][T] in `anc`, per-row and per-image state cleared
 int launch_sample_init(const SampleState& st, int* anc, cudaStream_t s);
 int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t s);
+// The step of a prompted decode (engine state only): at a step t < pfx_len[b] every row of image b takes pfx_ids[b][t] with no
+// draw; the sampling step after it.  pfx_ids [images][T] / pfx_len [images]: launch_prefix_load's buffers.
+int launch_sample_step_prefix(const SampleState& st, const int* pfx_ids, const int* pfx_len, const float* logits, cudaStream_t s);
 
 // ---- score.cu -----------------------------------------------------------------------------------
 // Caption scoring (fpnmt_score, include/fpnmt.h): row r = c * t + j is position j of caption c = b * N + n.

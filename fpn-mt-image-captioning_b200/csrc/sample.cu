@@ -128,7 +128,12 @@ __device__ uint32_t radix_select_desc(const float* s_row, int V, unsigned long l
   return prefix;
 }
 
-__global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step(SampleState st, const float* __restrict__ logits) {
+// The step body.  PREFIX (k_sample_step_prefix): a row of an image inside its prefix (step t < pfx_len[image]) takes the
+// prefix token pfx_ids[image][t] (top-k, top-p and the draw skipped) and adds its log-probability with the expression of the
+// free path.
+template <bool PREFIX>
+__device__ __forceinline__ void sample_step_body(const SampleState& st, const float* __restrict__ logits,
+                                                 const int* __restrict__ pfx_ids, const int* __restrict__ pfx_len) {
   extern __shared__ float4 s_row4[];
   float* s_row = reinterpret_cast<float*>(s_row4);
   __shared__ SampleSmem sm;
@@ -211,9 +216,15 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step(SampleState st, 
     for (int w = 0; w < NW; ++w) a += sm.ws[w];
     sm.lse1 = m + logf(a);
     sm.tok = sm.mi;                                      // temperature 0: arg-max, lowest token id on ties
+    if constexpr (PREFIX) {                              // forced step of a prompted decode: the prefix token
+      const int b = row / st.N;
+      if (t < pfx_len[b]) sm.tok = pfx_ids[(size_t)b * st.T + t];
+    }
   }
+  bool forced = false;
+  if constexpr (PREFIX) forced = t < pfx_len[row / st.N];
 
-  if (prm.temperature > 0.f) {
+  if (prm.temperature > 0.f && !forced) {
     // ---- top-k: K1 = {i : z_i >= z_(k)}, every token tied with the k-th largest logit kept
     uint32_t k1 = 0u;
     if (prm.top_k > 0 && prm.top_k < V)
@@ -317,6 +328,16 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step(SampleState st, 
   }
 }
 
+__global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step(SampleState st, const float* __restrict__ logits) {
+  sample_step_body<false>(st, logits, nullptr, nullptr);
+}
+// the step of a prompted decode (pfx_ids [images][T], pfx_len [images]: launch_prefix_load's buffers)
+__global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step_prefix(SampleState st, const float* __restrict__ logits,
+                                                                       const int* __restrict__ pfx_ids,
+                                                                       const int* __restrict__ pfx_len) {
+  sample_step_body<true>(st, logits, pfx_ids, pfx_len);
+}
+
 __global__ void k_sample_init(SampleState st, int* anc) {
   pdl_launch();
   pdl_wait();
@@ -340,6 +361,7 @@ __global__ void k_sample_init(SampleState st, int* anc) {
 
 int sample_set_attributes() {   // per device
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_sample_step, cudaFuncAttributeMaxDynamicSharedMemorySize, SAMPLE_MAX_SMEM));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_sample_step_prefix, cudaFuncAttributeMaxDynamicSharedMemorySize, SAMPLE_MAX_SMEM));
   return 0;
 }
 
@@ -353,13 +375,28 @@ int launch_sample_init(const SampleState& st, int* anc, cudaStream_t s) {
   return 0;
 }
 
-int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t s) {
+static size_t sample_smem(const SampleState& st) {   // 0: refused
   const size_t smem = ((size_t)st.V * 4 + 15) / 16 * 16;
   if (st.V < 1 || smem > (size_t)SAMPLE_MAX_SMEM || st.rows < 1 || st.N < 1) {
     set_last_error("sample_step: vocabulary must be 1 .. 51200 and rows >= 1");
+    return 0;
+  }
+  return smem;
+}
+int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t s) {
+  const size_t smem = sample_smem(st);
+  if (!smem) return 1;
+  FPNMT_CUDA_OK(launch_k(k_sample_step, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits));
+  return 0;
+}
+int launch_sample_step_prefix(const SampleState& st, const int* pfx_ids, const int* pfx_len, const float* logits, cudaStream_t s) {
+  if (!pfx_ids || !pfx_len || !st.ids) {
+    set_last_error("sample_step_prefix: needs the prefix buffers and the engine's decode state");
     return 1;
   }
-  FPNMT_CUDA_OK(launch_k(k_sample_step, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits));
+  const size_t smem = sample_smem(st);
+  if (!smem) return 1;
+  FPNMT_CUDA_OK(launch_k(k_sample_step_prefix, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits, pfx_ids, pfx_len));
   return 0;
 }
 

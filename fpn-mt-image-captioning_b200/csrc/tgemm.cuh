@@ -56,6 +56,10 @@ struct TgemmOp {
   int grid;
   int cluster;   // 1, or 4 (LayerNorm)
   double flops;
+  // vocabulary projection without logits (p.vs_stat) of a prompted beam search: tgemmw_target_kernel also writes
+  // tgt_logit[r] = z[r][tgt[r]] for every row r whose tgt[r] lies in [0, F) (device [R] each; nullptr = tgemmw_kernel)
+  const int* tgt = nullptr;
+  float* tgt_logit = nullptr;
 };
 
 size_t tgemm_smem_bytes(int BN);

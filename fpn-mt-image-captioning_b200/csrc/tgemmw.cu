@@ -109,9 +109,12 @@ __device__ __forceinline__ void tw_load_chunk(uint32_t taddr, const float* sBias
   }
 }
 
-__global__ void __launch_bounds__(TG_THREADS, 2)
-tgemmw_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX,
-              const __grid_constant__ CUtensorMap tmO, const TgemmParams p) {
+// The kernel body.  TGT (tgemmw_target_kernel, vocabulary tile without logits only): the row whose target id tgt[row] lies in
+// [0, F) also writes the fp32 logit of that feature, the value its tile's statistics and candidates are computed from, to
+// tgt_logit[row] (-1 or an id >= F: nothing written).
+template <bool TGT>
+__device__ __forceinline__ void tgemmw_body(const CUtensorMap& tmW, const CUtensorMap& tmX, const CUtensorMap& tmO,
+                                            const TgemmParams p, const int* __restrict__ tgt, float* __restrict__ tgt_logit) {
   constexpr int STAGES = TW_STAGES;
   constexpr int BN = 128;                          // features per tile == UMMA N == TMEM columns of one accumulator
   constexpr int CHUNKS = BN / 32;
@@ -284,6 +287,8 @@ tgemmw_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
         // slower, 65 vs 26 us for the C2 projection: the insertion body runs for nearly every element because some lane of the
         // warp always qualifies, so instruction count matters more than the length of the dependent chain.)
         float m = -INFINITY, ssum = 0.f;
+        int tg = -1;                                          // target feature of this row (TGT)
+        if constexpr (TGT) tg = row_ok ? __ldcg(tgt + row) : -1;
         float bv[TG_VS_N];
         int bi[TG_VS_N];
 #pragma unroll
@@ -305,6 +310,15 @@ tgemmw_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
           for (int i = 0; i < 32; ++i) {
             if (fo + i >= p.F) x[i] = -INFINITY;     // padding features of the last tile
             cm = fmaxf(cm, x[i]);
+          }
+          if constexpr (TGT) {
+            const int d = tg - fo;
+            if (d >= 0 && d < 32 && tg < p.F) {      // this chunk holds the target: select it without indexing the registers
+              float z = x[0];
+#pragma unroll
+              for (int i = 1; i < 32; ++i) z = d == i ? x[i] : z;
+              tgt_logit[row] = z;
+            }
           }
           if (cm > -INFINITY) {
             const float mn = fmaxf(m, cm);
@@ -494,6 +508,19 @@ tgemmw_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
   }
 }
 
+__global__ void __launch_bounds__(TG_THREADS, 2)
+tgemmw_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX,
+              const __grid_constant__ CUtensorMap tmO, const TgemmParams p) {
+  tgemmw_body<false>(tmW, tmX, tmO, p, nullptr, nullptr);
+}
+// The vocabulary projection of a prompted beam search on the logits-free tail: tgemmw_kernel + the target logit (TgemmOp::tgt)
+__global__ void __launch_bounds__(TG_THREADS, 2)
+tgemmw_target_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX,
+                     const __grid_constant__ CUtensorMap tmO, const TgemmParams p, const int* __restrict__ tgt,
+                     float* __restrict__ tgt_logit) {
+  tgemmw_body<true>(tmW, tmX, tmO, p, tgt, tgt_logit);
+}
+
 int tgemmw_launch(const TgemmOp& op, cudaStream_t stream) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(op.grid);
@@ -516,13 +543,16 @@ int tgemmw_launch(const TgemmOp& op, cudaStream_t stream) {
   }
   cfg.attrs = attr;
   cfg.numAttrs = n;
-  FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p));
+  if (op.tgt) FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_target_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p, op.tgt, op.tgt_logit));
+  else FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p));
   return 0;
 }
 
 int tgemmw_set_attributes() {
   FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tgemmw_smem_bytes(128)));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_target_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tgemmw_smem_bytes(128)));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_target_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   return 0;
 }
 

@@ -70,6 +70,7 @@ SIGNATURES = {
     "fpnmt_op_decode_jpeg": (_i, [_i, C.POINTER(_vp), C.POINTER(C.c_size_t), _i, _i, _vp, _vp, _vp]),
     "fpnmt_op_dense": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _i, _vp, _vp, _vp, C.c_float, _vp, _i, _vp]),
     "fpnmt_op_vocab_stats": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "fpnmt_op_vocab_stats_target": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "fpnmt_op_depthwise3x3": (_i, [_i, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
     "fpnmt_op_pool": (_i, [_i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
     "fpnmt_op_scale_shift_relu": (_i, [_i, _i, _vp, C.c_int64, _i, _i, _vp, _vp, _vp, _i, _vp]),
@@ -89,6 +90,8 @@ SIGNATURES = {
     "fpnmt_score": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp]),
     "fpnmt_beam_search": (_i, [_vp, _vp, _i, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
     "fpnmt_beam_search_diverse": (_i, [_vp, _vp, _i, _i, C.c_float, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
+    "fpnmt_sample_prefix": (_i, [_vp, _vp, _i, _vp, _vp, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _i, _i, _vp]),
+    "fpnmt_beam_search_prefix": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i, C.c_float, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
 }
 
 
@@ -122,6 +125,8 @@ SIGNATURES.update({
     "fpnmt_score_dl": (_i, [_vp, _dlp, _dlp, _dlp, _dlp, _dlp, _vp]),
     "fpnmt_beam_search_dl": (_i, [_vp, _dlp, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_beam_search_diverse_dl": (_i, [_vp, _dlp, _i, C.c_float, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
+    "fpnmt_sample_prefix_dl": (_i, [_vp, _dlp, _dlp, _dlp, C.POINTER(FpnmtSampling), _dlp, _dlp, _dlp, _i, _vp]),
+    "fpnmt_beam_search_prefix_dl": (_i, [_vp, _dlp, _dlp, _dlp, _i, C.c_float, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_comm_unique_id": (_i, [_vp]),
     "fpnmt_comm_create": (_i, [_i, _i, _vp, _i, C.POINTER(_vp)]),
     "fpnmt_comm_destroy": (_i, [_vp]),

@@ -248,26 +248,51 @@ class Engine:
                                            _stream_ptr(self.device)))
         return (ids, lens, scores) if return_scores else (ids, lens)
 
+    def _prefix(self, prefix, prefix_lens):
+        """(ids (B, p) int32, lens (B,) int32) on the device for a prompted call; ValueError for other shapes."""
+        if prefix is None:
+            if prefix_lens is not None:
+                raise ValueError("prefix_lens without prefix")
+            return None
+        ids = _as_cuda(prefix, torch.int32, self.device)
+        if ids.dim() != 2 or int(ids.shape[0]) != self.batch:
+            raise ValueError("prefix must be (%d, p), got %s" % (self.batch, tuple(ids.shape)))
+        if prefix_lens is None:
+            lens = torch.full((self.batch,), int(ids.shape[1]), dtype=torch.int32, device=self.device)
+        else:
+            lens = _as_cuda(prefix_lens, torch.int32, self.device)
+        if tuple(lens.shape) != (self.batch,):
+            raise ValueError("prefix_lens must be (%d,), got %s" % (self.batch, tuple(lens.shape)))
+        return ids, lens
+
     def sample(self, images=None, *, temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0,
-               early_stop: bool = True, to_host: bool = True, return_logprobs: bool = False):
+               early_stop: bool = True, to_host: bool = True, return_logprobs: bool = False, prefix=None, prefix_lens=None):
         """`beam` independent sampled captions per image (fpnmt_sample; semantics in include/fpnmt.h): softmax(z / temperature)
         restricted to the top_k logits (0 = off, ties kept) and then to the nucleus of top_p of that mass (1 = off), drawn with
         the Philox stream of (seed, step, image, sample).  temperature 0 is greedy.  images None = the memory of the last
         encode / generate.  Returns ids (B, N, T) int32 zero padded without <start> / <end>, lengths (B, N) and, with
-        return_logprobs, the captions' log-likelihoods (B, N) float32 (log_softmax at temperature 1, <end> included)."""
+        return_logprobs, the captions' log-likelihoods (B, N) float32 (log_softmax at temperature 1, <end> included).
+        prefix (B, p) int32 with prefix_lens (B,) (default: p for every image), on host or device: every sample of image b
+        continues prefix[b, :prefix_lens[b]] (fpnmt_sample_prefix); the returned captions and log-likelihoods include it."""
         ptr, on_host, keep = self._images_opt(images)
+        pfx = self._prefix(prefix, prefix_lens)
         B, N, T = self.batch, self.beam, self.max_len
         ids = self._result((B, N, T), torch.int32, to_host)
         lens = self._result((B, N), torch.int32, to_host)
         lp = self._result((B, N), torch.float32, to_host) if return_logprobs else None
         sp = _lib.sampling(temperature, top_k, top_p, seed)
-        _lib.check(self.lib.fpnmt_sample(self._h, ptr, on_host, C.byref(sp), ids.data_ptr(), lens.data_ptr(),
-                                         lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
-                                         _stream_ptr(self.device)))
+        lpp = lp.data_ptr() if lp is not None else None
+        if pfx is None:
+            _lib.check(self.lib.fpnmt_sample(self._h, ptr, on_host, C.byref(sp), ids.data_ptr(), lens.data_ptr(), lpp,
+                                             int(to_host), int(early_stop), _stream_ptr(self.device)))
+        else:
+            _lib.check(self.lib.fpnmt_sample_prefix(self._h, ptr, on_host, pfx[0].data_ptr(), pfx[1].data_ptr(),
+                                                    int(pfx[0].shape[1]), C.byref(sp), ids.data_ptr(), lens.data_ptr(), lpp,
+                                                    int(to_host), int(early_stop), _stream_ptr(self.device)))
         return (ids, lens, lp) if return_logprobs else (ids, lens)
 
     def beam_search(self, images=None, *, length_penalty: float = 0.0, early_stop: bool = True, to_host: bool = True,
-                    return_logprobs: bool = False, beam_groups: int = 1, diversity: float = 0.0):
+                    return_logprobs: bool = False, beam_groups: int = 1, diversity: float = 0.0, prefix=None, prefix_lens=None):
         """The `beam` most likely captions per image by a true beam search with frozen finished beams (fpnmt_beam_search;
         definition in include/fpnmt.h), ranked by log-likelihood / ((5 + n) / 6) ** length_penalty, n the scored positions.
         images None = the memory of the last encode / generate / sample / score.  Returns ids (B, N, T) int32 zero padded
@@ -275,13 +300,22 @@ class Engine:
         log-likelihoods (B, N) float32 (<end> included): what `score` gives for them with t = T.
         beam_groups G > 1 runs the diverse beam search instead (fpnmt_beam_search_diverse): G groups of N / G beams, each
         group's candidates lowered by `diversity` per earlier group's beam that chose the same token at the same step.  The
-        output is group-major (beams [g * N / G, (g + 1) * N / G) are group g), rank order within a group."""
+        output is group-major (beams [g * N / G, (g + 1) * N / G) are group g), rank order within a group.
+        prefix (B, p) int32 with prefix_lens (B,) (default: p for every image), on host or device: every beam of image b
+        continues prefix[b, :prefix_lens[b]] (fpnmt_beam_search_prefix); the returned captions and log-likelihoods include it."""
         ptr, on_host, keep = self._images_opt(images)
+        pfx = self._prefix(prefix, prefix_lens)
         B, N, T = self.batch, self.beam, self.max_len
         ids = self._result((B, N, T), torch.int32, to_host)
         lens = self._result((B, N), torch.int32, to_host)
         lp = self._result((B, N), torch.float32, to_host) if return_logprobs else None
-        if beam_groups == 1:
+        if pfx is not None:
+            _lib.check(self.lib.fpnmt_beam_search_prefix(self._h, ptr, on_host, pfx[0].data_ptr(), pfx[1].data_ptr(),
+                                                         int(pfx[0].shape[1]), int(beam_groups), float(diversity),
+                                                         float(length_penalty), ids.data_ptr(), lens.data_ptr(),
+                                                         lp.data_ptr() if lp is not None else None, int(to_host),
+                                                         int(early_stop), _stream_ptr(self.device)))
+        elif beam_groups == 1:
             _lib.check(self.lib.fpnmt_beam_search(self._h, ptr, on_host, float(length_penalty), ids.data_ptr(), lens.data_ptr(),
                                                   lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
                                                   _stream_ptr(self.device)))
@@ -493,6 +527,35 @@ def vocab_stats(x: torch.Tensor, kernel: np.ndarray, bias: Optional[np.ndarray] 
     _lib.check(_lib.load().fpnmt_op_vocab_stats(dev.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), r, k, _hptr(kn), f,
                                                 _hptr(b), stat.data_ptr(), val.data_ptr(), idx.data_ptr(), _stream_ptr(dev)))
     return stat, val, idx
+
+
+def vocab_stats_target(x: torch.Tensor, kernel: np.ndarray, target, bias: Optional[np.ndarray] = None,
+                       target_logit: Optional[torch.Tensor] = None, precision: str = "bf16"
+                       ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """`vocab_stats` with the target epilogue of a prompted beam search (fpnmt_op_vocab_stats_target): also
+    target_logit[r] = z[r, target[r]] (fp32, the value the tile's statistics come from) for every row whose target (R,) int32
+    lies in [0, F); the other entries of target_logit (R,) float32 (default: NaN) keep their contents.
+    Returns (stat, val, idx, target_logit)."""
+    x = _dev32(x)
+    r, k = x.shape
+    kn = _host32(kernel)
+    f = kn.shape[1]
+    ft = (f + 127) // 128
+    dev = x.device
+    stat = torch.full((r, ft, 2), float("nan"), device=dev)
+    val = torch.full((r, ft, 8), float("nan"), device=dev)
+    idx = torch.full((r, ft, 8), -1, dtype=torch.int32, device=dev)
+    tg = _as_cuda(target, torch.int32, dev)
+    if tuple(tg.shape) != (r,):
+        raise ValueError("target must be (%d,), got %s" % (r, tuple(tg.shape)))
+    tl = torch.full((r,), float("nan"), device=dev) if target_logit is None else target_logit
+    if tl.dtype != torch.float32 or not tl.is_contiguous() or tl.device != dev or tuple(tl.shape) != (r,):
+        raise ValueError("target_logit must be a contiguous float32 tensor of shape (%d,) on %s" % (r, dev))
+    b = _host32(bias)
+    _lib.check(_lib.load().fpnmt_op_vocab_stats_target(dev.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), r, k, _hptr(kn), f,
+                                                       _hptr(b), tg.data_ptr(), stat.data_ptr(), val.data_ptr(), idx.data_ptr(),
+                                                       tl.data_ptr(), _stream_ptr(dev)))
+    return stat, val, idx, tl
 
 
 # ---- stand-alone encoder bandwidth operators (kernel parity tests) --------------------------------------------------------

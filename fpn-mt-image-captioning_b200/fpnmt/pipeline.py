@@ -76,28 +76,58 @@ class Pipeline:
         attn = {k: v.cpu().numpy() for k, v in eng.caption_attention(ids, lens).items()}
         return ids.numpy(), lens.numpy(), attn
 
+    def _prefix_ids(self, prefix, B: int, T: int):
+        """B prefix strings -> (ids (B, p) int32, lens (B,)) tokenized as score_batch does (a leading <start> dropped), or
+        (None, None) for prefix None.  ValueError for a prefix holding <end> or max_seq_len or more tokens."""
+        if prefix is None:
+            return None, None
+        if len(prefix) != B:
+            raise ValueError("prefix: one string per image (%d), got %d" % (B, len(prefix)))
+        start, end = self.tokenizer.word_index["<start>"], self.tokenizer.word_index["<end>"]
+        seqs = []
+        for seq in self.tokenizer.texts_to_sequences(list(prefix)):
+            if seq and seq[0] == start:
+                seq = seq[1:]
+            if end in seq:
+                raise ValueError("prefix: a prefix may not contain <end>")
+            if len(seq) >= T:
+                raise ValueError("prefix: a prefix of %d tokens needs max_seq_len > %d (max_seq_len = %d)" % (len(seq), len(seq), T))
+            seqs.append(seq)
+        ids = np.zeros((B, max(1, max(len(q) for q in seqs))), np.int32)
+        for i, q in enumerate(seqs):
+            ids[i, :len(q)] = q
+        return ids, np.array([len(q) for q in seqs], np.int32)
+
     def sample_batch(self, imgs, max_seq_len: Optional[int] = None, num_samples: Optional[int] = None, *,
-                     temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0, return_logprobs: bool = False):
+                     temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0, return_logprobs: bool = False,
+                     prefix=None):
         """`num_samples` (default: the beam width) independent sampled captions per image (Engine.sample): imgs (B,S,S,3)
         float32 in [-1,1] -> (ids (B,num_samples,T) int32 zero padded, lengths (B,num_samples)), plus the captions'
-        log-likelihoods (B,num_samples) with return_logprobs.  temperature 0 is greedy."""
+        log-likelihoods (B,num_samples) with return_logprobs.  temperature 0 is greedy.  prefix: B strings, each image's
+        samples continue its string (tokenized as score_batch does; the returned captions include it)."""
         imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
-        eng = self.transformer.engine(int(imgs.shape[0]), num_samples or self.beam, max_seq_len or self.max_seq_len)
+        T = max_seq_len or self.max_seq_len
+        pids, plens = self._prefix_ids(prefix, int(imgs.shape[0]), T)
+        eng = self.transformer.engine(int(imgs.shape[0]), num_samples or self.beam, T)
         out = eng.sample(imgs, temperature=temperature, top_k=top_k, top_p=top_p, seed=seed, early_stop=True, to_host=True,
-                         return_logprobs=return_logprobs)
+                         return_logprobs=return_logprobs, prefix=pids, prefix_lens=plens)
         return tuple(o.numpy() for o in out)
 
     def beam_search_batch(self, imgs, max_seq_len: Optional[int] = None, num_beams: Optional[int] = None, *,
                           length_penalty: float = 0.0, return_logprobs: bool = False, beam_groups: int = 1,
-                          diversity: float = 0.0):
+                          diversity: float = 0.0, prefix=None):
         """The `num_beams` (default: the beam width) most likely captions per image (Engine.beam_search): imgs (B,S,S,3)
         float32 in [-1,1] -> (ids (B,num_beams,T) int32 zero padded, in rank order, lengths (B,num_beams)), plus the captions'
         log-likelihoods (B,num_beams) with return_logprobs.  Ranking by log-likelihood / ((5 + n) / 6) ** length_penalty.
-        beam_groups > 1: diverse beam search in that many groups with the given diversity penalty (group-major output)."""
+        beam_groups > 1: diverse beam search in that many groups with the given diversity penalty (group-major output).
+        prefix: B strings, each image's beams continue its string (tokenized as score_batch does; the returned captions
+        include it)."""
         imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
-        eng = self.transformer.engine(int(imgs.shape[0]), num_beams or self.beam, max_seq_len or self.max_seq_len)
+        T = max_seq_len or self.max_seq_len
+        pids, plens = self._prefix_ids(prefix, int(imgs.shape[0]), T)
+        eng = self.transformer.engine(int(imgs.shape[0]), num_beams or self.beam, T)
         out = eng.beam_search(imgs, length_penalty=length_penalty, early_stop=True, to_host=True, return_logprobs=return_logprobs,
-                              beam_groups=beam_groups, diversity=diversity)
+                              beam_groups=beam_groups, diversity=diversity, prefix=pids, prefix_lens=plens)
         return tuple(o.numpy() for o in out)
 
     def score_batch(self, imgs, captions, max_seq_len: Optional[int] = None, *, return_token_logprobs: bool = False):

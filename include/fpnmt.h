@@ -287,6 +287,38 @@ FPNMT_API int fpnmt_beam_search_diverse(fpnmt_handle* h, const float* images, in
                                         float length_penalty, int32_t* out_ids, int32_t* out_len, float* out_logprob,
                                         int outputs_on_host, int early_stop, void* stream);
 
+/* Prompted decoding: fpnmt_sample, fpnmt_beam_search and fpnmt_beam_search_diverse continuing a given caption prefix per image
+ * (no reference counterpart; completing a caption a user started, a fixed opening for every caption, keeping the first k
+ * words and asking for the best continuations).  prefix_ids DEVICE int32 [batch][p], 1 <= p <= max_len - 1, and prefix_len
+ * DEVICE int32 [batch]: image b's prefix is prefix_ids[b][0 .. prefix_len[b]), in the layout of fpnmt_score's ids (no
+ * <start>, no <end>), shared by all N = beam samples or beams of the image.  The call is its unprompted twin with one change:
+ *   forced step: at a step t < prefix_len[b] every row of image b, live or dead, takes the token prefix_ids[b][t] and keeps
+ *     its own parent (parent = self; the physical cache mode's reorder is the identity for that image).  A live row's score
+ *     grows by log_softmax(z)[token] at temperature 1 with no filtering, a dead beam stays at -inf.  Nothing is ranked, no
+ *     diversity penalty is applied, nothing is counted in h_g and no Philox draw is used: the counter stays (t, b, n, 0), so
+ *     the steps from prefix_len[b] on draw what they would draw anyway.
+ *   after the prefix: from t = prefix_len[b] the image decodes as the unprompted call does (true-beam start: only beam 0, or
+ *     the first beam of every group, is alive, and it now carries the prefix; frozen finished beams; lp(n) with n counting
+ *     the prefix tokens too; the N-best close and early stop as before).  A prompted call runs the same number of steps as an
+ *     unprompted one: the prefix fills positions 0 .. prefix_len[b] - 1 of the caption.
+ *   outputs: the layout of the unprompted call.  out_ids / out_len hold the whole caption, prefix included; out_logprob is the
+ *     whole caption's log-likelihood, prefix terms included, so fpnmt_score of a returned caption gives it back.
+ *   invalid prefix: an image whose prefix_len is outside [0, p], or one of whose first prefix_len ids is outside [0, vocab) or
+ *     equals end_id, comes back with out_len 0, zero ids and NaN out_logprob in all N rows; every other image's result is
+ *     bit-identical to what it would be anyway.  The host never reads prefix_ids / prefix_len; ids are clamped before any load.
+ * All prefix_len = 0 gives the unprompted call's results bit for bit.  Determinism and what the call leaves behind as the
+ * unprompted twin.  Errors: FPNMT_ERR_INVALID (nothing launched) for p outside [1, max_len - 1], NULL prefix_ids /
+ * prefix_len and every refusal of the unprompted twin; FPNMT_ERR_STATE with decode_path = FUSED, score_mode = PROB (beam
+ * search only) or while lane 0 holds a submitted batch.  fpnmt_generate has no prompted form. */
+FPNMT_API int fpnmt_sample_prefix(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                  const int32_t* prefix_len, int p, const fpnmt_sampling* sampling, int32_t* out_ids,
+                                  int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop, void* stream);
+/* beam_groups = 1: the prompted fpnmt_beam_search (diversity ignored); > 1: the prompted fpnmt_beam_search_diverse. */
+FPNMT_API int fpnmt_beam_search_prefix(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                       const int32_t* prefix_len, int p, int beam_groups, float diversity, float length_penalty,
+                                       int32_t* out_ids, int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
+                                       void* stream);
+
 /* Replaces: Pipeline.predict (utils/pipeline.py:82-154) for a batch: encoder + beam-search decode.
  * out_ids DEVICE-or-HOST int32 [batch, max_len] (0 padded), out_len int32 [batch]: exactly what predict() returns
  * per image (<start> stripped, trailing <end> stripped).  outputs_on_host != 0: results are copied to host and
@@ -368,6 +400,13 @@ FPNMT_API int fpnmt_op_dense(int device, int precision, const float* x, int R, i
  * and anything else the kernel does not write keep their contents.  K and F multiples of 8; bf16x3 is FPNMT_ERR_INVALID. */
 FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
                                    const float* bias, float* stat, float* val, int32_t* idx, void* stream);
+/* fpnmt_op_vocab_stats with the target epilogue of a prompted beam search on the logits-free tail: stat / val / idx as
+ * fpnmt_op_vocab_stats writes them, and for every row r < R whose target[r] lies in [0, F), target_logit[r] = z[r, target[r]],
+ * the fp32 value the tile's statistics and candidates are computed from (written in place; other entries keep their
+ * contents).  target DEVICE int32 [R] (-1 = none), target_logit DEVICE float32 [R]. */
+FPNMT_API int fpnmt_op_vocab_stats_target(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                          const float* bias, const int32_t* target, float* stat, float* val, int32_t* idx,
+                                          float* target_logit, void* stream);
 
 /* Encoder bandwidth kernels one at a time (the launchers of the engine's program, which choose the kernel by precision
  * and shape exactly as the engine does).  Activations are DEVICE float32, uploaded into bf16 (or bf16x3 hi + lo)

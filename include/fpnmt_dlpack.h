@@ -82,6 +82,14 @@ FPNMT_API int fpnmt_beam_search_dl(fpnmt_handle* h, const DLTensor* images, floa
 FPNMT_API int fpnmt_beam_search_diverse_dl(fpnmt_handle* h, const DLTensor* images, int beam_groups, float diversity,
                                            float length_penalty, DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob,
                                            int early_stop, void* stream);
+/* fpnmt_sample_prefix / fpnmt_beam_search_prefix: prefix_ids int32 [batch, p] (p from its shape) and prefix_len int32 [batch],
+ * both on the GPU; images and outputs as fpnmt_sample_dl / fpnmt_beam_search_dl. */
+FPNMT_API int fpnmt_sample_prefix_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids, const DLTensor* prefix_len,
+                                     const fpnmt_sampling* sampling, DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob,
+                                     int early_stop, void* stream);
+FPNMT_API int fpnmt_beam_search_prefix_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
+                                          const DLTensor* prefix_len, int beam_groups, float diversity, float length_penalty,
+                                          DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream);
 
 /* ---- in-library communicator: the ONE collective of the path (SURVEY §8e) -------------------------------------------
  * Image batches shard across the GPUs of a box; the only exchange is the all-gather of the caption ids.  The library opens

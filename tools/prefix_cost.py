@@ -1,0 +1,105 @@
+"""Cost of prompted decoding at the C2 size (ResNet-50-FPN 512x512, batch 64, beam 8, T = 64, V = 10000, 6 layers, bf16,
+synthetic weights, fixed length).
+
+    python tools/prefix_cost.py [--reps 10] [--out result.json]
+
+For the default kernels and for opts=("tgemm_wide",) (the logits-free decode tail):
+1. Engine.beam_search and Engine.sample unprompted and with prefixes of 0, 4 and 16 tokens for every image (all from the
+   images, early_stop=False, device outputs): CUDA events on the launching stream, the calls alternated, median over --reps.
+   A prompted call runs as many steps as an unprompted one; the forced steps only skip the ranking / the draw.
+2. In a run of its own, the vocabulary projection of the logits-free tail at the C2 shape (512 rows, K 512, V 10000) through
+   the stand-alone operators: tgemmw_kernel (fpnmt_op_vocab_stats, the unprompted search) against tgemmw_target_kernel
+   (fpnmt_op_vocab_stats_target, the prompted search), kernel time from torch.profiler (CUDA activity, mean over 50 launches
+   of each, alternated).
+
+The card's name and power limit are read in the same run and printed with the numbers.  Measured on one NVIDIA B200 at a
+1000 W power limit (--reps 7): beam_search 29.59 ms, with 0 / 4 / 16 prefix tokens 29.56 / 29.45 / 29.24 ms; sample 45.63 ms,
+45.71 / 44.69 / 41.72 ms; with tgemm_wide beam_search 35.57 ms, 35.86 / 35.75 / 35.66 ms, sample 51.56 ms, 51.62 / 50.63 /
+47.64 ms; the projection alone 34.3 us (tgemmw_kernel) against 35.2 us (tgemmw_target_kernel).
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "fpn-mt-image-captioning_b200"))
+
+
+def final_layer_us(reps=50):
+    import numpy as np
+    from torch.profiler import ProfilerActivity, profile
+    from fpnmt.engine import vocab_stats, vocab_stats_target
+    R, K, F = 512, 512, 10000
+    rng = np.random.default_rng(0)
+    x = torch.from_numpy(rng.standard_normal((R, K)).astype(np.float32)).cuda()
+    kern = (rng.standard_normal((K, F)) / np.sqrt(K)).astype(np.float32)
+    bias = (rng.standard_normal(F) * 0.1).astype(np.float32)
+    tgt = torch.from_numpy(rng.integers(0, F, R).astype(np.int32)).cuda()
+    vocab_stats(x, kern, bias)
+    vocab_stats_target(x, kern, tgt, bias)
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            vocab_stats(x, kern, bias)
+            vocab_stats_target(x, kern, tgt, bias)
+        torch.cuda.synchronize()
+    out = {}
+    for n in ("tgemmw_kernel", "tgemmw_target_kernel"):
+        ks = [e for e in prof.events() if n + "(" in e.name and e.device_type == torch.autograd.DeviceType.CUDA]
+        us = [e.device_time for e in ks] if ks and hasattr(ks[0], "device_time") else [e.cuda_time for e in ks]
+        out[n] = {"launches": len(us), "mean_us": sum(us) / max(1, len(us)), "median_us": sorted(us)[len(us) // 2] if us else None}
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=10)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    from fpnmt.engine import Engine
+    from fpnmt.weights import init_weights
+    B, N, T, V, S = 64, 8, 64, 10000, 512
+    w = init_weights("resnet50", vocab=V, seed=0)
+    g = torch.Generator(device="cuda").manual_seed(0)
+    img = torch.rand((B, S, S, 3), generator=g, device="cuda") * 2 - 1
+    prefix = torch.randint(4, V, (B, 16), generator=g, device="cuda", dtype=torch.int32)
+    res = {"config": "C2 size: resnet50 512x512, batch 64, beam 8, T 64, V 10000, 6 layers, bf16, fixed length; prefixes of "
+                     "random tokens, the same length for every image"}
+    for opts in ((), ("tgemm_wide",)):
+        eng = Engine(w, backbone="resnet50", batch=B, beam=N, vocab=V, max_len=T, image_size=S, opts=opts)
+        kw = dict(early_stop=False, to_host=False, return_logprobs=True)
+        sp = dict(temperature=0.9, top_k=50, top_p=0.95, seed=1)
+        calls = {"beam_search": lambda: eng.beam_search(img, **kw), "sample": lambda: eng.sample(img, **kw, **sp)}
+        for k in (0, 4, 16):
+            lens = torch.full((B,), k, dtype=torch.int32, device="cuda")
+            calls["beam_search_prefix%d" % k] = (lambda lens=lens: eng.beam_search(img, prefix=prefix, prefix_lens=lens, **kw))
+            calls["sample_prefix%d" % k] = (lambda lens=lens: eng.sample(img, prefix=prefix, prefix_lens=lens, **kw, **sp))
+        for f in calls.values():       # warm-up: module loads, graph capture, first-touch of the buffers
+            f()
+        torch.cuda.synchronize()
+        times = {k: [] for k in calls}
+        for _ in range(args.reps):
+            for k, f in calls.items():
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                f()
+                e1.record()
+                e1.synchronize()
+                times[k].append(e0.elapsed_time(e1))
+        res["default" if not opts else "+".join(opts)] = {"median_ms": {k: sorted(v)[len(v) // 2] for k, v in times.items()},
+                                                          "all_ms": times}
+        eng.close()
+    res["final_layer_C2_shape"] = final_layer_us()
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+    res["gpu"] = q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else torch.cuda.get_device_name()
+    print(json.dumps(res))
+    if args.out:
+        json.dump(res, open(args.out, "w"), indent=1)
+
+
+if __name__ == "__main__":
+    main()
