@@ -209,6 +209,35 @@ FPNMT_API int fpnmt_beam_search_prefix(fpnmt_handle* h, const float* images, int
   return h->eng->beam_search(images, images_on_host, beam_groups, diversity, length_penalty, out_ids, out_len, out_logprob,
                              outputs_on_host, early_stop, (cudaStream_t)stream, &pa);
 }
+FPNMT_API int fpnmt_sample_constrained(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                       const int32_t* prefix_len, int p, const fpnmt_sampling* sampling,
+                                       const fpnmt_constraints* constraints, int32_t* out_ids, int32_t* out_len,
+                                       float* out_logprob, int outputs_on_host, int early_stop, void* stream) {
+  CHECK_H(h);
+  if (!sampling || !constraints) {
+    set_last_error("sample_constrained: NULL sampling parameters / constraints");
+    return FPNMT_ERR_INVALID;
+  }
+  const PrefixArg pa{prefix_ids, prefix_len, p};
+  const bool prompted = prefix_ids || prefix_len || p;
+  return h->eng->sample(images, images_on_host, *sampling, out_ids, out_len, out_logprob, outputs_on_host, early_stop,
+                        (cudaStream_t)stream, prompted ? &pa : nullptr, constraints);
+}
+FPNMT_API int fpnmt_beam_search_constrained(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                            const int32_t* prefix_len, int p, int beam_groups, float diversity,
+                                            float length_penalty, const fpnmt_constraints* constraints, int32_t* out_ids,
+                                            int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
+                                            void* stream) {
+  CHECK_H(h);
+  if (!constraints) {
+    set_last_error("beam_search_constrained: NULL constraints");
+    return FPNMT_ERR_INVALID;
+  }
+  const PrefixArg pa{prefix_ids, prefix_len, p};
+  const bool prompted = prefix_ids || prefix_len || p;
+  return h->eng->beam_search(images, images_on_host, beam_groups, diversity, length_penalty, out_ids, out_len, out_logprob,
+                             outputs_on_host, early_stop, (cudaStream_t)stream, prompted ? &pa : nullptr, constraints);
+}
 FPNMT_API int fpnmt_stage_images(fpnmt_handle* h, const float* host_images, int slot) {
   CHECK_H(h);
   return h->eng->stage_images(host_images, slot);
@@ -727,9 +756,11 @@ FPNMT_API int fpnmt_op_layernorm_rows(int device, int precision, const float* x,
 
 }  // extern "C"
 
-// fpnmt_op_vocab_stats and, with target != nullptr, fpnmt_op_vocab_stats_target (tgemmw_target_kernel)
+// fpnmt_op_vocab_stats and, with target != nullptr, fpnmt_op_vocab_stats_target (tgemmw_target_kernel); with mask != nullptr,
+// fpnmt_op_vocab_stats_mask (tgemmw_mask_kernel)
 static int op_vocab_stats(int device, int precision, const float* x, int R, int K, const float* kernel, int F, const float* bias,
-                          const int32_t* target, float* target_logit, float* stat, float* val, int32_t* idx, void* stream) {
+                          const int32_t* target, float* target_logit, float* stat, float* val, int32_t* idx, void* stream,
+                          const uint32_t* mask = nullptr) {
   if (precision != FPNMT_PREC_BF16)
     return op_invalid("op_vocab_stats: the logits-free vocabulary projection is a bf16-mode kernel (the wide-row Dense kernel)");
   if (!x || !kernel || !stat || !val || !idx || R < 1 || K < 8 || K % 8 || F < 8 || F % 8 ||
@@ -756,6 +787,7 @@ static int op_vocab_stats(int device, int precision, const float* x, int R, int 
                         (float2*)stat, val, idx);
   op.tgt = target;
   op.tgt_logit = target_logit;
+  op.mask = mask;
   if (!o.rc) o.rc = tgemm_launch(op, o.s);
   return o.finish("op_vocab_stats");
 }
@@ -772,6 +804,39 @@ FPNMT_API int fpnmt_op_vocab_stats_target(int device, int precision, const float
                                           float* target_logit, void* stream) {
   if (!target || !target_logit) return op_invalid("op_vocab_stats_target: NULL target / target_logit");
   return op_vocab_stats(device, precision, x, R, K, kernel, F, bias, target, target_logit, stat, val, idx, stream);
+}
+
+FPNMT_API int fpnmt_op_vocab_stats_mask(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                        const float* bias, const uint32_t* mask, const int32_t* target, float* stat, float* val,
+                                        int32_t* idx, float* target_logit, void* stream) {
+  if (!mask) return op_invalid("op_vocab_stats_mask: NULL mask");
+  return op_vocab_stats(device, precision, x, R, K, kernel, F, bias, target, target_logit, stat, val, idx, stream, mask);
+}
+
+FPNMT_API int fpnmt_op_ban_mask(int device, const int32_t* hist, int ld, const int32_t* len, int rows, int vocab, int end_id,
+                                int no_repeat_ngram, int min_len, const int32_t* banned, int n_banned, uint32_t* mask,
+                                void* stream) {
+  if (!hist || !len || !mask || rows < 1 || ld < 1 || vocab < 1 || end_id < 0 || end_id >= vocab || no_repeat_ngram < 0 ||
+      no_repeat_ngram > ld || min_len < 0 || min_len > ld || n_banned < 0 || (n_banned > 0 && !banned))
+    return op_invalid("op_ban_mask: bad arguments (0 <= no_repeat_ngram, min_len <= ld; end_id in [0, vocab))");
+  const int W = (vocab + 31) / 32;
+  std::vector<uint32_t> hc(2 + W, 0u);
+  hc[0] = (uint32_t)no_repeat_ngram;
+  hc[1] = (uint32_t)min_len;
+  for (int i = 0; i < n_banned; ++i) {
+    if (banned[i] < 0 || banned[i] >= vocab || banned[i] == end_id)
+      return op_invalid("op_ban_mask: banned ids must lie in [0, vocab) and differ from end_id");
+    hc[2 + banned[i] / 32] |= 1u << (banned[i] % 32);
+  }
+  int rc = op_device(device, "op_ban_mask");
+  if (rc) return rc;
+  OpScratch o((cudaStream_t)stream, FPNMT_PREC_BF16);
+  uint32_t* dc = (uint32_t*)o.alloc(hc.size() * 4);
+  if (o.rc) return o.finish("op_ban_mask");
+  cudaMemcpyAsync(dc, hc.data(), hc.size() * 4, cudaMemcpyHostToDevice, o.s);
+  const BanMask bm{mask, dc, rows, W, vocab, end_id};
+  o.rc = launch_ban_rows(bm, 0, hist, ld, len, o.s);
+  return o.finish("op_ban_mask");
 }
 
 FPNMT_API int fpnmt_op_sample_step(int device, const float* logits, int rows, int V, int samples_per_image, int t,

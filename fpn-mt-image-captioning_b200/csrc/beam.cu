@@ -80,8 +80,12 @@ __device__ __forceinline__ void warp_argmax(float& v, int& i) {
 //                          last image advance the device step counter.
 //   PREFIX (prompted N-best decode, BeamState::pf): at a step inside the image's prefix every row's one candidate is the prefix
 //                          token, scored with the expression of the free branch, and phase 2 keeps every beam on its own row.
-template <int THREADS, bool NBEST = false, bool PREFIX = false>
-__global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(BeamState st, const float* __restrict__ logits, int ld, BeamEmbed em) {
+//   MASK (constrained decode, `ban`; only with NBEST and PREFIX): a live unforced row ranks allowed tokens only (its lse stays
+//                          over all V), and phase 2 writes every new beam's ban set of step t + 1.  `ban` is the last parameter,
+//                          so the other instantiations keep their parameter offsets and code.
+template <int THREADS, bool NBEST = false, bool PREFIX = false, bool MASK = false>
+__global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(BeamState st, const float* __restrict__ logits, int ld, BeamEmbed em,
+                                                                                BanMask ban) {
   constexpr int NW = THREADS / 32;
   extern __shared__ float4 s_row4[];                       // the row's logits (later: candidate scores), nv4*THREADS float4
   __shared__ float s_m[NW], s_s[NW];
@@ -143,8 +147,14 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
         s_s[warp] = wsum;
       }
     }
-    // tile maxima: the N-th largest of them bounds the N-th best logit of the row from below
-    for (int i = tid; i < nt; i += THREADS) s_cv[i] = __ldcg(stt + i).x;
+    // tile maxima: the N-th largest of them bounds the N-th best logit of the row from below.  MASK: each tile's best ALLOWED
+    // logit (its first candidate; the projection skipped the banned ones) - a banned tile maximum would lift tau above every
+    // allowed candidate.  N distinct tiles still reach tau, and a tile holds at most N - 1 <= 7 better allowed logits.
+    if constexpr (MASK) {
+      for (int i = tid; i < nt; i += THREADS) s_cv[i] = __ldcg(cvv + (size_t)i * 8);
+    } else {
+      for (int i = tid; i < nt; i += THREADS) s_cv[i] = __ldcg(stt + i).x;
+    }
     if (tid == 0) {
       s_cnt2 = 0;
       s_tau = -INFINITY;
@@ -252,7 +262,30 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       s_m[warp] = wm;
       s_s[warp] = sum;
     }
-    s_cv[warp * 32 + lane] = tmax_v;                        // thread maxima, for the selection threshold below
+    float tsel = tmax_v;
+    if constexpr (MASK) {
+      // banned tokens -> -inf in the staged row (own slots: no barrier), after the unmasked statistics above; the thread
+      // maxima behind tau, the pre-filter, the gather and the exact fallback below then see allowed tokens only.  A forced
+      // row keeps its row: it reads its prefix token's logit.
+      if (!(PREFIX && ftok >= 0)) {
+        const uint32_t* mk = ban_row(ban, t, row);
+        tsel = -INFINITY;
+        for (int i = 0; i < nv4; ++i) {
+          const int e = (i * THREADS + tid) * 4;
+          float4 q = s_row4[i * THREADS + tid];
+          const uint32_t bits = e < V ? (__ldcg(mk + (e >> 5)) >> (e & 31)) & 15u : 0u;
+          if (bits) {
+            if (bits & 1u) q.x = -INFINITY;
+            if (bits & 2u) q.y = -INFINITY;
+            if (bits & 4u) q.z = -INFINITY;
+            if (bits & 8u) q.w = -INFINITY;
+            s_row4[i * THREADS + tid] = q;
+          }
+          tsel = fmaxf(tsel, fmaxf(fmaxf(q.x, q.y), fmaxf(q.z, q.w)));
+        }
+      }
+    }
+    s_cv[warp * 32 + lane] = tsel;                          // thread maxima, for the selection threshold below
   }
   constexpr int CAP = 128;
   __shared__ float s_lv[CAP];
@@ -587,6 +620,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 4 : 2) k_beam_step(B
       if (lane == 0) danc[t] = rows0 + apar;
     }
     if (lane == 0) dseq[t + 1] = tok;
+    if constexpr (MASK) {                                             // the new beam's ban set of step t + 1 from its caption
+      __syncwarp();
+      if (t + 1 < T) ban_row_warp(ban_row(ban, t + 1, rows0 + n), ban, dseq + 1, t + 1);
+    }
   }
   BDBG(10);
   // next step's decoder input: x[row] = embedding[token] + pos[t + 1]   (transformer.py:326-329)
@@ -680,6 +717,8 @@ int beam_set_attributes() {   // per device (Engine::init)
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<256, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<256, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_beam_step<512, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return 0;
 }
 int check_beam_step(const BeamState& st, int ld) {
@@ -702,13 +741,14 @@ int check_beam_step(const BeamState& st, int ld) {
   }
   return 0;
 }
-template <bool NBEST, bool PREFIX = false>
-static int launch_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
+template <bool NBEST, bool PREFIX = false, bool MASK = false>
+static int launch_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s,
+                       const BanMask& ban = BanMask{}) {
   if (check_beam_step(st, ld)) return 1;
   if (st.vs_stat) {                                         // logits-free tail: merge the vocabulary projection's candidates
     size_t smem = (size_t)st.vs_tiles * 8 * 8;
     if (smem < 12288) smem = 12288;
-    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST, PREFIX>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST, PREFIX, MASK>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em, ban));
     return 0;
   }
   const int threads = st.V <= 16384 ? 256 : 512;
@@ -716,9 +756,9 @@ static int launch_step(const BeamState& st, const float* logits, int ld, const B
   size_t smem = (size_t)nv4 * threads * 16;
   if (smem < 12288) smem = 12288;                           // phase 2 keeps the N x N merge lists (values, flat ids, keys) there
   if (threads == 256)
-    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST, PREFIX>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<256, NBEST, PREFIX, MASK>, dim3(st.B * st.N), dim3(256), smem, s, st, logits, ld, em, ban));
   else
-    FPNMT_CUDA_OK(launch_k(k_beam_step<512, NBEST, PREFIX>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em));
+    FPNMT_CUDA_OK(launch_k(k_beam_step<512, NBEST, PREFIX, MASK>, dim3(st.B * st.N), dim3(512), smem, s, st, logits, ld, em, ban));
   return 0;
 }
 int launch_beam_step(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s) {
@@ -752,6 +792,35 @@ int launch_beam_step_prefix(const BeamState& st, const float* logits, int ld, co
     return 1;
   }
   return launch_step<true, true>(st, logits, ld, em, s);
+}
+int launch_beam_step_constrained(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, const BanMask& ban,
+                                 cudaStream_t s) {
+  if (!ban.mask || !ban.cfg || ban.rows != st.B * st.N || ban.V != st.V || ban.W != (st.V + 31) / 32) {
+    set_last_error("beam_step_constrained: needs the ban masks of every row");
+    return 1;
+  }
+  if (!st.pf.ids || !st.pf.len || (st.vs_stat && (!st.pf.tgt || !st.pf.tgt_logit))) {
+    set_last_error("beam_step_constrained: needs the prefix buffers (and on the logits-free tail the target ids and logits)");
+    return 1;
+  }
+  if (!st.finished_mode || st.prob_mode || !st.nb.ids || !st.nb.len || !st.nb.score || !st.nb.groups) {
+    set_last_error("beam_step_constrained: needs finished beams, log scores, the N-best outputs and the beam-group words");
+    return 1;
+  }
+  return launch_step<true, true, true>(st, logits, ld, em, s, ban);
+}
+
+// Step 0's ban sets (hist == nullptr) and fpnmt_op_ban_mask: one warp per row
+__global__ void k_ban_rows(BanMask bm, int t, const int* __restrict__ hist, int ld, const int* __restrict__ len) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= bm.rows) return;
+  const int n = len ? len[row] : 0;
+  ban_row_warp(ban_row(bm, t, row), bm, hist ? hist + (size_t)row * ld : nullptr, hist ? min(max(n, 0), ld) : 0);
+}
+int launch_ban_rows(const BanMask& bm, int t, const int* hist, int ld, const int* len, cudaStream_t s) {
+  k_ban_rows<<<(bm.rows + 3) / 4, 128, 0, s>>>(bm, t, hist, ld, len);
+  LAUNCH_CHECK();
+  return 0;
 }
 
 // Prompted decode: one block per image copies and checks its prefix (see kernels.cuh)

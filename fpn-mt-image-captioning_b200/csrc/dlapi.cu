@@ -328,6 +328,44 @@ FPNMT_API int fpnmt_beam_search_prefix_dl(fpnmt_handle* h, const DLTensor* image
                                   length_penalty, (int32_t*)pids, (int32_t*)plen, (float*)plp, ids_host, early_stop, stream);
 }
 
+// the optional prefix of a constrained call: both DLTensors NULL (unprompted: NULL / NULL / 0) or dl_prefix's checks
+static int dl_prefix_opt(fpnmt_handle* h, const std::string& fn, const DLTensor* prefix_ids, const DLTensor* prefix_len,
+                         void** pids, void** plen, int* p) {
+  if (!prefix_ids && !prefix_len) return 0;
+  return dl_prefix(h, fn, prefix_ids, prefix_len, pids, plen, p);
+}
+
+FPNMT_API int fpnmt_sample_constrained_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
+                                          const DLTensor* prefix_len, const fpnmt_sampling* sampling,
+                                          const fpnmt_constraints* constraints, DLTensor* out_ids, DLTensor* out_len,
+                                          DLTensor* out_logprob, int early_stop, void* stream) {
+  CHECK_H(h);
+  void *pi = nullptr, *pp = nullptr, *pl = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
+  int img_host = 0, ids_host = 0, p = 0;
+  int rc = dl_images_opt(h, "sample_constrained_dl", images, &pi, &img_host);
+  if (!rc) rc = dl_prefix_opt(h, "sample_constrained_dl", prefix_ids, prefix_len, &pp, &pl, &p);
+  if (!rc) rc = dl_captions(h, "sample_constrained_dl", out_ids, out_len, out_logprob, &pids, &plen, &plp, &ids_host);
+  if (rc) return rc;
+  return fpnmt_sample_constrained(h, (const float*)pi, img_host, (const int32_t*)pp, (const int32_t*)pl, p, sampling, constraints,
+                                  (int32_t*)pids, (int32_t*)plen, (float*)plp, ids_host, early_stop, stream);
+}
+
+FPNMT_API int fpnmt_beam_search_constrained_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
+                                               const DLTensor* prefix_len, int beam_groups, float diversity, float length_penalty,
+                                               const fpnmt_constraints* constraints, DLTensor* out_ids, DLTensor* out_len,
+                                               DLTensor* out_logprob, int early_stop, void* stream) {
+  CHECK_H(h);
+  void *pi = nullptr, *pp = nullptr, *pl = nullptr, *pids = nullptr, *plen = nullptr, *plp = nullptr;
+  int img_host = 0, ids_host = 0, p = 0;
+  int rc = dl_images_opt(h, "beam_search_constrained_dl", images, &pi, &img_host);
+  if (!rc) rc = dl_prefix_opt(h, "beam_search_constrained_dl", prefix_ids, prefix_len, &pp, &pl, &p);
+  if (!rc) rc = dl_captions(h, "beam_search_constrained_dl", out_ids, out_len, out_logprob, &pids, &plen, &plp, &ids_host);
+  if (rc) return rc;
+  return fpnmt_beam_search_constrained(h, (const float*)pi, img_host, (const int32_t*)pp, (const int32_t*)pl, p, beam_groups,
+                                       diversity, length_penalty, constraints, (int32_t*)pids, (int32_t*)plen, (float*)plp,
+                                       ids_host, early_stop, stream);
+}
+
 // fpnmt_beam_search_dl and fpnmt_beam_search_diverse_dl: the same shape checks, then the diverse entry (G = 1 is
 // fpnmt_beam_search)
 static int beam_search_dl(const char* name, fpnmt_handle* h, const DLTensor* images, int beam_groups, float diversity,

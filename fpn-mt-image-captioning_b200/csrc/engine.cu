@@ -48,6 +48,8 @@ Engine::~Engine() {
   if (nbest_graph_) cudaGraphExecDestroy(nbest_graph_);
   if (nbest_pfx_graph_) cudaGraphExecDestroy(nbest_pfx_graph_);
   if (sample_pfx_graph_) cudaGraphExecDestroy(sample_pfx_graph_);
+  if (nbest_con_graph_) cudaGraphExecDestroy(nbest_con_graph_);
+  if (sample_con_graph_) cudaGraphExecDestroy(sample_con_graph_);
   for (auto& kv : score_graphs_)
     if (kv.second) cudaGraphExecDestroy(kv.second);
   if (cap_stream_) cudaStreamDestroy(cap_stream_);
@@ -1792,13 +1794,15 @@ int Engine::generate(const float* images, int on_host, int32_t* out_ids, int32_t
 // k_sample_step draws its next token, so the N rows of an image are N independent samples.  The sampling parameters live in a
 // device struct the kernel reads: a captured sample_graph_ serves every parameter set.
 int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len,
-                   float* out_logprob, int out_on_host, int early_stop, cudaStream_t s, const PrefixArg* prefix) {
+                   float* out_logprob, int out_on_host, int early_stop, cudaStream_t s, const PrefixArg* prefix,
+                   const fpnmt_constraints* con) {
   RC(check_decode_entry("sample", "has no sampling tail"));
   const int B = cfg_.batch, N = cfg_.beam, T = cfg_.max_len, V = cfg_.vocab, R = B * N;
   if (check_sampling(sp, V))
     return fail(FPNMT_ERR_INVALID, "sample: temperature >= 0, top_p in (0, 1], 0 <= top_k <= vocab and reserved words 0");
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "sample: NULL out_ids / out_len");
-  RC(check_prefix("sample_prefix", prefix));
+  RC(check_prefix(con ? "sample_constrained" : "sample_prefix", prefix));
+  RC(check_constraints("sample_constrained", con));
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   if (!ss_.ids) {   // per-row buffers [R][T] + [R] x 3 and the per-image counters, on the first call
     SampleState st{};
@@ -1831,15 +1835,32 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
     o.name = "sample_step(prefix)";
     o.run = [st, lg, pid, pln](cudaStream_t q) { return launch_sample_step_prefix(st, pid, pln, lg, q); };
   }
+  if (con && sample_con_prog_.empty()) {      // constrained: the same program with the masked sample op
+    const SampleState st = ss_;
+    const float* lg = logits_;
+    const int *pid = pfx_ids_, *pln = pfx_len_;
+    const BanMask bm = ban_;
+    sample_con_prog_ = sample_prog_;
+    Op& o = sample_con_prog_.back();
+    o.name = "sample_step(constrained)";
+    o.run = [st, lg, pid, pln, bm](cudaStream_t q) { return launch_sample_step_constrained(st, pid, pln, lg, bm, q); };
+  }
   const SampleParams prm{sp.temperature, sp.top_k, sp.top_p, 0, (unsigned long long)sp.seed};
   if (images) RC(encode(images, on_host, nullptr, s, false));
   FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<SampleParams*>(ss_.params), &prm, sizeof prm, cudaMemcpyHostToDevice, s));
   RC(run_program(dec_init_prog_, s));
-  if (prefix) RC(load_prefix(*prefix, s));
+  if (con) RC(load_constraints(*con, prefix, s));
+  else if (prefix) RC(load_prefix(*prefix, s));
   RC(launch_sample_init(ss_, bs_.anc[0], s));
   launches += 1;
   FlagGuard forced(forced_mode_);   // the self-attention launches of the program stay in the first buffer pair, without representatives
-  if (prefix) {
+  if (con) {
+    RC(run_steps(sample_con_prog_, sample_con_graph_, bs_.n_done, early_stop, s));
+    if (prefix) {
+      RC(launch_prefix_flag(pfx_bad_, B, N, T, ss_.ids, ss_.len, ss_.lp, s));
+      launches += 1;
+    }
+  } else if (prefix) {
     RC(run_steps(sample_pfx_prog_, sample_pfx_graph_, bs_.n_done, early_stop, s));
     RC(launch_prefix_flag(pfx_bad_, B, N, T, ss_.ids, ss_.len, ss_.lp, s));
     launches += 1;
@@ -1861,14 +1882,15 @@ int Engine::sample(const float* images, int on_host, const fpnmt_sampling& sp, i
 // every (G, lambda, alpha) and bs_.lp, which generate reads, is never touched.  fpnmt_beam_search is G = 1.
 int Engine::beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty,
                         int32_t* out_ids, int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s,
-                        const PrefixArg* prefix) {
+                        const PrefixArg* prefix, const fpnmt_constraints* con) {
   RC(check_decode_entry("beam_search", "has no N-best tail"));
   if (cfg_.score_mode == FPNMT_SCORE_PROB)
     return fail(FPNMT_ERR_STATE, "beam_search: the length penalty and the log-likelihoods need score_mode = log");
   if (!std::isfinite(length_penalty)) return fail(FPNMT_ERR_INVALID, "beam_search: length_penalty must be finite");
   if (check_beam_groups(step_bsv_, beam_groups, diversity)) return FPNMT_ERR_INVALID;
   if (!out_ids || !out_len) return fail(FPNMT_ERR_INVALID, "beam_search: NULL out_ids / out_len");
-  RC(check_prefix("beam_search_prefix", prefix));
+  RC(check_prefix(con ? "beam_search_constrained" : "beam_search_prefix", prefix));
+  RC(check_constraints("beam_search_constrained", con));
   FPNMT_CUDA_OK(cudaSetDevice(dev_));
   const int B = cfg_.batch, T = cfg_.max_len, R = B * cfg_.beam;
   if (!nbest_bs_.nb.ids) {
@@ -1916,18 +1938,54 @@ int Engine::beam_search(const float* images, int on_host, int beam_groups, float
     o.run = [st, lg, V, em](cudaStream_t q) { return launch_beam_step_prefix(st, lg, V, em, q); };
     nbest_pfx_bs_ = st;
   }
+  if (con && nbest_con_prog_.empty()) {
+    // constrained: the prompted program's state (prefix buffers, target logits) with the masked beam op and, on the logits-free
+    // tail, the masked vocabulary projection (it reads the ban sets of the step parity in bs_.step)
+    BeamState st = nbest_bs_;
+    st.pf.ids = pfx_ids_;
+    st.pf.len = pfx_len_;
+    const BanMask bm = ban_;
+    nbest_con_prog_ = nbest_prog_;
+    if (st.vs_stat) {
+      st.pf.tgt = pfx_tgt_;
+      st.pf.tgt_logit = pfx_tgt_logit_;
+      TgemmOp op = vs_final_op_;
+      op.tgt = pfx_tgt_;
+      op.tgt_logit = pfx_tgt_logit_;
+      op.mask = bm.mask;
+      op.mask_step = st.step;
+      Op& f = nbest_con_prog_[step_final_at_];
+      f.name = "final_layer(softmax partials + allowed candidates + target logit)";
+      f.run = [op](cudaStream_t q) { return tgemm_launch(op, q); };
+    }
+    const float* lg = logits_;
+    const BeamEmbed em = beam_embed_;
+    const int V = cfg_.vocab;
+    Op& o = nbest_con_prog_[step_beam_at_];
+    o.name = "beam_step(n-best, constrained)";
+    o.run = [st, lg, V, em, bm](cudaStream_t q) { return launch_beam_step_constrained(st, lg, V, em, bm, q); };
+    nbest_con_bs_ = st;
+  }
   std::vector<float> lp(T + 4);
   for (int i = 0; i < T + 2; ++i) lp[i] = powf((5.f + (float)i) / 6.f, length_penalty);
   lp[T + 2] = (float)beam_groups;
   lp[T + 3] = beam_groups > 1 ? diversity : 0.f;
   if (images) RC(encode(images, on_host, nullptr, s, false));
   FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<float*>(nbest_bs_.lp), lp.data(), lp.size() * 4, cudaMemcpyHostToDevice, s));
-  if (prefix) RC(load_prefix(*prefix, s));                  // before the init kernel, which writes step 0's targets
-  RC(launch_beam_init(prefix ? nbest_pfx_bs_ : nbest_bs_, 1, s, beam_groups));
+  // before the init kernel, which writes step 0's targets
+  if (con) RC(load_constraints(*con, prefix, s));
+  else if (prefix) RC(load_prefix(*prefix, s));
+  RC(launch_beam_init(con ? nbest_con_bs_ : prefix ? nbest_pfx_bs_ : nbest_bs_, 1, s, beam_groups));
   launches += 1;
   RC(run_program(dec_init_prog_, s));
   RC(run_program(embed_prog_, s));
-  if (prefix) {
+  if (con) {
+    RC(run_steps(nbest_con_prog_, nbest_con_graph_, nbest_bs_.n_done, early_stop, s));
+    if (prefix) {
+      RC(launch_prefix_flag(pfx_bad_, B, cfg_.beam, T, nbest_bs_.nb.ids, nbest_bs_.nb.len, nbest_bs_.nb.score, s));
+      launches += 1;
+    }
+  } else if (prefix) {
     RC(run_steps(nbest_pfx_prog_, nbest_pfx_graph_, nbest_bs_.n_done, early_stop, s));
     RC(launch_prefix_flag(pfx_bad_, B, cfg_.beam, T, nbest_bs_.nb.ids, nbest_bs_.nb.len, nbest_bs_.nb.score, s));
     launches += 1;
@@ -1947,6 +2005,9 @@ int Engine::check_prefix(const char* entry, const PrefixArg* prefix) {
   const std::string e = entry;
   if (!prefix->ids || !prefix->len) return fail(FPNMT_ERR_INVALID, e + ": NULL prefix_ids / prefix_len");
   if (prefix->p < 1 || prefix->p > cfg_.max_len - 1) return fail(FPNMT_ERR_INVALID, e + ": p must be 1 .. max_len - 1");
+  return alloc_prefix();
+}
+int Engine::alloc_prefix() {
   if (!pfx_ids_) {
     FPNMT_CUDA_OK(cudaSetDevice(dev_));
     const int B = cfg_.batch, R = B * cfg_.beam;
@@ -1957,6 +2018,60 @@ int Engine::check_prefix(const char* entry, const PrefixArg* prefix) {
     pfx_tgt_logit_ = (float*)dalloc((size_t)R * 4);
     if (!pfx_ids_ || !pfx_len_ || !pfx_bad_ || !pfx_tgt_ || !pfx_tgt_logit_) return FPNMT_ERR_CUDA;
   }
+  return 0;
+}
+
+// The refusals of a constraint set (nothing launched) and, on the first constrained call, the ban masks and the prefix buffers
+// the constrained programs always carry.
+int Engine::check_constraints(const char* entry, const fpnmt_constraints* con) {
+  if (!con) return 0;
+  const std::string e = entry;
+  const int V = cfg_.vocab, T = cfg_.max_len;
+  if (con->reserved[0] || con->reserved[1] || con->reserved[2] || con->reserved[3])
+    return fail(FPNMT_ERR_INVALID, e + ": reserved words must be 0");
+  if (con->no_repeat_ngram < 0 || con->no_repeat_ngram > T) return fail(FPNMT_ERR_INVALID, e + ": no_repeat_ngram must be 0 .. max_len");
+  if (con->min_len < 0 || con->min_len > T) return fail(FPNMT_ERR_INVALID, e + ": min_len must be 0 .. max_len");
+  if (con->n_banned < 0 || (con->n_banned > 0 && !con->banned)) return fail(FPNMT_ERR_INVALID, e + ": NULL banned with n_banned > 0");
+  std::vector<char> seen(V, 0);
+  int distinct = 0;
+  for (int i = 0; i < con->n_banned; ++i) {
+    const int v = con->banned[i];
+    if (v < 0 || v >= V) return fail(FPNMT_ERR_INVALID, e + ": banned id " + std::to_string(v) + " outside [0, vocab)");
+    if (v == cfg_.end_id) return fail(FPNMT_ERR_INVALID, e + ": <end> cannot be banned (min_len holds it back)");
+    distinct += seen[v] ? 0 : 1;
+    seen[v] = 1;
+  }
+  if (V - distinct - T < cfg_.beam)
+    return fail(FPNMT_ERR_INVALID, e + ": vocab - distinct banned ids - max_len must be >= beam (allowed tokens at every step)");
+  RC(alloc_prefix());
+  if (!ban_.mask) {
+    FPNMT_CUDA_OK(cudaSetDevice(dev_));                      // the entry points set the device only after these checks
+    const int W = (V + 31) / 32, R = cfg_.batch * cfg_.beam;
+    ban_.mask = (uint32_t*)dalloc((size_t)2 * R * W * 4);
+    ban_.cfg = (const uint32_t*)dalloc((size_t)(2 + W) * 4);
+    if (!ban_.mask || !ban_.cfg) return FPNMT_ERR_CUDA;
+    ban_.rows = R;
+    ban_.W = W;
+    ban_.V = V;
+    ban_.end_id = cfg_.end_id;
+  }
+  return 0;
+}
+
+// (n, min_len, S) -> ban_.cfg, the prefixes (all prefix_len 0 for an unprompted call), then step 0's ban sets
+int Engine::load_constraints(const fpnmt_constraints& con, const PrefixArg* prefix, cudaStream_t s) {
+  std::vector<uint32_t> h(2 + ban_.W, 0u);
+  h[0] = (uint32_t)con.no_repeat_ngram;
+  h[1] = (uint32_t)con.min_len;
+  for (int i = 0; i < con.n_banned; ++i) h[2 + con.banned[i] / 32] |= 1u << (con.banned[i] % 32);
+  FPNMT_CUDA_OK(cudaMemcpyAsync(const_cast<uint32_t*>(ban_.cfg), h.data(), h.size() * 4, cudaMemcpyHostToDevice, s));
+  if (prefix) {
+    RC(load_prefix(*prefix, s));
+  } else {
+    FPNMT_CUDA_OK(cudaMemsetAsync(pfx_len_, 0, (size_t)cfg_.batch * 4, s));
+  }
+  RC(launch_ban_rows(ban_, 0, nullptr, 0, nullptr, s));
+  launches += 1;
   return 0;
 }
 

@@ -80,9 +80,11 @@ class Engine {
                float* step_scores, cudaStream_t s);
   // Sampled decode (fpnmt_sample): every row of the batch is one independent sample of its image; the teacher-forced step
   // program with k_sample_step in place of the teacher-forced tail.  images == nullptr: the memory of the last encode.
-  // prefix != nullptr: the prompted decode (fpnmt_sample_prefix) on sample_pfx_prog_.
+  // prefix != nullptr: the prompted decode (fpnmt_sample_prefix) on sample_pfx_prog_.  con != nullptr: the constrained decode
+  // (fpnmt_sample_constrained, prompted or not) on sample_con_prog_.
   int sample(const float* images, int on_host, const fpnmt_sampling& sp, int32_t* out_ids, int32_t* out_len, float* out_logprob,
-             int out_on_host, int early_stop, cudaStream_t s, const PrefixArg* prefix = nullptr);
+             int out_on_host, int early_stop, cudaStream_t s, const PrefixArg* prefix = nullptr,
+             const fpnmt_constraints* con = nullptr);
   // Caption scoring (fpnmt_score): the N captions ids [B][N][t] / lens [B][N] (device) of every image through the decoder
   // as B * N * t rows of one teacher-forced pass.  images == nullptr: the memory of the last encode.
   int score(const float* images, int on_host, const int32_t* ids, const int32_t* lens, int t, float* out_logprob,
@@ -90,10 +92,11 @@ class Engine {
   // N-best beam search (fpnmt_beam_search: beam_groups = 1) and diverse beam search (fpnmt_beam_search_diverse): the
   // whole-batch step program with k_beam_step's group ranking and N-best close, true-beam start (first beam of every group),
   // frozen finished beams and this call's length penalty.  images == nullptr: the memory of the last encode.
-  // prefix != nullptr: the prompted search (fpnmt_beam_search_prefix) on nbest_pfx_prog_.
+  // prefix != nullptr: the prompted search (fpnmt_beam_search_prefix) on nbest_pfx_prog_.  con != nullptr: the constrained
+  // search (fpnmt_beam_search_constrained, prompted or not) on nbest_con_prog_.
   int beam_search(const float* images, int on_host, int beam_groups, float diversity, float length_penalty, int32_t* out_ids,
                   int32_t* out_len, float* out_logprob, int out_on_host, int early_stop, cudaStream_t s,
-                  const PrefixArg* prefix = nullptr);
+                  const PrefixArg* prefix = nullptr, const fpnmt_constraints* con = nullptr);
   int profile(int iters, char* buf, size_t cap);
   int build_dstep(const Tensor& ckv, const float* d_emb, const float* d_pos);
   int get_tap_f32(const std::string& name, float* out, size_t cap, size_t* count, cudaStream_t s);
@@ -150,7 +153,18 @@ class Engine {
   int *pfx_ids_ = nullptr, *pfx_len_ = nullptr, *pfx_bad_ = nullptr, *pfx_tgt_ = nullptr;   // [B][T], [B], [B], [B*N]
   float* pfx_tgt_logit_ = nullptr;                                                          // [B*N]
   int check_prefix(const char* entry, const PrefixArg* prefix);
+  int alloc_prefix();
   int load_prefix(const PrefixArg& prefix, cudaStream_t s);
+  // constrained decode (built on its first call): copies of the prompted programs (an unprompted call runs them with every
+  // prefix_len 0) with the beam / sample op replaced by its MASK variant and, on the logits-free tail, the vocabulary projection
+  // by tgemmw_mask_kernel.  The ban sets live in ban_ (one buffer pair for both programs); each call uploads (n, min_len, S)
+  // and writes step 0's sets, so one captured graph serves every constraint set.
+  Program nbest_con_prog_, sample_con_prog_;
+  BeamState nbest_con_bs_{};
+  cudaGraphExec_t nbest_con_graph_ = nullptr, sample_con_graph_ = nullptr;
+  BanMask ban_{};
+  int check_constraints(const char* entry, const fpnmt_constraints* con);
+  int load_constraints(const fpnmt_constraints& con, const PrefixArg* prefix, cudaStream_t s);
   SampleState ss_{};                      // sampler state: per-row buffers allocated on the first sample call
   cudaGraphExec_t sample_graph_ = nullptr;   // sample_prog_ captured with forced_mode_ set (never step_graph_)
   // score pass: one program (and graph) per caption length t, built on its first call; activations for B * N * max_len rows

@@ -160,6 +160,42 @@ struct BeamState {
 };
 static_assert(sizeof(BeamState::NBest) == 32, "see BeamState::NBest::groups");
 static_assert(sizeof(BeamState::Prefix) == 32, "see BeamState::NBest::groups");
+// Constrained decoding (fpnmt_constraints, include/fpnmt.h): a row's ban set A(t) = S | E(t) | R(t) as a bit mask of
+// W = ceil(V / 32) words (bit v % 32 of word v / 32 set: token v is banned), double-buffered by step parity like the beam
+// scores: the row's set at step t is mask + ((t & 1) * rows + row) * W.  The step kernel of step t writes every row's set of
+// step t + 1; launch_ban_rows writes step 0's.  The (n, min_len) words and S are uploaded per call, so one captured graph
+// serves every constraint set.
+struct BanMask {
+  uint32_t* mask;            // [2][rows][W]
+  const uint32_t* cfg;       // [2 + W]: no_repeat_ngram n (0 = off), min_len, then the static mask S
+  int rows, W, V, end_id;
+};
+__device__ __forceinline__ uint32_t* ban_row(const BanMask& bm, int t, int row) {
+  return bm.mask + ((size_t)(t & 1) * bm.rows + row) * bm.W;
+}
+// One full warp writes dst[0 .. W) = the ban set of a row whose caption so far is w[0 .. len) (no <start>, prefix tokens
+// included), at step len: S; <end> while len < min_len; and, for n >= 1, R = every token w[j + n - 1] whose n - 1
+// predecessors w[j .. j + n - 2] equal the caption's last n - 1 tokens (n = 1: every token of the caption).  The shared
+// definition of the beam step, the sample step and fpnmt_op_ban_mask.  Readers are later kernels.
+__device__ __forceinline__ void ban_row_warp(uint32_t* dst, const BanMask& bm, const int* w, int len) {
+  const int lane = threadIdx.x & 31;
+  const int n = (int)bm.cfg[0], min_len = (int)bm.cfg[1];
+  for (int i = lane; i < bm.W; i += 32) dst[i] = bm.cfg[2 + i];
+  __syncwarp();
+  if (lane == 0 && len < min_len) atomicOr(dst + (bm.end_id >> 5), 1u << (bm.end_id & 31));
+  if (n >= 1) {
+    for (int j = lane; j <= len - n; j += 32) {
+      bool match = true;
+      for (int k = 0; k < n - 1 && match; ++k) match = w[j + k] == w[len - n + 1 + k];
+      const int v = w[j + n - 1];
+      if (match && v >= 0 && v < bm.V) atomicOr(dst + (v >> 5), 1u << (v & 31));
+    }
+  }
+}
+// dst rows [0, rows) of step t's parity: ban_row_warp of hist[r][0 .. len[r]) (hist [rows][ld]; hist / len nullptr: the
+// empty caption, step 0's sets)
+int launch_ban_rows(const BanMask& bm, int t, const int* hist, int ld, const int* len, cudaStream_t s);
+
 // true_beam = 0 reproduces the reference (all beams start identical, pipeline.py:101-102); 1 starts only the first beam of
 // each of beam_groups groups of N / beam_groups beams alive (beam_groups = 1: beams 1..N-1 dead)
 int launch_beam_init(const BeamState& st, int true_beam, cudaStream_t s, int beam_groups = 1);
@@ -178,6 +214,11 @@ int launch_beam_step(const BeamState& st, const float* logits, int ld, const Bea
 int launch_beam_step_nbest(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
 // The N-best step of a prompted decode: forced steps inside each image's prefix (BeamState::pf), the N-best step after it.
 int launch_beam_step_prefix(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, cudaStream_t s);
+// The prompted N-best step with a ban set per row (BanMask): a live, unforced row never ranks a banned token (the logits path
+// masks its row; on the logits-free tail the vocabulary projection's candidates already skip them and tau comes from each
+// tile's best allowed logit); its log-softmax stays over all V.  Phase 2 writes every new beam's set of step t + 1.
+int launch_beam_step_constrained(const BeamState& st, const float* logits, int ld, const BeamEmbed& em, const BanMask& ban,
+                                 cudaStream_t s);
 // Prompted decode, before the first step: dst_ids[b][j] = prefix_ids[b][j] for j < prefix_len[b] (ids clamped to [0, V)
 // before they are stored), 0 elsewhere ([B][T]); bad[b] = 1 when prefix_len[b] is outside [0, p] or one of its first
 // prefix_len[b] ids is outside [0, V) or equals end_id; dst_len[b] = bad[b] ? 0 : prefix_len[b].  prefix_ids DEVICE [B][p].
@@ -238,6 +279,11 @@ int launch_sample_step(const SampleState& st, const float* logits, cudaStream_t 
 // The step of a prompted decode (engine state only): at a step t < pfx_len[b] every row of image b takes pfx_ids[b][t] with no
 // draw; the sampling step after it.  pfx_ids [images][T] / pfx_len [images]: launch_prefix_load's buffers.
 int launch_sample_step_prefix(const SampleState& st, const int* pfx_ids, const int* pfx_len, const float* logits, cudaStream_t s);
+// The prompted step with a ban set per row (BanMask): the arg-max, top-k, the tempered masses (relative to the largest allowed
+// logit) and the draw see z with the banned logits at -inf; the log-probability stays log_softmax of the unmasked z.  The
+// row's CTA then writes its own set of step t + 1 from ids[row][0 .. len).
+int launch_sample_step_constrained(const SampleState& st, const int* pfx_ids, const int* pfx_len, const float* logits,
+                                   const BanMask& ban, cudaStream_t s);
 
 // ---- score.cu -----------------------------------------------------------------------------------
 // Caption scoring (fpnmt_score, include/fpnmt.h): row r = c * t + j is position j of caption c = b * N + n.

@@ -58,6 +58,15 @@ struct SampleSmem {
   int mi, tok;
   uint32_t u24;
 };
+// the step's shared state; MASK adds the largest allowed logit (per warp, of the row) and its lowest index (the other kernels
+// keep SampleSmem's layout)
+template <bool MASK>
+struct SampleStepSmem : SampleSmem {};
+template <>
+struct SampleStepSmem<true> : SampleSmem {
+  float wma[SAMPLE_THREADS / 32], ma;
+  int wmai[SAMPLE_THREADS / 32];
+};
 
 // Block sum of a uint64 (exact: integer addition), result in every thread.
 __device__ __forceinline__ unsigned long long block_sum_u64(unsigned long long v, SampleSmem& sm) {
@@ -130,13 +139,17 @@ __device__ uint32_t radix_select_desc(const float* s_row, int V, unsigned long l
 
 // The step body.  PREFIX (k_sample_step_prefix): a row of an image inside its prefix (step t < pfx_len[image]) takes the
 // prefix token pfx_ids[image][t] (top-k, top-p and the draw skipped) and adds its log-probability with the expression of the
-// free path.
-template <bool PREFIX>
+// free path.  MASK (k_sample_step_constrained): after the log-partition function, the banned logits of the staged row become
+// -inf, so the arg-max, top-k, the masses (taken relative to the largest ALLOWED logit: relative to a banned maximum the allowed
+// masses could all round to 0) and the draw see allowed tokens only; the log-probability still reads the unmasked logit.  The
+// row's CTA then writes its own ban set of step t + 1.
+template <bool PREFIX, bool MASK = false>
 __device__ __forceinline__ void sample_step_body(const SampleState& st, const float* __restrict__ logits,
-                                                 const int* __restrict__ pfx_ids, const int* __restrict__ pfx_len) {
+                                                 const int* __restrict__ pfx_ids, const int* __restrict__ pfx_len,
+                                                 const BanMask& ban) {
   extern __shared__ float4 s_row4[];
   float* s_row = reinterpret_cast<float*>(s_row4);
-  __shared__ SampleSmem sm;
+  __shared__ SampleStepSmem<MASK> sm;
   pdl_launch();
   pdl_wait();
   const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -206,7 +219,35 @@ __device__ __forceinline__ void sample_step_body(const SampleState& st, const fl
   m = sm.m;
   // ---- log-partition function at temperature 1 (fixed reduction tree: bit-identical run to run)
   float s1 = 0.f;
-  for (int i = tid; i < V; i += SAMPLE_THREADS) s1 += expf(s_row[i] - m);
+  float ma = -INFINITY;                                  // MASK: this thread's largest allowed logit (lowest index)
+  int mai = 0x7fffffff;
+  if constexpr (MASK) {
+    const uint32_t* mk = ban_row(ban, t, row);
+    for (int i = tid; i < V; i += SAMPLE_THREADS) {     // own entries: the same slots the sum reads, no barrier
+      const float v = s_row[i];
+      s1 += expf(v - m);
+      if ((__ldcg(mk + (i >> 5)) >> (i & 31)) & 1u) s_row[i] = -INFINITY;
+      else if (v > ma) {
+        ma = v;
+        mai = i;
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float om = __shfl_xor_sync(0xffffffffu, ma, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, mai, o);
+      if (om > ma || (om == ma && oi < mai)) {
+        ma = om;
+        mai = oi;
+      }
+    }
+    if (lane == 0) {
+      sm.wma[warp] = ma;
+      sm.wmai[warp] = mai;
+    }
+  } else {
+    for (int i = tid; i < V; i += SAMPLE_THREADS) s1 += expf(s_row[i] - m);
+  }
   s1 = warp_sum(s1);
   if (lane == 0) sm.ws[warp] = s1;
   __syncthreads();
@@ -216,6 +257,18 @@ __device__ __forceinline__ void sample_step_body(const SampleState& st, const fl
     for (int w = 0; w < NW; ++w) a += sm.ws[w];
     sm.lse1 = m + logf(a);
     sm.tok = sm.mi;                                      // temperature 0: arg-max, lowest token id on ties
+    if constexpr (MASK) {                                //   over the allowed tokens
+      float bm = sm.wma[0];
+      int bi = sm.wmai[0];
+#pragma unroll
+      for (int w = 1; w < NW; ++w)
+        if (sm.wma[w] > bm || (sm.wma[w] == bm && sm.wmai[w] < bi)) {
+          bm = sm.wma[w];
+          bi = sm.wmai[w];
+        }
+      sm.ma = bm;
+      sm.tok = bi;
+    }
     if constexpr (PREFIX) {                              // forced step of a prompted decode: the prefix token
       const int b = row / st.N;
       if (t < pfx_len[b]) sm.tok = pfx_ids[(size_t)b * st.T + t];
@@ -232,10 +285,12 @@ __device__ __forceinline__ void sample_step_body(const SampleState& st, const fl
                              [](float z, uint32_t* key) -> unsigned long long { *key = fkey(z); return 1ull; }, sm);
     // ---- tempered probabilities relative to the row maximum, 0 outside K1; fixed-point masses of those
     __syncthreads();
+    float mref = m;
+    if constexpr (MASK) mref = sm.ma;
     unsigned long long w1 = 0ull;
     for (int i = tid; i < V; i += SAMPLE_THREADS) {
       const float z = s_row[i];
-      const float e = fkey(z) >= k1 ? expf((z - m) / prm.temperature) : 0.f;
+      const float e = fkey(z) >= k1 ? expf((z - mref) / prm.temperature) : 0.f;
       s_row[i] = e;
       w1 += mass_of(e);
     }
@@ -326,16 +381,29 @@ __device__ __forceinline__ void sample_step_body(const SampleState& st, const fl
       }
     }
   }
+  if constexpr (MASK) {                                  // the row's ban set of step t + 1 from its caption (thread 0 is in warp 0)
+    if (warp == 0) {
+      __syncwarp();
+      if (t + 1 < st.T) ban_row_warp(ban_row(ban, t + 1, row), ban, st.ids + (size_t)row * st.T, __ldcg(st.len + row));
+    }
+  }
 }
 
 __global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step(SampleState st, const float* __restrict__ logits) {
-  sample_step_body<false>(st, logits, nullptr, nullptr);
+  sample_step_body<false>(st, logits, nullptr, nullptr, BanMask{});
 }
 // the step of a prompted decode (pfx_ids [images][T], pfx_len [images]: launch_prefix_load's buffers)
 __global__ void __launch_bounds__(SAMPLE_THREADS) k_sample_step_prefix(SampleState st, const float* __restrict__ logits,
                                                                        const int* __restrict__ pfx_ids,
                                                                        const int* __restrict__ pfx_len) {
-  sample_step_body<true>(st, logits, pfx_ids, pfx_len);
+  sample_step_body<true>(st, logits, pfx_ids, pfx_len, BanMask{});
+}
+// the step of a constrained decode (prompted or not: pfx_len 0), with the ban sets of `ban`.  The minimum of 5 blocks per SM
+// gives ptxas a 48-register budget: with the thread count alone it picks 40 and spills one register across the masses loop.
+__global__ void __launch_bounds__(SAMPLE_THREADS, 5) k_sample_step_constrained(SampleState st, const float* __restrict__ logits,
+                                                                            const int* __restrict__ pfx_ids,
+                                                                            const int* __restrict__ pfx_len, BanMask ban) {
+  sample_step_body<true, true>(st, logits, pfx_ids, pfx_len, ban);
 }
 
 __global__ void k_sample_init(SampleState st, int* anc) {
@@ -362,6 +430,7 @@ __global__ void k_sample_init(SampleState st, int* anc) {
 int sample_set_attributes() {   // per device
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_sample_step, cudaFuncAttributeMaxDynamicSharedMemorySize, SAMPLE_MAX_SMEM));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(k_sample_step_prefix, cudaFuncAttributeMaxDynamicSharedMemorySize, SAMPLE_MAX_SMEM));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(k_sample_step_constrained, cudaFuncAttributeMaxDynamicSharedMemorySize, SAMPLE_MAX_SMEM));
   return 0;
 }
 
@@ -397,6 +466,20 @@ int launch_sample_step_prefix(const SampleState& st, const int* pfx_ids, const i
   const size_t smem = sample_smem(st);
   if (!smem) return 1;
   FPNMT_CUDA_OK(launch_k(k_sample_step_prefix, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits, pfx_ids, pfx_len));
+  return 0;
+}
+
+int launch_sample_step_constrained(const SampleState& st, const int* pfx_ids, const int* pfx_len, const float* logits,
+                                   const BanMask& ban, cudaStream_t s) {
+  if (!pfx_ids || !pfx_len || !st.ids || !ban.mask || !ban.cfg || ban.rows != st.rows || ban.V != st.V ||
+      ban.W != (st.V + 31) / 32) {
+    set_last_error("sample_step_constrained: needs the prefix buffers, the ban masks of every row and the engine's decode state");
+    return 1;
+  }
+  const size_t smem = sample_smem(st);
+  if (!smem) return 1;
+  FPNMT_CUDA_OK(launch_k(k_sample_step_constrained, dim3(st.rows), dim3(SAMPLE_THREADS), smem, s, st, logits, pfx_ids, pfx_len,
+                         ban));
   return 0;
 }
 

@@ -60,6 +60,10 @@ struct TgemmOp {
   // tgt_logit[r] = z[r][tgt[r]] for every row r whose tgt[r] lies in [0, F) (device [R] each; nullptr = tgemmw_kernel)
   const int* tgt = nullptr;
   float* tgt_logit = nullptr;
+  // constrained beam search on the same tail: tgemmw_mask_kernel keeps banned features out of every row's candidates (mask
+  // [2][R][ceil(F / 32)] bits by the parity of *mask_step, nullptr: parity 0; tgt may then be nullptr)
+  const uint32_t* mask = nullptr;
+  const int* mask_step = nullptr;
 };
 
 size_t tgemm_smem_bytes(int BN);

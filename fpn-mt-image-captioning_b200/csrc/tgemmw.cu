@@ -111,10 +111,13 @@ __device__ __forceinline__ void tw_load_chunk(uint32_t taddr, const float* sBias
 
 // The kernel body.  TGT (tgemmw_target_kernel, vocabulary tile without logits only): the row whose target id tgt[row] lies in
 // [0, F) also writes the fp32 logit of that feature, the value its tile's statistics and candidates are computed from, to
-// tgt_logit[row] (-1 or an id >= F: nothing written).
-template <bool TGT>
+// tgt_logit[row] (-1 or an id >= F: nothing written).  MASK (tgemmw_mask_kernel, with TGT; tgt may then be nullptr): the
+// top-8 candidates of a row skip the features banned in its mask row, mask + (par * R + row) * ceil(F / 32) with par =
+// *mask_step & 1 (mask_step nullptr: 0); a 32-feature chunk is one mask word.  The (max, sum exp) statistics stay unmasked.
+template <bool TGT, bool MASK = false>
 __device__ __forceinline__ void tgemmw_body(const CUtensorMap& tmW, const CUtensorMap& tmX, const CUtensorMap& tmO,
-                                            const TgemmParams p, const int* __restrict__ tgt, float* __restrict__ tgt_logit) {
+                                            const TgemmParams p, const int* __restrict__ tgt, float* __restrict__ tgt_logit,
+                                            const uint32_t* __restrict__ mask = nullptr, const int* __restrict__ mask_step = nullptr) {
   constexpr int STAGES = TW_STAGES;
   constexpr int BN = 128;                          // features per tile == UMMA N == TMEM columns of one accumulator
   constexpr int CHUNKS = BN / 32;
@@ -288,7 +291,12 @@ __device__ __forceinline__ void tgemmw_body(const CUtensorMap& tmW, const CUtens
         // warp always qualifies, so instruction count matters more than the length of the dependent chain.)
         float m = -INFINITY, ssum = 0.f;
         int tg = -1;                                          // target feature of this row (TGT)
-        if constexpr (TGT) tg = row_ok ? __ldcg(tgt + row) : -1;
+        if constexpr (TGT) tg = (row_ok && (!MASK || tgt)) ? __ldcg(tgt + row) : -1;
+        const uint32_t* mrow = nullptr;                       // this row's ban mask (MASK)
+        if constexpr (MASK) {
+          const int par = mask_step ? (__ldcg(mask_step) & 1) : 0;
+          mrow = mask + ((size_t)par * p.R + row) * ((p.F + 31) / 32);
+        }
         float bv[TG_VS_N];
         int bi[TG_VS_N];
 #pragma unroll
@@ -328,10 +336,20 @@ __device__ __forceinline__ void tgemmw_body(const CUtensorMap& tmW, const CUtens
             ssum = ssum * __expf(m - mn) + cs;
             m = mn;
           }
-          if (cm > bv[TG_VS_N - 1]) {
+          uint32_t mw = 0u;                                   // banned features of this chunk (MASK): never candidates
+          float cma = cm;
+          if constexpr (MASK) {
+            mw = (row_ok && fo < p.F) ? __ldcg(mrow + (fo >> 5)) : 0u;   // padding chunks: no mask word (already -inf)
+            if (mw) {
+              cma = -INFINITY;
+#pragma unroll
+              for (int i = 0; i < 32; ++i) cma = ((mw >> i) & 1u) ? cma : fmaxf(cma, x[i]);
+            }
+          }
+          if (cma > bv[TG_VS_N - 1]) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
-              if (x[i] > bv[TG_VS_N - 1]) {
+              if (x[i] > bv[TG_VS_N - 1] && !((mw >> i) & 1u)) {
                 bv[TG_VS_N - 1] = x[i];
                 bi[TG_VS_N - 1] = fo + i;
 #pragma unroll
@@ -520,6 +538,14 @@ tgemmw_target_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_const
                      float* __restrict__ tgt_logit) {
   tgemmw_body<true>(tmW, tmX, tmO, p, tgt, tgt_logit);
 }
+// The vocabulary projection of a constrained beam search on the logits-free tail: tgemmw_target_kernel + the ban masks
+// (TgemmOp::mask): every row's candidates are its allowed features only
+__global__ void __launch_bounds__(TG_THREADS, 2)
+tgemmw_mask_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX,
+                   const __grid_constant__ CUtensorMap tmO, const TgemmParams p, const int* __restrict__ tgt,
+                   float* __restrict__ tgt_logit, const uint32_t* __restrict__ mask, const int* __restrict__ mask_step) {
+  tgemmw_body<true, true>(tmW, tmX, tmO, p, tgt, tgt_logit, mask, mask_step);
+}
 
 int tgemmw_launch(const TgemmOp& op, cudaStream_t stream) {
   cudaLaunchConfig_t cfg{};
@@ -543,7 +569,10 @@ int tgemmw_launch(const TgemmOp& op, cudaStream_t stream) {
   }
   cfg.attrs = attr;
   cfg.numAttrs = n;
-  if (op.tgt) FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_target_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p, op.tgt, op.tgt_logit));
+  if (op.mask)
+    FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_mask_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p, op.tgt, op.tgt_logit, op.mask,
+                                     op.mask_step));
+  else if (op.tgt) FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_target_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p, op.tgt, op.tgt_logit));
   else FPNMT_CUDA_OK(cudaLaunchKernelEx(&cfg, tgemmw_kernel, op.tmW, op.tmX_hi, op.tmX_lo, op.p));
   return 0;
 }
@@ -553,6 +582,8 @@ int tgemmw_set_attributes() {
   FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_target_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tgemmw_smem_bytes(128)));
   FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_target_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_mask_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tgemmw_smem_bytes(128)));
+  FPNMT_CUDA_OK(cudaFuncSetAttribute(tgemmw_mask_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   return 0;
 }
 

@@ -35,6 +35,12 @@ class FpnmtSampling(C.Structure):
                 ("reserved", C.c_int32 * 4)]
 
 
+class FpnmtConstraints(C.Structure):
+    """fpnmt_constraints (include/fpnmt.h): no-repeat n-gram size, minimum length and banned token ids (host array)."""
+    _fields_ = [("no_repeat_ngram", C.c_int32), ("min_len", C.c_int32), ("banned", C.POINTER(C.c_int32)),
+                ("n_banned", C.c_int32), ("reserved", C.c_int32 * 4)]
+
+
 class FpnmtError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__("fpnmt error %d: %s" % (code, msg))
@@ -92,6 +98,12 @@ SIGNATURES = {
     "fpnmt_beam_search_diverse": (_i, [_vp, _vp, _i, _i, C.c_float, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
     "fpnmt_sample_prefix": (_i, [_vp, _vp, _i, _vp, _vp, _i, C.POINTER(FpnmtSampling), _vp, _vp, _vp, _i, _i, _vp]),
     "fpnmt_beam_search_prefix": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i, C.c_float, C.c_float, _vp, _vp, _vp, _i, _i, _vp]),
+    "fpnmt_sample_constrained": (_i, [_vp, _vp, _i, _vp, _vp, _i, C.POINTER(FpnmtSampling), C.POINTER(FpnmtConstraints), _vp, _vp,
+                                      _vp, _i, _i, _vp]),
+    "fpnmt_beam_search_constrained": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i, C.c_float, C.c_float, C.POINTER(FpnmtConstraints),
+                                           _vp, _vp, _vp, _i, _i, _vp]),
+    "fpnmt_op_vocab_stats_mask": (_i, [_i, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "fpnmt_op_ban_mask": (_i, [_i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _i, _vp, _vp]),
 }
 
 
@@ -127,6 +139,10 @@ SIGNATURES.update({
     "fpnmt_beam_search_diverse_dl": (_i, [_vp, _dlp, _i, C.c_float, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_sample_prefix_dl": (_i, [_vp, _dlp, _dlp, _dlp, C.POINTER(FpnmtSampling), _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_beam_search_prefix_dl": (_i, [_vp, _dlp, _dlp, _dlp, _i, C.c_float, C.c_float, _dlp, _dlp, _dlp, _i, _vp]),
+    "fpnmt_sample_constrained_dl": (_i, [_vp, _dlp, _dlp, _dlp, C.POINTER(FpnmtSampling), C.POINTER(FpnmtConstraints), _dlp, _dlp,
+                                         _dlp, _i, _vp]),
+    "fpnmt_beam_search_constrained_dl": (_i, [_vp, _dlp, _dlp, _dlp, _i, C.c_float, C.c_float, C.POINTER(FpnmtConstraints),
+                                              _dlp, _dlp, _dlp, _i, _vp]),
     "fpnmt_comm_unique_id": (_i, [_vp]),
     "fpnmt_comm_create": (_i, [_i, _i, _vp, _i, C.POINTER(_vp)]),
     "fpnmt_comm_destroy": (_i, [_vp]),
@@ -176,6 +192,19 @@ def sampling(temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed:
     sp = FpnmtSampling()
     sp.temperature, sp.top_k, sp.top_p, sp.seed = float(temperature), int(top_k), float(top_p), int(seed) & 0xFFFFFFFFFFFFFFFF
     return sp
+
+
+def constraints(no_repeat_ngram: int = 0, min_len: int = 0, banned=None) -> FpnmtConstraints:
+    """An fpnmt_constraints with the reserved words zero.  `banned` (token ids) is copied into an int32 array the struct
+    keeps alive."""
+    c = FpnmtConstraints()
+    c.no_repeat_ngram, c.min_len = int(no_repeat_ngram), int(min_len)
+    ids = [int(v) for v in (banned if banned is not None else [])]
+    if ids:
+        c._banned = (C.c_int32 * len(ids))(*ids)
+        c.banned = C.cast(c._banned, C.POINTER(C.c_int32))
+    c.n_banned = len(ids)
+    return c
 
 
 def check(rc: int) -> None:

@@ -266,14 +266,17 @@ class Engine:
         return ids, lens
 
     def sample(self, images=None, *, temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0,
-               early_stop: bool = True, to_host: bool = True, return_logprobs: bool = False, prefix=None, prefix_lens=None):
+               early_stop: bool = True, to_host: bool = True, return_logprobs: bool = False, prefix=None, prefix_lens=None,
+               no_repeat_ngram: int = 0, min_len: int = 0, banned=None):
         """`beam` independent sampled captions per image (fpnmt_sample; semantics in include/fpnmt.h): softmax(z / temperature)
         restricted to the top_k logits (0 = off, ties kept) and then to the nucleus of top_p of that mass (1 = off), drawn with
         the Philox stream of (seed, step, image, sample).  temperature 0 is greedy.  images None = the memory of the last
         encode / generate.  Returns ids (B, N, T) int32 zero padded without <start> / <end>, lengths (B, N) and, with
         return_logprobs, the captions' log-likelihoods (B, N) float32 (log_softmax at temperature 1, <end> included).
         prefix (B, p) int32 with prefix_lens (B,) (default: p for every image), on host or device: every sample of image b
-        continues prefix[b, :prefix_lens[b]] (fpnmt_sample_prefix); the returned captions and log-likelihoods include it."""
+        continues prefix[b, :prefix_lens[b]] (fpnmt_sample_prefix); the returned captions and log-likelihoods include it.
+        no_repeat_ngram / min_len / banned (token ids): the constraints of fpnmt_sample_constrained (no n-gram twice, no <end>
+        before min_len tokens, banned ids never drawn); they remove tokens from the draw and never change a log-likelihood."""
         ptr, on_host, keep = self._images_opt(images)
         pfx = self._prefix(prefix, prefix_lens)
         B, N, T = self.batch, self.beam, self.max_len
@@ -282,7 +285,13 @@ class Engine:
         lp = self._result((B, N), torch.float32, to_host) if return_logprobs else None
         sp = _lib.sampling(temperature, top_k, top_p, seed)
         lpp = lp.data_ptr() if lp is not None else None
-        if pfx is None:
+        if no_repeat_ngram or min_len or banned is not None and len(banned):
+            con = _lib.constraints(no_repeat_ngram, min_len, banned)
+            _lib.check(self.lib.fpnmt_sample_constrained(
+                self._h, ptr, on_host, pfx[0].data_ptr() if pfx else None, pfx[1].data_ptr() if pfx else None,
+                int(pfx[0].shape[1]) if pfx else 0, C.byref(sp), C.byref(con), ids.data_ptr(), lens.data_ptr(), lpp,
+                int(to_host), int(early_stop), _stream_ptr(self.device)))
+        elif pfx is None:
             _lib.check(self.lib.fpnmt_sample(self._h, ptr, on_host, C.byref(sp), ids.data_ptr(), lens.data_ptr(), lpp,
                                              int(to_host), int(early_stop), _stream_ptr(self.device)))
         else:
@@ -292,7 +301,8 @@ class Engine:
         return (ids, lens, lp) if return_logprobs else (ids, lens)
 
     def beam_search(self, images=None, *, length_penalty: float = 0.0, early_stop: bool = True, to_host: bool = True,
-                    return_logprobs: bool = False, beam_groups: int = 1, diversity: float = 0.0, prefix=None, prefix_lens=None):
+                    return_logprobs: bool = False, beam_groups: int = 1, diversity: float = 0.0, prefix=None, prefix_lens=None,
+                    no_repeat_ngram: int = 0, min_len: int = 0, banned=None):
         """The `beam` most likely captions per image by a true beam search with frozen finished beams (fpnmt_beam_search;
         definition in include/fpnmt.h), ranked by log-likelihood / ((5 + n) / 6) ** length_penalty, n the scored positions.
         images None = the memory of the last encode / generate / sample / score.  Returns ids (B, N, T) int32 zero padded
@@ -302,14 +312,23 @@ class Engine:
         group's candidates lowered by `diversity` per earlier group's beam that chose the same token at the same step.  The
         output is group-major (beams [g * N / G, (g + 1) * N / G) are group g), rank order within a group.
         prefix (B, p) int32 with prefix_lens (B,) (default: p for every image), on host or device: every beam of image b
-        continues prefix[b, :prefix_lens[b]] (fpnmt_beam_search_prefix); the returned captions and log-likelihoods include it."""
+        continues prefix[b, :prefix_lens[b]] (fpnmt_beam_search_prefix); the returned captions and log-likelihoods include it.
+        no_repeat_ngram / min_len / banned (token ids): the constraints of fpnmt_beam_search_constrained (no n-gram twice, no
+        <end> before min_len tokens, banned ids never emitted); they remove candidates and never change a score."""
         ptr, on_host, keep = self._images_opt(images)
         pfx = self._prefix(prefix, prefix_lens)
         B, N, T = self.batch, self.beam, self.max_len
         ids = self._result((B, N, T), torch.int32, to_host)
         lens = self._result((B, N), torch.int32, to_host)
         lp = self._result((B, N), torch.float32, to_host) if return_logprobs else None
-        if pfx is not None:
+        if no_repeat_ngram or min_len or banned is not None and len(banned):
+            con = _lib.constraints(no_repeat_ngram, min_len, banned)
+            _lib.check(self.lib.fpnmt_beam_search_constrained(
+                self._h, ptr, on_host, pfx[0].data_ptr() if pfx else None, pfx[1].data_ptr() if pfx else None,
+                int(pfx[0].shape[1]) if pfx else 0, int(beam_groups), float(diversity), float(length_penalty), C.byref(con),
+                ids.data_ptr(), lens.data_ptr(), lp.data_ptr() if lp is not None else None, int(to_host), int(early_stop),
+                _stream_ptr(self.device)))
+        elif pfx is not None:
             _lib.check(self.lib.fpnmt_beam_search_prefix(self._h, ptr, on_host, pfx[0].data_ptr(), pfx[1].data_ptr(),
                                                          int(pfx[0].shape[1]), int(beam_groups), float(diversity),
                                                          float(length_penalty), ids.data_ptr(), lens.data_ptr(),
@@ -556,6 +575,55 @@ def vocab_stats_target(x: torch.Tensor, kernel: np.ndarray, target, bias: Option
                                                        _hptr(b), tg.data_ptr(), stat.data_ptr(), val.data_ptr(), idx.data_ptr(),
                                                        tl.data_ptr(), _stream_ptr(dev)))
     return stat, val, idx, tl
+
+
+def vocab_stats_mask(x: torch.Tensor, kernel: np.ndarray, mask: torch.Tensor, bias: Optional[np.ndarray] = None, target=None,
+                     precision: str = "bf16") -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, Optional[torch.Tensor]]:
+    """`vocab_stats` with the ban-mask epilogue of a constrained beam search (fpnmt_op_vocab_stats_mask): stat as
+    `vocab_stats` (unmasked), val / idx the 8 largest logits per tile among the features whose bit in mask (R, ceil(F / 32))
+    int32 (bit f % 32 of word f / 32) is clear.  With target (R,) also the target logits as `vocab_stats_target` (else None).
+    Returns (stat, val, idx, target_logit)."""
+    x = _dev32(x)
+    r, k = x.shape
+    kn = _host32(kernel)
+    f = kn.shape[1]
+    ft = (f + 127) // 128
+    dev = x.device
+    stat = torch.full((r, ft, 2), float("nan"), device=dev)
+    val = torch.full((r, ft, 8), float("nan"), device=dev)
+    idx = torch.full((r, ft, 8), -1, dtype=torch.int32, device=dev)
+    mk = _as_cuda(mask, torch.int32, dev)
+    if tuple(mk.shape) != (r, (f + 31) // 32):
+        raise ValueError("mask must be (%d, %d), got %s" % (r, (f + 31) // 32, tuple(mk.shape)))
+    tg = tl = None
+    if target is not None:
+        tg = _as_cuda(target, torch.int32, dev)
+        if tuple(tg.shape) != (r,):
+            raise ValueError("target must be (%d,), got %s" % (r, tuple(tg.shape)))
+        tl = torch.full((r,), float("nan"), device=dev)
+    b = _host32(bias)
+    _lib.check(_lib.load().fpnmt_op_vocab_stats_mask(dev.index or 0, _lib.PREC_IDS[precision], x.data_ptr(), r, k, _hptr(kn), f,
+                                                     _hptr(b), mk.data_ptr(), tg.data_ptr() if tg is not None else None,
+                                                     stat.data_ptr(), val.data_ptr(), idx.data_ptr(),
+                                                     tl.data_ptr() if tl is not None else None, _stream_ptr(dev)))
+    return stat, val, idx, tl
+
+
+def ban_mask(hist, lens, vocab: int, end_id: int, no_repeat_ngram: int = 0, min_len: int = 0, banned=None,
+             device: int = 0) -> torch.Tensor:
+    """The ban sets of fpnmt_constraints for given captions (fpnmt_op_ban_mask): hist (rows, ld) int32 caption tokens, lens
+    (rows,) -> mask (rows, ceil(vocab / 32)) int32, bit v % 32 of word v / 32 set when token v is banned at step lens[r]."""
+    dev = torch.device("cuda", device)
+    h = _as_cuda(hist, torch.int32, dev)
+    ln = _as_cuda(lens, torch.int32, dev)
+    rows, ld = h.shape
+    out = torch.full((rows, (vocab + 31) // 32), -1, dtype=torch.int32, device=dev)
+    ids = [int(v) for v in (banned if banned is not None else [])]
+    arr = (C.c_int32 * max(1, len(ids)))(*ids)
+    _lib.check(_lib.load().fpnmt_op_ban_mask(device, h.data_ptr(), ld, ln.data_ptr(), rows, int(vocab), int(end_id),
+                                             int(no_repeat_ngram), int(min_len), arr if ids else None, len(ids), out.data_ptr(),
+                                             _stream_ptr(dev)))
+    return out
 
 
 # ---- stand-alone encoder bandwidth operators (kernel parity tests) --------------------------------------------------------

@@ -98,36 +98,58 @@ class Pipeline:
             ids[i, :len(q)] = q
         return ids, np.array([len(q) for q in seqs], np.int32)
 
+    def _banned_ids(self, words):
+        """banned_words -> token ids through tokenizer.word_index; ValueError for an unknown word or <end> (min_len is how
+        <end> is held back)."""
+        if not words:
+            return None
+        if isinstance(words, str):
+            raise ValueError("banned_words: a list of words, got a string")
+        ids = []
+        for w in words:
+            if w not in self.tokenizer.word_index:
+                raise ValueError("banned_words: %r is not in the vocabulary" % (w,))
+            if w == "<end>":
+                raise ValueError("banned_words: <end> cannot be banned; use min_len")
+            ids.append(int(self.tokenizer.word_index[w]))
+        return ids
+
     def sample_batch(self, imgs, max_seq_len: Optional[int] = None, num_samples: Optional[int] = None, *,
                      temperature: float = 1.0, top_k: int = 0, top_p: float = 1.0, seed: int = 0, return_logprobs: bool = False,
-                     prefix=None):
+                     prefix=None, no_repeat_ngram: int = 0, min_len: int = 0, banned_words=None):
         """`num_samples` (default: the beam width) independent sampled captions per image (Engine.sample): imgs (B,S,S,3)
         float32 in [-1,1] -> (ids (B,num_samples,T) int32 zero padded, lengths (B,num_samples)), plus the captions'
         log-likelihoods (B,num_samples) with return_logprobs.  temperature 0 is greedy.  prefix: B strings, each image's
-        samples continue its string (tokenized as score_batch does; the returned captions include it)."""
+        samples continue its string (tokenized as score_batch does; the returned captions include it).  no_repeat_ngram,
+        min_len and banned_words (words of the tokenizer, e.g. "<start>", "<unk>") constrain the draw as Engine.sample does."""
         imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
         T = max_seq_len or self.max_seq_len
         pids, plens = self._prefix_ids(prefix, int(imgs.shape[0]), T)
+        banned = self._banned_ids(banned_words)
         eng = self.transformer.engine(int(imgs.shape[0]), num_samples or self.beam, T)
         out = eng.sample(imgs, temperature=temperature, top_k=top_k, top_p=top_p, seed=seed, early_stop=True, to_host=True,
-                         return_logprobs=return_logprobs, prefix=pids, prefix_lens=plens)
+                         return_logprobs=return_logprobs, prefix=pids, prefix_lens=plens, no_repeat_ngram=no_repeat_ngram,
+                         min_len=min_len, banned=banned)
         return tuple(o.numpy() for o in out)
 
     def beam_search_batch(self, imgs, max_seq_len: Optional[int] = None, num_beams: Optional[int] = None, *,
                           length_penalty: float = 0.0, return_logprobs: bool = False, beam_groups: int = 1,
-                          diversity: float = 0.0, prefix=None):
+                          diversity: float = 0.0, prefix=None, no_repeat_ngram: int = 0, min_len: int = 0, banned_words=None):
         """The `num_beams` (default: the beam width) most likely captions per image (Engine.beam_search): imgs (B,S,S,3)
         float32 in [-1,1] -> (ids (B,num_beams,T) int32 zero padded, in rank order, lengths (B,num_beams)), plus the captions'
         log-likelihoods (B,num_beams) with return_logprobs.  Ranking by log-likelihood / ((5 + n) / 6) ** length_penalty.
         beam_groups > 1: diverse beam search in that many groups with the given diversity penalty (group-major output).
         prefix: B strings, each image's beams continue its string (tokenized as score_batch does; the returned captions
-        include it)."""
+        include it).  no_repeat_ngram: no n-gram twice in a caption; min_len: no <end> before that many tokens; banned_words:
+        words of the tokenizer never emitted (e.g. "<start>" or the OOV token).  They remove candidates and never change a score."""
         imgs = torch.as_tensor(imgs) if not isinstance(imgs, torch.Tensor) else imgs
         T = max_seq_len or self.max_seq_len
         pids, plens = self._prefix_ids(prefix, int(imgs.shape[0]), T)
+        banned = self._banned_ids(banned_words)
         eng = self.transformer.engine(int(imgs.shape[0]), num_beams or self.beam, T)
         out = eng.beam_search(imgs, length_penalty=length_penalty, early_stop=True, to_host=True, return_logprobs=return_logprobs,
-                              beam_groups=beam_groups, diversity=diversity, prefix=pids, prefix_lens=plens)
+                              beam_groups=beam_groups, diversity=diversity, prefix=pids, prefix_lens=plens,
+                              no_repeat_ngram=no_repeat_ngram, min_len=min_len, banned=banned)
         return tuple(o.numpy() for o in out)
 
     def score_batch(self, imgs, captions, max_seq_len: Optional[int] = None, *, return_token_logprobs: bool = False):

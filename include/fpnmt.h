@@ -319,6 +319,51 @@ FPNMT_API int fpnmt_beam_search_prefix(fpnmt_handle* h, const float* images, int
                                        int32_t* out_ids, int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
                                        void* stream);
 
+/* Constrained decoding: the standard decoding controls for fpnmt_sample, fpnmt_beam_search and fpnmt_beam_search_diverse,
+ * prompted or not (no reference counterpart).
+ *   no_repeat_ngram  n: 0 = off; 1 <= n <= max_len: no n-gram occurs twice in a caption.
+ *   min_len          0 = off; <end> is banned while the caption has fewer than min_len tokens; 0 <= min_len <= max_len.
+ *   banned           HOST int32 [n_banned] token ids never emitted (e.g. the padding id 0, <start>, the OOV token), or NULL;
+ *                    duplicates allowed; <end> may not be listed (min_len is how <end> is held back).
+ * A live row at step t whose caption is w_0 .. w_{t-1} (no <start>, prefix tokens included) has the ban set
+ * A(t) = S | E(t) | R(t): S = the banned list; E(t) = {end_id} when t < min_len; R(t) = { w_{j+n-1} : 0 <= j <= t - n,
+ * w_{j .. j+n-2} = w_{t-n+1 .. t-1} } for n >= 1 (n = 1: every token already in the caption).  A constraint removes
+ * candidates and never changes a score:
+ *   beam search (N-best and diverse): a live candidate (parent p, token v) with v in A_p(t) is never ranked nor selected;
+ *     everything else is the unconstrained search (raw score = score + log_softmax(z)[v] over all V, length penalty,
+ *     diversity penalty and h_g; frozen beams unaffected), so out_logprob is still the caption's log-likelihood and
+ *     fpnmt_score of a returned caption gives it back.
+ *   sampling: steps 1-5 of fpnmt_sampling run on z' with z'_i = -inf for i in A(t) (top-k is the k-th largest allowed logit;
+ *     greedy is the arg-max over allowed tokens, lowest id on ties); step 6, the reported log-probability, is log_softmax of
+ *     the unmasked z; the Philox counter is unchanged.
+ *   prefix: a forced step (t < prefix_len[b]) takes the prefix token even if it is in A(t); forced tokens count in the
+ *     history of R and toward min_len.
+ * Errors: FPNMT_ERR_INVALID (nothing launched) for an id outside [0, vocab) or end_id in `banned`, NULL banned with
+ * n_banned > 0, n or min_len out of range, non-zero reserved words, vocab - |distinct banned ids| - max_len < beam (that
+ * bound keeps at least `beam` allowed tokens for every live row at every step, as |R(t)| + |E(t)| <= max_len), and every
+ * refusal of the unconstrained twin; FPNMT_ERR_STATE as the twin (decode_path = FUSED, score_mode = PROB for beam search,
+ * lane 0 busy).  All-zero constraints (banned NULL) give the twin's results bit for bit; determinism, graphs, cache modes
+ * and what the call leaves behind are as for the twin.  fpnmt_generate has no constrained form. */
+typedef struct fpnmt_constraints {
+  int32_t no_repeat_ngram;
+  int32_t min_len;
+  const int32_t* banned;
+  int32_t n_banned;
+  int32_t reserved[4]; /* must be 0 */
+} fpnmt_constraints;
+/* prefix_ids / prefix_len / p as fpnmt_sample_prefix, or NULL / NULL / 0 for an unprompted call. */
+FPNMT_API int fpnmt_sample_constrained(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                       const int32_t* prefix_len, int p, const fpnmt_sampling* sampling,
+                                       const fpnmt_constraints* constraints, int32_t* out_ids, int32_t* out_len,
+                                       float* out_logprob, int outputs_on_host, int early_stop, void* stream);
+/* beam_groups = 1: the constrained fpnmt_beam_search (diversity ignored); > 1: the constrained fpnmt_beam_search_diverse.
+ * prefix_ids / prefix_len / p as fpnmt_beam_search_prefix, or NULL / NULL / 0 for an unprompted call. */
+FPNMT_API int fpnmt_beam_search_constrained(fpnmt_handle* h, const float* images, int images_on_host, const int32_t* prefix_ids,
+                                            const int32_t* prefix_len, int p, int beam_groups, float diversity,
+                                            float length_penalty, const fpnmt_constraints* constraints, int32_t* out_ids,
+                                            int32_t* out_len, float* out_logprob, int outputs_on_host, int early_stop,
+                                            void* stream);
+
 /* Replaces: Pipeline.predict (utils/pipeline.py:82-154) for a batch: encoder + beam-search decode.
  * out_ids DEVICE-or-HOST int32 [batch, max_len] (0 padded), out_len int32 [batch]: exactly what predict() returns
  * per image (<start> stripped, trailing <end> stripped).  outputs_on_host != 0: results are copied to host and
@@ -407,6 +452,20 @@ FPNMT_API int fpnmt_op_vocab_stats(int device, int precision, const float* x, in
 FPNMT_API int fpnmt_op_vocab_stats_target(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
                                           const float* bias, const int32_t* target, float* stat, float* val, int32_t* idx,
                                           float* target_logit, void* stream);
+/* fpnmt_op_vocab_stats with the ban-mask epilogue of a constrained beam search on the logits-free tail: stat is written
+ * exactly as fpnmt_op_vocab_stats writes it (over every feature), and val / idx hold each tile's 8 largest ALLOWED
+ * logits (features f with bit f % 32 of mask[r][f / 32] clear), -inf / 0x7fffffff padded.  mask DEVICE uint32
+ * [R][ceil(F / 32)].  target / target_logit (both NULL, or both set) as fpnmt_op_vocab_stats_target. */
+FPNMT_API int fpnmt_op_vocab_stats_mask(int device, int precision, const float* x, int R, int K, const float* kernel, int F,
+                                        const float* bias, const uint32_t* mask, const int32_t* target, float* stat, float* val,
+                                        int32_t* idx, float* target_logit, void* stream);
+/* The ban sets of fpnmt_constraints for `rows` given captions: mask[r] (DEVICE uint32 [rows][ceil(vocab / 32)]) = the bits of
+ * A(len[r]) for the caption hist[r][0 .. len[r]) (DEVICE int32 hist [rows][ld], len [rows], clamped to [0, ld]; ids outside
+ * [0, vocab) never set a bit).  no_repeat_ngram, min_len and banned / n_banned as fpnmt_constraints (banned HOST; the refusals
+ * are those of the entry points, except the vocab - |S| - max_len bound). */
+FPNMT_API int fpnmt_op_ban_mask(int device, const int32_t* hist, int ld, const int32_t* len, int rows, int vocab, int end_id,
+                                int no_repeat_ngram, int min_len, const int32_t* banned, int n_banned, uint32_t* mask,
+                                void* stream);
 
 /* Encoder bandwidth kernels one at a time (the launchers of the engine's program, which choose the kernel by precision
  * and shape exactly as the engine does).  Activations are DEVICE float32, uploaded into bf16 (or bf16x3 hi + lo)

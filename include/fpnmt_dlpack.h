@@ -90,6 +90,16 @@ FPNMT_API int fpnmt_sample_prefix_dl(fpnmt_handle* h, const DLTensor* images, co
 FPNMT_API int fpnmt_beam_search_prefix_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
                                           const DLTensor* prefix_len, int beam_groups, float diversity, float length_penalty,
                                           DLTensor* out_ids, DLTensor* out_len, DLTensor* out_logprob, int early_stop, void* stream);
+/* fpnmt_sample_constrained / fpnmt_beam_search_constrained: prefix_ids / prefix_len as fpnmt_sample_prefix_dl, or both NULL
+ * for an unprompted call; constraints a host struct; images and outputs as fpnmt_sample_dl / fpnmt_beam_search_dl. */
+FPNMT_API int fpnmt_sample_constrained_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
+                                          const DLTensor* prefix_len, const fpnmt_sampling* sampling,
+                                          const fpnmt_constraints* constraints, DLTensor* out_ids, DLTensor* out_len,
+                                          DLTensor* out_logprob, int early_stop, void* stream);
+FPNMT_API int fpnmt_beam_search_constrained_dl(fpnmt_handle* h, const DLTensor* images, const DLTensor* prefix_ids,
+                                               const DLTensor* prefix_len, int beam_groups, float diversity, float length_penalty,
+                                               const fpnmt_constraints* constraints, DLTensor* out_ids, DLTensor* out_len,
+                                               DLTensor* out_logprob, int early_stop, void* stream);
 
 /* ---- in-library communicator: the ONE collective of the path (SURVEY §8e) -------------------------------------------
  * Image batches shard across the GPUs of a box; the only exchange is the all-gather of the caption ids.  The library opens
